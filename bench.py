@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
                     [--workload c2|c3|c4|c5] [--scaling weak|strong] [--no-cpu-baseline] [--no-extras]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic input.  Workloads (BASELINE.json `configs`):
 
@@ -36,6 +37,12 @@ One JSON line on rank 0:
 
 ``--impl reference`` times the CPU oracle alone (all host cores, bounded sample per step) on the headline
 workload's input format (int16 PCM -> decode -> peak normalise -> features).
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed device-resident step of the headline workload
+computed on rank 0: ``features.npy`` (float32 feature rows) and, for c3 / c4, ``collect_audio.npy`` /
+``collect_facial.npy`` (float32 augmented rows).  An output of more than DUMP_ROWS rows is a fixed, seeded sample of its
+rows, in order; ``<name>_rows.npy`` (float64) holds their indices.  The inputs are synthesised from fixed seeds, so two
+builds run with the same arguments can be compared array for array.
 """
 import os
 
@@ -76,6 +83,34 @@ WORKLOADS = {
                desc="C5: 10000 clips x 2 s @ 16 kHz, batched small clips"),
 }
 DEFAULT_SCALING = {"c2": "weak", "c3": "strong", "c4": "weak", "c5": "strong"}
+# --dump-outputs: rows kept per output array; the largest dump (c4: 256 + 256 + 61 float32 columns) stays under 64 MB
+DUMP_ROWS = 16384
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_row_index(n_rows):
+    """Rows of an n_rows output that --dump-outputs keeps: all of them, or a fixed seeded sample in ascending order."""
+    if n_rows <= DUMP_ROWS:
+        return np.arange(n_rows, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(n_rows, DUMP_ROWS, replace=False))
+
+
+def sample_rows(name, rows):
+    """{name: the kept rows of a (rows, cols) CUDA tensor as float32, name_rows: their indices as float64}."""
+    import torch
+    idx = dump_row_index(rows.shape[0])
+    kept = rows.index_select(0, torch.from_numpy(idx).to(rows.device)).cpu().numpy()
+    return {name: kept.astype(np.float32, copy=False), name + "_rows": idx.astype(np.float64)}
+
+
+def write_outputs(directory, arrays):
+    """One ``directory/<name>.npy`` per array: float32 / float64 only, DUMP_LIMIT_BYTES in all."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, total
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def algorithmic(sr, Fr, Hr, kp):
@@ -371,9 +406,10 @@ def make_inputs(name, rank, world, scaling):
     return packed, off, base, mine, n_total
 
 
-def measure_workload(name, scaling, steps, warmup, D, rank, world, local_rank, detail):
+def measure_workload(name, scaling, steps, warmup, D, rank, world, local_rank, detail, dump=False):
     """One workload on this rank's GPU: device-resident throughput, per-kernel stage times, end-to-end runs through
-    the host entry points.  Returns a dict on every rank (timings are already max-over-ranks)."""
+    the host entry points.  Returns a dict on every rank (timings are already max-over-ranks); with ``dump`` its
+    ``_outputs`` holds the rows of the last timed step (see --dump-outputs)."""
     import torch
     from neurosync_trainer_lite_b200 import _native as nv
     from neurosync_trainer_lite_b200 import engine, synth
@@ -421,6 +457,12 @@ def measure_workload(name, scaling, steps, warmup, D, rank, world, local_rank, d
     D.barrier()
     dev_ms = D.max(e0.elapsed_time(e1))
     launches = eng.launch_count() - launches0
+    outputs = None
+    if dump:                                           # read back after the timed region, before anything reuses `out`
+        outputs = sample_rows("features", out)
+        if col:
+            outputs.update(sample_rows("collect_audio", col["out_a"]))
+            outputs.update(sample_rows("collect_facial", col["out_f"]))
 
     # per-kernel stage times (CUDA events recorded by the library on the same stream)
     eng.set_profiling(True)
@@ -600,6 +642,7 @@ def measure_workload(name, scaling, steps, warmup, D, rank, world, local_rank, d
         ceiling["e2e_frac_of_ceiling"] = round(ceiling["ms_per_step"] / res["e2e"]["ms_per_step"], 4)
         res["copy_ceiling"] = ceiling
     res["_frames"] = frames
+    res["_outputs"] = outputs
     return res
 
 
@@ -843,8 +886,12 @@ def run_native(args, rank, world, local_rank):
     warm = max(args.warmup, 3)
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    main = measure_workload(name, scaling, args.steps, warm, D, rank, world, local_rank, detail=True)
+    main = measure_workload(name, scaling, args.steps, warm, D, rank, world, local_rank, detail=True,
+                            dump=args.dump_outputs is not None and rank == 0)
     clocks = sampler.stop() if sampler else None
+    outputs = main.pop("_outputs")
+    if outputs:
+        write_outputs(args.dump_outputs, outputs)
 
     extras = {}
     if not args.no_extras and name == "c2":
@@ -893,6 +940,7 @@ def run_native(args, rank, world, local_rank):
         c.close()
     for r in list(extras.values()) + [main]:
         r.pop("_frames", None)
+        r.pop("_outputs", None)
 
     line = {
         "metric": "audio_seconds_per_second", "value": main["value"], "unit": "audio-s/s", "n_gpus": world,
@@ -931,7 +979,14 @@ def main():
     ap.add_argument("--single-process", action="store_true",
                     help="c3 / c4 end to end from ONE process driving --gpus N devices (one thread + context each) into one "
                          "page-locked host array; run without torchrun")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 rows, "
+                         "seeded row sample of large outputs, rank 0's share)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl == "reference" or args.single_process):
+        ap.error("--dump-outputs writes the device-resident path's rows: not with --impl reference or --single-process")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

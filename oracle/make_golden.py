@@ -155,8 +155,9 @@ def main():
         write_wav(ps, short, 88200)
         assert quiet(ref_ef.extract_audio_features, ps, 88200) == (None, None)
         assert quiet(fo.extract_audio_features_from_array, short.astype(np.float32), 88200) == (None, None)
-        np.savez_compressed(os.path.join(OUT, "entry_points.npz"), pcm88=raw16, feats88=feats,
-                            y88=yn, pcm16=raw16k, feats16=f16, y16=y16)
+        # one file per rate: every golden file stays under 1 MB
+        np.savez_compressed(os.path.join(OUT, "entry_points.npz"), pcm88=raw16, feats88=feats, y88=yn)
+        np.savez_compressed(os.path.join(OUT, "entry_points_16k.npz"), pcm16=raw16k, feats16=f16, y16=y16)
         made.append(("entry_points", feats.shape))
 
         # ---- D. the reference's own fixture, first 3 s, native 44.1 kHz via from_bytes -----------
@@ -182,7 +183,7 @@ def main():
         acsv = os.path.join(td, "audio_features.csv")
         pd.DataFrame(c1_features).to_csv(acsv, index=False)
         cached = pd.read_csv(acsv).values
-        res = {}
+        shapes = {}
         for tag, kw in [("fast", dict()), ("fast_slow", dict(include_slow=True)),
                         ("noblend", dict(blend_boundaries=False)),
                         ("slow_only_b7", dict(include_fast=False, include_slow=True, blend_frames=7))]:
@@ -196,16 +197,15 @@ def main():
                      if 0 <= k < a.shape[0]]
             r = np.unique(np.concatenate([np.arange(0, a.shape[0], 97),
                                           np.array(extra, dtype=np.int64)]))
-            res[tag + "_rows"] = r
-            res[tag + "_shape"] = np.array(a.shape)
-            res[tag + "_audio"] = a[r]
-            res[tag + "_facial"] = f[r]
-        assert tuple(res["fast_shape"]) == (2670, 256) and tuple(res["fast_slow_shape"]) == (6239, 256)
+            # one file per setting: every golden file stays under 1 MB
+            np.savez_compressed(os.path.join(OUT, f"collect_c3_{tag}.npz"), **{
+                tag + "_rows": r, tag + "_shape": np.array(a.shape), tag + "_audio": a[r], tag + "_facial": f[r]})
+            shapes[tag] = a.shape
+        assert shapes["fast"] == (2670, 256) and shapes["fast_slow"] == (6239, 256)
         # facial rows are regenerated by the tests (synth_facial(1800, seed=0)); the CSV round trip
         # moves them by <= 1 ulp, far inside the test tolerance
         assert np.abs(facial_rt - facial).max() < 1e-15
-        np.savez_compressed(os.path.join(OUT, "collect_c3.npz"), **res)
-        made.append(("collect_c3", tuple(res["fast_shape"])))
+        made.append(("collect_c3", shapes["fast"]))
 
     # ---- F. small known-answer tests of the augmentation helpers (SURVEY 8(c)) ------------------
     A = np.arange(10, dtype=np.float64).reshape(5, 2)

@@ -44,6 +44,10 @@ def main():
             ref = ref_u.extract_overlapping_autocorr(y, sr, F, H, **kw)
             mine = fo.autocorr_block(y, sr, F, H, **kw)
             assert ref.dtype == mine.dtype and np.array_equal(ref, mine), (tag, name)
+            if name.endswith("trim"):
+                # identical to the unpadded result on these clips: stored once, which keeps the file under 1 MB
+                assert np.array_equal(ref, out[f"{tag}_nopad"]), (tag, name)
+                continue
             out[f"{tag}_{name}"] = ref
     # a clip whose leading frames are silent: constant padding makes frame 0 all-zero, the edge fix copies frame 1
     y = synth.synth_clip(0.3, 88200, seed=33, kind="voiced")

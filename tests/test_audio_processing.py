@@ -1,11 +1,10 @@
 """Inference-side chunker (SURVEY.md section 8(f)-4): the package's mirror of the reference's
-``utils/audio/processing/audio_processing.py`` against the reference file itself.
-
-The reference module needs only NumPy and torch, so when /root/reference is mounted (the build
-container) the two implementations are run side by side on a small deterministic model; on the GPU box
-the committed golden vectors (tests/golden/audio_processing.npz, made by oracle/make_golden_chunker.py)
-stand in for it."""
-import importlib.util
+``utils/audio/processing/audio_processing.py`` against what the reference module returned on a small
+deterministic model: its ``process_audio_features`` results (tests/golden/audio_processing.npz, made by
+oracle/make_golden_chunker.py) and digests of its helper results (tests/golden/audio_processing_helpers.json,
+oracle/make_golden_chunker_helpers.py)."""
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -15,7 +14,6 @@ import torch
 from neurosync_trainer_lite_b200.utils.audio.processing import audio_processing as ap
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/utils/audio/processing/audio_processing.py"
 
 
 class ToyModel(torch.nn.Module):
@@ -74,21 +72,24 @@ def test_matches_golden(n, frame, overlap):
         np.testing.assert_allclose(got, want, rtol=0, atol=0 if not batched else 2e-6)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not mounted (GPU box)")
 @pytest.mark.parametrize("n,frame,overlap", CASES)
 def test_matches_reference_module(n, frame, overlap):
-    spec = importlib.util.spec_from_file_location("ref_audio_processing", REF)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    """Chunk-by-chunk decoding reproduces the reference module's result, and the cross-fade / reflect-padding
+    helpers its results (dtype, shape and SHA-256 of the bytes: bit for bit)."""
+    gold = np.load(os.path.join(HERE, "golden", "audio_processing.npz"))
+    with open(os.path.join(HERE, "golden", "audio_processing_helpers.json")) as fh:
+        ref = json.load(fh)[str(n)]
     model = ToyModel()
     feats = _features(n, seed=n)
     cfg = {"frame_size": frame, "overlap": overlap}
-    want = ref.process_audio_features(feats, model, "cpu", cfg)
+    want = gold[f"out_{n}_{frame}_{overlap}"]
     got = ap.process_audio_features(feats, model, "cpu", cfg, batched=False)
     np.testing.assert_array_equal(got, want)
     a, b = feats[:40].astype(np.float32), feats[40:70].astype(np.float32)
-    np.testing.assert_array_equal(ap.blend_chunks(a, b, 16), ref.blend_chunks(a, b, 16))
-    np.testing.assert_array_equal(ap.pad_audio_chunk(a, 128, 256), ref.pad_audio_chunk(a, 128, 256))
+    for name, out in (("blend_chunks", ap.blend_chunks(a, b, 16)), ("pad_audio_chunk", ap.pad_audio_chunk(a, 128, 256))):
+        out = np.ascontiguousarray(out)
+        assert (out.dtype.str, list(out.shape)) == (ref[name]["dtype"], ref[name]["shape"]), name
+        assert hashlib.sha256(out.tobytes()).hexdigest() == ref[name]["sha256"], name
 
 
 @pytest.mark.gpu

@@ -193,3 +193,62 @@ def test_bench_workload_table_and_algorithmic_counts():
     # SURVEY section 8(d): per hop-frame at 88.2 kHz
     assert alg["stft_gemm"][1] == 4327680 and alg["autocorr"][1] == 517564
     assert alg["stft_gemm"][0] == alg["autocorr"][0] == "tensor" and alg["fold"][0] == "hbm"
+
+
+def _bench():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_dump_outputs_sample_is_fixed_and_bounded(tmp_path):
+    """--dump-outputs keeps every row of a short output and the same seeded, ordered row sample of a long one, and the
+    largest dump (C4: features + collected audio and facial rows, with their row indices) fits in 64 MB."""
+    import numpy as np
+    bench = _bench()
+    assert np.array_equal(bench.dump_row_index(1000), np.arange(1000))
+    big = bench.dump_row_index(60 * 6239)
+    assert np.array_equal(big, bench.dump_row_index(60 * 6239)) and len(big) == bench.DUMP_ROWS
+    assert np.all(np.diff(big) > 0) and big[-1] < 60 * 6239
+    worst = bench.DUMP_ROWS * ((256 + 256 + 61) * 4 + 3 * 8)
+    assert worst <= bench.DUMP_LIMIT_BYTES == 64 << 20
+    bench.write_outputs(str(tmp_path / "d"), {"features": np.ones((3, 256), np.float32),
+                                              "features_rows": np.arange(3.0)})
+    assert sorted(os.listdir(tmp_path / "d")) == ["features.npy", "features_rows.npy"]
+    with pytest.raises(AssertionError):
+        bench.write_outputs(str(tmp_path / "e"), {"features_rows": np.arange(3)})          # int64: not a float dump
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_steps_rows(tmp_path):
+    """bench.py --dump-outputs on C3 (features + collect_features): float arrays within 64 MB, and the sampled feature and
+    collected rows are the rows a direct device call on the same synthetic inputs returns, bit for bit."""
+    import subprocess
+    import sys
+
+    import numpy as np
+    import torch
+    out_dir = tmp_path / "dump"
+    subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c3", "--steps", "2", "--warmup", "1",
+                    "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(out_dir)],
+                   check=True, cwd=str(tmp_path), timeout=1200, stdout=subprocess.DEVNULL)
+    got = {f[:-len(".npy")]: np.load(out_dir / f) for f in os.listdir(out_dir)}
+    assert set(got) == {p + s for p in ("features", "collect_audio", "collect_facial") for s in ("", "_rows")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    bench = _bench()
+    from neurosync_trainer_lite_b200 import engine, synth
+    w = bench.WORKLOADS["c3"]
+    packed, off, _, mine, _ = bench.make_inputs("c3", 0, 1, "strong")
+    eng = engine.get_engine(w["sr"], w["F"], w["H"], device=0)
+    dev = torch.device("cuda", 0)
+    rows, _ = eng.extract_device(torch.from_numpy(packed).to(dev), off)
+    facial = np.concatenate([synth.synth_facial(bench.FACIAL_ROWS, seed=int(i) % 6) for i in mine]).astype(np.float32)
+    f_off = np.arange(len(mine) + 1, dtype=np.int64) * bench.FACIAL_ROWS
+    col_a, col_f, _ = eng.collect_device(rows, eng.row_offsets(off), torch.from_numpy(facial).to(dev), f_off, **w["collect"])
+    for name, full in (("features", rows), ("collect_audio", col_a), ("collect_facial", col_f)):
+        idx = got[name + "_rows"].astype(np.int64)
+        assert np.array_equal(idx, bench.dump_row_index(full.shape[0])), name
+        np.testing.assert_array_equal(got[name], full[torch.from_numpy(idx).to(dev)].cpu().numpy(), err_msg=name)

@@ -166,9 +166,10 @@ def test_entry_points_file_bytes_and_too_short(golden, ef, tmp_path, capsys):
     assert y.dtype == np.float32
     fb, yb = ef.extract_audio_features(synth.wav_bytes(g["pcm88"], 88200), 88200, True)
     np.testing.assert_array_equal(fb, feats)
-    f16, y16 = ef.extract_audio_features(synth.wav_bytes(g["pcm16"], 16000), 16000, True)
-    check_rows(f16, g["feats16"])
-    np.testing.assert_array_equal(y16, g["y16"])
+    g16 = golden("entry_points_16k")
+    f16, y16 = ef.extract_audio_features(synth.wav_bytes(g16["pcm16"], 16000), 16000, True)
+    check_rows(f16, g16["feats16"])
+    np.testing.assert_array_equal(y16, g16["y16"])
     short = np.zeros(8 * 735 + 1469, dtype=np.int16)
     short[100] = 1000
     capsys.readouterr()
@@ -307,7 +308,7 @@ def test_augmentation_kats_bit_exact(golden, dp):
                                                           blend_frames=7))])
 def test_collect_matches_reference_golden(tag, kw, golden, dp, oracle):
     """C3 shapes: 1801 audio rows (oracle features of the C1 clip) + 1800 facial rows -> bit-exact."""
-    g = golden("collect_c3")
+    g = golden("collect_c3_" + tag)
     y = synth.synth_clip(30.0, 88200, seed=0, kind="voiced")
     audio = oracle.extract_and_combine_features(y, 88200, 1470, 735)   # the checker makes the input
     facial = synth.synth_facial(1800, seed=0)

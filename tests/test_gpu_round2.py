@@ -46,6 +46,8 @@ KNOBS = {
     "trim": dict(trim_padded=True),
     "edge_trim": dict(padding_mode="edge", trim_padded=True),
 }
+# the reference returned identical arrays for these knobs on both clips: autocorr_knobs.npz stores them once
+KNOB_STORED_AS = {"trim": "nopad", "edge_trim": "nopad"}
 
 
 @pytest.mark.parametrize("clip", ["a", "b"])
@@ -55,7 +57,7 @@ def test_autocorr_knobs_match_reference_golden(clip, knob, golden, efu, oracle):
     y, sr = g[f"{clip}_y"], int(g[f"{clip}_sr"])
     F, H = oracle.frame_params(sr)
     got = efu.extract_overlapping_autocorr(y, sr, F, H, **KNOBS[knob])
-    want = g[f"{clip}_{knob}"]
+    want = g[f"{clip}_{KNOB_STORED_AS.get(knob, knob)}"]
     assert got.shape == want.shape and got.dtype == np.float64     # frame counts bit-exact
     assert np.abs(got - want).max() <= TOL_AC
 
