@@ -311,6 +311,51 @@ NSF_API int64_t nsf_resample_design(int32_t orig_sr, int32_t target_sr, double* 
 NSF_API nsf_status nsf_resample_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_format, int64_t n_in,
                                      int32_t orig_sr, int32_t target_sr, float* out_host, int64_t out_capacity);
 
+/* ---- WAV conversion: decode + downmix + resample for a ragged batch ---------------------------------
+ * Raw WAV data-chunk bytes in (any encoding decode_wav of utils/audio/load_audio.py accepts, any channel count,
+ * any rate), mono float32 at target_sr out.  Clip i is described by sources[i]: `frames` interleaved frames of
+ * `channels` samples of `encoding` starting `byte_offset` bytes into the payload.  Per clip the output is, bit for
+ * bit, what decode_wav followed by nsf_resample_host (at the context's NSF_OPT_RESAMPLE_QUALITY) produces:
+ *   decode   u8 (v - 128) / 128, i16 v / 32768, i24 v / 2^23, i32 v / 2^31 (rounded once to float32), f32 as is,
+ *            f64 rounded to nearest float32;
+ *   downmix  the channel mean in NumPy's order (mean(axis=1, dtype=float32): pairwise summation, then one
+ *            division by the channel count); mono clips are not touched;
+ *   resample the polyphase filter of nsf_resample_host when sample_rate != target_sr (same float64 FMA chain per
+ *            output); a clip already at target_sr is decode-only.
+ * Every descriptor is validated on the host before anything is launched (NSF_ERR_BAD_ARG): a known encoding,
+ * 1 <= channels <= 65535, frames >= 0, sample_rate > 0, the byte range inside payload_bytes, and 2-, 4- and 8-byte
+ * containers at addresses that are multiples of their size (a misaligned device load would fault).
+ *   nsf_convert_offsets  out_offsets[0] = 0, out_offsets[i + 1] = out_offsets[i] + output length of clip i
+ *                        (frames at target_sr, else nsf_resample_len(frames, sample_rate, target_sr)); runs without
+ *                        a GPU; out_offsets has n + 1 entries.
+ *   nsf_convert_batch    device payload -> device float32, stream-ordered; clip i writes
+ *                        out_dev[out_offsets[i], out_offsets[i + 1]) (out_offsets_host NULL = the prefix sum).
+ *                        Descriptors go through the descriptor ring.  Filter tables are cached in the context per
+ *                        (rate pair, quality): the FIRST use of a pair uploads its table synchronously and may wait.
+ *   nsf_convert_host     host payload -> host float32 at the prefix-sum packing; pipelined over clip groups like
+ *                        nsf_extract_host (pageable buffers staged through pinned arenas).  Synchronous. */
+#define NSF_ENC_U8 0
+#define NSF_ENC_I16 1
+#define NSF_ENC_I24 2
+#define NSF_ENC_I32 3
+#define NSF_ENC_F32 4
+#define NSF_ENC_F64 5
+typedef struct nsf_pcm_source {
+  int64_t byte_offset;  /* first byte of the clip's frames in the payload                */
+  int64_t frames;       /* interleaved frames (data bytes // (bytes per sample * channels)) */
+  int32_t encoding;     /* NSF_ENC_*                                                     */
+  int32_t channels;
+  int32_t sample_rate;
+  int32_t reserved;     /* 0 */
+} nsf_pcm_source;
+NSF_API nsf_status nsf_convert_offsets(const nsf_pcm_source* sources, int32_t n, int32_t target_sr,
+                                       int64_t payload_bytes, int64_t* out_offsets);
+NSF_API nsf_status nsf_convert_batch(nsf_ctx* ctx, void* cuda_stream, const void* payload_dev, int64_t payload_bytes,
+                                     const nsf_pcm_source* sources_host, int32_t n, int32_t target_sr, float* out_dev,
+                                     const int64_t* out_offsets_host);
+NSF_API nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes,
+                                    const nsf_pcm_source* sources, int32_t n, int32_t target_sr, float* out_host);
+
 /* ---- instrumentation -------------------------------------------------------------------------
  * Kernel launches issued by this context since creation (bench.py reports it as gpu_launches). */
 NSF_API int64_t nsf_launch_count(const nsf_ctx* ctx);

@@ -29,6 +29,11 @@ OPT_EDGE_ZERO_THRESHOLD = 0
 OPT_RESAMPLE_QUALITY = 1
 RESAMPLE_POLY, RESAMPLE_HQ = 0, 1
 POST_EDGEFIX, POST_CMVN, POST_DELTAS, POST_REDUCE = 0x1, 0x2, 0x4, 0x8
+ENC_U8, ENC_I16, ENC_I24, ENC_I32, ENC_F32, ENC_F64 = range(6)
+# nsf_pcm_source: one clip of the WAV conversion calls (raw data-chunk bytes -> mono float32)
+PCM_SOURCE = np.dtype([("byte_offset", "<i8"), ("frames", "<i8"), ("encoding", "<i4"), ("channels", "<i4"),
+                       ("sample_rate", "<i4"), ("reserved", "<i4")], align=True)
+assert PCM_SOURCE.itemsize == 32
 STAGE_NAMES = ("peak_normalize", "fold", "stft_gemm", "mel_db", "dct_stats", "cmvn_delta_reduce",
                "autocorr", "post")
 
@@ -98,6 +103,9 @@ _SIGS = {
     "nsf_resample_design": (_i64, [_i32, _i32, _f64p, _i64, _i32p, _i32p, _i32p, _i32p]),
     "nsf_resample_design_q": (_i64, [_i32, _i32, _i32, _f64p, _i64, _i32p, _i32p, _i32p, _i32p]),
     "nsf_resample_host": (_i32, [_vp, _vp, _i32, _i64, _i32, _i32, _vp, _i64]),
+    "nsf_convert_offsets": (_i32, [_vp, _i32, _i32, _i64, _i64p]),
+    "nsf_convert_batch": (_i32, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _i64p]),
+    "nsf_convert_host": (_i32, [_vp, _vp, _i64, _vp, _i32, _i32, _vp]),
     "nsf_launch_count": (_i64, [_vp]),
     "nsf_set_profiling": (None, [_vp, _i32]),
     "nsf_stage_times_ms": (_i32, [_vp, _f32p, _i32]),
@@ -133,3 +141,23 @@ def ptr(array):
         return None
     assert array.flags["C_CONTIGUOUS"]
     return C.c_void_p(array.ctypes.data)
+
+
+def pcm_sources(sources):
+    """C-contiguous ``PCM_SOURCE`` array from an array of that dtype or from (byte_offset, frames, encoding,
+    channels, sample_rate) tuples."""
+    if isinstance(sources, np.ndarray) and sources.dtype == PCM_SOURCE:
+        return np.ascontiguousarray(sources)
+    out = np.zeros(len(sources), dtype=PCM_SOURCE)
+    for i, s in enumerate(sources):
+        out[i] = tuple(s[:5]) + (0,)
+    return out
+
+
+def convert_offsets(sources, target_sr, payload_bytes):
+    """Prefix sum of the per-clip output lengths of a conversion (``nsf_convert_offsets``; validates every
+    descriptor, needs no GPU)."""
+    src = pcm_sources(sources)
+    out = np.empty(len(src) + 1, dtype=np.int64)
+    check(lib.nsf_convert_offsets(ptr(src), len(src), int(target_sr), int(payload_bytes), out.ctypes.data_as(_i64p)))
+    return out

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libnsf.so")
-SOURCES = ["nsf_plan.cpp", "nsf_kernels.cu", "nsf_autocorr_mma.cu", "nsf_stft_tc.cu", "nsf_api.cu"]
+SOURCES = ["nsf_plan.cpp", "nsf_kernels.cu", "nsf_autocorr_mma.cu", "nsf_stft_tc.cu", "nsf_convert.cu", "nsf_api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xptxas=-v", "-Xcompiler", "-fPIC,-O3,-fvisibility=hidden",

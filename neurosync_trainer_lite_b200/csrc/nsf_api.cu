@@ -174,8 +174,16 @@ struct Slot {  // one in-flight clip group of the host pipeline
 constexpr int kDescRing = 8;
 struct DescEntry {
   PinnedArena mem;
+  Arena dev;              // device copy of the entry, for calls whose descriptors have no other home (nsf_convert_batch)
   cudaEvent_t copied = nullptr;
   bool pending = false;
+};
+
+// Polyphase filter of one (rate pair, quality), k-major [kmax][up], resident on the device (nsf_convert_*).
+struct TapTable {
+  int orig = 0, target = 0, quality = 0;
+  int up = 1, down = 1, n_pre_pad = 0, n_pre_remove = 0, kmax = 0;
+  Arena mem;
 };
 
 // Host-side descriptor arrays of a batch (kept in the context: no heap traffic per call after the first).
@@ -206,6 +214,10 @@ struct nsf_ctx {
   cudaEvent_t stage_ev[nsf::kStages + 1] = {};
   bool stage_valid = false;
   nsf::Arena collect_in_a, collect_in_f, collect_out_a, collect_out_f, collect_desc;
+  std::vector<nsf::TapTable*> tap_tables;   // filter cache of the conversion calls, one per (rate pair, quality)
+  std::vector<nsf::ConvClip> conv_clips;    // scratch of convert_enqueue
+  std::vector<nsf_pcm_source> conv_src;     // scratch of nsf_convert_host (one group's rebased descriptors)
+  std::vector<int64_t> conv_off, conv_group_off;
 };
 
 namespace nsf {
@@ -535,7 +547,8 @@ nsf_status nsf_ctx_create(const nsf_plan* plan, int32_t device, nsf_ctx** out_ct
     }
   }
   // opt-in shared-memory limits of every kernel, once per device: no launch path touches function attributes
-  if (!init_kernel_attributes() || !init_autocorr_mma_attributes() || !init_stft_tc_attributes()) {
+  if (!init_kernel_attributes() || !init_autocorr_mma_attributes() || !init_stft_tc_attributes() ||
+      !init_convert_attributes()) {
     set_error(cuda_msg("cudaFuncSetAttribute", cudaGetLastError())); nsf_ctx_destroy(ctx); return NSF_ERR_CUDA;
   }
   for (int i = 0; i <= kStages; ++i) {
@@ -562,7 +575,9 @@ void nsf_ctx_destroy(nsf_ctx* ctx) {
   for (auto& d : ctx->desc) {
     if (d.copied) cudaEventDestroy(d.copied);
     d.mem.release();
+    d.dev.release();
   }
+  for (TapTable* t : ctx->tap_tables) { t->mem.release(); delete t; }
   ctx->table_mem.release();
   ctx->collect_in_a.release(); ctx->collect_in_f.release();
   ctx->collect_out_a.release(); ctx->collect_out_f.release(); ctx->collect_desc.release();
@@ -934,16 +949,170 @@ nsf_status nsf_normalize_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_fo
   return NSF_OK;
 }
 
-// ---- sample-rate conversion ------------------------------------------------------------------------
+// ---- sample-rate conversion + WAV conversion -----------------------------------------------------------
+namespace {
+int enc_bytes(int enc) {
+  switch (enc) {
+    case NSF_ENC_U8: return 1;
+    case NSF_ENC_I16: return 2;
+    case NSF_ENC_I24: return 3;
+    case NSF_ENC_I32: case NSF_ENC_F32: return 4;
+    case NSF_ENC_F64: return 8;
+    default: return 0;
+  }
+}
+int enc_align(int enc) { const int b = enc_bytes(enc); return b == 3 ? 1 : b; }
+
+// Validates every descriptor (nothing is launched for a bad batch) and writes the output prefix sum.  `base` is the
+// address the byte offsets are relative to (0 when only the offsets' own alignment matters).
+nsf_status convert_offsets(const nsf_pcm_source* src, int32_t n, int32_t target_sr, int64_t payload_bytes,
+                           uintptr_t base, int64_t* out_off) {
+  if (!src || !out_off || n <= 0) { set_error("nsf_convert: NULL sources / offsets or n <= 0"); return NSF_ERR_BAD_ARG; }
+  if (target_sr <= 0) { set_error("nsf_convert: target_sr must be positive"); return NSF_ERR_BAD_ARG; }
+  if (payload_bytes < 0) { set_error("nsf_convert: negative payload_bytes"); return NSF_ERR_BAD_ARG; }
+  out_off[0] = 0;
+  for (int i = 0; i < n; ++i) {
+    const nsf_pcm_source& c = src[i];
+    char buf[200];
+    auto fail = [&](const char* what) {
+      std::snprintf(buf, sizeof buf, "nsf_convert: source %d: %s", i, what);
+      set_error(buf);
+      return NSF_ERR_BAD_ARG;
+    };
+    const int bps = enc_bytes(c.encoding);
+    if (bps == 0) return fail("unknown encoding");
+    if (c.channels < 1 || c.channels > 65535) return fail("channels must be in [1, 65535]");
+    if (c.frames < 0) return fail("negative frame count");
+    if (c.sample_rate <= 0) return fail("sample_rate must be positive");
+    if (c.byte_offset < 0 || c.byte_offset > payload_bytes) return fail("byte_offset outside the payload");
+    const int64_t frame_bytes = static_cast<int64_t>(c.channels) * bps;
+    if (c.frames > (payload_bytes - c.byte_offset) / frame_bytes) return fail("byte range past payload_bytes");
+    if ((base + static_cast<uintptr_t>(c.byte_offset)) % static_cast<uintptr_t>(enc_align(c.encoding)) != 0)
+      return fail("samples are not aligned to their container size");
+    const int64_t len = c.sample_rate == target_sr ? c.frames : nsf_resample_len(c.frames, c.sample_rate, target_sr);
+    out_off[i + 1] = out_off[i] + len;
+  }
+  return NSF_OK;
+}
+
+// The context's filter table for (orig, target, its current quality); built and uploaded on first use (synchronous).
+nsf_status get_taps(nsf_ctx* ctx, int orig, int target, const TapTable** out) {
+  const int q = ctx->resample_quality;
+  for (const TapTable* t : ctx->tap_tables)
+    if (t->orig == orig && t->target == target && t->quality == q) { *out = t; return NSF_OK; }
+  ResampleDesign d;
+  if (!(q == NSF_RESAMPLE_HQ ? design_resampler_hq(orig, target, &d) : design_resampler(orig, target, &d))) {
+    set_error("nsf_convert: rates must be positive"); return NSF_ERR_BAD_ARG;
+  }
+  // k-major table [kmax][up]: entry (k, p) = h[p + k up] (zero beyond the last tap).  Neighbouring threads of
+  // k_convert_resample hold different phases at the same k, so their loads fall into one short row
+  const int n_taps = static_cast<int>(d.h.size());
+  const int kmax = (n_taps + d.up - 1) / d.up;
+  std::vector<double> pm(static_cast<size_t>(d.up) * kmax, 0.0);
+  for (int i = 0; i < n_taps; ++i) pm[static_cast<size_t>(i / d.up) * d.up + i % d.up] = d.h[i];
+  TapTable* t = new TapTable();
+  t->orig = orig; t->target = target; t->quality = q;
+  t->up = d.up; t->down = d.down; t->n_pre_pad = d.n_pre_pad; t->n_pre_remove = d.n_pre_remove; t->kmax = kmax;
+  nsf_status st = t->mem.reserve(pm.size() * sizeof(double));
+  if (st == NSF_OK && cudaMemcpy(t->mem.ptr, pm.data(), pm.size() * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) {
+    set_error(cuda_msg("nsf_convert: filter upload", cudaGetLastError()));
+    st = NSF_ERR_CUDA;
+  }
+  if (st != NSF_OK) { t->mem.release(); delete t; return st; }
+  ctx->tap_tables.push_back(t);
+  *out = t;
+  return NSF_OK;
+}
+
+// Input frames of the window a k_convert_resample block of `span` outputs reads (upper bound over every tile).
+int64_t window_frames(const TapTable& t, int64_t span) { return ((span - 1) * t.down + t.up - 1) / t.up + 1 + t.kmax; }
+
+// Enqueues the conversion of n validated clips: clip i reads payload_dev + src[i].byte_offset and writes
+// out_dev[out_off[i], out_off[i + 1]).  Same-rate clips are decode-only unless always_resample (nsf_resample_host
+// filters at every rate pair, 1:1 included).  At most two launches (decode, resample); the descriptors travel through
+// the ring, whose entry is released only after the kernels that read it.
+nsf_status convert_enqueue(nsf_ctx* ctx, cudaStream_t s, const void* payload_dev, const nsf_pcm_source* src, int n,
+                           int32_t target_sr, const int64_t* out_off, float* out_dev, bool always_resample) {
+  std::vector<ConvClip>& cl = ctx->conv_clips;
+  cl.clear();
+  int64_t tiles[2] = {0, 0};
+  int n_kind[2] = {0, 0};
+  int64_t max_window = 0;
+  for (int pass = 0; pass < 2; ++pass) {            // decode-only clips first, then the resampled ones
+    for (int i = 0; i < n; ++i) {
+      const nsf_pcm_source& c = src[i];
+      const bool resample = always_resample || c.sample_rate != target_sr;
+      if (resample != (pass == 1)) continue;
+      const int64_t n_out = out_off[i + 1] - out_off[i];
+      if (n_out <= 0) continue;
+      ConvClip v{};
+      v.byte_off = c.byte_offset; v.frames = c.frames; v.out_off = out_off[i]; v.n_out = n_out;
+      v.enc = c.encoding; v.channels = c.channels; v.bps = enc_bytes(c.encoding);
+      int64_t nt;
+      if (!resample) {
+        nt = (c.frames + kConvDecodeTile - 1) / kConvDecodeTile;
+      } else {
+        const TapTable* t = nullptr;
+        const nsf_status st = get_taps(ctx, c.sample_rate, target_sr, &t);
+        if (st != NSF_OK) return st;
+        v.taps = static_cast<const double*>(t->mem.ptr);
+        v.up = t->up; v.down = t->down; v.n_pre_pad = t->n_pre_pad; v.n_pre_remove = t->n_pre_remove; v.kmax = t->kmax;
+        // tile: `slots` outputs (a multiple of up, >= 256 when up allows it) x `reps` outputs per slot, as large as
+        // the float64 input window in shared memory allows
+        // the slot count keeps the 256 threads busy: the multiple of up (up to 32 up) whose passes over the
+        // block waste the fewest threads, preferring more outputs per slot
+        const int64_t budget = static_cast<int64_t>(kConvMaxSmem / sizeof(double));
+        int64_t slots = 0;
+        int reps = 0;
+        double best = -1.0;
+        for (int r = kConvMaxReps; r >= 1 && best < 0.9; r /= 2)
+          for (int64_t m = 1; m <= 32; ++m) {
+            const int64_t sl = m * t->up;
+            if (window_frames(*t, sl * r) > budget) break;
+            const double eff = static_cast<double>(sl) / (256.0 * ((sl + 255) / 256));
+            if (eff > best + 1e-9) { best = eff; slots = sl; reps = r; }
+          }
+        if (slots == 0) { set_error("nsf_convert: rate pair needs a larger filter window than one block holds"); return NSF_ERR_UNSUPPORTED; }
+        if (slots > (int64_t(1) << 30)) { set_error("nsf_convert: rate pair too large"); return NSF_ERR_UNSUPPORTED; }
+        v.slots = static_cast<int32_t>(slots); v.reps = reps;
+        max_window = std::max(max_window, window_frames(*t, slots * reps));
+        nt = (n_out + slots * reps - 1) / (slots * reps);
+      }
+      if (nt <= 0) continue;
+      v.tile0 = tiles[pass];
+      tiles[pass] += nt;
+      ++n_kind[pass];
+      cl.push_back(v);
+    }
+  }
+  if (cl.empty()) return NSF_OK;
+  if (tiles[0] > INT32_MAX || tiles[1] > INT32_MAX) { set_error("nsf_convert: batch too large for one launch"); return NSF_ERR_UNSUPPORTED; }
+  const size_t bytes = cl.size() * sizeof(ConvClip);
+  DescEntry* de = nullptr;
+  nsf_status st = desc_acquire(ctx, bytes, &de);
+  if (st != NSF_OK) return st;
+  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
+  std::memcpy(de->mem.ptr, cl.data(), bytes);
+  const ConvClip* d = static_cast<const ConvClip*>(de->dev.ptr);
+  NSF_CUDA(cudaMemcpyAsync(de->dev.ptr, de->mem.ptr, bytes, cudaMemcpyHostToDevice, s));
+  int launched = 0;
+  for (int kind = 0; kind < 2; ++kind) {
+    const ConvClip* first = d + (kind == 0 ? 0 : n_kind[0]);
+    const int m = launch_convert(s, kind == 1, first, n_kind[kind], tiles[kind],
+                                 kind == 1 ? static_cast<size_t>(max_window) * sizeof(double) : 0, payload_dev, out_dev);
+    if (m < 0) { set_error(cuda_msg("launch_convert", cudaGetLastError())); return NSF_ERR_CUDA; }
+    launched += m;
+  }
+  ctx->launches += launched;
+  return desc_commit(de, s);     // recorded after the kernels: the entry (host and device) is reused only after them
+}
+}  // namespace
+
 nsf_status nsf_resample_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_format, int64_t n_in, int32_t orig_sr,
                              int32_t target_sr, float* out_host, int64_t out_capacity) {
   if (!ctx || !pcm_host || !out_host || n_in <= 0) { set_error("nsf_resample_host: NULL argument or empty input"); return NSF_ERR_BAD_ARG; }
   if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
-  ResampleDesign d;
-  if (!(ctx->resample_quality == NSF_RESAMPLE_HQ ? design_resampler_hq(orig_sr, target_sr, &d)
-                                                 : design_resampler(orig_sr, target_sr, &d))) {
-    set_error("nsf_resample_host: rates must be positive"); return NSF_ERR_BAD_ARG;
-  }
+  if (orig_sr <= 0 || target_sr <= 0) { set_error("nsf_resample_host: rates must be positive"); return NSF_ERR_BAD_ARG; }
   const int64_t n_out = nsf_resample_len(n_in, orig_sr, target_sr);
   if (out_capacity < n_out) { set_error("nsf_resample_host: out_capacity < nsf_resample_len()"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
@@ -951,23 +1120,109 @@ nsf_status nsf_resample_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_for
   nsf_status st = ensure_slot(sl);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  // phase-major tap table [up][kmax]: row p holds h[p], h[p + up], h[p + 2 up], ...
-  const int n_taps = static_cast<int>(d.h.size());
-  const int kmax = (n_taps + d.up - 1) / d.up;
-  std::vector<double> pm(static_cast<size_t>(d.up) * kmax, 0.0);
-  for (int i = 0; i < n_taps; ++i) pm[static_cast<size_t>(i % d.up) * kmax + i / d.up] = d.h[i];
+  // one mono clip of the conversion kernel (float32 samples are its f32 encoding, int16 its i16 encoding)
+  const nsf_pcm_source src{0, n_in, pcm_format == NSF_PCM_I16 ? NSF_ENC_I16 : NSF_ENC_F32, 1, orig_sr, 0};
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
+  const int64_t off[2] = {0, n_out};
   if ((st = sl->pcm.reserve(static_cast<size_t>(n_in) * esz)) != NSF_OK) return st;
   if ((st = sl->ynorm.reserve(static_cast<size_t>(n_out) * sizeof(float))) != NSF_OK) return st;
-  if ((st = sl->work.reserve(pm.size() * sizeof(double))) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(sl->work.ptr, pm.data(), pm.size() * sizeof(double), cudaMemcpyHostToDevice, sl->stream));
   NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, pcm_host, static_cast<size_t>(n_in) * esz, cudaMemcpyHostToDevice, sl->stream));
-  const int n = launch_resample(sl->stream, sl->pcm.ptr, pcm_format, n_in, d.up, d.down, d.n_pre_pad, d.n_pre_remove,
-                                static_cast<const double*>(sl->work.ptr), kmax, static_cast<float*>(sl->ynorm.ptr), n_out);
-  if (n < 0) { set_error(cuda_msg("launch_resample", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n;
+  if ((st = convert_enqueue(ctx, sl->stream, sl->pcm.ptr, &src, 1, target_sr, off, static_cast<float*>(sl->ynorm.ptr),
+                            true)) != NSF_OK) return st;
   NSF_CUDA(cudaMemcpyAsync(out_host, sl->ynorm.ptr, static_cast<size_t>(n_out) * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));     // pm (host vector) must outlive its async copy
+  NSF_CUDA(cudaStreamSynchronize(sl->stream));
+  return NSF_OK;
+}
+
+nsf_status nsf_convert_offsets(const nsf_pcm_source* sources, int32_t n, int32_t target_sr, int64_t payload_bytes,
+                               int64_t* out_offsets) {
+  return convert_offsets(sources, n, target_sr, payload_bytes, 0, out_offsets);
+}
+
+nsf_status nsf_convert_batch(nsf_ctx* ctx, void* cuda_stream, const void* payload_dev, int64_t payload_bytes,
+                             const nsf_pcm_source* sources, int32_t n, int32_t target_sr, float* out_dev,
+                             const int64_t* out_offsets_host) {
+  if (!ctx || !payload_dev || !out_dev) { set_error("nsf_convert_batch: NULL argument"); return NSF_ERR_BAD_ARG; }
+  std::vector<int64_t>& off = ctx->conv_off;
+  off.resize(n > 0 ? n + 1 : 1);
+  nsf_status st = convert_offsets(sources, n, target_sr, payload_bytes, reinterpret_cast<uintptr_t>(payload_dev), off.data());
+  if (st != NSF_OK) return st;
+  if (out_offsets_host) {
+    for (int i = 0; i < n; ++i)
+      if (out_offsets_host[i + 1] - out_offsets_host[i] != off[i + 1] - off[i]) {
+        set_error("nsf_convert_batch: out_offsets is not a prefix sum of the output lengths"); return NSF_ERR_BAD_ARG;
+      }
+    for (int i = 0; i <= n; ++i) off[i] = out_offsets_host[i];
+  }
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  return convert_enqueue(ctx, static_cast<cudaStream_t>(cuda_stream), payload_dev, sources, n, target_sr, off.data(),
+                         out_dev, false);
+}
+
+nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes, const nsf_pcm_source* sources,
+                            int32_t n, int32_t target_sr, float* out_host) {
+  if (!ctx || !payload_host || !out_host) { set_error("nsf_convert_host: NULL argument"); return NSF_ERR_BAD_ARG; }
+  std::vector<int64_t>& all = ctx->conv_group_off;
+  all.resize(n > 0 ? n + 1 : 1);
+  nsf_status st = convert_offsets(sources, n, target_sr, payload_bytes, 0, all.data());
+  if (st != NSF_OK) return st;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  for (auto& sl : ctx->slot) sl.n_pending = 0;
+  const bool in_dma = dma_reachable(payload_host), out_dma = dma_reachable(out_host);
+  // clip groups by output budget, rotating over the slots: the upload of group g + 1, the kernels of group g and the
+  // download of group g - 1 overlap (see nsf_extract_host)
+  int first = 0, turn = 0;
+  while (first < n) {
+    int last = first;
+    while (last < n && (last == first || all[last + 1] - all[first] <= group_budget(turn))) ++last;
+    Slot* sl = &ctx->slot[turn % kSlots];
+    if ((st = ensure_slot(sl)) != NSF_OK) return st;
+    if ((st = drain_slot(sl)) != NSF_OK) return st;
+    // the group's input bytes [b0, b1), b0 rounded down to 8 so every container keeps its alignment in the arena
+    int64_t b0 = INT64_MAX, b1 = 0;
+    for (int i = first; i < last; ++i) {
+      const nsf_pcm_source& c = sources[i];
+      const int64_t end = c.byte_offset + c.frames * c.channels * enc_bytes(c.encoding);
+      if (c.frames > 0) { b0 = std::min(b0, c.byte_offset); b1 = std::max(b1, end); }
+    }
+    if (b0 > b1) b0 = b1 = 0;
+    b0 &= ~int64_t(7);
+    const int64_t in_bytes = b1 - b0, n_out = all[last] - all[first];
+    std::vector<nsf_pcm_source>& g = ctx->conv_src;
+    std::vector<int64_t>& goff = ctx->conv_off;
+    g.assign(sources + first, sources + last);
+    goff.resize(last - first + 1);
+    for (int i = first; i < last; ++i) { g[i - first].byte_offset = sources[i].frames > 0 ? sources[i].byte_offset - b0 : 0; }
+    for (int i = first; i <= last; ++i) goff[i - first] = all[i] - all[first];
+    if ((st = sl->pcm.reserve(std::max<int64_t>(in_bytes, 1))) != NSF_OK) return st;
+    if ((st = sl->out.reserve(std::max<int64_t>(n_out, 1) * sizeof(float))) != NSF_OK) return st;
+    if (in_bytes > 0) {
+      const char* src = static_cast<const char*>(payload_host) + b0;
+      if (!in_dma) {
+        if ((st = sl->stage_in.reserve(in_bytes)) != NSF_OK) return st;
+        host_copy(sl->stage_in.ptr, src, in_bytes);
+        src = static_cast<const char*>(sl->stage_in.ptr);
+      }
+      NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, src, in_bytes, cudaMemcpyHostToDevice, sl->stream));
+    }
+    if ((st = convert_enqueue(ctx, sl->stream, sl->pcm.ptr, g.data(), last - first, target_sr, goff.data(),
+                              static_cast<float*>(sl->out.ptr), false)) != NSF_OK) return st;
+    if (n_out > 0) {
+      float* dst = out_host + all[first];
+      const size_t bytes = static_cast<size_t>(n_out) * sizeof(float);
+      if (!out_dma) {
+        if ((st = sl->stage_out.reserve(bytes)) != NSF_OK) return st;
+        NSF_CUDA(cudaMemcpyAsync(sl->stage_out.ptr, sl->out.ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
+        sl->pending[sl->n_pending++] = Slot::CopyOut{dst, sl->stage_out.ptr, bytes, 0, 0, 0, 1};
+      } else {
+        NSF_CUDA(cudaMemcpyAsync(dst, sl->out.ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
+      }
+    }
+    first = last;
+    ++turn;
+  }
+  for (auto& sl : ctx->slot)
+    if (sl.stream && (st = drain_slot(&sl)) != NSF_OK) return st;
   return NSF_OK;
 }
 

@@ -151,36 +151,6 @@ __global__ void __launch_bounds__(256) k_normalize(const T* __restrict__ pcm, Ba
 // ------------------------------------------------------------------------------------------------
 // Validation STFT path, fp32 on CUDA cores: fold (signed 4-tap gather) + small GEMMs + |.|^2
 // ------------------------------------------------------------------------------------------------
-// Sample-rate conversion: out[j] = sum_n h[(j + n_pre_remove) down - n_pre_pad - n up] x[n], the
-// polyphase form of scipy.signal.resample_poly (librosa.resample / librosa.load(sr=) stand-in, see
-// nsf.h).  One thread per output sample: t = (j + n_pre_remove) down - n_pre_pad selects the phase
-// t mod up (one contiguous row of the phase-major tap table) and the newest input sample t / up; the
-// ~21 (upsampling) to 20 down + 1 taps are accumulated in float64 and rounded once.  Neighbouring
-// threads read overlapping input windows (L1) and at most `up` distinct tap rows, so the kernel is
-// bound by the 4 (or 2) bytes in + 4 bytes out per sample.
-// ------------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256) k_resample(const T* __restrict__ x, int64_t n_in, int up, int down,
-                                                  int n_pre_pad, int n_pre_remove,
-                                                  const double* __restrict__ taps_pm, int kmax,
-                                                  float* __restrict__ out, int64_t n_out) {
-  for (int64_t j = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; j < n_out;
-       j += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int64_t t = (j + n_pre_remove) * down - n_pre_pad;     // > 0 by construction of the padding
-    const int64_t n_hi = t / up;
-    const int phase = static_cast<int>(t - n_hi * up);
-    const double* h = taps_pm + static_cast<int64_t>(phase) * kmax;
-    double acc = 0.0;
-    for (int k = 0; k < kmax; ++k) {
-      const int64_t n = n_hi - k;
-      if (n < 0) break;
-      if (n < n_in) acc = fma(__ldg(h + k), static_cast<double>(decode_pcm<T>(x[n])), acc);
-    }
-    out[j] = static_cast<float>(acc);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_fold32(DeviceTables t, BatchView b,
                                                 const float* __restrict__ y,
                                                 float* __restrict__ a32) {
@@ -1661,20 +1631,6 @@ int launch_mel_db(cudaStream_t s, const DeviceTables& t, const BatchView& b, con
   per_sm = per_sm < 1 ? 1 : (per_sm > 4 ? 4 : per_sm);
   const int grid = grid_for((b.total_frames + kMelFrames - 1) / kMelFrames, 1, kSmCount * per_sm);
   k_mel_db<<<grid, kMelWarps * 32, smem, s>>>(t, b, power, db, dbmax_key, chain_cols);
-  NSF_CHECK_LAUNCH();
-  return 1;
-}
-
-int launch_resample(cudaStream_t s, const void* pcm, int pcm_format, int64_t n_in, int up, int down,
-                    int n_pre_pad, int n_pre_remove, const double* taps_pm, int kmax, float* out, int64_t n_out) {
-  if (n_out <= 0) return 0;
-  const int grid = grid_for(n_out, 256, kSmCount * 8);
-  if (pcm_format == NSF_PCM_I16)
-    k_resample<int16_t><<<grid, 256, 0, s>>>(static_cast<const int16_t*>(pcm), n_in, up, down, n_pre_pad, n_pre_remove,
-                                              taps_pm, kmax, out, n_out);
-  else
-    k_resample<float><<<grid, 256, 0, s>>>(static_cast<const float*>(pcm), n_in, up, down, n_pre_pad, n_pre_remove,
-                                            taps_pm, kmax, out, n_out);
   NSF_CHECK_LAUNCH();
   return 1;
 }

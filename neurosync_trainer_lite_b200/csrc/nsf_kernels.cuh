@@ -106,10 +106,25 @@ int launch_collect(cudaStream_t s, int dtype, const CollectView& v, const void* 
 // stand-alone row helpers (interpolate_slower / smooth / one stack_with_blend step)
 int launch_rows_op(cudaStream_t s, int op, int dtype, const void* a, int64_t na, const void* b,
                    int64_t nb, int cols, int64_t k_blend, void* out, int64_t out_rows);
-// polyphase sample-rate conversion (scipy.signal.resample_poly arithmetic); taps_pm is the filter in
-// phase-major float64 layout [up][kmax] (zero beyond the last tap of a phase)
-int launch_resample(cudaStream_t s, const void* pcm, int pcm_format, int64_t n_in, int up, int down,
-                    int n_pre_pad, int n_pre_remove, const double* taps_pm, int kmax, float* out, int64_t n_out);
+// WAV conversion (nsf_convert.cu): one descriptor per clip.  `taps` is the clip's polyphase filter in k-major
+// float64 layout [kmax][up] (zero beyond the last tap of a phase); decode-only clips leave the resampling fields 0.
+struct ConvClip {
+  int64_t byte_off;   // clip's first byte in the payload
+  int64_t frames;     // input frames
+  int64_t out_off;    // first output sample
+  int64_t n_out;      // output samples
+  int64_t tile0;      // first block of the clip in its launch
+  const double* taps;
+  int32_t enc, channels, bps;
+  int32_t up, down, n_pre_pad, n_pre_remove, kmax;
+  int32_t slots, reps;   // resampling tile: `slots` (a multiple of up) x `reps` outputs per block
+};
+constexpr int kConvDecodeTile = 4096;          // frames per block of k_convert_decode
+constexpr int kConvMaxReps = 8;                // outputs per thread slot of k_convert_resample
+constexpr size_t kConvMaxSmem = 96 * 1024;     // input window of one k_convert_resample block (float64)
+// resample = false: k_convert_decode, else k_convert_resample with `smem_bytes` of dynamic shared memory
+int launch_convert(cudaStream_t s, bool resample, const ConvClip* clips_dev, int n_clips, int64_t tiles,
+                   size_t smem_bytes, const void* payload, float* out);
 // generic per-channel statistics of one [T][C] matrix and the edge fix
 int launch_col_stats(cudaStream_t s, const float* in, int64_t T, int C, double* sum, double* sumsq);
 int launch_edge_fix(cudaStream_t s, float* data, int64_t T, int C, float zero_threshold);
@@ -126,6 +141,7 @@ int launch_chunk_blend(cudaStream_t s, const float* decoded, int64_t n_rows, int
 bool init_kernel_attributes();        // nsf_kernels.cu
 bool init_autocorr_mma_attributes();  // nsf_autocorr_mma.cu
 bool init_stft_tc_attributes();       // nsf_stft_tc.cu
+bool init_convert_attributes();       // nsf_convert.cu
 
 }  // namespace nsf
 #endif  // NSF_KERNELS_CUH_

@@ -9,7 +9,8 @@ arithmetic of the reference (same operation order, IEEE add/mul, no FMA contract
 
 ``load_data`` keeps the reference signature but builds the whole dataset in ONE pipelined device pass
 (``load_data_batched``): the folders are scanned first, every take without a feature cache is read straight
-into a page-locked int16 arena, ``nsf_extract_collect_host`` turns PCM + facial rows into augmented rows
+into a page-locked arena (int16 samples when every take is mono PCM16 at 88.2 kHz, else the raw WAV bytes, which
+``nsf_convert_host`` decodes, downmixes and resamples on the device), ``nsf_extract_collect_host`` turns PCM + facial rows into augmented rows
 without the feature rows ever leaving the GPU, and the examples are float32 (``dataset/dataset.py:75`` casts to
 float32 anyway).  ``process_folder`` / ``collect_features`` remain the
 per-take float64 route, bit-identical to the reference's NumPy arithmetic.
@@ -242,6 +243,47 @@ def _pcm16_payload(path, sr):
         return None
 
 
+_WAV_ENCODINGS = {(1, 8): nv.ENC_U8, (1, 16): nv.ENC_I16, (1, 24): nv.ENC_I24, (1, 32): nv.ENC_I32,
+                  (3, 32): nv.ENC_F32, (3, 64): nv.ENC_F64}
+_ENC_BYTES = {nv.ENC_U8: 1, nv.ENC_I16: 2, nv.ENC_I24: 3, nv.ENC_I32: 4, nv.ENC_F32: 4, nv.ENC_F64: 8}
+
+
+def _wav_source(path):
+    """(data offset, data bytes, encoding, channels, rate) of a RIFF/WAVE file, read from its headers only.
+
+    The chunk walk of ``decode_wav`` (utils/audio/load_audio.py), step for step: WAVE_FORMAT_EXTENSIBLE takes its
+    format tag from the sub-format GUID, odd-sized chunks are padded, the first ``data`` chunk ends the walk and is
+    truncated at the end of the file.  Raises ``decode_wav``'s ``ValueError`` for what ``decode_wav`` rejects.  A
+    header declaring 0 channels (which ``decode_wav`` reads as mono) reports 1."""
+    import struct
+    size_all = os.path.getsize(path)
+    with open(path, "rb") as fh:
+        head = fh.read(12)
+        if len(head) < 12 or head[:4] != b"RIFF" or head[8:12] != b"WAVE":
+            raise ValueError("not a RIFF/WAVE stream (only WAV decoding is built in)")
+        pos, fmt, data = 12, None, None
+        while pos + 8 <= size_all:
+            fh.seek(pos)
+            hdr = fh.read(8)
+            tag, size = hdr[:4], struct.unpack_from("<I", hdr, 4)[0]
+            if tag == b"fmt ":
+                body = fh.read(size)
+                fmt = struct.unpack_from("<HHIIHH", body, 0)
+                if fmt[0] == 0xFFFE and len(body) >= 26:
+                    fmt = (struct.unpack_from("<H", body, 24)[0],) + fmt[1:]
+            elif tag == b"data":
+                data = (pos + 8, min(size, size_all - (pos + 8)))
+                break
+            pos += 8 + size + (size & 1)
+    if fmt is None or data is None:
+        raise ValueError("WAV stream lacks a fmt or data chunk")
+    code, channels, rate, _, _, bits = fmt
+    enc = _WAV_ENCODINGS.get((code, bits))
+    if enc is None:
+        raise ValueError(f"unsupported WAV encoding (format {code}, {bits} bit)")
+    return data[0], data[1], enc, max(int(channels), 1), int(rate)
+
+
 def _read_into(path, offset, dst):
     with open(path, "rb", buffering=0) as fh:
         fh.seek(offset)
@@ -289,7 +331,8 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
     extracted); a rank only touches - and only runs ffmpeg for - its own takes.
 
     ``dtype=np.float32`` (default, the training format): takes without a feature cache are read straight
-    into page-locked int16 memory by a thread pool, go through ``nsf_extract_collect_host`` (features and
+    into page-locked memory by a thread pool (int16 samples, or raw WAV bytes converted to float32 at 88.2 kHz by
+    ``nsf_convert_host`` exactly as ``decode_for_path`` would when any take is in another format or rate), go through ``nsf_extract_collect_host`` (features and
     augmentation fused, rows never leave the device in between) and come back as float32 arrays; cached takes are augmented by one float32 ``nsf_collect_host`` call.
     ``dtype=np.float64``: extraction batched, augmentation through the float64 kernel - bit-identical to
     the per-folder builder.  A take shorter than 9 frames raises ``TypeError`` exactly where the
@@ -299,7 +342,7 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
 
     from .. import shard
     from ..utils.audio.extraction.extract_features import MIN_FRAMES
-    from ..utils.audio.load_audio import REFERENCE_RATE, decode_for_path
+    from ..utils.audio.load_audio import REFERENCE_RATE
 
     t_start = time.perf_counter()
     timing = {}
@@ -357,7 +400,8 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
         facial_jobs = {}
 
         # ---- PCM of the takes to extract: mono PCM16 files at 88.2 kHz are read straight into page-locked
-        # int16 memory (2 bytes per sample over PCIe); anything else is decoded / resampled to float32 ----------
+        # int16 memory (2 bytes per sample over PCIe); every other take's raw bytes are decoded, downmixed and
+        # resampled to float32 on the device by nsf_convert_host ------------------------------------------------
         n_rows = {}
         pcm_arena = pcm = off = None
         if todo:
@@ -366,8 +410,26 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
             if fast:
                 lens = [n for _, n in info]
             else:
-                decoded = list(pool.map(lambda tp: _as_float32(decode_for_path(tp[1], sr)[0]), todo))
-                lens = [len(d) for d in decoded]
+                # every other take: raw data-chunk bytes, converted on the device (decode_for_path's arithmetic)
+                heads = list(pool.map(lambda tp: _wav_source(tp[1]), todo))
+                for (_, p), h in zip(todo, heads):
+                    print(f"Loaded audio file '{p}' with sample rate {sr if sr is not None else h[4]}")
+                # sr=None keeps the native rate in decode(): one conversion, native -> 88.2 kHz
+                sr1 = sr if sr is not None else REFERENCE_RATE
+                src = np.zeros(len(todo), dtype=nv.PCM_SOURCE)
+                pos = 0
+                for k, (_, nbytes, enc, ch, rate) in enumerate(heads):
+                    frames = nbytes // (_ENC_BYTES[enc] * ch)
+                    src[k] = (pos, frames, enc, ch, rate, 0)
+                    pos += (frames * _ENC_BYTES[enc] * ch + 7) // 8 * 8          # every take 8-byte aligned
+                mid_off = nv.convert_offsets(src, sr1, pos)                       # native rate -> sr
+                if sr1 != REFERENCE_RATE:                                          # then sr -> 88.2 kHz (load_audio.py:8-10)
+                    mid = np.zeros(len(todo), dtype=nv.PCM_SOURCE)
+                    for k in range(len(todo)):
+                        mid[k] = (int(mid_off[k]) * 4, int(mid_off[k + 1] - mid_off[k]), nv.ENC_F32, 1, sr1, 0)
+                    lens = np.diff(nv.convert_offsets(mid, REFERENCE_RATE, int(mid_off[-1]) * 4))
+                else:
+                    lens = np.diff(mid_off)
             for (i, _), n in zip(todo, lens):
                 g = eng.plan.guard_frames(n)
                 if g < MIN_FRAMES:                                             # extract_features.py:16-20 -> :143
@@ -386,9 +448,21 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
                 for r in reads:
                     r.result()
             else:
-                for k, d in enumerate(decoded):
-                    pcm[off[k]:off[k + 1]] = d
-                del decoded
+                wav_arena = _engine.scratch_pinned("dataset_wav", max(pos, 1))
+                raw = wav_arena.view(np.uint8, (pos,))
+                reads = [pool.submit(_read_into, todo[k][1], heads[k][0], raw[int(src[k]["byte_offset"]):
+                                     int(src[k]["byte_offset"]) + int(src[k]["frames"]) * _ENC_BYTES[heads[k][2]] *
+                                     heads[k][3]]) for k in range(len(todo)) if src[k]["frames"] > 0]
+                facial_jobs = {i: pool.submit(_facial_rows, takes[i][4], dtype) for i in keep}
+                for r in reads:
+                    r.result()
+                if sr1 != REFERENCE_RATE:
+                    y_sr = _engine.scratch_pinned("dataset_wav_mid", max(int(mid_off[-1]) * 4, 1)).view(
+                        np.float32, (int(mid_off[-1]),))
+                    eng.convert_host(raw, src, sr1, out=y_sr)
+                    eng.convert_host(y_sr.view(np.uint8), mid, REFERENCE_RATE, out=pcm)
+                else:
+                    eng.convert_host(raw, src, sr1, out=pcm)
             roff = eng.row_offsets(off)
             for k, (i, _) in enumerate(todo):
                 n_rows[i] = int(roff[k + 1] - roff[k])
@@ -479,6 +553,3 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
     last_timing.update(timing)
     return examples, indices
 
-
-def _as_float32(pcm):
-    return pcm if pcm.dtype == np.float32 else pcm.astype(np.float32) / np.float32(32768)

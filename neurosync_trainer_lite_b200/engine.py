@@ -233,6 +233,54 @@ class Engine:
                                               int(target_sr), nv.ptr(out), n_out))
         return out
 
+    def _set_quality(self, quality):
+        q = {"hq": nv.RESAMPLE_HQ, "poly": nv.RESAMPLE_POLY}[quality]
+        nv.check(nv.lib.nsf_ctx_set_option(self.handle, nv.OPT_RESAMPLE_QUALITY, float(q)))
+
+    # ---- WAV conversion: raw data-chunk bytes -> mono float32 at a target rate -----------------------
+    @staticmethod
+    def convert_offsets(sources, target_sr, payload_bytes):
+        """Output packing of a conversion: prefix sum of the per-clip lengths (``nsf_convert_offsets``)."""
+        return nv.convert_offsets(sources, target_sr, payload_bytes)
+
+    def convert_host(self, payload, sources, target_sr, quality="hq", out=None):
+        """Decode + downmix + resample a ragged batch of WAV clips on the device (``nsf_convert_host``).
+
+        ``payload``: 1-D uint8 host array of raw data-chunk bytes; ``sources``: ``nv.PCM_SOURCE`` array (or
+        tuples ``(byte_offset, frames, encoding, channels, sample_rate)``).  Returns ``(float32 samples,
+        offsets)``; clip i is ``out[offsets[i]:offsets[i + 1]]``, bit for bit ``decode_wav`` followed by
+        ``resample_host(.., quality)``."""
+        payload = np.ascontiguousarray(payload).view(np.uint8).reshape(-1)
+        src = nv.pcm_sources(sources)
+        off = nv.convert_offsets(src, target_sr, payload.nbytes)
+        if out is None:
+            out = np.empty(int(off[-1]), dtype=np.float32)
+        assert out.dtype == np.float32 and out.flags["C_CONTIGUOUS"] and out.size >= int(off[-1])
+        with self._lock:
+            self._set_quality(quality)
+            nv.check(nv.lib.nsf_convert_host(self.handle, nv.ptr(payload), payload.nbytes, nv.ptr(src), len(src),
+                                             int(target_sr), nv.ptr(out)))
+        return out[:int(off[-1])], off
+
+    def convert_device(self, payload, sources, target_sr, quality="hq", out=None, stream=None):
+        """``convert_host`` on device memory (``nsf_convert_batch``, stream-ordered): ``payload`` is a 1-D uint8
+        CUDA tensor; returns ``(float32 CUDA tensor, offsets)``, ready for ``extract_device``."""
+        import torch
+        assert payload.is_cuda and payload.device.index == self.device and payload.is_contiguous()
+        assert payload.dtype == torch.uint8
+        src = nv.pcm_sources(sources)
+        off = nv.convert_offsets(src, target_sr, payload.numel())
+        if out is None:
+            out = torch.empty(int(off[-1]), dtype=torch.float32, device=payload.device)
+        assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() >= int(off[-1])
+        s = torch.cuda.current_stream(payload.device) if stream is None else stream
+        with self._lock:
+            self._set_quality(quality)
+            nv.check(nv.lib.nsf_convert_batch(self.handle, C.c_void_p(s.cuda_stream), C.c_void_p(payload.data_ptr()),
+                                              payload.numel(), nv.ptr(src), len(src), int(target_sr),
+                                              C.c_void_p(out.data_ptr()), off.ctypes.data_as(nv._i64p)))
+        return out[:int(off[-1])], off
+
     # ---- device buffers (torch used for memory and streams only) -------------------------------
     def workspace_bytes(self, total_samples, n_clips, flags=0):
         return nv.lib.nsf_workspace_bytes(self.plan.handle, int(total_samples), int(n_clips), flags)

@@ -11,7 +11,10 @@ Division of labour
   ``NSF_PEAK_NORMALIZE`` so the PCM crosses PCIe once, as int16 when the file is int16.
 * **resampling** (only when the file's rate differs from the requested one) runs on the GPU through
   ``nsf_resample_host``: a rational polyphase filter with the arithmetic of
-  ``scipy.signal.resample_poly`` (Kaiser-windowed sinc), checked against a float64 NumPy oracle.  The
+  ``scipy.signal.resample_poly`` (Kaiser-windowed sinc), checked against a float64 NumPy oracle.
+* ``decode_wav`` + resampling is also the host statement of the batched device conversion
+  (``nsf_convert_*``, ``Engine.convert_host``) that ``load_data`` uses for every take that is not mono PCM16 at
+  88.2 kHz; that route reproduces these functions bit for bit.  The
   reference uses ``soxr_hq``, whose filter is not reproducible here, so this step is *not*
   parity-pinned against the reference; the synthetic benchmark configurations never resample.
 """
