@@ -356,6 +356,32 @@ NSF_API nsf_status nsf_convert_batch(nsf_ctx* ctx, void* cuda_stream, const void
 NSF_API nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes,
                                     const nsf_pcm_source* sources, int32_t n, int32_t target_sr, float* out_host);
 
+/* ---- training windows ------------------------------------------------------------------------------
+ * The consumer of the augmented rows at training time, AudioFacialDataset (dataset/dataset.py:58-98): every stride-1
+ * window of `window` rows of each clip, plus one reflected tail window when the clip's length is not a multiple of
+ * `window`.  Clip i owns audio rows [audio_offsets[i], audio_offsets[i+1]) and facial rows [facial_offsets[i],
+ * facial_offsets[i+1]); top = max(n_audio, n_facial).  Regular window j < top - window + 1 starts at row j; a stream
+ * shorter than j + window is zero-padded.  The tail window starts at row top - window: with seg = min(top, n_rows) -
+ * (top - window) valid rows, row r >= seg is the reflection rows[start + 2 seg - 1 - r] (torch.flip of the segment;
+ * a one-row segment is repeated, which is what torch's broadcast makes of it).  A clip with top < window, or with a
+ * stream whose tail segment is shorter than half a window and not one row (the host route raises for both), is
+ * rejected with NSF_ERR_BAD_ARG, as are decreasing or negative offsets and window < 1.
+ *   nsf_window_offsets  window_offsets[0] = 0, window_offsets[i+1] = window_offsets[i] + (top - window + 1) +
+ *                       (top % window != 0); validates the geometry; host only, no GPU.  n_clips + 1 entries.
+ *   nsf_window_gather   out_audio [n][window][audio_cols], out_facial [n][window][facial_cols] float32, contiguous:
+ *                       windows indices[k] of the dataset (global numbering of nsf_window_offsets), what
+ *                       collate_fn(stack of __getitem__) yields, bit for bit.  Stream-ordered; geometry and every
+ *                       index (in [0, total)) are validated on the host before anything is launched; the offsets and
+ *                       indices go through the descriptor ring.  n == 0 launches nothing (the outputs and indices
+ *                       may then be NULL). */
+NSF_API nsf_status nsf_window_offsets(const int64_t* audio_offsets, const int64_t* facial_offsets, int32_t n_clips,
+                                      int32_t window, int64_t* window_offsets);
+NSF_API nsf_status nsf_window_gather(nsf_ctx* ctx, void* cuda_stream,
+                                     const float* audio_dev, int32_t audio_cols, const int64_t* audio_offsets_host,
+                                     const float* facial_dev, int32_t facial_cols, const int64_t* facial_offsets_host,
+                                     int32_t n_clips, int32_t window, const int64_t* indices_host, int64_t n,
+                                     float* out_audio_dev, float* out_facial_dev);
+
 /* ---- instrumentation -------------------------------------------------------------------------
  * Kernel launches issued by this context since creation (bench.py reports it as gpu_launches). */
 NSF_API int64_t nsf_launch_count(const nsf_ctx* ctx);

@@ -106,6 +106,8 @@ _SIGS = {
     "nsf_convert_offsets": (_i32, [_vp, _i32, _i32, _i64, _i64p]),
     "nsf_convert_batch": (_i32, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _i64p]),
     "nsf_convert_host": (_i32, [_vp, _vp, _i64, _vp, _i32, _i32, _vp]),
+    "nsf_window_offsets": (_i32, [_i64p, _i64p, _i32, _i32, _i64p]),
+    "nsf_window_gather": (_i32, [_vp, _vp, _vp, _i32, _i64p, _vp, _i32, _i64p, _i32, _i32, _i64p, _i64, _vp, _vp]),
     "nsf_launch_count": (_i64, [_vp]),
     "nsf_set_profiling": (None, [_vp, _i32]),
     "nsf_stage_times_ms": (_i32, [_vp, _f32p, _i32]),
@@ -160,4 +162,16 @@ def convert_offsets(sources, target_sr, payload_bytes):
     src = pcm_sources(sources)
     out = np.empty(len(src) + 1, dtype=np.int64)
     check(lib.nsf_convert_offsets(ptr(src), len(src), int(target_sr), int(payload_bytes), out.ctypes.data_as(_i64p)))
+    return out
+
+
+def window_offsets(audio_offsets, facial_offsets, window):
+    """Prefix sum of the per-clip training-window counts of a packed dataset (``nsf_window_offsets``; validates the
+    geometry the way ``_WindowedClip`` fails, needs no GPU)."""
+    a_off, a_p = i64_array(audio_offsets)
+    f_off, f_p = i64_array(facial_offsets)
+    if len(a_off) != len(f_off) or len(a_off) < 2:
+        raise ValueError("audio and facial offsets need the same length, at least 2")
+    out = np.empty(len(a_off), dtype=np.int64)
+    check(lib.nsf_window_offsets(a_p, f_p, len(a_off) - 1, int(window), out.ctypes.data_as(_i64p)))
     return out

@@ -1498,6 +1498,92 @@ nsf_status nsf_chunk_blend(nsf_ctx* ctx, void* cuda_stream, const float* decoded
   return NSF_OK;
 }
 
+// ---- training windows --------------------------------------------------------------------------------------
+nsf_status nsf_window_offsets(const int64_t* a_off, const int64_t* f_off, int32_t n_clips, int32_t window,
+                              int64_t* w_off) {
+  if (!a_off || !f_off || !w_off || n_clips < 1) { set_error("nsf_window_offsets: NULL argument or n_clips < 1"); return NSF_ERR_BAD_ARG; }
+  if (window < 1) { set_error("nsf_window_offsets: window must be >= 1"); return NSF_ERR_BAD_ARG; }
+  if (a_off[0] < 0 || f_off[0] < 0) { set_error("nsf_window_offsets: negative offset"); return NSF_ERR_BAD_ARG; }
+  w_off[0] = 0;
+  char buf[200];
+  for (int i = 0; i < n_clips; ++i) {
+    const int64_t na = a_off[i + 1] - a_off[i], nf = f_off[i + 1] - f_off[i];
+    if (na < 0 || nf < 0) { set_error("nsf_window_offsets: offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+    const int64_t top = std::max(na, nf);
+    if (top < window) {   // dataset.py:77-91 fails on such a clip (broadcast error in the tail branch)
+      std::snprintf(buf, sizeof buf, "clip %d has %lld rows, fewer than the window of %d", i, static_cast<long long>(top), window);
+      set_error(buf);
+      return NSF_ERR_BAD_ARG;
+    }
+    const bool tail = top % window != 0;
+    if (tail) {
+      // the tail window mirrors the last seg rows of each stream into the rest of the window: the host route fails
+      // when a stream has fewer than window / 2 rows there, unless it has exactly one (which torch broadcasts)
+      for (int64_t n : {na, nf}) {
+        const int64_t seg = std::max<int64_t>(0, std::min(top, n) - (top - window));
+        if (2 * seg < window && seg != 1) {
+          std::snprintf(buf, sizeof buf, "clip %d: a stream of %lld rows leaves %lld rows for the tail window of %d (at least half are needed)",
+                        i, static_cast<long long>(n), static_cast<long long>(seg), window);
+          set_error(buf);
+          return NSF_ERR_BAD_ARG;
+        }
+      }
+    }
+    w_off[i + 1] = w_off[i] + (top - window + 1) + (tail ? 1 : 0);
+  }
+  return NSF_OK;
+}
+
+nsf_status nsf_window_gather(nsf_ctx* ctx, void* cuda_stream, const float* audio_dev, int32_t audio_cols,
+                             const int64_t* a_off, const float* facial_dev, int32_t facial_cols, const int64_t* f_off,
+                             int32_t n_clips, int32_t window, const int64_t* indices, int64_t n, float* out_audio_dev,
+                             float* out_facial_dev) {
+  // an empty batch writes nothing: its outputs may be NULL (what a zero-size tensor's data pointer is)
+  if (!ctx || !audio_dev || !facial_dev || audio_cols < 1 || facial_cols < 1 || n < 0 ||
+      (n > 0 && (!indices || !out_audio_dev || !out_facial_dev))) {
+    set_error("nsf_window_gather: bad argument"); return NSF_ERR_BAD_ARG;
+  }
+  if (n_clips < 1) { set_error("nsf_window_gather: n_clips < 1"); return NSF_ERR_BAD_ARG; }
+  const size_t n1 = static_cast<size_t>(n_clips) + 1;
+  std::vector<int64_t> w_off(n1);
+  nsf_status st = nsf_window_offsets(a_off, f_off, n_clips, window, w_off.data());
+  if (st != NSF_OK) return st;
+  const int64_t total = w_off[n_clips];
+  for (int64_t k = 0; k < n; ++k)
+    if (indices[k] < 0 || indices[k] >= total) {
+      char buf[120];
+      std::snprintf(buf, sizeof buf, "nsf_window_gather: index %lld at position %lld is outside [0, %lld)",
+                    static_cast<long long>(indices[k]), static_cast<long long>(k), static_cast<long long>(total));
+      set_error(buf);
+      return NSF_ERR_BAD_ARG;
+    }
+  if (n == 0) return NSF_OK;
+  const int64_t tiles = (window + kWindowTileRows - 1) / kWindowTileRows;
+  if (n > INT32_MAX / tiles) { set_error("nsf_window_gather: too many windows for one launch"); return NSF_ERR_UNSUPPORTED; }
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  // one descriptor block [a_off | f_off | w_off | indices] through the ring; its device copy lives in the ring entry,
+  // which is reused only after this call's kernel has run
+  const size_t bytes = (3 * n1 + static_cast<size_t>(n)) * sizeof(int64_t);
+  DescEntry* de = nullptr;
+  if ((st = desc_acquire(ctx, bytes, &de)) != NSF_OK) return st;
+  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
+  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
+  std::memcpy(h, a_off, n1 * sizeof(int64_t));
+  std::memcpy(h + n1, f_off, n1 * sizeof(int64_t));
+  std::memcpy(h + 2 * n1, w_off.data(), n1 * sizeof(int64_t));
+  std::memcpy(h + 3 * n1, indices, static_cast<size_t>(n) * sizeof(int64_t));
+  int64_t* d = static_cast<int64_t*>(de->dev.ptr);
+  NSF_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s));
+  WindowView v;
+  v.a_off = d; v.f_off = d + n1; v.w_off = d + 2 * n1; v.index = d + 3 * n1;
+  v.n_clips = n_clips; v.window = window; v.n = n;
+  const int m = launch_window_gather(s, v, audio_dev, audio_cols, facial_dev, facial_cols, out_audio_dev, out_facial_dev);
+  if (m < 0) { set_error(cuda_msg("launch_window_gather", cudaGetLastError())); return NSF_ERR_CUDA; }
+  ctx->launches += m;
+  return desc_commit(de, s);
+}
+
 nsf_status nsf_rows_host(nsf_ctx* ctx, int32_t op, int32_t dtype, const void* a_host, int64_t na,
                          const void* b_host, int64_t nb, int32_t cols, int32_t blend_frames, void* out_host) {
   if (!ctx || !a_host || !out_host || na <= 0 || cols <= 0) { set_error("nsf_rows_host: bad argument"); return NSF_ERR_BAD_ARG; }

@@ -1548,6 +1548,100 @@ __global__ void __launch_bounds__(256) k_chunk_blend(const float* __restrict__ d
   }
 }
 
+// ---- training windows (dataset/dataset.py:58-98, _WindowedClip) --------------------------------------------
+// One stream (audio or facial) of a resolved window: output row r reads rows[base + r] while r < seg; past seg it
+// mirrors (rows[base + 2 seg - 1 - r], the tail window; a one-row segment repeats, as torch broadcasts it) or is zero
+// (a regular window past the stream's end).
+struct WinStream {
+  int64_t base;
+  int32_t seg, reflect;
+};
+
+__device__ __forceinline__ int64_t win_src(const WinStream& s, int r) {
+  if (r < s.seg) return s.base + r;
+  if (!s.reflect) return -1;
+  return s.seg == 1 ? s.base : s.base + 2 * s.seg - 1 - r;
+}
+
+template <int V> struct WinVec;
+template <> struct WinVec<1> {
+  using T = float;
+  static __device__ __forceinline__ T zero() { return 0.0f; }
+};
+template <> struct WinVec<4> {
+  using T = float4;
+  static __device__ __forceinline__ T zero() { return make_float4(0.0f, 0.0f, 0.0f, 0.0f); }
+};
+
+constexpr int kWinThreads = 256, kWinUnroll = 8;
+
+// `n_rows` rows of one stream of the block's tile into the contiguous `out`, V floats per access: every thread issues
+// up to kWinUnroll independent loads before its first store (a 32-row tile of 256 float4 columns is exactly one round).
+template <int V>
+__device__ __forceinline__ void win_copy(const float* __restrict__ rows, int cols, const WinStream& s, int r0, int n_rows,
+                                         float* __restrict__ out) {
+  using T = typename WinVec<V>::T;
+  const int cv = cols / V;
+  const int total = n_rows * cv;
+  for (int e0 = threadIdx.x; e0 < total; e0 += kWinThreads * kWinUnroll) {
+    T v[kWinUnroll];
+#pragma unroll
+    for (int u = 0; u < kWinUnroll; ++u) {
+      const int e = e0 + u * kWinThreads;
+      v[u] = WinVec<V>::zero();
+      if (e < total) {
+        const int r = e / cv;
+        const int64_t src = win_src(s, r0 + r);
+        if (src >= 0) v[u] = __ldg(reinterpret_cast<const T*>(rows + src * cols) + (e - r * cv));
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < kWinUnroll; ++u) {
+      const int e = e0 + u * kWinThreads;
+      if (e < total) reinterpret_cast<T*>(out)[e] = v[u];
+    }
+  }
+}
+
+// Block b copies rows [r0, r0 + kWindowTileRows) of output window b / tiles.  Thread 0 resolves the window to its clip
+// (binary search over the window offsets) and to the two streams' sources once; the copy itself is pure data movement.
+// V = 4: audio rows as float4 (cols % 4 == 0 and 16-byte aligned bases); facial rows are always scalar (61 columns,
+// 244-byte rows), read by consecutive threads.
+template <int V>
+__global__ void __launch_bounds__(kWinThreads) k_window_gather(WindowView v, int tiles, const float* __restrict__ audio,
+                                                               int a_cols, const float* __restrict__ facial, int f_cols,
+                                                               float* __restrict__ out_a, float* __restrict__ out_f) {
+  __shared__ WinStream s_st[2];
+  const int64_t k = blockIdx.x / tiles;
+  const int r0 = static_cast<int>(blockIdx.x % tiles) * kWindowTileRows;
+  const int n_rows = min(kWindowTileRows, v.window - r0);
+  if (threadIdx.x == 0) {
+    const int64_t idx = v.index[k];
+    int lo = 0, hi = v.n_clips;                 // last clip c with w_off[c] <= idx (every clip has >= 1 window)
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (__ldg(v.w_off + mid) <= idx) lo = mid; else hi = mid;
+    }
+    const int64_t j = idx - __ldg(v.w_off + lo);
+    const int64_t a0 = __ldg(v.a_off + lo), f0 = __ldg(v.f_off + lo);
+    const int64_t na = __ldg(v.a_off + lo + 1) - a0, nf = __ldg(v.f_off + lo + 1) - f0;
+    const int64_t top = max(na, nf), w = v.window;
+    const bool tail = j >= top - w + 1;
+    const int64_t start = tail ? top - w : j;
+    // regular: rows of the stream left from `start`, at most a window (zero past them); tail: min(top, n) - start,
+    // at least half a window (validated on the host)
+    const int64_t seg_a = max(int64_t(0), min(w, min(top, na) - start));
+    const int64_t seg_f = max(int64_t(0), min(w, min(top, nf) - start));
+    s_st[0] = WinStream{a0 + start, static_cast<int32_t>(seg_a), tail ? 1 : 0};
+    s_st[1] = WinStream{f0 + start, static_cast<int32_t>(seg_f), tail ? 1 : 0};
+  }
+  __syncthreads();
+  const WinStream sa = s_st[0], sf = s_st[1];
+  const int64_t out_row = k * v.window + r0;
+  win_copy<V>(audio, a_cols, sa, r0, n_rows, out_a + out_row * a_cols);
+  win_copy<1>(facial, f_cols, sf, r0, n_rows, out_f + out_row * f_cols);
+}
+
 int grid_for(int64_t items, int per_block, int max_blocks) {
   int64_t g = (items + per_block - 1) / per_block;
   if (g < 1) g = 1;
@@ -1783,6 +1877,19 @@ int launch_chunk_blend(cudaStream_t s, const float* decoded, int64_t n_rows, int
                        int64_t n_chunks, int scale_cols, float divisor, float* out) {
   const int grid = grid_for(n_rows * cols, 256, kSmCount * 8);
   k_chunk_blend<<<grid, 256, 0, s>>>(decoded, n_rows, cols, frame, frame - overlap, overlap, n_chunks, scale_cols, divisor, out);
+  NSF_CHECK_LAUNCH();
+  return 1;
+}
+
+int launch_window_gather(cudaStream_t s, const WindowView& v, const float* audio, int a_cols, const float* facial,
+                         int f_cols, float* out_a, float* out_f) {
+  if (v.n <= 0) return 0;
+  const int tiles = (v.window + kWindowTileRows - 1) / kWindowTileRows;
+  const unsigned blocks = static_cast<unsigned>(v.n * tiles);   // <= INT32_MAX (checked by nsf_window_gather)
+  if (a_cols % 4 == 0 && aligned16(audio) && aligned16(out_a))
+    k_window_gather<4><<<blocks, kWinThreads, 0, s>>>(v, tiles, audio, a_cols, facial, f_cols, out_a, out_f);
+  else
+    k_window_gather<1><<<blocks, kWinThreads, 0, s>>>(v, tiles, audio, a_cols, facial, f_cols, out_a, out_f);
   NSF_CHECK_LAUNCH();
   return 1;
 }

@@ -136,6 +136,20 @@ int launch_chunk_gather(cudaStream_t s, const float* rows, int64_t n_rows, int c
 int launch_chunk_blend(cudaStream_t s, const float* decoded, int64_t n_rows, int cols, int frame, int overlap,
                        int64_t n_chunks, int scale_cols, float divisor, float* out);
 
+// training windows of a packed dataset (nsf_window_gather): every array in device memory, geometry validated on the
+// host.  One block per kWindowTileRows output rows of a window.
+struct WindowView {
+  const int64_t* a_off;    // [n_clips+1] audio rows of each clip
+  const int64_t* f_off;    // [n_clips+1] facial rows of each clip
+  const int64_t* w_off;    // [n_clips+1] first window of each clip (nsf_window_offsets)
+  const int64_t* index;    // [n] windows to gather
+  int32_t n_clips, window;
+  int64_t n;
+};
+constexpr int kWindowTileRows = 32;
+int launch_window_gather(cudaStream_t s, const WindowView& v, const float* audio, int a_cols, const float* facial,
+                         int f_cols, float* out_a, float* out_f);
+
 // One-time (per device) cudaFuncSetAttribute calls of each translation unit; nsf_ctx_create runs them so that no
 // launch path touches function attributes.
 bool init_kernel_attributes();        // nsf_kernels.cu

@@ -281,6 +281,53 @@ class Engine:
                                               C.c_void_p(out.data_ptr()), off.ctypes.data_as(nv._i64p)))
         return out[:int(off[-1])], off
 
+    # ---- training windows of a packed dataset (dataset/dataset.py:58-98) ------------------------------
+    @staticmethod
+    def window_offsets(audio_offsets, facial_offsets, window):
+        """First window of every clip, plus the total (``nsf_window_offsets``): the numbering of
+        ``AudioFacialDataset``'s items.  Raises ``NsfError`` for the clips the host windowing rejects."""
+        return nv.window_offsets(audio_offsets, facial_offsets, window)
+
+    def window_gather(self, audio, audio_offsets, facial, facial_offsets, window, indices, out_audio=None,
+                      out_facial=None, stream=None):
+        """Windows ``indices`` of a packed dataset on the device (``nsf_window_gather``, stream-ordered):
+        ``audio [sum N, a_cols]`` / ``facial [sum N, f_cols]`` float32 CUDA tensors, clip i owning rows
+        ``[offsets[i], offsets[i + 1])`` of each; ``indices`` a host sequence (list, NumPy array or CPU tensor).
+        Returns ``(out_audio [n, window, a_cols], out_facial [n, window, f_cols])``, bit for bit what
+        ``collate_fn([dataset[i] for i in indices])`` gives.  Indices and geometry are checked on the host first:
+        on error nothing is launched and the outputs are not touched."""
+        import torch
+        for t in (audio, facial):
+            assert t.is_cuda and t.device.index == self.device and t.dtype == torch.float32
+            assert t.dim() == 2 and t.is_contiguous()
+        if isinstance(indices, torch.Tensor):
+            if indices.is_cuda:
+                raise ValueError("window_gather: indices are validated on the host; pass a host sequence")
+            indices = indices.numpy()
+        idx, idx_p = nv.i64_array(np.asarray(indices).reshape(-1))
+        a_off, a_p = nv.i64_array(audio_offsets)
+        f_off, f_p = nv.i64_array(facial_offsets)
+        if len(a_off) != len(f_off) or len(a_off) < 2:
+            raise ValueError("audio and facial offsets need the same length, at least 2")
+        if a_off[-1] > audio.shape[0] or f_off[-1] > facial.shape[0]:
+            raise ValueError("offsets run past the rows of the packed tensors")
+        n, window = len(idx), int(window)
+        a_cols, f_cols = audio.shape[1], facial.shape[1]
+        if out_audio is None:
+            out_audio = torch.empty((n, window, a_cols), dtype=torch.float32, device=audio.device)
+        if out_facial is None:
+            out_facial = torch.empty((n, window, f_cols), dtype=torch.float32, device=audio.device)
+        for t, cols in ((out_audio, a_cols), (out_facial, f_cols)):
+            assert t.is_cuda and t.device.index == self.device and t.dtype == torch.float32 and t.is_contiguous()
+            assert tuple(t.shape) == (n, window, cols), (tuple(t.shape), (n, window, cols))
+        s = torch.cuda.current_stream(audio.device) if stream is None else stream
+        with self._lock:
+            nv.check(nv.lib.nsf_window_gather(
+                self.handle, C.c_void_p(s.cuda_stream), C.c_void_p(audio.data_ptr()), a_cols, a_p,
+                C.c_void_p(facial.data_ptr()), f_cols, f_p, len(a_off) - 1, window, idx_p, n,
+                C.c_void_p(out_audio.data_ptr()), C.c_void_p(out_facial.data_ptr())))
+        return out_audio, out_facial
+
     # ---- device buffers (torch used for memory and streams only) -------------------------------
     def workspace_bytes(self, total_samples, n_clips, flags=0):
         return nv.lib.nsf_workspace_bytes(self.plan.handle, int(total_samples), int(n_clips), flags)
