@@ -199,8 +199,6 @@ struct nsf_ctx {
   int device = 0;
   nsf::DeviceTables tables{};
   nsf::StftTcTables tc{};
-  nsf::DctCoef dct_coef{};       // DCT matrix as a kernel parameter (default 128 -> 23 shape only)
-  bool dct_coef_ok = false;
   nsf::Arena table_mem;
   nsf::DescEntry desc[nsf::kDescRing];
   int desc_next = 0;
@@ -279,7 +277,7 @@ nsf_status upload_tables(nsf_ctx* ctx) {
   // k_dct_mma: B[k][n] = 2^10 dct[n][k] (n < n_mfcc, else 0) split into fp16 hi + lo, in m16n8k16 fragment order:
   // lane (g, tq) of k-step ks, column tile nt holds b0 = (k = 16 ks + 2 tq, + 1; n = 8 nt + g), b1 = (k + 8, k + 9)
   std::vector<uint32_t> dct_frag;
-  const bool dct_frag_ok = p.n_mels == kDctConstMels && p.n_mfcc == kDctConstMfcc;
+  const bool dct_frag_ok = p.n_mels == kDctMmaMels && p.n_mfcc == kDctMmaMfcc;
   if (dct_frag_ok) {
     dct_frag.assign(static_cast<size_t>(8) * 3 * 2 * 32 * 2, 0u);
     auto half_bits = [](float v) { const __half h = __float2half_rn(v); uint16_t u; std::memcpy(&u, &h, 2); return u; };
@@ -303,11 +301,6 @@ nsf_status upload_tables(nsf_ctx* ctx) {
         }
   }
   const size_t off_dct_frag = dct_frag_ok ? put(dct_frag.data(), dct_frag.size() * sizeof(uint32_t)) : 0;
-  ctx->dct_coef_ok = p.n_mels == kDctConstMels && p.n_mfcc == kDctConstMfcc;
-  if (ctx->dct_coef_ok)
-    for (int m = 0; m < kDctConstMels; ++m)
-      for (int k = 0; k < kDctConstMfcc; ++k)
-        ctx->dct_coef.v[m * kDctConstLd + k] = p.dct[static_cast<size_t>(k) * p.n_mels + m];
   // column -> (first filter, two weights) table for the fused mel epilogue of the tcgen05 kernel
   size_t off_melcol[2] = {0, 0};
   int mel_col_ok = 1;
@@ -727,8 +720,7 @@ nsf_status nsf_extract_batch(nsf_ctx* ctx, void* cuda_stream, const void* pcm_de
   // stage 4: floor + DCT + CMVN statistics
   timer.mark(4);
   if (do_mfcc) {
-    NSF_LAUNCH(launch_dct_sum(s, t, b, L.db, L.dbmax_key, L.mfcc_raw, L.sum, L.sumsq,
-                              ctx->dct_coef_ok ? &ctx->dct_coef : nullptr));
+    NSF_LAUNCH(launch_dct_sum(s, t, b, L.db, L.dbmax_key, L.mfcc_raw, L.sum, L.sumsq));
   }
   // stage 5: CMVN + deltas + pair reduce -> columns [0, mfcc_cols)
   timer.mark(5);

@@ -24,7 +24,6 @@
 //                    frame woven into the compile-time unrolled five-tile MMA loop of the current one (am_mma5_pipe)
 //   k_autocorr_sym   every other frame length: every warp stages, then multiplies, its own frames (am_mma5 /
 //                    am_mma5_static<17> / am_mma); NSF_AC_KERNEL=sym forces it at F = 1470
-//   k_autocorr_mma   warp-specialised producer / consumer pairs of round 1 (NSF_AC_KERNEL=pairs)
 #include <cuda_fp16.h>
 
 #include <cstdint>
@@ -124,7 +123,7 @@ __device__ __forceinline__ void am_issue_fast(const float* __restrict__ src, int
 // hann: np.hanning(F) staged in shared memory and ZERO from F up to 64 n_it, so elements beyond the
 // frame come out as exact zeros without a branch (they land in the zero margin of the copies).
 // Both passes over the frame (mean / max, then window + scale + split) run out of registers and the
-// hot path has no divergent or data-dependent branches: a producer warp is alone on its latency.
+// hot path has no divergent or data-dependent branches.
 // When `next` is a fast frame every register pair is refilled with ITS samples as soon as the pair
 // has been consumed, so the next memory round trip overlaps the rest of this frame.
 template <int kIters, bool kExact>
@@ -199,7 +198,7 @@ __device__ __forceinline__ void am_process(const DeviceTables& t, const float* h
 
 // Any frame, start to finish, without register staging: three plain passes (mean / max, window +
 // split, shifted copies).  Cold path - the two clip-edge frames with np.pad(..., mode='reflect')
-// indexing, the tail of a batch, and the consumers' rare edge-fix refill - kept out of line so that it
+// indexing, the tail of a batch, and the rare edge-fix refill - kept out of line so that it
 // costs the hot paths neither registers nor instruction-cache space.
 __device__ __noinline__ void am_fill_simple(const DeviceTables& t, const float* hann, const AmSrc& s, __half* copies,
                                             const AmGeom& geo, int lane) {
@@ -547,14 +546,8 @@ template <int NBLK, int kIters>
 __device__ __forceinline__ void am_mma5_pipe(const __half* copies, const AmGeom& geo, int lane, float (&val)[kVals],
                                              const DeviceTables& t, const float* hann, float (&v0)[kIters],
                                              float (&v1)[kIters], __half* next_copies) {
-#ifndef NSF_PIPE_PASS1
-#define NSF_PIPE_PASS1 12
-#endif
-#ifndef NSF_PIPE_GAP
-#define NSF_PIPE_GAP 2
-#endif
-  constexpr int kPass1 = NBLK >= 40 ? NSF_PIPE_PASS1 : 5;           // block after which the loads are consumed
-  constexpr int kPass2 = kPass1 + NSF_PIPE_GAP;
+  constexpr int kPass1 = NBLK >= 40 ? 12 : 5;           // block after which the loads are consumed
+  constexpr int kPass2 = kPass1 + 2;                    // block of the first pass-2 iteration
   constexpr int kStride = (NBLK - 2 - kPass2) / kIters > 0 ? (NBLK - 2 - kPass2) / kIters : 1;
   static_assert(kPass2 + kStride * (kIters - 1) < NBLK, "every staging iteration must fall inside the loop");
   const int g = lane >> 2, tq = lane & 3;
@@ -651,140 +644,15 @@ __device__ __forceinline__ bool am_all_small(const float (&val)[kVals], int lane
   return __all_sync(0xffffffffu, small);
 }
 
-// ---- mbarrier helpers (producer / consumer hand-off of the frame buffers) -------------------------
-__device__ __forceinline__ void am_bar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(am_smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void am_bar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(am_smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void am_bar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0;
-  for (uint32_t spins = 0; !ok; ++spins) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(am_smem_u32(bar)), "r"(parity) : "memory");
-    if (spins > (1u << 26)) __trap();      // a hand-off bug traps instead of hanging the GPU
-  }
-}
-
-// (A 3-consumer : 1-producer grouping over a ring of four buffers - 12 MMA warps per SM instead of 8 in
-// the same shared memory - was measured too: 1.37 vs 1.39 ms at 88.2 kHz, 6.3 vs 4.3 ms on the 16 kHz
-// small-clip batch; the lone producer becomes the bottleneck, so the pairs stayed.)
-// Warp-specialised kernel.  A block is kAmPairs (consumer, producer) warp pairs; each pair owns two
-// frame buffers.  The producer warp fetches, windows, scales and splits frame after frame; the
-// consumer warp runs nothing but the MMA loop (plus the cheap normalise / pair-mean / store), so the
-// tensor pipe is fed continuously while memory latency and the fp32->fp16 conversion hide behind it.
-// Round 2: this kernel is the alternative (NSF_AC_KERNEL=pairs); the symmetric kernel below is the product path.
-constexpr int kAmPairs = 4;
-
-template <int kIters, bool kExact>
-__global__ void __launch_bounds__(kAmPairs * 64, 2) k_autocorr_mma(DeviceTables t, BatchView b,
-                                                                   const float* __restrict__ y, bool reduce,
-                                                                   float* __restrict__ out, int64_t out_ld,
-                                                                   int col0) {
-  extern __shared__ __align__(16) __half s_am[];
-  __shared__ uint64_t s_bar[kAmPairs][4];          // per pair: full[2], empty[2]
-  const AmGeom geo = am_geom(t.F);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_pairs = static_cast<int>(blockDim.x >> 6);   // kAmPairs, fewer when the frame buffers of four do not fit
-  const int pair = warp % n_pairs;
-  const bool producer = warp >= n_pairs;
-  __half* bufs = s_am + static_cast<size_t>(pair) * 2 * 4 * geo.len;      // two buffers of 4 copies
-  // np.hanning(F) staged in shared memory: with ~220 KB of the SM carved out for buffers the L1 is too
-  // small to keep the table resident next to the streaming frame loads
-  float* hann = reinterpret_cast<float*>(s_am + static_cast<size_t>(n_pairs) * 2 * 4 * geo.len);
-  const int n_it = (t.F / 2 + 1 + 31) / 32;          // register-staging iterations the frame needs
-  for (int n = threadIdx.x; n < 64 * n_it; n += blockDim.x) hann[n] = n < t.F ? __ldg(t.hann_sym + n) : 0.0f;
-  uint64_t* full = s_bar[pair];
-  uint64_t* empty = s_bar[pair] + 2;
-  if (!producer) {
-    // zero once: the margins are never written again, the frame region is rewritten per frame
-    for (int i = lane; i < 2 * 4 * geo.len / 2; i += 32) reinterpret_cast<uint32_t*>(bufs)[i] = 0u;
-    if (lane == 0) {
-      am_bar_init(full + 0, 1); am_bar_init(full + 1, 1);
-      am_bar_init(empty + 0, 1); am_bar_init(empty + 1, 1);
-    }
-  }
-  __syncthreads();
-  // Every pair owns a CONTIGUOUS run of rows: consecutive frames share half of their samples (L1 / L2 hits
-  // for the producer) and almost always the clip, whose descriptor - a chain of dependent loads - is then
-  // looked up once per clip instead of once per row, on both sides of the hand-off.
-  const int64_t n_pairs_total = static_cast<int64_t>(gridDim.x) * n_pairs;
-  const int64_t chunk = (b.total_rows + n_pairs_total - 1) / n_pairs_total;
-  const int64_t r_begin = (static_cast<int64_t>(blockIdx.x) * n_pairs + pair) * chunk;
-  const int64_t r_end = min(r_begin + chunk, b.total_rows);
-  uint32_t it = 0;                                  // frames handed over so far (buffer = it & 1)
-  int64_t base = 0, len = 0, T = 0, clip_row0 = 0, clip_row_end = -1;
-  for (int64_t r = r_begin; r < r_end; ++r) {
-    if (r >= clip_row_end) {
-      const int clip = find_segment(b.row_off, b.n_clips, r);
-      base = __ldg(b.clip_off + clip);
-      len = __ldg(b.clip_off + clip + 1) - base;
-      T = __ldg(b.frame_off + clip + 1) - __ldg(b.frame_off + clip);
-      clip_row0 = __ldg(b.row_off + clip);
-      clip_row_end = __ldg(b.row_off + clip + 1);
-    }
-    const int64_t lr = r - clip_row0;
-    const int64_t tf0 = reduce ? 2 * lr : lr;
-    const int n_frames = (reduce && tf0 + 1 < T) ? 2 : 1;   // odd T: the last row passes through
-    if (producer) {
-      for (int f = 0; f < n_frames; ++f, ++it) {
-        const uint32_t buf = it & 1u;
-        am_bar_wait(empty + buf, ((it >> 1) & 1u) ^ 1u);
-        const AmSrc src = am_src(t, b, y, base, len, tf0 + f, n_it);
-        if (src.fast) {
-          float v0[kIters], v1[kIters];
-          am_issue_fast<kIters, kExact>(src.clip + src.first, n_it, lane, v0, v1);
-          am_process<kIters, kExact>(t, hann, n_it, v0, v1, bufs + buf * 4 * geo.len, geo, lane, nullptr);
-        } else {
-          am_fill_simple(t, hann, src, bufs + buf * 4 * geo.len, geo, lane);
-        }                                                 // both end with __syncwarp
-        if (lane == 0) am_bar_arrive(full + buf);
-      }
-    } else {
-      float acc[kVals];
-#pragma unroll
-      for (int v = 0; v < kVals; ++v) acc[v] = 0.0f;
-      for (int f = 0; f < n_frames; ++f, ++it) {
-        const uint32_t buf = it & 1u;
-        __half* copies = bufs + buf * 4 * geo.len;
-        const int64_t tf = tf0 + f;
-        float val[kVals];
-        am_bar_wait(full + buf, (it >> 1) & 1u);
-        am_mma(copies, geo, lane, val);
-        // fix_edge_frames_autocorr: a near-silent first (last) frame takes the values of frame 1 (T-2);
-        // rare, so the consumer refills the buffer it still owns itself
-        if (T > 1 && (tf == 0 || tf == T - 1) && am_all_small(val, lane, t.n_lags, t.edge_thr)) {
-          am_fill_simple(t, hann, am_src(t, b, y, base, len, tf == 0 ? 1 : T - 2, n_it), copies, geo, lane);
-          am_mma(copies, geo, lane, val);
-        }
-        __syncwarp();
-        if (lane == 0) am_bar_arrive(empty + buf);
-#pragma unroll
-        for (int v = 0; v < kVals; ++v) acc[v] += val[v];
-      }
-      const float wgt = n_frames == 2 ? 0.5f : 1.0f;
-      float* o = out + r * out_ld + col0;
-#pragma unroll
-      for (int v = 0; v < kVals; ++v) {
-        const int lag = lag_of(lane, v);
-        if (lag >= 1 && lag <= t.n_lags) o[lag - 1] = acc[v] * wgt;
-      }
-    }
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // Symmetric kernel: every warp stages AND multiplies its own frames (one frame buffer per warp, no mbarriers).
-// The warp-specialised kernel above keeps two MMA warps per scheduler busy and two producer warps idle two thirds of
-// the time (ncu, round 2: 25 % of all stall samples are producers spinning on `empty`), and whenever both MMA warps
-// of a scheduler wait for a fragment or a hand-off at the same moment the tensor pipe idles (67 % active).  Here the
-// same sixteen warps per SM all issue MMAs, each in its own phase of the stage / multiply cycle, so on average
-// two to three warps per scheduler have MMAs ready while the others convert their next frame.  Same shared-memory
-// footprint (sixteen frame buffers per SM), same registers, same arithmetic in the same order: bit-identical rows.
+// Round 1's warp-specialised producer / consumer pairs kept two MMA warps per scheduler busy and two producer warps
+// idle two thirds of the time (ncu, round 2: 25 % of all stall samples were producers spinning on `empty`), and
+// whenever both MMA warps of a scheduler waited for a fragment or a hand-off at the same moment the tensor pipe idled
+// (67 % active).  Here the same sixteen warps per SM all issue MMAs, each in its own phase of the stage / multiply
+// cycle, so on average two to three warps per scheduler have MMAs ready while the others convert their next frame.
+// Same shared-memory footprint (sixteen frame buffers per SM), same registers, same arithmetic in the same order as
+// the pairs: bit-identical rows.
 // ------------------------------------------------------------------------------------------------
 constexpr int kSymWarps = 8;       // per block, two blocks per SM
 
@@ -1049,11 +917,6 @@ int launch_autocorr_mma(cudaStream_t s, const DeviceTables& t, const BatchView& 
   if (t.n_lags > 191) return -1;
   const int iters = (t.F / 2 + 1 + 31) / 32;      // register-staging iterations the frame needs
   const size_t hann_bytes = static_cast<size_t>(64) * iters * sizeof(float);   // np.hanning(F), zero padded
-  // NSF_AC_KERNEL=pairs selects the warp-specialised kernel of round 1 (A/B timing; bit-identical results)
-  static const bool use_pairs = [] {
-    const char* v = std::getenv("NSF_AC_KERNEL");
-    return v != nullptr && v[0] == 'p' && v[1] == 'a';      // "pairs" ("pipe" forces the pipelined kernel, below)
-  }();
   // MMA loop of the symmetric kernel: the five-tile loop (am_mma5) for frames of at least 44 K-blocks (F >= 689:
   // 44.1 kHz and up), where most blocks run in its unchecked body; the six-MMA loop (am_mma) for short frames, where the
   // eight lead-in blocks and the range checks of the five-tile loop cost more than the MMAs it saves (B200, F = 266:
@@ -1069,24 +932,17 @@ int launch_autocorr_mma(cudaStream_t s, const DeviceTables& t, const BatchView& 
   // symmetric kernel: as many warps per block as fit twice per SM (eight up to F ~ 1530, fewer for long frames);
   // two blocks of 113 KB (+ 1 KB reserved each) are what an SM's 228 KB hold
   int warps = kSymWarps;
-  size_t sym_smem = 0;
-  for (; warps >= 1; --warps) {
-    sym_smem = static_cast<size_t>(warps) * (kExtraFront + 4 * static_cast<size_t>(geo.len)) * sizeof(__half) + hann_bytes;
-    if (sym_smem <= (warps > 2 ? 113 : 220) * 1024) break;      // long frames: one block per SM
-  }
-  // pairs kernel: four (consumer, producer) pairs per block when their eight frame buffers fit, else three or two
-  int pairs = kAmPairs;
   size_t smem = 0;
-  for (; pairs >= 1; --pairs) {
-    smem = static_cast<size_t>(pairs) * 2 * 4 * geo.len * sizeof(__half) + hann_bytes;
-    if (smem <= 220 * 1024) break;
+  for (; warps >= 1; --warps) {
+    smem = static_cast<size_t>(warps) * (kExtraFront + 4 * static_cast<size_t>(geo.len)) * sizeof(__half) + hann_bytes;
+    if (smem <= (warps > 2 ? 113 : 220) * 1024) break;      // long frames: one block per SM
   }
-  if (warps < 1 && pairs < 1) return -1;
+  if (warps < 1) return -1;
   // Software-pipelined kernel (k_autocorr_pipe): the 88.2 kHz plan (23 staging iterations, 92 K-blocks).
-  // NSF_AC_KERNEL=sym / pairs select the earlier kernels (validation, A/B; bit-identical rows)
+  // NSF_AC_KERNEL=sym selects the symmetric kernel instead (validation; bit-identical rows)
   static const bool no_pipe = [] {
     const char* v = std::getenv("NSF_AC_KERNEL");
-    return v != nullptr && (v[0] == 's' || (v[0] == 'p' && v[1] == 'a'));
+    return v != nullptr && v[0] == 's';
   }();
   // Short frames stay on the symmetric kernel: at F = 266 (16 kHz) the pipelined kernel is bit-identical but SLOWER
   // (B200, C5: 2.93 ms at twelve warps per SM / 168 registers with one or two frames of look-ahead, 3.10 - 4.70 ms at
@@ -1101,31 +957,17 @@ int launch_autocorr_mma(cudaStream_t s, const DeviceTables& t, const BatchView& 
     k_autocorr_pipe<23, 92, kPipeWarps, 1><<<static_cast<int>(pgrid), kPipeWarps * 32, pipe_smem, s>>>(t, b, y, reduce, out, out_ld, col0);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
   }
-  const bool sym = !use_pairs && warps >= 1;
-  int64_t grid;
-  int threads;
-  if (sym) {
-    const int per_sm = sym_smem <= 113 * 1024 ? 2 : 1;
-    grid = (b.total_rows + warps - 1) / warps;
-    if (grid > static_cast<int64_t>(kSmCount) * per_sm) grid = static_cast<int64_t>(kSmCount) * per_sm;
-    threads = warps * 32;
-    smem = sym_smem;
-  } else {
-    if (pairs < 1) return -1;
-    int per_sm = static_cast<int>((224 * 1024) / (smem + 1024));
-    per_sm = per_sm < 1 ? 1 : (per_sm > 2 ? 2 : per_sm);
-    grid = (b.total_rows + pairs - 1) / pairs;
-    if (grid > static_cast<int64_t>(kSmCount) * per_sm) grid = static_cast<int64_t>(kSmCount) * per_sm;
-    threads = pairs * 64;
-  }
+  const int per_sm = smem <= 113 * 1024 ? 2 : 1;
+  int64_t grid = (b.total_rows + warps - 1) / warps;
+  if (grid > static_cast<int64_t>(kSmCount) * per_sm) grid = static_cast<int64_t>(kSmCount) * per_sm;
   if (grid < 1) grid = 1;
-  auto go = [&](auto k_five, auto k_six, auto k_pairs) {
-    if (sym && !use_six) k_five<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
-    else if (sym) k_six<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
-    else k_pairs<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
+  const int threads = warps * 32;
+  auto go = [&](auto k_five, auto k_six) {
+    if (use_six) k_six<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
+    else k_five<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
   };
-#define NSF_AC_GO(IT, EX) go(k_autocorr_sym<IT, EX, true>, k_autocorr_sym<IT, EX, false>, k_autocorr_mma<IT, EX>)
+#define NSF_AC_GO(IT, EX) go(k_autocorr_sym<IT, EX, true>, k_autocorr_sym<IT, EX, false>)
   if (iters == 23) return NSF_AC_GO(23, true);    // 88.2 kHz: F = 1470
   if (iters == 5) return NSF_AC_GO(5, true);      // 16 kHz: F = 266
   if (iters <= 6) return NSF_AC_GO(6, false);     // F <= 382   (22.05 kHz: 367)
@@ -1143,9 +985,6 @@ bool init_autocorr_mma_attributes() {
   auto set = [&](auto kernel) {
     ok = ok && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024) == cudaSuccess;
   };
-  set(k_autocorr_mma<23, true>); set(k_autocorr_mma<5, true>); set(k_autocorr_mma<6, false>);
-  set(k_autocorr_mma<12, false>); set(k_autocorr_mma<24, false>); set(k_autocorr_mma<40, false>);
-  set(k_autocorr_mma<66, false>);
 #define NSF_AC_SET(IT, EX) set(k_autocorr_sym<IT, EX, true>); set(k_autocorr_sym<IT, EX, false>)
   NSF_AC_SET(23, true); NSF_AC_SET(5, true); NSF_AC_SET(6, false); NSF_AC_SET(12, false);
   NSF_AC_SET(24, false); NSF_AC_SET(40, false); NSF_AC_SET(66, false);

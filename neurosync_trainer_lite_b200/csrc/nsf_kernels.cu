@@ -10,7 +10,7 @@
 //   k_autocorr               reflect-pad framing, DC removal, np.hanning, 188 lags, normalise,
 //                            edge fix, pair reduction  (fp32 FMA bound; extract_features_utils.py:54-113)
 //   k_smooth                 smooth_features (extract_features_utils.py:47-51)
-//   k_collect                collect_features augmentation (dataset/data_processing.py:126-197)
+//   k_collect_rows           collect_features augmentation (dataset/data_processing.py:126-197)
 #include <cuda_fp16.h>
 
 #include "nsf.h"
@@ -559,89 +559,18 @@ __global__ void __launch_bounds__(kDct2Warps * 32, 2) k_dct_rows(DeviceTables t,
 }
 
 // ------------------------------------------------------------------------------------------------
-// K2 (product variant for the reference's 128 mels -> 23 MFCCs): k_dct_rows with the coefficients in the
-// CONSTANT BANK.  k_dct_rows issues 768 broadcast LDS.128 per 32 frames and stalls on the shared-memory
-// instruction queue (ncu: short_scoreboard + mio_throttle, 0.089 ms on C2 = 22 % of the HBM roofline).  Here
-// the matrix is a kernel parameter, the mel loop is fully unrolled, and ptxas turns every coefficient into
-// a uniform-register FFMA operand fetched by LDCU.128 on the uniform datapath: per frame-lane 2944 FFMA +
-// 128 FMNMX + 32 LDG.128, no LDS.  Same accumulation order over the mels as k_dct_rows / k_dct_sum
-// (bit-identical MFCCs); the staging / moment tail is the same code.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kDct2Warps * 32, 3) k_dct_const(const __grid_constant__ DctCoef c, BatchView b,
-                                                                  const float* __restrict__ db,
-                                                                  const uint32_t* __restrict__ dbmax_key,
-                                                                  float* __restrict__ mfcc_raw,
-                                                                  double* __restrict__ sum,
-                                                                  double* __restrict__ sumsq) {
-  constexpr int NM = kDctConstMels, NC = kDctConstMfcc, LD = kDctConstLd;
-  __shared__ float s_stage[kDct2Warps * 32 * NC];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  float* s_o = s_stage + warp * 32 * NC;
-  const int64_t n_tiles = (b.total_frames + 31) / 32;
-  for (int64_t tile = static_cast<int64_t>(blockIdx.x) * kDct2Warps + warp; tile < n_tiles;
-       tile += static_cast<int64_t>(gridDim.x) * kDct2Warps) {
-    const int64_t g0 = tile * 32;
-    const int nf = static_cast<int>(min(static_cast<int64_t>(32), b.total_frames - g0));
-    const bool valid = lane < nf;
-    const int clip = valid ? find_segment(b.frame_off, b.n_clips, g0 + lane) : -1;
-    const float floor_db = valid ? key_float(__ldg(dbmax_key + clip)) - 80.0f : 0.0f;
-    const float4* row = reinterpret_cast<const float4*>(db + (g0 + (valid ? lane : 0)) * NM);
-    float acc[NC];
-#pragma unroll
-    for (int k = 0; k < NC; ++k) acc[k] = 0.0f;
-#pragma unroll
-    for (int q = 0; q < NM / 4; ++q) {
-      const float4 x4 = __ldg(row + q);
-      const float xs[4] = {x4.x, x4.y, x4.z, x4.w};
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const float x = fmaxf(xs[e], floor_db);
-#pragma unroll
-        for (int k = 0; k < NC; ++k) acc[k] = fmaf(c.v[(4 * q + e) * LD + k], x, acc[k]);
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < NC; ++k) s_o[lane * NC + k] = valid ? acc[k] : 0.0f;
-    __syncwarp();
-    for (int i = lane; i < nf * NC; i += 32) mfcc_raw[g0 * NC + i] = s_o[i];
-    const int first_clip = __shfl_sync(0xffffffffu, clip, 0);
-    const bool uniform = __all_sync(0xffffffffu, clip == first_clip || clip < 0);
-    if (uniform) {
-      if (lane < NC && first_clip >= 0) {
-        double ts = 0.0, tq = 0.0;
-        for (int f = 0; f < nf; ++f) {
-          const double a = static_cast<double>(s_o[f * NC + lane]);
-          ts += a;
-          tq = fma(a, a, tq);
-        }
-        atomicAdd(sum + static_cast<int64_t>(first_clip) * NC + lane, ts);
-        atomicAdd(sumsq + static_cast<int64_t>(first_clip) * NC + lane, tq);
-      }
-    } else if (valid) {
-#pragma unroll
-      for (int k = 0; k < NC; ++k) {
-        const double a = static_cast<double>(acc[k]);
-        atomicAdd(sum + static_cast<int64_t>(clip) * NC + k, a);
-        atomicAdd(sumsq + static_cast<int64_t>(clip) * NC + k, a * a);
-      }
-    }
-    __syncwarp();
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // K2 on the tensor pipe: the DCT-II of the default shape (128 mels -> 23 coefficients) as warp-level MMAs
 // (mma.sync m16n8k16, fp16 split operands, fp32 accumulation).  north_star lists the DCT among the dense contractions
-// that belong on tensor cores; as FFMAs it costs 2944 instructions per frame (k_dct_const: issue bound at 0.46 of the
-// HBM roofline), as MMAs 4.5 per frame: [32 frames x 128] x [128 x 24] per warp tile = 8 k-steps x 2 row tiles x 3
-// column tiles x 3 split products.
+// that belong on tensor cores; as FFMAs it costs 2944 instructions per frame (round 2's constant-bank FFMA kernel:
+// issue bound at 0.46 of the HBM roofline), as MMAs 4.5 per frame: [32 frames x 128] x [128 x 24] per warp tile =
+// 8 k-steps x 2 row tiles x 3 column tiles x 3 split products.
 //   A  floored dB rows, CENTRED per row: x' = max(x, clip_max - 80) - (clip_max - 40) lies in [-40, 40], so the fp16
 //      hi + lo split carries 2^-22 x 64 = 1.5e-5 of absolute error per element instead of 3e-5 at |x| ~ 100.  The
 //      offset only reaches coefficient 0 (the other DCT rows sum to zero) and is added back there in float32.
 //   B  the DCT matrix scaled by 2^10 (exact), pre-split on the host into hi / lo and laid out in fragment order
 //      (one 64-bit shared-memory load per lane, k-step, column tile and part).
 // hi.hi + hi.lo + lo.hi: fp32-class like the other split GEMMs of the path.  Staging, store and the float64 CMVN
-// moments are those of k_dct_const.
+// moments are those of k_dct_rows.
 // ------------------------------------------------------------------------------------------------
 constexpr int kDctMmaFragWords = 8 * 3 * 2 * 32 * 2;      // [k-step][column tile][hi, lo][lane] x {b0, b1}
 constexpr float kDctMmaScale = 1024.0f;
@@ -666,7 +595,7 @@ __global__ void __launch_bounds__(kDct2Warps * 32, 3) k_dct_mma(const uint2* __r
                                                                 const uint32_t* __restrict__ dbmax_key,
                                                                 float* __restrict__ mfcc_raw,
                                                                 double* __restrict__ sum, double* __restrict__ sumsq) {
-  constexpr int NM = kDctConstMels, NC = kDctConstMfcc;
+  constexpr int NM = kDctMmaMels, NC = kDctMmaMfcc;
   __shared__ uint2 s_frag[kDctMmaFragWords / 2];
   __shared__ float s_stage[kDct2Warps * 32 * NC];
   for (int i = threadIdx.x; i < kDctMmaFragWords / 2; i += blockDim.x) s_frag[i] = __ldg(frag + i);
@@ -1139,8 +1068,8 @@ __global__ void __launch_bounds__(256) k_smooth(BatchView b, const float* __rest
 }
 
 // ------------------------------------------------------------------------------------------------
-// collect_features augmentation.  One block per output row; the row's provenance (which version,
-// blend weights) is resolved once, then threads stream the 256 + 61 columns.
+// collect_features augmentation.  One warp per output row, every warp walking short runs of consecutive rows;
+// the row's provenance (which version, blend weights) is resolved once, then the lanes stream the 256 + 61 columns.
 // ------------------------------------------------------------------------------------------------
 template <typename T> struct Arith;
 template <> struct Arith<double> {
@@ -1201,77 +1130,11 @@ __device__ __forceinline__ float4 version_value4(const float* __restrict__ src, 
   return mul4(add4(slow(j - 1), slow(j)), 0.5f);
 }
 
-template <typename T>
-__global__ void __launch_bounds__(128) k_collect(CollectView v, const T* __restrict__ audio,
-                                                 int a_cols, const T* __restrict__ facial, int f_cols,
-                                                 T* __restrict__ out_audio, T* __restrict__ out_facial) {
-  using A = Arith<T>;
-  for (int64_t r = blockIdx.x; r < v.total_out_rows; r += gridDim.x) {
-    const int clip = find_segment(v.o_off, v.n_clips, r);
-    const int64_t p = r - __ldg(v.o_off + clip);
-    int64_t a0 = __ldg(v.a_off + clip), na = __ldg(v.a_off + clip + 1) - a0;
-    int64_t f0 = __ldg(v.f_off + clip), nf = __ldg(v.f_off + clip + 1) - f0;
-    // centre-trim the longer stream (data_processing.py:126-145)
-    if (na > nf) a0 += (na - nf) / 2; else if (nf > na) f0 += (nf - na) / 2;
-    const int64_t n = min(na, nf);
-    // version lengths and blend zones (stack_with_blend, data_processing.py:179-197)
-    int ver[3]; int64_t vlen[3]; int nv = 0;
-    ver[nv] = 0; vlen[nv++] = n;
-    if (v.flags & NSF_COLLECT_FAST) { ver[nv] = 1; vlen[nv++] = (n + 1) / 2; }
-    if (v.flags & NSF_COLLECT_SLOW) { ver[nv] = 2; vlen[nv++] = n > 0 ? 2 * n - 1 : 0; }
-    const bool blend = (v.flags & NSF_COLLECT_BLEND) != 0;
-    int64_t len_before[3], nb[3];  // result length before stacking version i, blend rows used
-    int64_t total = vlen[0];
-    len_before[0] = 0; nb[0] = 0;
-    for (int i = 1; i < nv; ++i) {
-      int64_t k = blend ? min(min(static_cast<int64_t>(v.blend_frames), total), vlen[i]) : 0;
-      if (k < 0) k = 0;
-      len_before[i] = total; nb[i] = k;
-      total += vlen[i] - k;
-    }
-    // Resolve row p by walking from the last stacked version down.  Level i of the stack is
-    //   [ result_{i-1}[: L-k] | w1*result_{i-1}[L-k+q] + w2*V_i[q], q < k | V_i[k:] ],  L = len(result_{i-1})
-    // so a row is one "terminal" version row plus at most two enclosing cross-fades.
-    int term_ver = ver[0];
-    int64_t term_row = p;
-    int n_blend = 0, blend_level[2];
-    int64_t blend_q[2];
-    for (int level = nv - 1; level >= 1; --level) {
-      const int64_t L = len_before[level], k = nb[level];
-      if (p >= L) { term_ver = ver[level]; term_row = p - L + k; break; }
-      if (p >= L - k) { blend_level[n_blend] = level; blend_q[n_blend] = p - (L - k); ++n_blend; }
-    }
-    // evaluate per column, innermost first
-    const int cols_total = a_cols + f_cols;
-    for (int c = threadIdx.x; c < cols_total; c += blockDim.x) {
-      const bool is_a = c < a_cols;
-      const T* src = is_a ? audio + a0 * a_cols : facial + f0 * f_cols;
-      const int64_t ld = is_a ? a_cols : f_cols;
-      const int cc = is_a ? c : c - a_cols;
-      const bool smooth_slow = !is_a;
-      T val = version_value<T>(src, ld, term_ver, term_row, cc, smooth_slow);
-      for (int bi = n_blend - 1; bi >= 0; --bi) {
-        const int lv = blend_level[bi];
-        const int64_t q = blend_q[bi], k = nb[lv];
-        const T w1 = static_cast<T>(linspace_at(1.0, 0.0, k, q));
-        const T w2 = static_cast<T>(linspace_at(0.0, 1.0, k, q));
-        const T nv_val = version_value<T>(src, ld, ver[lv], q, cc, smooth_slow);
-        val = A::add(A::mul(w1, val), A::mul(w2, nv_val));
-      }
-      if (is_a) out_audio[r * a_cols + cc] = val; else out_facial[r * f_cols + cc] = val;
-    }
-  }
-}
-
-// Product variant of k_collect: a WARP per output row, every warp walking a contiguous run of rows.  The
-// stack geometry of a clip (trim offsets, version lengths, blend zones) is derived once per clip and kept in
-// registers - it was recomputed, behind a chain of dependent loads, by all 128 threads of a block for every
-// single row - and the lanes stream the 256 + 61 columns of the row with fully coalesced 128-byte requests.
-// Same arithmetic (Arith<T>, linspace_at, version_value), so the float64 variant stays bit-exact.
-#ifndef NSF_COLLECT_RUN
-#define NSF_COLLECT_RUN 4
-#endif
-constexpr int kCollectRun = NSF_COLLECT_RUN;      // consecutive rows per warp and tile
+// The stack geometry of a clip (trim offsets, version lengths, blend zones) is derived once per clip and kept in
+// registers - round 1's block-per-row kernel recomputed it, behind a chain of dependent loads, with all 128 threads
+// of a block for every single row - and the lanes stream the 256 + 61 columns of the row with fully coalesced
+// 128-byte requests.  Arith<T>, linspace_at and version_value keep the float64 variant bit-exact.
+constexpr int kCollectRun = 4;      // consecutive rows per warp and tile
 template <typename T>
 __global__ void __launch_bounds__(256, 5) k_collect_rows(CollectView v, const T* __restrict__ audio, int a_cols,
                                                       const T* __restrict__ facial, int f_cols,
@@ -1319,7 +1182,9 @@ __global__ void __launch_bounds__(256, 5) k_collect_rows(CollectView v, const T*
       }
     }
     const int64_t p = r - clip_o0;
-    // Resolve row p by walking from the last stacked version down (see k_collect).
+    // Resolve row p by walking from the last stacked version down.  Level i of the stack is
+    //   [ result_{i-1}[: L-k] | w1*result_{i-1}[L-k+q] + w2*V_i[q], q < k | V_i[k:] ],  L = len(result_{i-1})
+    // so a row is one "terminal" version row plus at most two enclosing cross-fades.
     int term_ver = ver[0];
     int64_t term_row = p;
     int n_blend = 0, blend_level[2] = {0, 0};
@@ -1730,31 +1595,20 @@ int launch_mel_db(cudaStream_t s, const DeviceTables& t, const BatchView& b, con
 }
 
 int launch_dct_sum(cudaStream_t s, const DeviceTables& t, const BatchView& b, const float* db,
-                   const uint32_t* dbmax_key, float* mfcc_raw, double* sum, double* sumsq,
-                   const DctCoef* coef) {
+                   const uint32_t* dbmax_key, float* mfcc_raw, double* sum, double* sumsq) {
   if (t.n_mels > 128 || t.n_mfcc > 32) return -1;
   const int kp = t.n_mfcc <= 24 ? 24 : 32;
-  // default shape: the tensor-pipe kernel.  NSF_DCT_CONST=1 keeps the constant-bank FFMA kernel (validation / A-B timing)
-  static const bool force_const = std::getenv("NSF_DCT_CONST") != nullptr;
-  static const bool force_other = std::getenv("NSF_DCT_SMEM") != nullptr || std::getenv("NSF_DCT_TILE") != nullptr;
-  if (t.dct_frag && !force_const && !force_other && t.n_mels == kDctConstMels && t.n_mfcc == kDctConstMfcc) {
+  // default shape: the tensor-pipe kernel.  NSF_DCT_SMEM=1 keeps the shared-memory coefficient kernels for the
+  // default shape too (the FFMA reference of test_dct_mma_kernel_agrees_with_ffma_kernel)
+  static const bool force_smem = std::getenv("NSF_DCT_SMEM") != nullptr;
+  if (t.dct_frag && !force_smem && t.n_mels == kDctMmaMels && t.n_mfcc == kDctMmaMfcc) {
     const int grid_m = grid_for((b.total_frames + 31) / 32, kDct2Warps, kSmCount * 3);
     k_dct_mma<<<grid_m, kDct2Warps * 32, 0, s>>>(t.dct_frag, b, db, dbmax_key, mfcc_raw, sum, sumsq);
     NSF_CHECK_LAUNCH();
     return 1;
   }
-  // NSF_DCT_SMEM=1 keeps the shared-memory coefficient kernels for the default shape too (validation / A-B timing)
-  static const bool force_smem = std::getenv("NSF_DCT_SMEM") != nullptr;
-  if (coef && !force_smem && t.n_mels == kDctConstMels && t.n_mfcc == kDctConstMfcc) {
-    const int grid_c = grid_for((b.total_frames + 31) / 32, kDct2Warps, kSmCount * 3);
-    k_dct_const<<<grid_c, kDct2Warps * 32, 0, s>>>(*coef, b, db, dbmax_key, mfcc_raw, sum, sumsq);
-    NSF_CHECK_LAUNCH();
-    return 1;
-  }
-  // NSF_DCT_TILE=1 keeps the transposing-tile kernel (validation / A-B timing); it is also the path for
-  // mel counts that are not a multiple of 4 (rows would not be 16-byte aligned)
-  static const bool force_tile = std::getenv("NSF_DCT_TILE") != nullptr;
-  if (!force_tile && (t.n_mels & 3) == 0) {
+  // k_dct_rows reads 16-byte aligned rows; mel counts that are not a multiple of 4 take the transposing-tile kernel
+  if ((t.n_mels & 3) == 0) {
     const size_t smem2 = (static_cast<size_t>(t.n_mels) * kp + static_cast<size_t>(kDct2Warps) * 32 * t.n_mfcc) * sizeof(float);
     const int grid2 = grid_for((b.total_frames + 31) / 32, kDct2Warps, kSmCount * 2);
     if (kp == 24) k_dct_rows<24><<<grid2, kDct2Warps * 32, smem2, s>>>(t, b, db, dbmax_key, mfcc_raw, sum, sumsq);
@@ -1809,32 +1663,17 @@ int launch_smooth(cudaStream_t s, const BatchView& b, const float* in, int64_t i
 int launch_collect(cudaStream_t s, int dtype, const CollectView& v, const void* audio, int a_cols,
                    const void* facial, int f_cols, void* out_audio, void* out_facial) {
   if (v.total_out_rows == 0) return 0;
-  // NSF_COLLECT_BLOCKROW=1 keeps the block-per-row kernel (validation / A-B timing)
-  static const bool block_row = std::getenv("NSF_COLLECT_BLOCKROW") != nullptr;
-  if (!block_row) {
-    // one wave of resident blocks (48 registers: five blocks of 256 threads per SM), >= 8 rows per warp when there are
-    // enough: with 8 blocks per SM the second wave ran 60 % full (ncu: 1.6 waves)
-    const int grid = grid_for(v.total_out_rows, 8 * 8, kSmCount * 5);
-    if (dtype == NSF_F64)
-      k_collect_rows<double><<<grid, 256, 0, s>>>(v, static_cast<const double*>(audio), a_cols,
-                                                  static_cast<const double*>(facial), f_cols,
-                                                  static_cast<double*>(out_audio), static_cast<double*>(out_facial));
-    else
-      k_collect_rows<float><<<grid, 256, 0, s>>>(v, static_cast<const float*>(audio), a_cols,
-                                                 static_cast<const float*>(facial), f_cols,
-                                                 static_cast<float*>(out_audio), static_cast<float*>(out_facial));
-    NSF_CHECK_LAUNCH();
-    return 1;
-  }
-  const int grid = grid_for(v.total_out_rows, 1, kSmCount * 32);
+  // one wave of resident blocks (48 registers: five blocks of 256 threads per SM), >= 8 rows per warp when there are
+  // enough: with 8 blocks per SM the second wave ran 60 % full (ncu: 1.6 waves)
+  const int grid = grid_for(v.total_out_rows, 8 * 8, kSmCount * 5);
   if (dtype == NSF_F64)
-    k_collect<double><<<grid, 128, 0, s>>>(v, static_cast<const double*>(audio), a_cols,
-                                          static_cast<const double*>(facial), f_cols,
-                                          static_cast<double*>(out_audio), static_cast<double*>(out_facial));
+    k_collect_rows<double><<<grid, 256, 0, s>>>(v, static_cast<const double*>(audio), a_cols,
+                                                static_cast<const double*>(facial), f_cols,
+                                                static_cast<double*>(out_audio), static_cast<double*>(out_facial));
   else
-    k_collect<float><<<grid, 128, 0, s>>>(v, static_cast<const float*>(audio), a_cols,
-                                         static_cast<const float*>(facial), f_cols,
-                                         static_cast<float*>(out_audio), static_cast<float*>(out_facial));
+    k_collect_rows<float><<<grid, 256, 0, s>>>(v, static_cast<const float*>(audio), a_cols,
+                                               static_cast<const float*>(facial), f_cols,
+                                               static_cast<float*>(out_audio), static_cast<float*>(out_facial));
   NSF_CHECK_LAUNCH();
   return 1;
 }

@@ -68,15 +68,11 @@ int launch_dft_simt(cudaStream_t s, const DeviceTables& t, const BatchView& b, c
                     float* power);
 int launch_mel_db(cudaStream_t s, const DeviceTables& t, const BatchView& b, const float* power,
                   float* db, uint32_t* dbmax_key);
-// DCT-II matrix of the reference's default shape (128 mels -> 23 MFCCs) as a KERNEL PARAMETER: it lands in
-// the constant bank, the unrolled kernel reads it with uniform loads and feeds the FFMAs uniform-register
-// operands, so the 3 k multiply-adds per frame need no shared-memory traffic at all (k_dct_const).
-constexpr int kDctConstMels = 128, kDctConstMfcc = 23, kDctConstLd = 24;
-struct DctCoef { float v[kDctConstMels * kDctConstLd]; };   // [mel][24], column 23 unused
-// coef: host pointer, non-NULL only when the plan has exactly that shape (else the shared-memory kernels run)
+// Shape of the tensor-pipe DCT kernel k_dct_mma: the reference's default 128 mels -> 23 MFCCs.  Other shapes run the
+// shared-memory coefficient kernels.
+constexpr int kDctMmaMels = 128, kDctMmaMfcc = 23;
 int launch_dct_sum(cudaStream_t s, const DeviceTables& t, const BatchView& b, const float* db,
-                   const uint32_t* dbmax_key, float* mfcc_raw, double* sum, double* sumsq,
-                   const DctCoef* coef);
+                   const uint32_t* dbmax_key, float* mfcc_raw, double* sum, double* sumsq);
 // generic normalise + delta + pair-reduce over a [frames][C] matrix
 int launch_delta_reduce(cudaStream_t s, const BatchView& b, const float* in, int C, int in_ld,
                         const double* sum, const double* sumsq, bool cmvn, bool deltas, bool reduce,

@@ -19,7 +19,6 @@
 #include <cuda_fp16.h>
 
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include <algorithm>
@@ -737,20 +736,17 @@ k_tc_gemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
 // (dm / d0 / d1) and applies them after the hand-shake with its partner (apply_deferred), so every element of
 // the mel tile still receives its contributions in a fixed order.
 struct MelDeferred { int m[2]; float s0[2], s1[2]; int n; };
-constexpr bool kDefaultRolledEpilogue = true;   // 0.653 -> 0.641 ms on C2, 2.13 -> 2.07 ms on C5 (round 2, r2o_ab)
 
-// kRolled: the four 16-column chunks run as a ROLLED loop (one chunk body in the instruction stream instead of four:
-// the fully unrolled epilogue is ~2400 instructions per instantiation, ncu shows 19 % of the fused kernel's stall
-// samples as instruction-fetch starvation); the chunk in flight lands in a second register set that is copied over
-// the working set after the wait (32 moves per chunk).  Same arithmetic in the same order.
-// c_begin, c_end (rolled loop only): the 16-column chunks this warp walks.  The callers split the LIVE chunks of the
-// sub-tile between the two warps (67 of 128 columns hold bins at F = 266: chunks 0-2 and 3-4 instead of four chunks
-// each, of which the upper warp's were 61 / 64 padding); the unrolled variant keeps the fixed 4 + 4 split.
-template <bool kUpper, bool kRolled>
+// The 16-column chunks run as a ROLLED loop (one chunk body in the instruction stream: a fully unrolled epilogue is
+// ~2400 instructions per instantiation, ncu showed 19 % of the fused kernel's stall samples as instruction-fetch
+// starvation; rolling it took C2 from 0.653 to 0.641 ms and C5 from 2.13 to 2.07 ms, round 2); the chunk in flight
+// lands in a second register set that is copied over the working set after the wait (32 moves per chunk).
+// c_begin, c_end: the 16-column chunks this warp walks.  The callers split the LIVE chunks of the sub-tile between the
+// two warps (67 of 128 columns hold bins at F = 266: chunks 0-2 and 3-4 instead of four chunks each, of which the
+// upper warp's were 61 / 64 padding).
+template <bool kUpper>
 __device__ __forceinline__ void mel_accumulate_half(uint32_t acc_addr, const float4* __restrict__ tab,
                                                     float* my_acc, float sc2, MelDeferred& def, int c_begin, int c_end) {
-  constexpr int kCols = BN / 2, kChunks = kCols / 16;
-  constexpr int c0 = kUpper ? kCols : 0;
   int cur_m = -1;
   float s0 = 0.0f, s1 = 0.0f;
   def.n = 0;
@@ -765,70 +761,39 @@ __device__ __forceinline__ void mel_accumulate_half(uint32_t acc_addr, const flo
       my_acc[cur_m + 1] += s1 * sc2;
     }
   };
-  if constexpr (kRolled) {
-    if (c_begin >= c_end) return;
-    float re[16], im[16], nre[16], nim[16];
-    tmem_ld_32x16_async(acc_addr + 16 * c_begin, re);
-    tmem_ld_32x16_async(acc_addr + BN + 16 * c_begin, im);
-    tmem_wait_ld(re, im);
+  if (c_begin >= c_end) return;
+  float re[16], im[16], nre[16], nim[16];
+  tmem_ld_32x16_async(acc_addr + 16 * c_begin, re);
+  tmem_ld_32x16_async(acc_addr + BN + 16 * c_begin, im);
+  tmem_wait_ld(re, im);
 #pragma unroll 1
-    for (int c = c_begin; c < c_end; ++c) {
-      if (c + 1 < c_end) {
-        tmem_ld_32x16_async(acc_addr + 16 * (c + 1), nre);
-        tmem_ld_32x16_async(acc_addr + BN + 16 * (c + 1), nim);
-      }
+  for (int c = c_begin; c < c_end; ++c) {
+    if (c + 1 < c_end) {
+      tmem_ld_32x16_async(acc_addr + 16 * (c + 1), nre);
+      tmem_ld_32x16_async(acc_addr + BN + 16 * (c + 1), nim);
+    }
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        float4 e[8];
+    for (int h = 0; h < 2; ++h) {
+      float4 e[8];
 #pragma unroll
-        for (int q = 0; q < 8; ++q) e[q] = __ldg(tab + 16 * c + 8 * h + q);     // warp-uniform addresses: broadcast
+      for (int q = 0; q < 8; ++q) e[q] = __ldg(tab + 16 * c + 8 * h + q);     // warp-uniform addresses: broadcast
 #pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          const int m0 = __float_as_int(e[q].x);
-          const float pw = fmaf(re[8 * h + q], re[8 * h + q], im[8 * h + q] * im[8 * h + q]);
-          if (m0 != cur_m) {                               // uniform branch
-            flush();
-            cur_m = m0; s0 = 0.0f; s1 = 0.0f;
-          }
-          s0 = fmaf(pw, e[q].y, s0);
-          s1 = fmaf(pw, e[q].z, s1);
+      for (int q = 0; q < 8; ++q) {
+        const int m0 = __float_as_int(e[q].x);
+        const float pw = fmaf(re[8 * h + q], re[8 * h + q], im[8 * h + q] * im[8 * h + q]);
+        if (m0 != cur_m) {                               // uniform branch
+          flush();
+          cur_m = m0; s0 = 0.0f; s1 = 0.0f;
         }
-      }
-      if (c + 1 < c_end) {
-        tmem_wait_ld(nre, nim);
-#pragma unroll
-        for (int q = 0; q < 16; ++q) { re[q] = nre[q]; im[q] = nim[q]; }
+        s0 = fmaf(pw, e[q].y, s0);
+        s1 = fmaf(pw, e[q].z, s1);
       }
     }
-    flush();
-    return;
-  }
-  float re[2][16], im[2][16];
-  tmem_ld_32x16_async(acc_addr + c0, re[0]);
-  tmem_ld_32x16_async(acc_addr + BN + c0, im[0]);
-  tmem_wait_ld(re[0], im[0]);
+    if (c + 1 < c_end) {
+      tmem_wait_ld(nre, nim);
 #pragma unroll
-  for (int c = 0; c < kChunks; ++c) {
-    const int cur = c & 1, nxt = cur ^ 1;
-    if (c + 1 < kChunks) {
-      tmem_ld_32x16_async(acc_addr + c0 + 16 * (c + 1), re[nxt]);
-      tmem_ld_32x16_async(acc_addr + BN + c0 + 16 * (c + 1), im[nxt]);
+      for (int q = 0; q < 16; ++q) { re[q] = nre[q]; im[q] = nim[q]; }
     }
-    float4 e[16];
-#pragma unroll
-    for (int q = 0; q < 16; ++q) e[q] = __ldg(tab + c0 + 16 * c + q);     // warp-uniform addresses: broadcast
-#pragma unroll
-    for (int q = 0; q < 16; ++q) {
-      const int m0 = __float_as_int(e[q].x);
-      const float pw = fmaf(re[cur][q], re[cur][q], im[cur][q] * im[cur][q]);
-      if (m0 != cur_m) {                               // uniform branch
-        flush();
-        cur_m = m0; s0 = 0.0f; s1 = 0.0f;
-      }
-      s0 = fmaf(pw, e[q].y, s0);
-      s1 = fmaf(pw, e[q].z, s1);
-    }
-    if (c + 1 < kChunks) tmem_wait_ld(re[nxt], im[nxt]);
   }
   flush();
 }
@@ -889,7 +854,6 @@ constexpr size_t kMelTileBytes = (static_cast<size_t>(BM + 1) * kMelPitch * size
 constexpr size_t kFusedSmem = 1024 + static_cast<size_t>(kFStages) * kStageBytes +
                               kMelTileBytes + 256;
 
-template <bool kRolled>
 __global__ void __launch_bounds__(kFusedThreads, 1)
 k_tc_stft_mel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
               DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
@@ -1015,8 +979,8 @@ k_tc_stft_mel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
         tcgen05_fence_after();
         MelDeferred def;
         const int live_chunks = (min(BN, t.np[chain] - n0) + 15) / 16, lower_chunks = (live_chunks + 1) / 2;
-        if (upper) mel_accumulate_half<true, kRolled>(lane_addr + buf * 256u, tab, acc_row, sc2, def, lower_chunks, live_chunks);
-        else mel_accumulate_half<false, kRolled>(lane_addr + buf * 256u, tab, acc_row, sc2, def, 0, lower_chunks);
+        if (upper) mel_accumulate_half<true>(lane_addr + buf * 256u, tab, acc_row, sc2, def, lower_chunks, live_chunks);
+        else mel_accumulate_half<false>(lane_addr + buf * 256u, tab, acc_row, sc2, def, 0, lower_chunks);
         // all TMEM reads of this warp are complete (tcgen05.wait::ld inside the routine)
         tcgen05_fence_before();
         __syncwarp();
@@ -1098,7 +1062,6 @@ constexpr int kPStageBytes = 2 * kPTileA + 2 * kPTileB;
 constexpr size_t kPairSmem = 1024 + static_cast<size_t>(kPStages) * kPStageBytes +
                              kMelTileBytes + 256;
 
-template <bool kRolled>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1)
 k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                    DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
@@ -1228,8 +1191,8 @@ k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_const
         tcgen05_fence_after();
         MelDeferred def;
         const int live_chunks = (min(BN, t.np[chain] - n0) + 15) / 16, lower_chunks = (live_chunks + 1) / 2;
-        if (upper) mel_accumulate_half<true, kRolled>(lane_addr + buf * 256u, tab, acc_row, sc2, def, lower_chunks, live_chunks);
-        else mel_accumulate_half<false, kRolled>(lane_addr + buf * 256u, tab, acc_row, sc2, def, 0, lower_chunks);
+        if (upper) mel_accumulate_half<true>(lane_addr + buf * 256u, tab, acc_row, sc2, def, lower_chunks, live_chunks);
+        else mel_accumulate_half<false>(lane_addr + buf * 256u, tab, acc_row, sc2, def, 0, lower_chunks);
         // all TMEM reads of this warp are complete (tcgen05.wait::ld inside the routine)
         tcgen05_fence_before();
         __syncwarp();
@@ -1399,9 +1362,7 @@ int launch_stft_tc_fold(cudaStream_t s, const StftTcTables& tc, const DeviceTabl
   const int buf_floats = ((t.F + 3) & ~3) + 8;   // frame + up to 3 floats of skew + tail, 16-byte multiple
   const int kp = tc.kp;
   const int iters = (kp + 63) / 64;
-  // NSF_FOLD_LEGACY=1 keeps the two-pass kernel for every F (validation / A-B timing)
-  static const bool fold_legacy = std::getenv("NSF_FOLD_LEGACY") != nullptr;
-  const bool reg_path = iters <= 8 && !fold_legacy;
+  const bool reg_path = iters <= 8;              // longer frames take the two-pass kernel k_tc_fold
   const int wp_pairs = iters * 64;               // float2 window pairs, zero beyond K
   const size_t head = reg_path ? static_cast<size_t>(2) * wp_pairs : static_cast<size_t>((t.F + 3) & ~3);
   const size_t smem = (head + static_cast<size_t>(kFoldWarps) * 2 * buf_floats) * sizeof(float);
@@ -1432,37 +1393,22 @@ int launch_stft_tc_mel(cudaStream_t s, const StftTcTables& tc, const DeviceTable
   const OperandView v = view_operands(tc, b.total_frames, operands);
   CUtensorMap map_a;
   if (!encode_map(&map_a, v.planes, static_cast<uint64_t>(tc.chains) * 4 * v.rows, tc.kp, BM)) return -1;
-  // NSF_STFT_1CTA=1 keeps the single-CTA kernel (validation / A-B timing)
-  static const bool one_cta = std::getenv("NSF_STFT_1CTA") != nullptr;
-  // NSF_STFT_EPILOGUE=rolled|unrolled: the mel epilogue's chunk loop (A/B timing; identical results)
-  static const bool rolled = [] {
-    const char* v = std::getenv("NSF_STFT_EPILOGUE");
-    return v ? v[0] == 'r' : kDefaultRolledEpilogue;
-  }();
   // short K (16 kHz: two 64-column stages per accumulator) leaves the pair's longer hand-off exposed:
   // measured 3.31 vs 3.06 ms on the C5 batch, so pairs are used from four K stages on
   const int kblocks = (tc.kp + BK - 1) / BK;
-  if (!one_cta && kblocks >= 4) {
+  if (kblocks >= 4) {
     int64_t pairs = v.rows / (2 * BM);
     if (pairs > 74) pairs = 74;
     if (pairs < 1) pairs = 1;
-    if (rolled)
-      k_tc_stft_mel_pair<true><<<static_cast<unsigned>(2 * pairs), kFusedThreads, kPairSmem, s>>>(
-          map_a, tc.map_b_half, t, b, v.rows, tc.kp, tc.np_ld, v.row_exp, db, dbmax_key);
-    else
-      k_tc_stft_mel_pair<false><<<static_cast<unsigned>(2 * pairs), kFusedThreads, kPairSmem, s>>>(
-          map_a, tc.map_b_half, t, b, v.rows, tc.kp, tc.np_ld, v.row_exp, db, dbmax_key);
+    k_tc_stft_mel_pair<<<static_cast<unsigned>(2 * pairs), kFusedThreads, kPairSmem, s>>>(
+        map_a, tc.map_b_half, t, b, v.rows, tc.kp, tc.np_ld, v.row_exp, db, dbmax_key);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
   }
   int64_t grid = v.rows / BM;
   if (grid > 148) grid = 148;
   if (grid < 1) grid = 1;
-  if (rolled)
-    k_tc_stft_mel<true><<<static_cast<unsigned>(grid), kFusedThreads, kFusedSmem, s>>>(map_a, tc.map_b, t, b, v.rows, tc.kp,
-                                                                                   tc.np_ld, v.row_exp, db, dbmax_key);
-  else
-    k_tc_stft_mel<false><<<static_cast<unsigned>(grid), kFusedThreads, kFusedSmem, s>>>(map_a, tc.map_b, t, b, v.rows, tc.kp,
-                                                                                    tc.np_ld, v.row_exp, db, dbmax_key);
+  k_tc_stft_mel<<<static_cast<unsigned>(grid), kFusedThreads, kFusedSmem, s>>>(map_a, tc.map_b, t, b, v.rows, tc.kp,
+                                                                             tc.np_ld, v.row_exp, db, dbmax_key);
   return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
 
@@ -1490,10 +1436,8 @@ bool init_stft_tc_attributes() {
   };
   set(k_tc_fold_r<2>, 220 * 1024); set(k_tc_fold_r<3>, 220 * 1024); set(k_tc_fold_r<4>, 220 * 1024);
   set(k_tc_fold_r<6>, 220 * 1024); set(k_tc_fold_r<8>, 220 * 1024); set(k_tc_fold, 220 * 1024);
-  set(k_tc_stft_mel_pair<false>, static_cast<int>(kPairSmem));
-  set(k_tc_stft_mel_pair<true>, static_cast<int>(kPairSmem));
-  set(k_tc_stft_mel<false>, static_cast<int>(kFusedSmem));
-  set(k_tc_stft_mel<true>, static_cast<int>(kFusedSmem));
+  set(k_tc_stft_mel_pair, static_cast<int>(kPairSmem));
+  set(k_tc_stft_mel, static_cast<int>(kFusedSmem));
   set(k_tc_gemm, static_cast<int>(kSmemBytes));
   return ok;
 }

@@ -4,7 +4,7 @@
     python scripts/prof_step.py [--workload c2] [--warmup 2] [--steps 1]
 
 Prints the mean step time (CUDA events) and the library's per-stage times as one JSON line.  Environment switches
-of the library (NSF_AC_LOOP, NSF_STFT_1CTA, ...) apply as usual.  Experiments only."""
+of the library (NSF_AC_LOOP, NSF_AC_KERNEL, ...) apply as usual.  Experiments only."""
 import argparse
 import json
 import os

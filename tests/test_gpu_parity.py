@@ -553,12 +553,11 @@ def test_fused_extract_collect_equals_two_calls(engine, nv):
         np.testing.assert_array_equal(gf, wf)
 
 
-def test_dct_kernels_agree(engine, tmp_path):
-    """Three DCT kernels: k_dct_mma (default: tensor-pipe, split fp16), k_dct_const (NSF_DCT_CONST: coefficients as a
-    kernel parameter, uniform-register FFMA operands) and k_dct_rows (NSF_DCT_SMEM: shared-memory coefficients).  The
-    two FFMA kernels keep one accumulation order: bit-identical feature matrices.  The MMA kernel sums in another order
-    and from split operands: MFCC / delta columns within 2e-5 / 5e-6 of them, autocorrelation columns identical.  The
-    environment switches are read once per process, so the FFMA kernels run in child processes."""
+def test_dct_mma_kernel_agrees_with_ffma_kernel(engine, tmp_path):
+    """Two DCT kernels: k_dct_mma (default: tensor-pipe, split fp16) and k_dct_rows (NSF_DCT_SMEM: shared-memory
+    coefficients, FFMA).  The MMA kernel sums in another order and from split operands: MFCC / delta columns within
+    2e-5 / 5e-6 of the FFMA kernel's, autocorrelation columns identical.  The environment switch is read once per
+    process, so the FFMA kernel runs in a child process."""
     import os
     import subprocess
     import sys
@@ -572,19 +571,15 @@ def test_dct_kernels_agree(engine, tmp_path):
     np.save(tmp_path / "off.npy", off)
     got = engine.get_engine(88200, 1470, 735).extract_host(y, off, 0)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    refs = {}
-    for tag in ("NSF_DCT_CONST", "NSF_DCT_SMEM"):
-        out = tmp_path / (tag + ".npy")
-        code = ("import sys, numpy as np; sys.path.insert(0, %r)\n"
-                "from neurosync_trainer_lite_b200 import engine\n"
-                "y, off = np.load(%r), np.load(%r)\n"
-                "np.save(%r, engine.get_engine(88200, 1470, 735).extract_host(y, off, 0))\n"
-                % (root, str(tmp_path / "y.npy"), str(tmp_path / "off.npy"), str(out)))
-        subprocess.run([sys.executable, "-c", code], check=True, env=dict(os.environ, **{tag: "1"}), timeout=600)
-        refs[tag] = np.load(out)
-    want = refs["NSF_DCT_CONST"]
+    out = tmp_path / "NSF_DCT_SMEM.npy"
+    code = ("import sys, numpy as np; sys.path.insert(0, %r)\n"
+            "from neurosync_trainer_lite_b200 import engine\n"
+            "y, off = np.load(%r), np.load(%r)\n"
+            "np.save(%r, engine.get_engine(88200, 1470, 735).extract_host(y, off, 0))\n"
+            % (root, str(tmp_path / "y.npy"), str(tmp_path / "off.npy"), str(out)))
+    subprocess.run([sys.executable, "-c", code], check=True, env=dict(os.environ, NSF_DCT_SMEM="1"), timeout=600)
+    want = np.load(out)
     assert got.shape == want.shape and got.shape[0] > 0
-    assert np.array_equal(want, refs["NSF_DCT_SMEM"])
     assert np.array_equal(got[:, 69:], want[:, 69:])
     d = np.abs(got - want)
     assert d[:, :23].max() <= 2e-5 and d[:, 23:69].max() <= 5e-6, (d[:, :23].max(), d[:, 23:69].max())
