@@ -155,16 +155,14 @@ inline int64_t group_budget(int turn) {
 // Grid caps of the two front-end kernels inside the pipelined passes (nsf_kernels.cu, launch_absmax).
 constexpr int kPipelinedAbsmaxBlocks = 74, kPipelinedNormalizeBlocks = 148;
 
-struct Slot {  // one in-flight clip group of the host pipeline
+struct Slot {  // one in-flight clip group of the host pipeline; slot 0 also serves the synchronous one-shot calls
   cudaStream_t stream = nullptr;
-  Arena pcm, out, work, ynorm;
-  Arena fac_in, col_a, col_f, col_desc;   // fused extract + collect path
-  cudaEvent_t done = nullptr;
-  // pageable callers: the group's PCM is gathered into `stage_in` (pinned) before its upload and its rows
-  // come back through `stage_out` (pinned); `pending_*` describe the copy-out owed to the caller's buffers
-  PinnedArena stage_in, stage_out, stage_aux, stage_fac, stage_feat;
-  struct CopyOut { void* dst; const void* src; size_t bytes; size_t dst_pitch, src_pitch, width; int64_t rows; };
-  CopyOut pending[4];
+  Arena in[2], out[3], work;   // device: the group's inputs, its results, kernel workspace
+  // pinned twins of `in` / `out` for pageable caller buffers: an input is gathered into stage_in[i] before its
+  // upload, a result comes back through stage_out[i]; `pending` lists the copy-outs owed to the caller's buffers
+  PinnedArena stage_in[2], stage_out[3];
+  struct CopyOut { void* dst; const void* src; size_t dst_pitch, width; int64_t rows; };   // rows of `width` bytes
+  CopyOut pending[3];
   int n_pending = 0;
 };
 
@@ -174,7 +172,7 @@ struct Slot {  // one in-flight clip group of the host pipeline
 constexpr int kDescRing = 8;
 struct DescEntry {
   PinnedArena mem;
-  Arena dev;              // device copy of the entry, for calls whose descriptors have no other home (nsf_convert_batch)
+  Arena dev;              // device copy of the entry, for calls whose descriptors have no other home (convert, collect, windows)
   cudaEvent_t copied = nullptr;
   bool pending = false;
 };
@@ -211,7 +209,6 @@ struct nsf_ctx {
   bool pipelined = false;     // set by the host passes around their nsf_extract_batch calls (front-end grid caps)
   cudaEvent_t stage_ev[nsf::kStages + 1] = {};
   bool stage_valid = false;
-  nsf::Arena collect_in_a, collect_in_f, collect_out_a, collect_out_f, collect_desc;
   std::vector<nsf::TapTable*> tap_tables;   // filter cache of the conversion calls, one per (rate pair, quality)
   std::vector<nsf::ConvClip> conv_clips;    // scratch of convert_enqueue
   std::vector<nsf_pcm_source> conv_src;     // scratch of nsf_convert_host (one group's rebased descriptors)
@@ -454,6 +451,166 @@ struct StageTimer {
   }
 };
 
+// ---- host-buffer pipeline ------------------------------------------------------------------------
+nsf_status ensure_slot(Slot* sl) {
+  if (!sl->stream) NSF_CUDA(cudaStreamCreateWithFlags(&sl->stream, cudaStreamNonBlocking));
+  return NSF_OK;
+}
+
+// Is `p` memory the copy engines can reach directly (cudaHostAlloc / cudaHostRegister / managed)?  Pageable
+// buffers are staged through the slot's pinned arenas so that uploads and downloads stay asynchronous.
+bool dma_reachable(const void* p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
+}
+
+// memcpy split over a few threads once it is large enough to be bound by one core's copy bandwidth.
+void host_copy(void* dst, const void* src, size_t bytes) {
+  constexpr size_t kChunk = size_t(8) << 20;
+  unsigned hw = std::thread::hardware_concurrency();
+  size_t n = bytes / kChunk;
+  if (n > 8) n = 8;
+  if (hw && n > hw) n = hw;
+  if (n < 2) { std::memcpy(dst, src, bytes); return; }
+  const size_t part = (bytes / n + 63) & ~size_t(63);
+  std::vector<std::thread> th;
+  th.reserve(n - 1);
+  for (size_t i = 1; i < n; ++i) {
+    const size_t off = i * part;
+    if (off >= bytes) break;
+    const size_t len = std::min(part, bytes - off);
+    th.emplace_back([=] { std::memcpy(static_cast<char*>(dst) + off, static_cast<const char*>(src) + off, len); });
+  }
+  std::memcpy(dst, src, std::min(part, bytes));
+  for (auto& t : th) t.join();
+}
+
+// Waits for the slot's stream, then makes the copy-outs it owes to pageable caller buffers.
+nsf_status drain_slot(Slot* sl) {
+  NSF_CUDA(cudaStreamSynchronize(sl->stream));
+  for (int i = 0; i < sl->n_pending; ++i) {
+    const Slot::CopyOut& c = sl->pending[i];
+    if (c.dst_pitch == c.width) {
+      host_copy(c.dst, c.src, c.width * static_cast<size_t>(c.rows));
+    } else {
+      for (int64_t r = 0; r < c.rows; ++r)
+        std::memcpy(static_cast<char*>(c.dst) + r * c.dst_pitch, static_cast<const char*>(c.src) + r * c.width, c.width);
+    }
+  }
+  sl->n_pending = 0;
+  return NSF_OK;
+}
+
+// Slot 0, ready for a synchronous one-shot call: created, drained, owing no copy-out.
+nsf_status oneshot_slot(nsf_ctx* ctx, Slot** out) {
+  Slot* sl = &ctx->slot[0];
+  const nsf_status st = ensure_slot(sl);
+  if (st != NSF_OK) return st;
+  NSF_CUDA(cudaStreamSynchronize(sl->stream));
+  sl->n_pending = 0;
+  *out = sl;
+  return NSF_OK;
+}
+
+// Queues the copy of `bytes` of caller memory into the slot's device input i (reserved by the caller).  Pageable
+// memory is first gathered into the pinned stage_in[i] by the host, so that the copy itself stays asynchronous.
+nsf_status upload(Slot* sl, int i, const void* src, size_t bytes, bool dma) {
+  if (!dma) {
+    const nsf_status st = sl->stage_in[i].reserve(bytes);
+    if (st != NSF_OK) return st;
+    host_copy(sl->stage_in[i].ptr, src, bytes);
+    src = sl->stage_in[i].ptr;
+  }
+  NSF_CUDA(cudaMemcpyAsync(sl->in[i].ptr, src, bytes, cudaMemcpyHostToDevice, sl->stream));
+  return NSF_OK;
+}
+
+// Queues the copy of the slot's device output i, `rows` packed rows of `width` bytes, to caller memory whose rows
+// start `dst_pitch` bytes apart.  The copy engine writes page-locked memory itself; pageable memory gets the rows
+// from the pinned stage_out[i] when the slot drains.
+nsf_status download(Slot* sl, int i, void* dst, size_t dst_pitch, size_t width, int64_t rows, bool dma) {
+  const size_t bytes = width * static_cast<size_t>(rows);
+  if (dma && dst_pitch == width) {
+    NSF_CUDA(cudaMemcpyAsync(dst, sl->out[i].ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
+  } else if (dma) {
+    NSF_CUDA(cudaMemcpy2DAsync(dst, dst_pitch, sl->out[i].ptr, width, width, rows, cudaMemcpyDeviceToHost, sl->stream));
+  } else {
+    const nsf_status st = sl->stage_out[i].reserve(bytes);
+    if (st != NSF_OK) return st;
+    NSF_CUDA(cudaMemcpyAsync(sl->stage_out[i].ptr, sl->out[i].ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
+    sl->pending[sl->n_pending++] = Slot::CopyOut{dst, sl->stage_out[i].ptr, dst_pitch, width, rows};
+  }
+  return NSF_OK;
+}
+
+// Runs a host call as clip groups.  cost[0..n] is a prefix sum over the n clips; a group is the longest run of clips
+// [first, last) with cost[last] - cost[first] <= group_budget(turn), and at least one clip.  Groups rotate over the
+// slots, and a slot drains before it takes its next group, so the upload of group g + 1, the kernels of group g and
+// the download of group g - 1 overlap.  body(first, last, slot) reserves the slot's arenas and queues the group's
+// uploads, kernels and downloads.  Every slot drains before the call returns: the caller's buffers are final on
+// success and no copy into them is still running on error.  On error the owed copy-outs are dropped and the first
+// error is returned.
+template <typename Body>
+nsf_status run_groups(nsf_ctx* ctx, const int64_t* cost, int32_t n, Body&& body) {
+  nsf_status st = NSF_OK;
+  for (int first = 0, turn = 0; first < n && st == NSF_OK; ++turn) {
+    int last = first + 1;
+    while (last < n && cost[last + 1] - cost[first] <= group_budget(turn)) ++last;
+    Slot* sl = &ctx->slot[turn % kSlots];
+    if ((st = ensure_slot(sl)) == NSF_OK && (st = drain_slot(sl)) == NSF_OK) st = body(first, last, sl);
+    first = last;
+  }
+  for (auto& sl : ctx->slot) {
+    if (!sl.stream) continue;
+    if (st == NSF_OK) { st = drain_slot(&sl); continue; }
+    sl.n_pending = 0;
+    cudaStreamSynchronize(sl.stream);   // the first error is the one reported
+  }
+  return st;
+}
+
+// nsf_extract_batch of one group, from the slot's in[0] into its out[0], with the front-end grid caps of a pipelined
+// pass.
+nsf_status extract_group(nsf_ctx* ctx, Slot* sl, int32_t pcm_format, const int64_t* clip_offsets, int32_t n,
+                         uint32_t flags, int cols, float* y_norm_dev) {
+  ctx->pipelined = true;
+  const nsf_status st = nsf_extract_batch(ctx, sl->stream, sl->in[0].ptr, pcm_format, clip_offsets, n, flags,
+                                          static_cast<float*>(sl->out[0].ptr), cols, nullptr, y_norm_dev, sl->work.ptr,
+                                          static_cast<int64_t>(sl->work.bytes));
+  ctx->pipelined = false;
+  return st;
+}
+
+// Enqueues k_collect_rows over n clips whose rows start at `audio` / `facial` and whose results start at `out_a` /
+// `out_f`.  a_off / f_off / o_off (n + 1 entries each, rebased here to their first entry) place the clips in each.  The
+// three arrays travel through the descriptor ring into the entry's device copy, which is reused only after the kernel.
+nsf_status collect_enqueue(nsf_ctx* ctx, cudaStream_t s, int32_t dtype, const void* audio, int32_t a_cols,
+                           const int64_t* a_off, const void* facial, int32_t f_cols, const int64_t* f_off,
+                           const int64_t* o_off, int32_t n, uint32_t flags, int32_t blend_frames, void* out_a,
+                           void* out_f) {
+  const size_t n1 = static_cast<size_t>(n) + 1, bytes = 3 * n1 * sizeof(int64_t);
+  DescEntry* de = nullptr;
+  nsf_status st = desc_acquire(ctx, bytes, &de);
+  if (st != NSF_OK) return st;
+  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
+  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
+  for (size_t i = 0; i < n1; ++i) {
+    h[i] = a_off[i] - a_off[0];
+    h[n1 + i] = f_off[i] - f_off[0];
+    h[2 * n1 + i] = o_off[i] - o_off[0];
+  }
+  int64_t* d = static_cast<int64_t*>(de->dev.ptr);
+  NSF_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s));
+  CollectView v;
+  v.a_off = d; v.f_off = d + n1; v.o_off = d + 2 * n1;
+  v.n_clips = n; v.total_out_rows = o_off[n] - o_off[0]; v.flags = flags; v.blend_frames = blend_frames;
+  const int m = launch_collect(s, dtype, v, audio, a_cols, facial, f_cols, out_a, out_f);
+  if (m < 0) { set_error(cuda_msg("launch_collect", cudaGetLastError())); return NSF_ERR_CUDA; }
+  ctx->launches += m;
+  return desc_commit(de, s);     // recorded after the kernel: the entry (host and device) is reused only after it
+}
+
 }  // namespace
 }  // namespace nsf
 
@@ -559,10 +716,11 @@ void nsf_ctx_destroy(nsf_ctx* ctx) {
   cudaDeviceSynchronize();
   for (auto& s : ctx->slot) {
     if (s.stream) cudaStreamDestroy(s.stream);
-    if (s.done) cudaEventDestroy(s.done);
-    s.pcm.release(); s.out.release(); s.work.release(); s.ynorm.release();
-    s.fac_in.release(); s.col_a.release(); s.col_f.release(); s.col_desc.release();
-    s.stage_in.release(); s.stage_out.release(); s.stage_aux.release(); s.stage_fac.release(); s.stage_feat.release();
+    for (auto& a : s.in) a.release();
+    for (auto& a : s.out) a.release();
+    s.work.release();
+    for (auto& a : s.stage_in) a.release();
+    for (auto& a : s.stage_out) a.release();
   }
   for (auto& e : ctx->stage_ev) if (e) cudaEventDestroy(e);
   for (auto& d : ctx->desc) {
@@ -572,8 +730,6 @@ void nsf_ctx_destroy(nsf_ctx* ctx) {
   }
   for (TapTable* t : ctx->tap_tables) { t->mem.release(); delete t; }
   ctx->table_mem.release();
-  ctx->collect_in_a.release(); ctx->collect_in_f.release();
-  ctx->collect_out_a.release(); ctx->collect_out_f.release(); ctx->collect_desc.release();
   delete ctx;
 }
 
@@ -752,60 +908,6 @@ nsf_status nsf_extract_batch(nsf_ctx* ctx, void* cuda_stream, const void* pcm_de
 }
 
 // ---- host-buffer pipeline ------------------------------------------------------------------------
-static nsf_status ensure_slot(Slot* sl) {
-  if (!sl->stream) NSF_CUDA(cudaStreamCreateWithFlags(&sl->stream, cudaStreamNonBlocking));
-  if (!sl->done) NSF_CUDA(cudaEventCreateWithFlags(&sl->done, cudaEventDisableTiming));
-  return NSF_OK;
-}
-
-// Is `p` memory the copy engines can reach directly (cudaHostAlloc / cudaHostRegister / managed)?  Pageable
-// buffers are staged through the slot's pinned arenas so that uploads and downloads stay asynchronous.
-static bool dma_reachable(const void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
-}
-
-// memcpy split over a few threads once it is large enough to be bound by one core's copy bandwidth.
-static void host_copy(void* dst, const void* src, size_t bytes) {
-  constexpr size_t kChunk = size_t(8) << 20;
-  unsigned hw = std::thread::hardware_concurrency();
-  size_t n = bytes / kChunk;
-  if (n > 8) n = 8;
-  if (hw && n > hw) n = hw;
-  if (n < 2) { std::memcpy(dst, src, bytes); return; }
-  const size_t part = (bytes / n + 63) & ~size_t(63);
-  std::vector<std::thread> th;
-  th.reserve(n - 1);
-  for (size_t i = 1; i < n; ++i) {
-    const size_t off = i * part;
-    if (off >= bytes) break;
-    const size_t len = std::min(part, bytes - off);
-    th.emplace_back([=] { std::memcpy(static_cast<char*>(dst) + off, static_cast<const char*>(src) + off, len); });
-  }
-  std::memcpy(dst, src, std::min(part, bytes));
-  for (auto& t : th) t.join();
-}
-
-// Copy-outs a slot owes to pageable caller buffers; run once the slot's stream has drained.
-static void flush_pending(Slot* sl) {
-  for (int i = 0; i < sl->n_pending; ++i) {
-    const Slot::CopyOut& c = sl->pending[i];
-    if (c.rows <= 1 || (c.dst_pitch == c.width && c.src_pitch == c.width)) {
-      host_copy(c.dst, c.src, c.rows <= 1 ? c.bytes : c.width * static_cast<size_t>(c.rows));
-    } else {
-      for (int64_t r = 0; r < c.rows; ++r)
-        std::memcpy(static_cast<char*>(c.dst) + r * c.dst_pitch, static_cast<const char*>(c.src) + r * c.src_pitch, c.width);
-    }
-  }
-  sl->n_pending = 0;
-}
-static nsf_status drain_slot(Slot* sl) {
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  flush_pending(sl);
-  return NSF_OK;
-}
-
 nsf_status nsf_extract_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_format,
                             const int64_t* clip_offsets, int32_t n_clips, uint32_t flags,
                             float* out_host, int64_t out_ld, float* y_norm_host) {
@@ -821,76 +923,29 @@ nsf_status nsf_extract_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_form
   nsf_status st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  for (auto& sl : ctx->slot) sl.n_pending = 0;   // nothing is owed from an earlier call (errors drop their copy-outs)
-  const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
+  const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4, row_bytes = static_cast<size_t>(cols) * sizeof(float);
   // pageable caller buffers go through the slot's pinned staging arenas: the host copies group g + 1 in (and
   // group g - 2 out) while the copy engines and kernels work on the groups in between
   const bool in_dma = dma_reachable(pcm_host), out_dma = dma_reachable(out_host);
   const bool y_dma = y_norm_host ? dma_reachable(y_norm_host) : true;
-  int first = 0, turn = 0;
-  while (first < n_clips) {
-    int last = first;
-    int64_t samples = 0;
-    while (last < n_clips && (last == first || samples + (clip_offsets[last + 1] - clip_offsets[last]) <= group_budget(turn))) {
-      samples += clip_offsets[last + 1] - clip_offsets[last];
-      ++last;
-    }
-    const int gn = last - first;
-    Slot* sl = &ctx->slot[turn % kSlots];
-    st = ensure_slot(sl);
-    if (st != NSF_OK) return st;
-    // the slot's previous group must have fully drained before its buffers are reused
-    if ((st = drain_slot(sl)) != NSF_OK) return st;
+  return run_groups(ctx, clip_offsets, n_clips, [&](int first, int last, Slot* sl) -> nsf_status {
+    const int64_t samples = clip_offsets[last] - clip_offsets[first];
     const int64_t rows = all.row_off[last] - all.row_off[first];
-    const int64_t wbytes = nsf_workspace_bytes(ctx->plan, samples, gn, flags);
-    const size_t out_bytes = static_cast<size_t>(rows) * cols * sizeof(float);
-    if ((st = sl->pcm.reserve(samples * esz)) != NSF_OK) return st;
-    if ((st = sl->out.reserve(out_bytes)) != NSF_OK) return st;
-    if ((st = sl->work.reserve(wbytes)) != NSF_OK) return st;
-    if (y_norm_host && (st = sl->ynorm.reserve(samples * sizeof(float))) != NSF_OK) return st;
-    const char* src = static_cast<const char*>(pcm_host) + clip_offsets[first] * esz;
-    if (!in_dma) {
-      if ((st = sl->stage_in.reserve(samples * esz)) != NSF_OK) return st;
-      host_copy(sl->stage_in.ptr, src, samples * esz);
-      src = static_cast<const char*>(sl->stage_in.ptr);
-    }
-    NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, src, samples * esz, cudaMemcpyHostToDevice, sl->stream));
-    ctx->pipelined = true;
-    st = nsf_extract_batch(ctx, sl->stream, sl->pcm.ptr, pcm_format, clip_offsets + first, gn, flags,
-                           static_cast<float*>(sl->out.ptr), cols, nullptr,
-                           y_norm_host ? static_cast<float*>(sl->ynorm.ptr) : nullptr, sl->work.ptr,
-                           static_cast<int64_t>(sl->work.bytes));
-    ctx->pipelined = false;
-    if (st != NSF_OK) return st;
-    float* dst = out_host + all.row_off[first] * out_ld;
-    if (!out_dma) {
-      if ((st = sl->stage_out.reserve(out_bytes)) != NSF_OK) return st;
-      NSF_CUDA(cudaMemcpyAsync(sl->stage_out.ptr, sl->out.ptr, out_bytes, cudaMemcpyDeviceToHost, sl->stream));
-      sl->pending[sl->n_pending++] = Slot::CopyOut{dst, sl->stage_out.ptr, out_bytes, static_cast<size_t>(out_ld) * sizeof(float),
-                                                   static_cast<size_t>(cols) * sizeof(float),
-                                                   static_cast<size_t>(cols) * sizeof(float), rows};
-    } else if (out_ld == cols) {
-      NSF_CUDA(cudaMemcpyAsync(dst, sl->out.ptr, out_bytes, cudaMemcpyDeviceToHost, sl->stream));
-    } else {
-      NSF_CUDA(cudaMemcpy2DAsync(dst, out_ld * sizeof(float), sl->out.ptr, cols * sizeof(float),
-                                 cols * sizeof(float), rows, cudaMemcpyDeviceToHost, sl->stream));
-    }
-    if (y_norm_host) {
-      float* ydst = y_norm_host + (clip_offsets[first] - clip_offsets[0]);
-      if (!y_dma) {
-        if ((st = sl->stage_aux.reserve(samples * sizeof(float))) != NSF_OK) return st;
-        NSF_CUDA(cudaMemcpyAsync(sl->stage_aux.ptr, sl->ynorm.ptr, samples * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-        sl->pending[sl->n_pending++] = Slot::CopyOut{ydst, sl->stage_aux.ptr, samples * sizeof(float), 0, 0, 0, 1};
-      } else {
-        NSF_CUDA(cudaMemcpyAsync(ydst, sl->ynorm.ptr, samples * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-      }
-    }
-    first = last;
-    ++turn;
-  }
-  for (auto& sl : ctx->slot)
-    if (sl.stream && (st = drain_slot(&sl)) != NSF_OK) return st;
-  return NSF_OK;
+    nsf_status st;
+    if ((st = sl->in[0].reserve(samples * esz)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(rows * row_bytes)) != NSF_OK) return st;
+    if ((st = sl->work.reserve(nsf_workspace_bytes(ctx->plan, samples, last - first, flags))) != NSF_OK) return st;
+    if (y_norm_host && (st = sl->out[1].reserve(samples * sizeof(float))) != NSF_OK) return st;
+    if ((st = upload(sl, 0, static_cast<const char*>(pcm_host) + clip_offsets[first] * esz, samples * esz, in_dma)) != NSF_OK)
+      return st;
+    if ((st = extract_group(ctx, sl, pcm_format, clip_offsets + first, last - first, flags, cols,
+                            y_norm_host ? static_cast<float*>(sl->out[1].ptr) : nullptr)) != NSF_OK) return st;
+    if ((st = download(sl, 0, out_host + all.row_off[first] * out_ld, static_cast<size_t>(out_ld) * sizeof(float),
+                       row_bytes, rows, out_dma)) != NSF_OK) return st;
+    if (!y_norm_host) return NSF_OK;
+    const size_t y_bytes = samples * sizeof(float);
+    return download(sl, 1, y_norm_host + (clip_offsets[first] - clip_offsets[0]), y_bytes, y_bytes, 1, y_dma);
+  });
 }
 
 nsf_status nsf_normalize_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_format,
@@ -902,18 +957,17 @@ nsf_status nsf_normalize_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_fo
   for (int i = 0; i < n_clips; ++i)
     if (clip_offsets[i + 1] < clip_offsets[i]) { set_error("clip_offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = &ctx->slot[0];
-  nsf_status st = ensure_slot(sl);
+  Slot* sl = nullptr;
+  nsf_status st = oneshot_slot(ctx, &sl);
   if (st != NSF_OK) return st;
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
   const int64_t samples = clip_offsets[n_clips] - clip_offsets[0];
   if (samples == 0) return NSF_OK;
   const size_t n1 = static_cast<size_t>(n_clips) + 1;
   // work arena: [clip_off n1 x int64][peak n x u32]
   const size_t off_b = align_up(n1 * sizeof(int64_t));
-  if ((st = sl->pcm.reserve(samples * esz)) != NSF_OK) return st;
-  if ((st = sl->ynorm.reserve(samples * sizeof(float))) != NSF_OK) return st;
+  if ((st = sl->in[0].reserve(samples * esz)) != NSF_OK) return st;
+  if ((st = sl->out[0].reserve(samples * sizeof(float))) != NSF_OK) return st;
   if ((st = sl->work.reserve(off_b + align_up(n_clips * sizeof(uint32_t)))) != NSF_OK) return st;
   DescEntry* de = nullptr;
   if ((st = desc_acquire(ctx, n1 * sizeof(int64_t), &de)) != NSF_OK) return st;
@@ -925,16 +979,16 @@ nsf_status nsf_normalize_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_fo
   if ((st = desc_commit(de, sl->stream)) != NSF_OK) return st;
   NSF_CUDA(cudaMemsetAsync(d_peak, 0, n_clips * sizeof(uint32_t), sl->stream));
   const char* src = static_cast<const char*>(pcm_host) + clip_offsets[0] * esz;
-  NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, src, samples * esz, cudaMemcpyHostToDevice, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, src, samples * esz, cudaMemcpyHostToDevice, sl->stream));
   BatchView b{};
   b.clip_off = d_off; b.frame_off = d_off; b.row_off = d_off;
   b.n_clips = n_clips; b.total_samples = samples;
-  int n = launch_absmax(sl->stream, sl->pcm.ptr, pcm_format, b, d_peak);
+  int n = launch_absmax(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak);
   if (n < 0) { set_error(cuda_msg("launch_absmax", cudaGetLastError())); return NSF_ERR_CUDA; }
-  int m = launch_normalize(sl->stream, sl->pcm.ptr, pcm_format, b, d_peak, true, static_cast<float*>(sl->ynorm.ptr));
+  int m = launch_normalize(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak, true, static_cast<float*>(sl->out[0].ptr));
   if (m < 0) { set_error(cuda_msg("launch_normalize", cudaGetLastError())); return NSF_ERR_CUDA; }
   ctx->launches += n + m;
-  NSF_CUDA(cudaMemcpyAsync(y_host, sl->ynorm.ptr, samples * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(y_host, sl->out[0].ptr, samples * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
   if (peaks_host)  // float bits of a non-negative float: copy as-is
     NSF_CUDA(cudaMemcpyAsync(peaks_host, d_peak, n_clips * sizeof(uint32_t), cudaMemcpyDeviceToHost, sl->stream));
   NSF_CUDA(cudaStreamSynchronize(sl->stream));
@@ -1108,20 +1162,19 @@ nsf_status nsf_resample_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_for
   const int64_t n_out = nsf_resample_len(n_in, orig_sr, target_sr);
   if (out_capacity < n_out) { set_error("nsf_resample_host: out_capacity < nsf_resample_len()"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = &ctx->slot[0];
-  nsf_status st = ensure_slot(sl);
+  Slot* sl = nullptr;
+  nsf_status st = oneshot_slot(ctx, &sl);
   if (st != NSF_OK) return st;
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
   // one mono clip of the conversion kernel (float32 samples are its f32 encoding, int16 its i16 encoding)
   const nsf_pcm_source src{0, n_in, pcm_format == NSF_PCM_I16 ? NSF_ENC_I16 : NSF_ENC_F32, 1, orig_sr, 0};
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
   const int64_t off[2] = {0, n_out};
-  if ((st = sl->pcm.reserve(static_cast<size_t>(n_in) * esz)) != NSF_OK) return st;
-  if ((st = sl->ynorm.reserve(static_cast<size_t>(n_out) * sizeof(float))) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, pcm_host, static_cast<size_t>(n_in) * esz, cudaMemcpyHostToDevice, sl->stream));
-  if ((st = convert_enqueue(ctx, sl->stream, sl->pcm.ptr, &src, 1, target_sr, off, static_cast<float*>(sl->ynorm.ptr),
+  if ((st = sl->in[0].reserve(static_cast<size_t>(n_in) * esz)) != NSF_OK) return st;
+  if ((st = sl->out[0].reserve(static_cast<size_t>(n_out) * sizeof(float))) != NSF_OK) return st;
+  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, pcm_host, static_cast<size_t>(n_in) * esz, cudaMemcpyHostToDevice, sl->stream));
+  if ((st = convert_enqueue(ctx, sl->stream, sl->in[0].ptr, &src, 1, target_sr, off, static_cast<float*>(sl->out[0].ptr),
                             true)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(out_host, sl->ynorm.ptr, static_cast<size_t>(n_out) * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(out_host, sl->out[0].ptr, static_cast<size_t>(n_out) * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
   NSF_CUDA(cudaStreamSynchronize(sl->stream));
   return NSF_OK;
 }
@@ -1159,17 +1212,9 @@ nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payl
   nsf_status st = convert_offsets(sources, n, target_sr, payload_bytes, 0, all.data());
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  for (auto& sl : ctx->slot) sl.n_pending = 0;
   const bool in_dma = dma_reachable(payload_host), out_dma = dma_reachable(out_host);
-  // clip groups by output budget, rotating over the slots: the upload of group g + 1, the kernels of group g and the
-  // download of group g - 1 overlap (see nsf_extract_host)
-  int first = 0, turn = 0;
-  while (first < n) {
-    int last = first;
-    while (last < n && (last == first || all[last + 1] - all[first] <= group_budget(turn))) ++last;
-    Slot* sl = &ctx->slot[turn % kSlots];
-    if ((st = ensure_slot(sl)) != NSF_OK) return st;
-    if ((st = drain_slot(sl)) != NSF_OK) return st;
+  // clip groups by output samples
+  return run_groups(ctx, all.data(), n, [&](int first, int last, Slot* sl) -> nsf_status {
     // the group's input bytes [b0, b1), b0 rounded down to 8 so every container keeps its alignment in the arena
     int64_t b0 = INT64_MAX, b1 = 0;
     for (int i = first; i < last; ++i) {
@@ -1186,36 +1231,16 @@ nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payl
     goff.resize(last - first + 1);
     for (int i = first; i < last; ++i) { g[i - first].byte_offset = sources[i].frames > 0 ? sources[i].byte_offset - b0 : 0; }
     for (int i = first; i <= last; ++i) goff[i - first] = all[i] - all[first];
-    if ((st = sl->pcm.reserve(std::max<int64_t>(in_bytes, 1))) != NSF_OK) return st;
-    if ((st = sl->out.reserve(std::max<int64_t>(n_out, 1) * sizeof(float))) != NSF_OK) return st;
-    if (in_bytes > 0) {
-      const char* src = static_cast<const char*>(payload_host) + b0;
-      if (!in_dma) {
-        if ((st = sl->stage_in.reserve(in_bytes)) != NSF_OK) return st;
-        host_copy(sl->stage_in.ptr, src, in_bytes);
-        src = static_cast<const char*>(sl->stage_in.ptr);
-      }
-      NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, src, in_bytes, cudaMemcpyHostToDevice, sl->stream));
-    }
-    if ((st = convert_enqueue(ctx, sl->stream, sl->pcm.ptr, g.data(), last - first, target_sr, goff.data(),
-                              static_cast<float*>(sl->out.ptr), false)) != NSF_OK) return st;
-    if (n_out > 0) {
-      float* dst = out_host + all[first];
-      const size_t bytes = static_cast<size_t>(n_out) * sizeof(float);
-      if (!out_dma) {
-        if ((st = sl->stage_out.reserve(bytes)) != NSF_OK) return st;
-        NSF_CUDA(cudaMemcpyAsync(sl->stage_out.ptr, sl->out.ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
-        sl->pending[sl->n_pending++] = Slot::CopyOut{dst, sl->stage_out.ptr, bytes, 0, 0, 0, 1};
-      } else {
-        NSF_CUDA(cudaMemcpyAsync(dst, sl->out.ptr, bytes, cudaMemcpyDeviceToHost, sl->stream));
-      }
-    }
-    first = last;
-    ++turn;
-  }
-  for (auto& sl : ctx->slot)
-    if (sl.stream && (st = drain_slot(&sl)) != NSF_OK) return st;
-  return NSF_OK;
+    nsf_status st;
+    if ((st = sl->in[0].reserve(std::max<int64_t>(in_bytes, 1))) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(std::max<int64_t>(n_out, 1) * sizeof(float))) != NSF_OK) return st;
+    if (in_bytes > 0 && (st = upload(sl, 0, static_cast<const char*>(payload_host) + b0, in_bytes, in_dma)) != NSF_OK)
+      return st;
+    if ((st = convert_enqueue(ctx, sl->stream, sl->in[0].ptr, g.data(), last - first, target_sr, goff.data(),
+                              static_cast<float*>(sl->out[0].ptr), false)) != NSF_OK) return st;
+    const size_t bytes = static_cast<size_t>(n_out) * sizeof(float);
+    return n_out > 0 ? download(sl, 0, out_host + all[first], bytes, bytes, 1, out_dma) : NSF_OK;
+  });
 }
 
 // ---- collect ---------------------------------------------------------------------------------------
@@ -1253,34 +1278,14 @@ nsf_status nsf_collect_batch(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, con
                                   blend_frames, out_offsets_host, &o_off);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  const size_t n1 = static_cast<size_t>(n_clips) + 1;
-  DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, 3 * n1 * sizeof(int64_t), &de)) != NSF_OK) return st;
-  if ((st = ctx->collect_desc.reserve(3 * n1 * sizeof(int64_t))) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  const int64_t a0 = audio_offsets_host[0], f0 = facial_offsets_host[0];
-  const int64_t o0 = out_offsets_host ? out_offsets_host[0] : 0;
-  for (size_t i = 0; i < n1; ++i) {
-    h[i] = audio_offsets_host[i] - a0;
-    h[n1 + i] = facial_offsets_host[i] - f0;
-    h[2 * n1 + i] = o_off[i];
-  }
-  int64_t* d = static_cast<int64_t*>(ctx->collect_desc.ptr);
-  NSF_CUDA(cudaMemcpyAsync(d, h, 3 * n1 * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-  if ((st = desc_commit(de, s)) != NSF_OK) return st;
-  CollectView v;
-  v.a_off = d; v.f_off = d + n1; v.o_off = d + 2 * n1;
-  v.n_clips = n_clips; v.total_out_rows = o_off[n_clips]; v.flags = collect_flags; v.blend_frames = blend_frames;
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
-  const char* a = static_cast<const char*>(audio_dev) + a0 * audio_cols * esz;
-  const char* f = static_cast<const char*>(facial_dev) + f0 * facial_cols * esz;
-  char* oa = static_cast<char*>(out_audio_dev) + o0 * audio_cols * esz;
-  char* of = static_cast<char*>(out_facial_dev) + o0 * facial_cols * esz;
-  const int n = launch_collect(s, dtype, v, a, audio_cols, f, facial_cols, oa, of);
-  if (n < 0) { set_error(cuda_msg("launch_collect", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n;
-  return NSF_OK;
+  const int64_t a0 = audio_offsets_host[0], f0 = facial_offsets_host[0], o0 = out_offsets_host ? out_offsets_host[0] : 0;
+  return collect_enqueue(ctx, static_cast<cudaStream_t>(cuda_stream), dtype,
+                         static_cast<const char*>(audio_dev) + a0 * audio_cols * esz, audio_cols, audio_offsets_host,
+                         static_cast<const char*>(facial_dev) + f0 * facial_cols * esz, facial_cols, facial_offsets_host,
+                         o_off.data(), n_clips, collect_flags, blend_frames,
+                         static_cast<char*>(out_audio_dev) + o0 * audio_cols * esz,
+                         static_cast<char*>(out_facial_dev) + o0 * facial_cols * esz);
 }
 
 nsf_status nsf_collect_host(nsf_ctx* ctx, int32_t dtype, const void* audio_host, int32_t audio_cols,
@@ -1290,32 +1295,31 @@ nsf_status nsf_collect_host(nsf_ctx* ctx, int32_t dtype, const void* audio_host,
   if (!ctx || !audio_host || !facial_host || !out_audio_host || !out_facial_host) {
     set_error("nsf_collect_host: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_collect_host: bad dtype"); return NSF_ERR_BAD_ARG; }
+  if ((dtype != NSF_F32 && dtype != NSF_F64) || audio_cols <= 0 || facial_cols <= 0) {
+    set_error("nsf_collect_host: bad dtype or column count"); return NSF_ERR_BAD_ARG;
+  }
   std::vector<int64_t> o_off;
   nsf_status st = collect_offsets(a_off, f_off, n_clips, collect_flags, blend_frames, nullptr, &o_off);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = &ctx->slot[0];
-  if ((st = ensure_slot(sl)) != NSF_OK) return st;
+  Slot* sl = nullptr;
+  if ((st = oneshot_slot(ctx, &sl)) != NSF_OK) return st;
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
-  const size_t a_rows = a_off[n_clips] - a_off[0], f_rows = f_off[n_clips] - f_off[0];
-  const size_t o_rows = o_off[n_clips];
-  if ((st = ctx->collect_in_a.reserve(a_rows * audio_cols * esz)) != NSF_OK) return st;
-  if ((st = ctx->collect_in_f.reserve(f_rows * facial_cols * esz)) != NSF_OK) return st;
-  if ((st = ctx->collect_out_a.reserve(o_rows * audio_cols * esz)) != NSF_OK) return st;
-  if ((st = ctx->collect_out_f.reserve(o_rows * facial_cols * esz)) != NSF_OK) return st;
+  const size_t a_bytes = (a_off[n_clips] - a_off[0]) * audio_cols * esz, f_bytes = (f_off[n_clips] - f_off[0]) * facial_cols * esz;
+  const size_t oa_bytes = o_off[n_clips] * audio_cols * esz, of_bytes = o_off[n_clips] * facial_cols * esz;
+  if ((st = sl->in[0].reserve(a_bytes)) != NSF_OK) return st;
+  if ((st = sl->in[1].reserve(f_bytes)) != NSF_OK) return st;
+  if ((st = sl->out[0].reserve(oa_bytes)) != NSF_OK) return st;
+  if ((st = sl->out[1].reserve(of_bytes)) != NSF_OK) return st;
   const char* ah = static_cast<const char*>(audio_host) + a_off[0] * audio_cols * esz;
   const char* fh = static_cast<const char*>(facial_host) + f_off[0] * facial_cols * esz;
-  NSF_CUDA(cudaMemcpyAsync(ctx->collect_in_a.ptr, ah, a_rows * audio_cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  NSF_CUDA(cudaMemcpyAsync(ctx->collect_in_f.ptr, fh, f_rows * facial_cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  std::vector<int64_t> a_rel(n_clips + 1), f_rel(n_clips + 1);
-  for (int i = 0; i <= n_clips; ++i) { a_rel[i] = a_off[i] - a_off[0]; f_rel[i] = f_off[i] - f_off[0]; }
-  st = nsf_collect_batch(ctx, sl->stream, dtype, ctx->collect_in_a.ptr, audio_cols, a_rel.data(),
-                         ctx->collect_in_f.ptr, facial_cols, f_rel.data(), n_clips, collect_flags,
-                         blend_frames, ctx->collect_out_a.ptr, ctx->collect_out_f.ptr, nullptr);
-  if (st != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(out_audio_host, ctx->collect_out_a.ptr, o_rows * audio_cols * esz, cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaMemcpyAsync(out_facial_host, ctx->collect_out_f.ptr, o_rows * facial_cols * esz, cudaMemcpyDeviceToHost, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, ah, a_bytes, cudaMemcpyHostToDevice, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(sl->in[1].ptr, fh, f_bytes, cudaMemcpyHostToDevice, sl->stream));
+  if ((st = collect_enqueue(ctx, sl->stream, dtype, sl->in[0].ptr, audio_cols, a_off, sl->in[1].ptr, facial_cols, f_off,
+                            o_off.data(), n_clips, collect_flags, blend_frames, sl->out[0].ptr, sl->out[1].ptr)) != NSF_OK)
+    return st;
+  NSF_CUDA(cudaMemcpyAsync(out_audio_host, sl->out[0].ptr, oa_bytes, cudaMemcpyDeviceToHost, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(out_facial_host, sl->out[1].ptr, of_bytes, cudaMemcpyDeviceToHost, sl->stream));
   NSF_CUDA(cudaStreamSynchronize(sl->stream));
   return NSF_OK;
 }
@@ -1337,104 +1341,39 @@ nsf_status nsf_extract_collect_host(nsf_ctx* ctx, const void* pcm_host, int32_t 
   nsf_status st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all);
   if (st != NSF_OK) return st;
   // output packing over the whole batch (validates the facial offsets)
-  std::vector<int64_t> a_rows(n_clips + 1), o_all;
-  for (int i = 0; i <= n_clips; ++i) a_rows[i] = all.row_off[i];
-  if ((st = collect_offsets(a_rows.data(), f_off, n_clips, collect_flags, blend_frames, nullptr, &o_all)) != NSF_OK) return st;
+  std::vector<int64_t> o_all;
+  if ((st = collect_offsets(all.row_off.data(), f_off, n_clips, collect_flags, blend_frames, nullptr, &o_all)) != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  for (auto& sl : ctx->slot) sl.n_pending = 0;
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
-  // pageable caller buffers are staged through the slot's pinned arenas (see nsf_extract_host)
+  const size_t row_bytes = static_cast<size_t>(cols) * sizeof(float), fac_row_bytes = static_cast<size_t>(facial_cols) * sizeof(float);
   const bool pcm_dma = dma_reachable(pcm_host), fac_dma = dma_reachable(facial_host);
   const bool oa_dma = dma_reachable(out_audio_host), of_dma = dma_reachable(out_facial_host);
   const bool ft_dma = features_host ? dma_reachable(features_host) : true;
-  int first = 0, turn = 0;
-  while (first < n_clips) {
-    int last = first;
-    int64_t samples = 0;
-    while (last < n_clips && (last == first || samples + (clip_offsets[last + 1] - clip_offsets[last]) <= group_budget(turn))) {
-      samples += clip_offsets[last + 1] - clip_offsets[last];
-      ++last;
-    }
-    const int gn = last - first;
-    Slot* sl = &ctx->slot[turn % kSlots];
-    if ((st = ensure_slot(sl)) != NSF_OK) return st;
-    if ((st = drain_slot(sl)) != NSF_OK) return st;   // the slot's previous group has fully drained
+  // device: in = [PCM, facial rows], out = [feature rows, collected audio rows, collected facial rows]
+  return run_groups(ctx, clip_offsets, n_clips, [&](int first, int last, Slot* sl) -> nsf_status {
+    const int64_t samples = clip_offsets[last] - clip_offsets[first];
     const int64_t rows = all.row_off[last] - all.row_off[first];
-    const int64_t frows = f_off[last] - f_off[first];
-    const int64_t orows = o_all[last] - o_all[first];
-    const int64_t wbytes = nsf_workspace_bytes(ctx->plan, samples, gn, flags);
-    const size_t n1 = static_cast<size_t>(gn) + 1;
-    if ((st = sl->pcm.reserve(samples * esz)) != NSF_OK) return st;
-    if ((st = sl->out.reserve(static_cast<size_t>(rows) * cols * sizeof(float))) != NSF_OK) return st;
-    if ((st = sl->work.reserve(wbytes)) != NSF_OK) return st;
-    if ((st = sl->fac_in.reserve(static_cast<size_t>(frows) * facial_cols * sizeof(float))) != NSF_OK) return st;
-    if ((st = sl->col_a.reserve(static_cast<size_t>(orows) * cols * sizeof(float))) != NSF_OK) return st;
-    if ((st = sl->col_f.reserve(static_cast<size_t>(orows) * facial_cols * sizeof(float))) != NSF_OK) return st;
-    if ((st = sl->col_desc.reserve(3 * n1 * sizeof(int64_t))) != NSF_OK) return st;
-    const char* src = static_cast<const char*>(pcm_host) + clip_offsets[first] * esz;
-    if (!pcm_dma) {
-      if ((st = sl->stage_in.reserve(samples * esz)) != NSF_OK) return st;
-      host_copy(sl->stage_in.ptr, src, samples * esz);
-      src = static_cast<const char*>(sl->stage_in.ptr);
-    }
-    NSF_CUDA(cudaMemcpyAsync(sl->pcm.ptr, src, samples * esz, cudaMemcpyHostToDevice, sl->stream));
-    const size_t fac_bytes = static_cast<size_t>(frows) * facial_cols * sizeof(float);
-    const float* fsrc = facial_host + f_off[first] * facial_cols;
-    if (!fac_dma) {
-      if ((st = sl->stage_fac.reserve(fac_bytes)) != NSF_OK) return st;
-      host_copy(sl->stage_fac.ptr, fsrc, fac_bytes);
-      fsrc = static_cast<const float*>(sl->stage_fac.ptr);
-    }
-    NSF_CUDA(cudaMemcpyAsync(sl->fac_in.ptr, fsrc, fac_bytes, cudaMemcpyHostToDevice, sl->stream));
-    // collect descriptors of this group (relative offsets) through the guarded pinned staging buffer.  Staged
-    // BEFORE the extraction kernels are enqueued: the next wait on the staging buffer then ends as soon as this
-    // group's uploads have run, so the host can start the next group's upload while these kernels execute
-    DescEntry* de = nullptr;
-    if ((st = desc_acquire(ctx, 3 * n1 * sizeof(int64_t), &de)) != NSF_OK) return st;
-    int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-    for (size_t i = 0; i < n1; ++i) {
-      h[i] = all.row_off[first + i] - all.row_off[first];
-      h[n1 + i] = f_off[first + i] - f_off[first];
-      h[2 * n1 + i] = o_all[first + i] - o_all[first];
-    }
-    int64_t* d = static_cast<int64_t*>(sl->col_desc.ptr);
-    NSF_CUDA(cudaMemcpyAsync(d, h, 3 * n1 * sizeof(int64_t), cudaMemcpyHostToDevice, sl->stream));
-    if ((st = desc_commit(de, sl->stream)) != NSF_OK) return st;
-    ctx->pipelined = true;
-    st = nsf_extract_batch(ctx, sl->stream, sl->pcm.ptr, pcm_format, clip_offsets + first, gn, flags,
-                           static_cast<float*>(sl->out.ptr), cols, nullptr, nullptr, sl->work.ptr,
-                           static_cast<int64_t>(sl->work.bytes));
-    ctx->pipelined = false;
-    if (st != NSF_OK) return st;
-    CollectView v;
-    v.a_off = d; v.f_off = d + n1; v.o_off = d + 2 * n1;
-    v.n_clips = gn; v.total_out_rows = orows; v.flags = collect_flags; v.blend_frames = blend_frames;
-    const int n = launch_collect(sl->stream, NSF_F32, v, sl->out.ptr, cols, sl->fac_in.ptr, facial_cols, sl->col_a.ptr,
-                                 sl->col_f.ptr);
-    if (n < 0) { set_error(cuda_msg("launch_collect", cudaGetLastError())); return NSF_ERR_CUDA; }
-    ctx->launches += n;
-    // downloads: straight into page-locked caller memory, else through a pinned stage + host copy at drain time
-    auto download = [&](void* dst, const void* dev, size_t bytes, bool dma, PinnedArena* stage) -> nsf_status {
-      if (dma) { NSF_CUDA(cudaMemcpyAsync(dst, dev, bytes, cudaMemcpyDeviceToHost, sl->stream)); return NSF_OK; }
-      const nsf_status r = stage->reserve(bytes);
-      if (r != NSF_OK) return r;
-      NSF_CUDA(cudaMemcpyAsync(stage->ptr, dev, bytes, cudaMemcpyDeviceToHost, sl->stream));
-      sl->pending[sl->n_pending++] = Slot::CopyOut{dst, stage->ptr, bytes, 0, 0, 0, 1};
-      return NSF_OK;
-    };
+    const int64_t frows = f_off[last] - f_off[first], orows = o_all[last] - o_all[first];
+    nsf_status st;
+    if ((st = sl->in[0].reserve(samples * esz)) != NSF_OK) return st;
+    if ((st = sl->in[1].reserve(frows * fac_row_bytes)) != NSF_OK) return st;
+    if ((st = sl->work.reserve(nsf_workspace_bytes(ctx->plan, samples, last - first, flags))) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(rows * row_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[1].reserve(orows * row_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[2].reserve(orows * fac_row_bytes)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, static_cast<const char*>(pcm_host) + clip_offsets[first] * esz, samples * esz, pcm_dma)) != NSF_OK)
+      return st;
+    if ((st = upload(sl, 1, facial_host + f_off[first] * facial_cols, frows * fac_row_bytes, fac_dma)) != NSF_OK) return st;
+    if ((st = extract_group(ctx, sl, pcm_format, clip_offsets + first, last - first, flags, cols, nullptr)) != NSF_OK) return st;
+    if ((st = collect_enqueue(ctx, sl->stream, NSF_F32, sl->out[0].ptr, cols, all.row_off.data() + first, sl->in[1].ptr,
+                              facial_cols, f_off + first, o_all.data() + first, last - first, collect_flags, blend_frames,
+                              sl->out[1].ptr, sl->out[2].ptr)) != NSF_OK) return st;
     if (features_host &&   // the un-augmented rows as well (what collect_features caches as audio_features.csv)
-        (st = download(features_host + all.row_off[first] * cols, sl->out.ptr,
-                       static_cast<size_t>(rows) * cols * sizeof(float), ft_dma, &sl->stage_feat)) != NSF_OK) return st;
-    if ((st = download(out_audio_host + o_all[first] * cols, sl->col_a.ptr,
-                       static_cast<size_t>(orows) * cols * sizeof(float), oa_dma, &sl->stage_out)) != NSF_OK) return st;
-    if ((st = download(out_facial_host + o_all[first] * facial_cols, sl->col_f.ptr,
-                       static_cast<size_t>(orows) * facial_cols * sizeof(float), of_dma, &sl->stage_aux)) != NSF_OK) return st;
-    first = last;
-    ++turn;
-  }
-  for (auto& sl : ctx->slot)
-    if (sl.stream && (st = drain_slot(&sl)) != NSF_OK) return st;
-  return NSF_OK;
+        (st = download(sl, 0, features_host + all.row_off[first] * cols, row_bytes, row_bytes, rows, ft_dma)) != NSF_OK)
+      return st;
+    if ((st = download(sl, 1, out_audio_host + o_all[first] * cols, row_bytes, row_bytes, orows, oa_dma)) != NSF_OK) return st;
+    return download(sl, 2, out_facial_host + o_all[first] * facial_cols, fac_row_bytes, fac_row_bytes, orows, of_dma);
+  });
 }
 
 // ---- inference-side chunker ---------------------------------------------------------------------------
@@ -1589,21 +1528,21 @@ nsf_status nsf_rows_host(nsf_ctx* ctx, int32_t op, int32_t dtype, const void* a_
     out_rows = na + nb - k;
   } else { set_error("nsf_rows_host: unknown op"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = &ctx->slot[0];
-  nsf_status st = ensure_slot(sl);
+  Slot* sl = nullptr;
+  nsf_status st = oneshot_slot(ctx, &sl);
   if (st != NSF_OK) return st;
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
   const bool two = op == NSF_ROWS_BLEND_STACK;
-  if ((st = ctx->collect_in_a.reserve(na * cols * esz)) != NSF_OK) return st;
-  if (two && (st = ctx->collect_in_f.reserve(nb * cols * esz)) != NSF_OK) return st;
-  if ((st = ctx->collect_out_a.reserve(out_rows * cols * esz)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(ctx->collect_in_a.ptr, a_host, na * cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  if (two) NSF_CUDA(cudaMemcpyAsync(ctx->collect_in_f.ptr, b_host, nb * cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  const int n = launch_rows_op(sl->stream, op, dtype, ctx->collect_in_a.ptr, na, two ? ctx->collect_in_f.ptr : nullptr,
-                               nb, cols, k, ctx->collect_out_a.ptr, out_rows);
+  if ((st = sl->in[0].reserve(na * cols * esz)) != NSF_OK) return st;
+  if (two && (st = sl->in[1].reserve(nb * cols * esz)) != NSF_OK) return st;
+  if ((st = sl->out[0].reserve(out_rows * cols * esz)) != NSF_OK) return st;
+  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, a_host, na * cols * esz, cudaMemcpyHostToDevice, sl->stream));
+  if (two) NSF_CUDA(cudaMemcpyAsync(sl->in[1].ptr, b_host, nb * cols * esz, cudaMemcpyHostToDevice, sl->stream));
+  const int n = launch_rows_op(sl->stream, op, dtype, sl->in[0].ptr, na, two ? sl->in[1].ptr : nullptr,
+                               nb, cols, k, sl->out[0].ptr, out_rows);
   if (n < 0) { set_error(cuda_msg("launch_rows_op", cudaGetLastError())); return NSF_ERR_CUDA; }
   ctx->launches += n;
-  NSF_CUDA(cudaMemcpyAsync(out_host, ctx->collect_out_a.ptr, out_rows * cols * esz, cudaMemcpyDeviceToHost, sl->stream));
+  NSF_CUDA(cudaMemcpyAsync(out_host, sl->out[0].ptr, out_rows * cols * esz, cudaMemcpyDeviceToHost, sl->stream));
   NSF_CUDA(cudaStreamSynchronize(sl->stream));
   return NSF_OK;
 }
@@ -1613,8 +1552,8 @@ nsf_status nsf_post_host(nsf_ctx* ctx, const float* in_host, int64_t T, int32_t 
   if ((pf & NSF_POST_DELTAS) && T < 9) { set_error("nsf_post_host: delta needs at least 9 frames"); return NSF_ERR_TOO_SHORT; }
   if ((pf & NSF_POST_EDGEFIX) && T < 2) { set_error("nsf_post_host: edge fix needs 2 frames"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = &ctx->slot[0];
-  nsf_status st = ensure_slot(sl);
+  Slot* sl = nullptr;
+  nsf_status st = oneshot_slot(ctx, &sl);
   if (st != NSF_OK) return st;
   const bool reduce = (pf & NSF_POST_REDUCE) != 0, deltas = (pf & NSF_POST_DELTAS) != 0, cmvn = (pf & NSF_POST_CMVN) != 0;
   const int64_t rows = reduce ? (T + 1) / 2 : T;
@@ -1622,8 +1561,8 @@ nsf_status nsf_post_host(nsf_ctx* ctx, const float* in_host, int64_t T, int32_t 
   // device layout: [in T*C floats][out rows*out_c floats][desc 6 x int64][sum C][sumsq C]
   const size_t in_b = align_up(T * Cc * sizeof(float)), out_b = align_up(rows * out_c * sizeof(float));
   const size_t desc_b = align_up(6 * sizeof(int64_t)), st_b = align_up(Cc * sizeof(double));
-  if ((st = ctx->collect_in_a.reserve(in_b + out_b + desc_b + 2 * st_b)) != NSF_OK) return st;
-  char* base = static_cast<char*>(ctx->collect_in_a.ptr);
+  if ((st = sl->work.reserve(in_b + out_b + desc_b + 2 * st_b)) != NSF_OK) return st;
+  char* base = static_cast<char*>(sl->work.ptr);
   float* d_in = reinterpret_cast<float*>(base);
   float* d_out = reinterpret_cast<float*>(base + in_b);
   int64_t* d_desc = reinterpret_cast<int64_t*>(base + in_b + out_b);

@@ -220,17 +220,15 @@ class Engine:
         "hq" = band-limited windowed sinc (64 zero crossings, Kaiser beta 14.77; torchaudio's
         sinc_interp_kaiser arithmetic, the class of the reference's soxr_hq), "poly" = the
         scipy.signal.resample_poly design (see include/nsf.h)."""
-        q = {"hq": nv.RESAMPLE_HQ, "poly": nv.RESAMPLE_POLY}[quality]
-        nv.check(nv.lib.nsf_ctx_set_option(self.handle, nv.OPT_RESAMPLE_QUALITY, float(q)))
         pcm = np.ascontiguousarray(pcm)
         fmt = self._pcm_format(pcm)
         n_out = int(nv.lib.nsf_resample_len(len(pcm), int(orig_sr), int(target_sr)))
         out = np.empty(n_out, dtype=np.float32)
-        if n_out == 0:
-            return out
         with self._lock:
-            nv.check(nv.lib.nsf_resample_host(self.handle, nv.ptr(pcm), fmt, len(pcm), int(orig_sr),
-                                              int(target_sr), nv.ptr(out), n_out))
+            self._set_quality(quality)
+            if n_out > 0:
+                nv.check(nv.lib.nsf_resample_host(self.handle, nv.ptr(pcm), fmt, len(pcm), int(orig_sr),
+                                                  int(target_sr), nv.ptr(out), n_out))
         return out
 
     def _set_quality(self, quality):
@@ -446,10 +444,7 @@ class Engine:
         f_off, f_p = nv.i64_array(facial_offsets)
         n = len(a_off) - 1
         flags = self.collect_flags(include_fast, include_slow, blend_boundaries)
-        rows = [nv.lib.nsf_collect_rows(int(a_off[i + 1] - a_off[i]), int(f_off[i + 1] - f_off[i]), flags,
-                                        int(blend_frames)) for i in range(n)]
-        o_off = np.zeros(n + 1, dtype=np.int64)
-        np.cumsum(rows, out=o_off[1:])
+        o_off = self.collect_rows(a_off, f_off, include_fast, include_slow, blend_boundaries, blend_frames)
         out_a = np.empty((int(o_off[-1]), audio.shape[1]), dtype=audio.dtype)
         out_f = np.empty((int(o_off[-1]), facial.shape[1]), dtype=audio.dtype)
         with self._lock:
