@@ -16,13 +16,15 @@ float32 anyway).  ``process_folder`` / ``collect_features`` remain the
 per-take float64 route, bit-identical to the reference's NumPy arithmetic.
 """
 import os
+from collections import namedtuple
 
 import numpy as np
 import pandas as pd
 
 from .. import _native as nv
 from .. import engine as _engine
-from ..utils.audio.extraction.extract_features import extract_audio_features
+from ..utils.audio.extraction.extract_features import MIN_FRAMES, extract_audio_features
+from ..utils.audio.load_audio import REFERENCE_RATE, WAV_ENCODINGS, wav_layout
 from ..utils.video.mov_extraction import find_files, get_audio
 
 COLUMNS_TO_DROP = ['Timecode', 'BlendshapeCount']
@@ -112,8 +114,39 @@ def collect_arrays(audio_features, facial_data, include_fast=True, include_slow=
     return out_a, out_f
 
 
+def _cache_format(cache_format):
+    """``cache_format``, else ``NSF_FEATURE_CACHE``, else "csv"; validated."""
+    cache_format = cache_format or os.environ.get("NSF_FEATURE_CACHE", "csv")
+    if cache_format not in ("csv", "npy", "both"):
+        raise ValueError("cache_format must be 'csv', 'npy' or 'both'")
+    return cache_format
+
+
 def _binary_cache_path(audio_features_csv_path):
     return os.path.splitext(audio_features_csv_path)[0] + ".npy"
+
+
+def _cached_features_path(cache_csv, cache_format):
+    """The feature cache to read (:112-114): the CSV if it exists, else the ``.npy`` unless the format is "csv"."""
+    if os.path.exists(cache_csv):
+        return cache_csv
+    npy_path = _binary_cache_path(cache_csv)
+    return npy_path if cache_format != "csv" and os.path.exists(npy_path) else None
+
+
+def _read_feature_cache(path):
+    return np.load(path) if path.endswith(".npy") else pd.read_csv(path).values
+
+
+def _write_feature_cache(cache_csv, rows, cache_format):
+    """The cache files of one take's feature rows (:115-120): the CSV from float64, the ``.npy`` from float32."""
+    if cache_format in ("csv", "both"):
+        pd.DataFrame(np.asarray(rows, dtype=np.float64)).to_csv(cache_csv, index=False)
+        print(f"Audio features saved to {cache_csv}")
+    if cache_format in ("npy", "both"):
+        npy_path = _binary_cache_path(cache_csv)
+        np.save(npy_path, np.asarray(rows, dtype=np.float32))
+        print(f"Audio features saved to {npy_path}")
 
 
 def collect_features(audio_path, audio_features_csv_path, facial_csv_path, sr,
@@ -125,26 +158,16 @@ def collect_features(audio_path, audio_features_csv_path, facial_csv_path, sr,
     "csv" = the reference's ``audio_features.csv`` (1.3 s and 9 MB per 30 s clip to write);
     "npy" = a float32 ``audio_features.npy`` beside it (milliseconds, 1.8 MB); "both" writes both.
     An existing CSV cache is always honoured first, exactly like the reference."""
-    cache_format = cache_format or os.environ.get("NSF_FEATURE_CACHE", "csv")
-    if cache_format not in ("csv", "npy", "both"):
-        raise ValueError("cache_format must be 'csv', 'npy' or 'both'")
-    npy_path = _binary_cache_path(audio_features_csv_path)
-    if os.path.exists(audio_features_csv_path):                           # :112-114
-        print(f"Loading audio features from {audio_features_csv_path}")
-        audio_features = pd.read_csv(audio_features_csv_path).values
-    elif cache_format != "csv" and os.path.exists(npy_path):
-        print(f"Loading audio features from {npy_path}")
-        audio_features = np.load(npy_path).astype(np.float64)
+    cache_format = _cache_format(cache_format)
+    cache_path = _cached_features_path(audio_features_csv_path, cache_format)
+    if cache_path:
+        print(f"Loading audio features from {cache_path}")
+        audio_features = np.asarray(_read_feature_cache(cache_path), dtype=np.float64)
     else:                                                                 # :115-120
         print(f"Extracting audio features from {audio_path}")
         audio_features, _ = extract_audio_features(audio_path, sr)
         if audio_features is not None:
-            if cache_format in ("csv", "both"):
-                pd.DataFrame(audio_features).to_csv(audio_features_csv_path, index=False)
-                print(f"Audio features saved to {audio_features_csv_path}")
-            if cache_format in ("npy", "both"):
-                np.save(npy_path, audio_features.astype(np.float32))
-                print(f"Audio features saved to {npy_path}")
+            _write_feature_cache(audio_features_csv_path, audio_features, cache_format)
     facial_data = pd.read_csv(facial_csv_path).drop(columns=COLUMNS_TO_DROP).values   # :123
     if audio_features is None:
         # the reference fails here with TypeError: object of type 'NoneType' has no len() (:143)
@@ -213,75 +236,51 @@ def collect_batch(audio_rows, facial_rows, include_fast=True, include_slow=False
                             blend_frames)
 
 
-def _pcm16_payload(path, sr):
-    """(byte offset, sample count) of the data chunk when ``path`` is a mono PCM16 RIFF/WAVE file at ``sr`` -
-    the format ffmpeg writes for the takes (utils/video/mov_extraction.py:50-57) - else None."""
-    import struct
-    try:
-        with open(path, "rb") as fh:
-            head = fh.read(12)
-            if len(head) < 12 or head[:4] != b"RIFF" or head[8:12] != b"WAVE":
-                return None
-            fmt, pos = None, 12
-            while True:
-                hdr = fh.read(8)
-                if len(hdr) < 8:
-                    return None
-                tag, size = hdr[:4], struct.unpack("<I", hdr[4:])[0]
-                if tag == b"fmt ":
-                    fmt = struct.unpack("<HHIIHH", fh.read(16))
-                    fh.seek(pos + 8 + size + (size & 1))
-                elif tag == b"data":
-                    if fmt is None or fmt[0] != 1 or fmt[1] != 1 or fmt[5] != 16 or fmt[2] != sr:
-                        return None
-                    avail = os.path.getsize(path) - (pos + 8)
-                    return pos + 8, min(size, max(avail, 0)) // 2
-                else:
-                    fh.seek(pos + 8 + size + (size & 1))
-                pos += 8 + size + (size & 1)
-    except OSError:
-        return None
+def _prefix(lengths):
+    """``[0, l0, l0 + l1, ...]`` as int64 offsets."""
+    off = np.zeros(len(lengths) + 1, dtype=np.int64)
+    np.cumsum(lengths, out=off[1:])
+    return off
 
 
-_WAV_ENCODINGS = {(1, 8): nv.ENC_U8, (1, 16): nv.ENC_I16, (1, 24): nv.ENC_I24, (1, 32): nv.ENC_I32,
-                  (3, 32): nv.ENC_F32, (3, 64): nv.ENC_F64}
 _ENC_BYTES = {nv.ENC_U8: 1, nv.ENC_I16: 2, nv.ENC_I24: 3, nv.ENC_I32: 4, nv.ENC_F32: 4, nv.ENC_F64: 8}
 
 
 def _wav_source(path):
-    """(data offset, data bytes, encoding, channels, rate) of a RIFF/WAVE file, read from its headers only.
-
-    The chunk walk of ``decode_wav`` (utils/audio/load_audio.py), step for step: WAVE_FORMAT_EXTENSIBLE takes its
-    format tag from the sub-format GUID, odd-sized chunks are padded, the first ``data`` chunk ends the walk and is
-    truncated at the end of the file.  Raises ``decode_wav``'s ``ValueError`` for what ``decode_wav`` rejects.  A
-    header declaring 0 channels (which ``decode_wav`` reads as mono) reports 1."""
-    import struct
-    size_all = os.path.getsize(path)
+    """(data offset, data bytes, encoding, declared channels, rate) of a WAV file, from its headers only
+    (``wav_layout``: ``decode_wav``'s chunk walk and its ``ValueError`` for what it cannot decode)."""
     with open(path, "rb") as fh:
-        head = fh.read(12)
-        if len(head) < 12 or head[:4] != b"RIFF" or head[8:12] != b"WAVE":
-            raise ValueError("not a RIFF/WAVE stream (only WAV decoding is built in)")
-        pos, fmt, data = 12, None, None
-        while pos + 8 <= size_all:
-            fh.seek(pos)
-            hdr = fh.read(8)
-            tag, size = hdr[:4], struct.unpack_from("<I", hdr, 4)[0]
-            if tag == b"fmt ":
-                body = fh.read(size)
-                fmt = struct.unpack_from("<HHIIHH", body, 0)
-                if fmt[0] == 0xFFFE and len(body) >= 26:
-                    fmt = (struct.unpack_from("<H", body, 24)[0],) + fmt[1:]
-            elif tag == b"data":
-                data = (pos + 8, min(size, size_all - (pos + 8)))
-                break
-            pos += 8 + size + (size & 1)
-    if fmt is None or data is None:
-        raise ValueError("WAV stream lacks a fmt or data chunk")
-    code, channels, rate, _, _, bits = fmt
-    enc = _WAV_ENCODINGS.get((code, bits))
-    if enc is None:
-        raise ValueError(f"unsupported WAV encoding (format {code}, {bits} bit)")
-    return data[0], data[1], enc, max(int(channels), 1), int(rate)
+        h = wav_layout(fh)
+    return h.data_offset, h.data_bytes, WAV_ENCODINGS[h.tag, h.bits], h.channels, h.rate
+
+
+# sources: nv.PCM_SOURCE per take, offsets into the read arena of nbytes bytes; lengths: samples at 88.2 kHz;
+# rate: the first conversion's target; mid: the second conversion's sources (float32 at rate), None at 88.2 kHz
+_AudioPlan = namedtuple("_AudioPlan", "int16 sources lengths nbytes rate mid")
+
+
+def _plan_audio(heads, sr):
+    """How takes with these WAV headers become ``decode_for_path``'s PCM at 88.2 kHz; host only.  The int16 route,
+    when ``sr`` and every take are mono PCM16 at 88.2 kHz (what ffmpeg writes, mov_extraction.py:50-57): the data
+    chunks are read back to back and are the samples.  Else each is read 8-byte aligned and ``nsf_convert_host``
+    converts it to ``sr`` (88.2 kHz if None: decode() keeps the native rate), then to 88.2 kHz (load_audio.py:8-10)."""
+    int16 = sr == REFERENCE_RATE and all(h[2:] == (nv.ENC_I16, 1, REFERENCE_RATE) for h in heads)
+    sources = np.zeros(len(heads), dtype=nv.PCM_SOURCE)
+    pos = 0
+    for k, (_, nbytes, enc, channels, native) in enumerate(heads):
+        channels = max(channels, 1)                                 # decode_wav reads 0 declared channels as mono
+        frames = nbytes // (_ENC_BYTES[enc] * channels)
+        sources[k] = (pos, frames, enc, channels, native, 0)
+        pos += frames * _ENC_BYTES[enc] * channels
+        if not int16:
+            pos += -pos % 8                                         # converted takes start 8-byte aligned
+    rate = sr if sr is not None else REFERENCE_RATE
+    off = nv.convert_offsets(sources, rate, pos)
+    mid = None
+    if rate != REFERENCE_RATE:
+        mid = nv.pcm_sources([(int(a) * 4, int(b - a), nv.ENC_F32, 1, rate) for a, b in zip(off[:-1], off[1:])])
+        off = nv.convert_offsets(mid, REFERENCE_RATE, int(off[-1]) * 4)
+    return _AudioPlan(int16, sources, np.diff(off), pos, rate, mid)
 
 
 def _read_into(path, offset, dst):
@@ -315,6 +314,155 @@ def _facial_rows(path, dtype):
     return np.ascontiguousarray(pd.read_csv(path).drop(columns=COLUMNS_TO_DROP).values, dtype=dtype)
 
 
+_Take = namedtuple("_Take", "folder video wav cache_csv facial_csv path")
+
+
+def _scan(root_dir, processed_folders, cache_format):
+    """The takes ``process_folder`` would not skip (:72-79), in ``os.listdir`` order, minus ``processed_folders``."""
+    takes = []
+    for folder in os.listdir(root_dir):
+        path = os.path.join(root_dir, folder)
+        if not os.path.isdir(path) or folder in processed_folders:
+            continue
+        mov, mp4, wav, facial_csv, cache_csv, _ = find_files(path)
+        video = mov or mp4
+        if facial_csv and (video or wav or _cached_features_path(cache_csv, cache_format)):
+            takes.append(_Take(folder, video, wav, cache_csv, facial_csv, path))
+    return takes
+
+
+def _partition(takes, rank, world):
+    """This rank's take indices.  The partition weighs files every rank sees identically BEFORE any rank extracts
+    audio (never on audio.wav, which another rank may be writing): the take's video, else its wav, else its cache."""
+    if world <= 1:
+        return list(range(len(takes)))
+    from .. import shard
+
+    def weight(t):
+        for cand in (t.video, t.wav, t.cache_csv):
+            if cand and os.path.exists(cand):
+                return max(1, os.path.getsize(cand))
+        return 1
+    return shard.lpt_partition([weight(t) for t in takes], world)[rank]
+
+
+def _classify(takes, mine, cache_format, pool):
+    """``(loaded, extract)``: take -> pool job loading its feature cache, and take -> the audio file to extract
+    (``get_audio`` may run ffmpeg).  A take with neither is dropped, as ``process_folder`` returns (None, None)."""
+    loaded, extract = {}, {}
+    for i in mine:
+        t = takes[i]
+        cache_path = _cached_features_path(t.cache_csv, cache_format)
+        if cache_path:
+            print(f"Loading audio features from {cache_path}")
+            loaded[i] = pool.submit(_read_feature_cache, cache_path)
+            continue
+        audio_path = get_audio(t.video, t.wav, t.path) if (t.video or t.wav) else None
+        if audio_path:
+            print(f"Extracting audio features from {audio_path}")
+            extract[i] = audio_path
+    return loaded, extract
+
+
+def _read_audio(eng, pool, paths, sr, then):
+    """``(pcm, offsets, then())``: the WAV files ``paths`` as packed PCM at 88.2 kHz (``_plan_audio``), int16 or float32
+    in library-owned page-locked memory.  Headers, then data chunks are read on ``pool``; ``then()`` runs once the
+    reads are queued, so what it submits runs behind them.  A take under 9 frames raises ``TypeError`` (:143)."""
+    if not paths:
+        return None, None, then()
+    heads = list(pool.map(_wav_source, paths))
+    plan = _plan_audio(heads, sr)
+    loaded = [f"Loaded audio file '{p}' with sample rate {sr if sr is not None else h[4]}"
+              for p, h in zip(paths, heads)]
+    if not plan.int16:                          # the int16 route announces its takes after the length check
+        print(*loaded, sep="\n")
+    for n in plan.lengths:
+        frames = eng.plan.guard_frames(n)
+        if frames < MIN_FRAMES:                                            # extract_features.py:16-20 -> :143
+            print(f"Audio file is too short: {frames} frames, required: {MIN_FRAMES} frames")
+            raise TypeError("object of type 'NoneType' has no len()")
+    if plan.int16:
+        print(*loaded, sep="\n")
+    off = _prefix(plan.lengths)
+    sample = np.dtype(np.int16 if plan.int16 else np.float32)
+    pcm = _engine.scratch_pinned("dataset_pcm", int(off[-1]) * sample.itemsize).view(sample, (int(off[-1]),))
+    dst = pcm.view(np.uint8) if plan.int16 else \
+        _engine.scratch_pinned("dataset_wav", max(plan.nbytes, 1)).view(np.uint8, (plan.nbytes,))
+    reads = [pool.submit(_read_into, p, h[0], dst[s["byte_offset"]:][:s["frames"] * s["channels"] * _ENC_BYTES[h[2]]])
+             for p, h, s in zip(paths, heads, plan.sources)]
+    queued = then()
+    for r in reads:
+        r.result()
+    if plan.mid is not None:
+        n_mid = int(plan.mid["frames"].sum())
+        y_mid = _engine.scratch_pinned("dataset_wav_mid", max(n_mid * 4, 1)).view(np.float32, (n_mid,))
+        eng.convert_host(dst, plan.sources, plan.rate, out=y_mid)
+        eng.convert_host(y_mid.view(np.uint8), plan.mid, REFERENCE_RATE, out=pcm)
+    elif not plan.int16:
+        eng.convert_host(dst, plan.sources, plan.rate, out=pcm)
+    return pcm, off, queued
+
+
+def _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw):
+    """``(results, features)``: take -> augmented (audio, facial) rows, for the takes ``extract`` (PCM ``pcm`` at
+    ``off``) and those with ``loaded`` rows; take -> feature rows extracted.  float32 with augmentation fuses
+    extraction and augmentation in one ``nsf_extract_collect_host`` call; otherwise the extracted rows join the
+    loaded ones in the collect pass."""
+    results, features, rows = {}, {}, dict(loaded)
+    augment = kw["include_fast"] or kw["include_slow"]
+    if extract:
+        roff = eng.row_offsets(off)
+        f_off = _prefix([len(facial[i]) for i in extract])
+        if dtype == np.float32 and augment and all(roff[k + 1] > roff[k] and len(facial[i])
+                                                   for k, i in enumerate(extract)):
+            f_cols = facial[extract[0]].shape[1]
+            fac = _engine.scratch_pinned("dataset_facial", int(f_off[-1]) * f_cols * 4).view(
+                np.float32, (int(f_off[-1]), f_cols))
+            np.concatenate([facial[i] for i in extract], out=fac)
+            o_off = eng.collect_rows(roff, f_off, **kw)
+            # results go to ordinary (pageable) arrays the caller owns: the library stages the downloads through
+            # its own page-locked arenas, which costs a host copy but not a cudaHostAlloc of ~300 MB per call
+            out_a = np.empty((int(o_off[-1]), 256), dtype=np.float32)
+            out_f = np.empty((int(o_off[-1]), f_cols), dtype=np.float32)
+            feats = np.empty((int(roff[-1]), 256), dtype=np.float32)
+            eng.extract_collect_host(pcm, off, fac, f_off, nv.PEAK_NORMALIZE, out_audio=out_a, out_facial=out_f,
+                                     features_out=feats, **kw)
+            for k, i in enumerate(extract):
+                results[i] = (out_a[o_off[k]:o_off[k + 1]], out_f[o_off[k]:o_off[k + 1]])
+                features[i] = feats[roff[k]:roff[k + 1]]
+        else:
+            feats = eng.extract_host(pcm, off, nv.PEAK_NORMALIZE)
+            for k, i in enumerate(extract):
+                features[i] = rows[i] = feats[roff[k]:roff[k + 1]]
+    if rows:
+        order = sorted(rows)
+        rows_in = [np.ascontiguousarray(rows[i], dtype=dtype) for i in order]
+        if augment and all(len(r) for r in rows_in) and all(len(facial[i]) for i in order):
+            out_a, out_f, o_off = eng.collect_host(np.concatenate(rows_in, axis=0), _prefix([len(r) for r in rows_in]),
+                                                   np.concatenate([facial[i] for i in order], axis=0),
+                                                   _prefix([len(facial[i]) for i in order]), **kw)
+            for k, i in enumerate(order):
+                results[i] = (out_a[o_off[k]:o_off[k + 1]], out_f[o_off[k]:o_off[k + 1]])
+        else:
+            for r, i in zip(rows_in, order):
+                results[i] = tuple(np.array(x) for x in collect_arrays(r, facial[i], **kw))
+    return results, features
+
+
+def _assemble(takes, mine, results, processed_folders):
+    """``(examples, indices)`` in take order with ``facial[:, :61] *= 100`` (:68); records the folders (:24)."""
+    examples, indices = [], []
+    for i in mine:
+        if i not in results:
+            continue
+        a, f = results[i]
+        f[:, :61] *= 100
+        examples.append((a, f))
+        indices.append(i)
+        processed_folders.add(takes[i].folder)
+    return examples, indices
+
+
 last_timing = {}     # phase -> seconds of the most recent load_data_batched call (bench.py reports it)
 
 
@@ -340,216 +488,42 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
     import time
     from concurrent.futures import ThreadPoolExecutor
 
-    from .. import shard
-    from ..utils.audio.extraction.extract_features import MIN_FRAMES
-    from ..utils.audio.load_audio import REFERENCE_RATE
-
     t_start = time.perf_counter()
     timing = {}
-    cache_format = cache_format or os.environ.get("NSF_FEATURE_CACHE", "csv")
-    if cache_format not in ("csv", "npy", "both"):
-        raise ValueError("cache_format must be 'csv', 'npy' or 'both'")
+    cache_format = _cache_format(cache_format)
     if dtype not in (np.float32, np.float64):
         raise ValueError("dtype must be numpy.float32 or numpy.float64")
-    takes = []                      # (folder, source audio/video, wav, cache_csv, facial_csv, folder_path)
-    for folder in os.listdir(root_dir):
-        folder_path = os.path.join(root_dir, folder)
-        if not os.path.isdir(folder_path) or folder in processed_folders:
-            continue
-        mov, mp4, wav, facial_csv, cache_csv, _ = find_files(folder_path)
-        video = mov or mp4
-        have_cache = os.path.exists(cache_csv) or (cache_format != "csv" and
-                                                   os.path.exists(_binary_cache_path(cache_csv)))
-        if not (facial_csv and (video or wav or have_cache)):
-            continue
-        takes.append((folder, video, wav, cache_csv, facial_csv, folder_path))
-    # partition on files every rank sees identically BEFORE any rank extracts audio (never on audio.wav, which
-    # another rank may be writing): the take's video, else its wav, else its cache
-    def weight(t):
-        for cand in (t[1], t[2], t[3]):
-            if cand and os.path.exists(cand):
-                return max(1, os.path.getsize(cand))
-        return 1
-    mine = shard.lpt_partition([weight(t) for t in takes], world)[rank] if world > 1 else list(range(len(takes)))
+    takes = _scan(root_dir, processed_folders, cache_format)
+    mine = _partition(takes, rank, world)
     timing["scan"] = time.perf_counter() - t_start
 
     f_len, h_len = _engine.frame_params(REFERENCE_RATE)     # file-path mode always lands at 88.2 kHz
     eng = _engine.get_engine(REFERENCE_RATE, f_len, h_len, device=device)
+    kw = dict(include_fast=include_fast, include_slow=include_slow, blend_boundaries=blend_boundaries,
+              blend_frames=blend_frames)
     threads = io_threads or min(32, len(os.sched_getaffinity(0)) or 1)
     pool = ThreadPoolExecutor(max_workers=threads)
     try:
-        # ---- which takes need extraction; where their audio is -------------------------------------------
         t0 = time.perf_counter()
-        cached, todo = {}, []            # take -> rows | (take, audio_path)
-        for i in mine:
-            folder, video, wav, cache_csv, facial_csv, folder_path = takes[i]
-            if os.path.exists(cache_csv):                                      # :112-114
-                print(f"Loading audio features from {cache_csv}")
-                cached[i] = pool.submit(lambda p=cache_csv: pd.read_csv(p).values)
-            elif cache_format != "csv" and os.path.exists(_binary_cache_path(cache_csv)):
-                print(f"Loading audio features from {_binary_cache_path(cache_csv)}")
-                cached[i] = pool.submit(np.load, _binary_cache_path(cache_csv))
-            else:
-                audio_path = get_audio(video, wav, folder_path) if (video or wav) else None
-                if not audio_path:
-                    continue                                                   # process_folder returns (None, None)
-                print(f"Extracting audio features from {audio_path}")
-                todo.append((i, audio_path))
-        todo_set = {j for j, _ in todo}
-        keep = [i for i in mine if i in cached or i in todo_set]
-        facial_jobs = {}
-
-        # ---- PCM of the takes to extract: mono PCM16 files at 88.2 kHz are read straight into page-locked
-        # int16 memory (2 bytes per sample over PCIe); every other take's raw bytes are decoded, downmixed and
-        # resampled to float32 on the device by nsf_convert_host ------------------------------------------------
-        n_rows = {}
-        pcm_arena = pcm = off = None
-        if todo:
-            info = [_pcm16_payload(p, REFERENCE_RATE) if sr == REFERENCE_RATE else None for _, p in todo]
-            fast = all(x is not None for x in info)
-            if fast:
-                lens = [n for _, n in info]
-            else:
-                # every other take: raw data-chunk bytes, converted on the device (decode_for_path's arithmetic)
-                heads = list(pool.map(lambda tp: _wav_source(tp[1]), todo))
-                for (_, p), h in zip(todo, heads):
-                    print(f"Loaded audio file '{p}' with sample rate {sr if sr is not None else h[4]}")
-                # sr=None keeps the native rate in decode(): one conversion, native -> 88.2 kHz
-                sr1 = sr if sr is not None else REFERENCE_RATE
-                src = np.zeros(len(todo), dtype=nv.PCM_SOURCE)
-                pos = 0
-                for k, (_, nbytes, enc, ch, rate) in enumerate(heads):
-                    frames = nbytes // (_ENC_BYTES[enc] * ch)
-                    src[k] = (pos, frames, enc, ch, rate, 0)
-                    pos += (frames * _ENC_BYTES[enc] * ch + 7) // 8 * 8          # every take 8-byte aligned
-                mid_off = nv.convert_offsets(src, sr1, pos)                       # native rate -> sr
-                if sr1 != REFERENCE_RATE:                                          # then sr -> 88.2 kHz (load_audio.py:8-10)
-                    mid = np.zeros(len(todo), dtype=nv.PCM_SOURCE)
-                    for k in range(len(todo)):
-                        mid[k] = (int(mid_off[k]) * 4, int(mid_off[k + 1] - mid_off[k]), nv.ENC_F32, 1, sr1, 0)
-                    lens = np.diff(nv.convert_offsets(mid, REFERENCE_RATE, int(mid_off[-1]) * 4))
-                else:
-                    lens = np.diff(mid_off)
-            for (i, _), n in zip(todo, lens):
-                g = eng.plan.guard_frames(n)
-                if g < MIN_FRAMES:                                             # extract_features.py:16-20 -> :143
-                    print(f"Audio file is too short: {g} frames, required: {MIN_FRAMES} frames")
-                    raise TypeError("object of type 'NoneType' has no len()")
-            off = np.zeros(len(todo) + 1, dtype=np.int64)
-            np.cumsum(lens, out=off[1:])
-            item = 2 if fast else 4
-            pcm_arena = _engine.scratch_pinned("dataset_pcm", int(off[-1]) * item)   # library-owned, reused
-            pcm = pcm_arena.view(np.int16 if fast else np.float32, (int(off[-1]),))
-            if fast:
-                for (_, p) in todo:
-                    print(f"Loaded audio file '{p}' with sample rate {REFERENCE_RATE}")
-                reads = [pool.submit(_read_into, todo[k][1], info[k][0], pcm[off[k]:off[k + 1]]) for k in range(len(todo))]
-                facial_jobs = {i: pool.submit(_facial_rows, takes[i][4], dtype) for i in keep}   # queued behind the reads
-                for r in reads:
-                    r.result()
-            else:
-                wav_arena = _engine.scratch_pinned("dataset_wav", max(pos, 1))
-                raw = wav_arena.view(np.uint8, (pos,))
-                reads = [pool.submit(_read_into, todo[k][1], heads[k][0], raw[int(src[k]["byte_offset"]):
-                                     int(src[k]["byte_offset"]) + int(src[k]["frames"]) * _ENC_BYTES[heads[k][2]] *
-                                     heads[k][3]]) for k in range(len(todo)) if src[k]["frames"] > 0]
-                facial_jobs = {i: pool.submit(_facial_rows, takes[i][4], dtype) for i in keep}
-                for r in reads:
-                    r.result()
-                if sr1 != REFERENCE_RATE:
-                    y_sr = _engine.scratch_pinned("dataset_wav_mid", max(int(mid_off[-1]) * 4, 1)).view(
-                        np.float32, (int(mid_off[-1]),))
-                    eng.convert_host(raw, src, sr1, out=y_sr)
-                    eng.convert_host(y_sr.view(np.uint8), mid, REFERENCE_RATE, out=pcm)
-                else:
-                    eng.convert_host(raw, src, sr1, out=pcm)
-            roff = eng.row_offsets(off)
-            for k, (i, _) in enumerate(todo):
-                n_rows[i] = int(roff[k + 1] - roff[k])
+        loaded, extract = _classify(takes, mine, cache_format, pool)
+        keep = [i for i in mine if i in loaded or i in extract]
+        pcm, off, facial = _read_audio(eng, pool, list(extract.values()), sr, then=lambda: {
+            i: pool.submit(_facial_rows, takes[i].facial_csv, dtype) for i in keep})
         timing["read_audio"] = time.perf_counter() - t0
         t0 = time.perf_counter()
-        for i in keep:
-            if i not in facial_jobs:
-                facial_jobs[i] = pool.submit(_facial_rows, takes[i][4], dtype)
-        facial = {i: j.result() for i, j in facial_jobs.items()}
-        cached = {i: j.result() for i, j in cached.items()}
+        facial = {i: j.result() for i, j in facial.items()}
+        loaded = {i: j.result() for i, j in loaded.items()}
         timing["facial_csv_wait"] = time.perf_counter() - t0
-
-        # ---- device pass ------------------------------------------------------------------------------------
         t0 = time.perf_counter()
-        results = {}                    # take -> (audio rows, facial rows)
-        feats_by_take = {}
-        kw = dict(include_fast=include_fast, include_slow=include_slow, blend_boundaries=blend_boundaries,
-                  blend_frames=blend_frames)
-        augment = include_fast or include_slow
-        if todo:
-            order = [i for i, _ in todo]
-            f_off = np.zeros(len(order) + 1, dtype=np.int64)
-            np.cumsum([len(facial[i]) for i in order], out=f_off[1:])
-            if dtype == np.float32 and augment and all(n_rows[i] and len(facial[i]) for i in order):
-                f_cols = facial[order[0]].shape[1]
-                fac_arena = _engine.scratch_pinned("dataset_facial", int(f_off[-1]) * f_cols * 4)
-                fac = fac_arena.view(np.float32, (int(f_off[-1]), f_cols))
-                for k, i in enumerate(order):
-                    fac[f_off[k]:f_off[k + 1]] = facial[i]
-                o_off = eng.collect_rows(roff, f_off, **kw)
-                # results go to ordinary (pageable) arrays the caller owns: the library stages the downloads through
-                # its own page-locked arenas, which costs a host copy but not a cudaHostAlloc of ~300 MB per call
-                out_a = np.empty((int(o_off[-1]), 256), dtype=np.float32)
-                out_f = np.empty((int(o_off[-1]), f_cols), dtype=np.float32)
-                feats = np.empty((int(roff[-1]), 256), dtype=np.float32)
-                eng.extract_collect_host(pcm, off, fac, f_off, nv.PEAK_NORMALIZE, out_audio=out_a, out_facial=out_f,
-                                         features_out=feats, **kw)
-                for k, i in enumerate(order):
-                    results[i] = (out_a[o_off[k]:o_off[k + 1]], out_f[o_off[k]:o_off[k + 1]])
-                    feats_by_take[i] = feats[roff[k]:roff[k + 1]]
-            else:
-                rows = eng.extract_host(pcm, off, nv.PEAK_NORMALIZE)
-                for k, i in enumerate(order):
-                    feats_by_take[i] = rows[roff[k]:roff[k + 1]]
-                    cached[i] = feats_by_take[i]
-        if cached:
-            order = sorted(cached)
-            rows_in = [np.ascontiguousarray(cached[i], dtype=dtype) for i in order]
-            if augment and all(len(r) for r in rows_in) and all(len(facial[i]) for i in order):
-                a_off = np.zeros(len(order) + 1, dtype=np.int64)
-                np.cumsum([len(r) for r in rows_in], out=a_off[1:])
-                f_off = np.zeros(len(order) + 1, dtype=np.int64)
-                np.cumsum([len(facial[i]) for i in order], out=f_off[1:])
-                out_a, out_f, o_off = eng.collect_host(np.concatenate(rows_in, axis=0), a_off,
-                                                       np.concatenate([facial[i] for i in order], axis=0), f_off, **kw)
-                for k, i in enumerate(order):
-                    results[i] = (out_a[o_off[k]:o_off[k + 1]], out_f[o_off[k]:o_off[k + 1]])
-            else:
-                for r, i in zip(rows_in, order):
-                    results[i] = tuple(np.array(x) for x in collect_arrays(r, facial[i], **kw))
+        results, features = _device_pass(eng, pcm, off, list(extract), loaded, facial, dtype, kw)
         timing["device"] = time.perf_counter() - t0
-
-        # ---- side effects: feature caches (:115-120), facial scaling (:68), processed_folders (:24) ---------
         t0 = time.perf_counter()
-        def write_cache(i):
-            cache_csv, f = takes[i][3], feats_by_take[i]
-            if cache_format in ("csv", "both"):
-                pd.DataFrame(np.asarray(f, dtype=np.float64)).to_csv(cache_csv, index=False)
-                print(f"Audio features saved to {cache_csv}")
-            if cache_format in ("npy", "both"):
-                np.save(_binary_cache_path(cache_csv), np.asarray(f, dtype=np.float32))
-                print(f"Audio features saved to {_binary_cache_path(cache_csv)}")
-        list(pool.map(write_cache, list(feats_by_take)))
+        list(pool.map(lambda i: _write_feature_cache(takes[i].cache_csv, features[i], cache_format), features))
         timing["write_cache"] = time.perf_counter() - t0
     finally:
         pool.shutdown(wait=True)
-    examples, indices = [], []
-    for i in mine:
-        if i not in results:
-            continue
-        a, f = results[i]
-        f[:, :61] *= 100                                                   # process_folder :68
-        examples.append((a, f))
-        indices.append(i)
-        processed_folders.add(takes[i][0])
+    examples, indices = _assemble(takes, mine, results, processed_folders)
     timing["total"] = time.perf_counter() - t_start
     last_timing.clear()
     last_timing.update(timing)
     return examples, indices
-

@@ -20,34 +20,58 @@ Division of labour
 """
 import io
 import struct
+from collections import namedtuple
 
 import numpy as np
 
+from ... import _native as nv
 from ... import engine as _engine
 
 REFERENCE_RATE = 88200  # load_audio.py:8-10: file-path mode always ends at 88.2 kHz
+
+# (format tag, bits per sample) -> nsf_pcm_source encoding: every encoding decode_wav reads
+WAV_ENCODINGS = {(1, 8): nv.ENC_U8, (1, 16): nv.ENC_I16, (1, 24): nv.ENC_I24, (1, 32): nv.ENC_I32,
+                 (3, 32): nv.ENC_F32, (3, 64): nv.ENC_F64}
+
+WavLayout = namedtuple("WavLayout", "tag channels rate bits data_offset data_bytes")
+
+
+def wav_layout(fh):
+    """``WavLayout`` of the seekable binary RIFF/WAVE stream ``fh``, read from its headers.  ``tag`` is the format tag
+    (WAVE_FORMAT_EXTENSIBLE's from its sub-format GUID), ``channels`` as declared (0 included).  Odd-sized chunks are
+    padded; the first ``data`` chunk ends the walk, truncated at the end of the stream.  ``ValueError`` for every
+    stream ``decode_wav`` cannot decode."""
+    size = fh.seek(0, io.SEEK_END)
+    fh.seek(0)
+    head = fh.read(12)
+    if len(head) < 12 or head[:4] != b"RIFF" or head[8:12] != b"WAVE":
+        raise ValueError("not a RIFF/WAVE stream (only WAV decoding is built in)")
+    pos, fmt, data = 12, None, None
+    while pos + 8 <= size:
+        fh.seek(pos)
+        tag, n = struct.unpack("<4sI", fh.read(8))
+        if tag == b"fmt ":
+            body = fh.read(n)
+            fmt = struct.unpack_from("<HHIIHH", body, 0)
+            if fmt[0] == 0xFFFE and len(body) >= 26:       # WAVE_FORMAT_EXTENSIBLE: real tag in GUID
+                fmt = (struct.unpack_from("<H", body, 24)[0],) + fmt[1:]
+        elif tag == b"data":
+            data = (pos + 8, min(n, size - (pos + 8)))
+            break
+        pos += 8 + n + (n & 1)
+    if fmt is None or data is None:
+        raise ValueError("WAV stream lacks a fmt or data chunk")
+    code, channels, rate, _, _, bits = fmt
+    if (code, bits) not in WAV_ENCODINGS:
+        raise ValueError(f"unsupported WAV encoding (format {code}, {bits} bit)")
+    return WavLayout(code, channels, rate, bits, *data)
 
 
 def decode_wav(data):
     """RIFF/WAVE bytes -> (pcm, native_sr).  pcm is int16 (mono PCM16 files, kept as is so it can
     be uploaded at 2 bytes/sample) or float32 in [-1, 1) (everything else, soundfile scaling)."""
-    if len(data) < 12 or data[:4] != b"RIFF" or data[8:12] != b"WAVE":
-        raise ValueError("not a RIFF/WAVE stream (only WAV decoding is built in)")
-    pos, fmt, payload = 12, None, None
-    while pos + 8 <= len(data):
-        tag, size = data[pos:pos + 4], struct.unpack_from("<I", data, pos + 4)[0]
-        body = data[pos + 8: pos + 8 + size]
-        if tag == b"fmt ":
-            fmt = struct.unpack_from("<HHIIHH", body, 0)
-            if fmt[0] == 0xFFFE and len(body) >= 26:       # WAVE_FORMAT_EXTENSIBLE: real tag in GUID
-                fmt = (struct.unpack_from("<H", body, 24)[0],) + fmt[1:]
-        elif tag == b"data":
-            payload = body
-            break
-        pos += 8 + size + (size & 1)
-    if fmt is None or payload is None:
-        raise ValueError("WAV stream lacks a fmt or data chunk")
-    code, channels, sr, _, _, bits = fmt
+    code, channels, sr, bits, off, n = wav_layout(io.BytesIO(data))
+    payload = data[off:off + n]
     if code == 1 and bits == 16:
         pcm = np.frombuffer(payload, dtype="<i2", count=len(payload) // 2)
         if channels == 1:
@@ -65,10 +89,8 @@ def decode_wav(data):
         x = (v.astype(np.float64) / float(1 << 31)).astype(np.float32)
     elif code == 3 and bits == 32:
         x = np.frombuffer(payload, dtype="<f4", count=len(payload) // 4).copy()
-    elif code == 3 and bits == 64:
+    else:                                                   # (3, 64): wav_layout rejected every other encoding
         x = np.frombuffer(payload, dtype="<f8", count=len(payload) // 8).astype(np.float32)
-    else:
-        raise ValueError(f"unsupported WAV encoding (format {code}, {bits} bit)")
     if channels > 1:
         x = x[: len(x) // channels * channels].reshape(-1, channels).mean(axis=1, dtype=np.float32)
     return np.ascontiguousarray(x, dtype=np.float32), sr

@@ -6,6 +6,7 @@ route must give exactly what the per-take decode_for_path route gave."""
 import ctypes as C
 import os
 import struct
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -147,6 +148,83 @@ def test_wav_source_rejects_what_decode_wav_rejects(tmp_path):
         assert str(e1.value) == str(e2.value)
 
 
+# ---- the dataset builder's audio route (host planning, no GPU) --------------------------------------------
+PCM16_TAKES = [("i16", 1, 88200, n, False) for n in (1000, 777, 4001)]
+
+
+def _wav_tree(root, specs):
+    """One take folder per (enc, channels, rate, frames, extensible) holding its audio.wav; returns the paths."""
+    paths = []
+    for k, (enc, ch, rate, n, ext) in enumerate(specs):
+        take = root / f"take_{k:03d}"
+        take.mkdir(parents=True)
+        (take / "audio.wav").write_bytes(wav_file(samples(enc, n * max(ch, 1), seed=k), enc, ch, rate, extensible=ext))
+        paths.append(str(take / "audio.wav"))
+    return paths
+
+
+def _plan(paths, sr):
+    from neurosync_trainer_lite_b200.dataset import data_processing as dp
+    return dp._plan_audio([dp._wav_source(p) for p in paths], sr)
+
+
+@pytest.mark.parametrize("extensible", [False, True])
+def test_mono_pcm16_takes_at_88200_take_the_int16_route(tmp_path, nv, extensible):
+    from neurosync_trainer_lite_b200.dataset import data_processing as dp
+    specs = list(PCM16_TAKES)
+    specs[1] = specs[1][:4] + (extensible,)
+    paths = _wav_tree(tmp_path, specs)
+    plan = _plan(paths, 88200)
+    data_bytes = [dp._wav_source(p)[1] for p in paths]
+    assert plan.int16 and plan.mid is None
+    assert list(plan.lengths) == [b // 2 for b in data_bytes] == [1000, 777, 4001]
+    assert list(plan.sources["byte_offset"]) == [0, 2000, 3554] and plan.nbytes == sum(data_bytes)
+    assert set(plan.sources["encoding"]) == {nv.ENC_I16} and set(plan.sources["channels"]) == {1}
+
+
+@pytest.mark.parametrize("enc,ch,rate", [("i16", 0, 88200), ("i16", 2, 88200), ("i16", 1, 48000), ("i24", 1, 88200),
+                                         ("f32", 1, 88200), ("u8", 1, 88200)])
+def test_any_other_take_sends_every_take_through_the_conversion(tmp_path, nv, enc, ch, rate):
+    from neurosync_trainer_lite_b200.utils.audio.load_audio import decode_wav
+    paths = _wav_tree(tmp_path, PCM16_TAKES + [(enc, ch, rate, 999, False)])
+    plan = _plan(paths, 88200)
+    assert not plan.int16 and plan.rate == 88200 and plan.mid is None
+    assert all(plan.sources["byte_offset"] % 8 == 0) and plan.sources[-1]["channels"] == max(ch, 1)
+    assert [len(decode_wav(Path(p).read_bytes())[0]) for p in paths] == list(plan.sources["frames"])
+    assert list(plan.lengths) == list(np.diff(nv.convert_offsets(plan.sources, 88200, plan.nbytes)))
+    # the int16 route also needs sr == 88200 (sr=None keeps the native rate in decode())
+    for sr in (None, 44100):
+        assert not _plan(paths[:3], sr).int16
+
+
+def test_a_rate_below_88200_converts_in_two_stages(tmp_path, nv):
+    paths = _wav_tree(tmp_path, PCM16_TAKES + [("i24", 2, 48000, 999, False)])
+    plan = _plan(paths, 44100)
+    first = nv.convert_offsets(plan.sources, 44100, plan.nbytes)
+    mid = nv.pcm_sources([(int(first[k]) * 4, int(first[k + 1] - first[k]), nv.ENC_F32, 1, 44100)
+                          for k in range(len(paths))])
+    assert not plan.int16 and plan.rate == 44100 and np.array_equal(plan.mid, mid)
+    assert list(plan.lengths) == list(np.diff(nv.convert_offsets(mid, 88200, int(first[-1]) * 4)))
+
+
+def test_unsupported_encoding_is_rejected_before_anything_is_read(tmp_path):
+    from concurrent.futures import ThreadPoolExecutor
+
+    from neurosync_trainer_lite_b200.dataset import data_processing as dp
+    from neurosync_trainer_lite_b200.utils.audio.load_audio import decode_wav
+    paths = _wav_tree(tmp_path, PCM16_TAKES + [("i16", 1, 88200, 6, False)])
+    blob = Path(paths[-1]).read_bytes().replace(struct.pack("<HHIIHH", 1, 1, 88200, 176400, 2, 16),
+                                                struct.pack("<HHIIHH", 1, 1, 88200, 176400, 2, 12))
+    Path(paths[-1]).write_bytes(blob)
+    with pytest.raises(ValueError) as want:
+        decode_wav(blob)
+    queued = []
+    # no engine: the header pass must fail before the length check, the reads and the jobs queued behind them
+    with ThreadPoolExecutor(4) as pool, pytest.raises(ValueError) as got:
+        dp._read_audio(None, pool, paths, 88200, then=lambda: queued.append(1))
+    assert str(got.value) == str(want.value) and not queued
+
+
 # ---- GPU ---------------------------------------------------------------------------------------------
 def _engine():
     from neurosync_trainer_lite_b200 import engine
@@ -232,11 +310,11 @@ MIXED = [("i16", 1, 88200, 2.1), ("i16", 2, 48000, 1.7), ("i24", 1, 44100, 2.4),
          ("u8", 1, 22050, 1.9), ("i24x", 2, 44100, 1.5)]
 
 
-def _mixed_tree(root, facial_rows=140):
+def _mixed_tree(root, specs=MIXED, facial_rows=140):
     import pandas as pd
     from neurosync_trainer_lite_b200 import synth
     cols = ["Timecode", "BlendshapeCount"] + [f"bs{i}" for i in range(61)]
-    for k, (enc, ch, rate, secs) in enumerate(MIXED):
+    for k, (enc, ch, rate, secs) in enumerate(specs):
         take = root / f"take_{k:03d}"
         take.mkdir(parents=True)
         y = np.stack([synth.synth_clip(secs, rate, seed=70 + k + c, kind=("voiced", "gated", "noise")[(k + c) % 3])
@@ -307,6 +385,27 @@ def test_mixed_format_dataset_equals_the_per_take_route(tmp_path, sr):
             assert ga.dtype == wa.dtype == dtype
             assert np.array_equal(ga, wa) and np.array_equal(gf, wf)
         assert all((root / f"take_{k:03d}" / "audio_features.csv").exists() for k in range(len(MIXED)))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dtype", [np.float32, np.float64])
+def test_extensible_pcm16_dataset_equals_the_plain_one(tmp_path, dtype):
+    """WAVE_FORMAT_EXTENSIBLE mono PCM16 takes at 88.2 kHz go the int16 route like plain ones: same examples, same
+    cache files, bit for bit."""
+    from neurosync_trainer_lite_b200.dataset import data_processing as dp
+    out = []
+    for enc in ("i16", "i16x"):
+        root = tmp_path / enc
+        _mixed_tree(root, [(enc, 1, 88200, secs) for secs in (2.1, 1.3, 1.8)])
+        got, _ = dp.load_data_batched(str(root), 88200, set(), cache_format="both", dtype=dtype)
+        caches = [(root / take / name).read_bytes() for take in sorted(os.listdir(root))
+                  for name in ("audio_features.csv", "audio_features.npy")]
+        out.append((got, caches))
+    (want, want_caches), (got, got_caches) = out
+    assert len(got) == len(want) == 3 and got_caches == want_caches
+    for (ga, gf), (wa, wf) in zip(got, want):
+        assert ga.dtype == wa.dtype == dtype
+        assert ga.tobytes() == wa.tobytes() and gf.tobytes() == wf.tobytes()
 
 
 @pytest.mark.gpu
