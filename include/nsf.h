@@ -382,6 +382,32 @@ NSF_API nsf_status nsf_window_gather(nsf_ctx* ctx, void* cuda_stream,
                                      int32_t n_clips, int32_t window, const int64_t* indices_host, int64_t n,
                                      float* out_audio_dev, float* out_facial_dev);
 
+/* ---- feature cache as CSV text ----------------------------------------------------------------------
+ * The reference's audio_features.csv cache (dataset/data_processing.py:115-120): pd.DataFrame(rows.astype(float64))
+ * .to_csv(path, index=False), formatted on the device byte for byte.  Each file is the header line "0,1,...,cols-1\n"
+ * followed by one line per row, fields separated by ',' and each line ended by '\n' (a file without rows is the
+ * header alone).  A finite field is Python's repr(float(v)): the shortest digits that round back to the double (the
+ * nearest such string when several have that length), positional for 1e-4 <= |v| < 1e16 with ".0" on integers
+ * (0.00015, 123.0, -0.0), scientific otherwise with a signed exponent of at least two digits (1e-05, 1e+16,
+ * 5e-324).  float32 rows are widened to double first (0.1f -> 0.10000000149011612).  inf / -inf are written as
+ * such, NaN as an empty field, or as "" when it is the row's only field. */
+/* Upper bound of the text nsf_format_csv_host writes for n_files files, n_rows rows in total, cols columns
+ * (24 characters per field + separator, plus one header per file); -1 for negative counts or cols < 1.  Host only.
+ * (data_processing.py:115-120) */
+NSF_API int64_t nsf_csv_bytes_bound(int64_t n_rows, int32_t cols, int32_t n_files);
+/* rows_host: [row_offsets[n_files] - row_offsets[0]] x cols, row-major, NSF_F32 or NSF_F64.  File i = header +
+ * rows [row_offsets[i], row_offsets[i+1]) -> text_host[text_offsets[i], text_offsets[i+1]), text_offsets[0] = 0
+ * (n_files + 1 entries).  Synchronous, pipelined over file groups (one wait per group for its text size); pageable
+ * or page-locked buffers.  NSF_ERR_BAD_ARG for NULLs, cols < 1, a bad dtype, decreasing offsets or text_capacity
+ * below nsf_csv_bytes_bound, before anything is launched.  (data_processing.py:115-120) */
+NSF_API nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_host, int32_t cols,
+                                       const int64_t* row_offsets_host, int32_t n_files,
+                                       char* text_host, int64_t text_capacity, int64_t* text_offsets_host);
+/* Verification aid, like nsf_plan_fold_check: the device's digit routine run on the host, value i -> out[32 i ..],
+ * lengths[i] characters (0 for NaN).  Exists so the formatting can be checked against repr without a GPU; not a
+ * compute path.  (data_processing.py:115-120) */
+NSF_API nsf_status nsf_format_check(const double* values, int64_t n, char* out, int32_t* lengths);
+
 /* ---- instrumentation -------------------------------------------------------------------------
  * Kernel launches issued by this context since creation (bench.py reports it as gpu_launches). */
 NSF_API int64_t nsf_launch_count(const nsf_ctx* ctx);

@@ -108,6 +108,9 @@ _SIGS = {
     "nsf_convert_host": (_i32, [_vp, _vp, _i64, _vp, _i32, _i32, _vp]),
     "nsf_window_offsets": (_i32, [_i64p, _i64p, _i32, _i32, _i64p]),
     "nsf_window_gather": (_i32, [_vp, _vp, _vp, _i32, _i64p, _vp, _i32, _i64p, _i32, _i32, _i64p, _i64, _vp, _vp]),
+    "nsf_csv_bytes_bound": (_i64, [_i64, _i32, _i32]),
+    "nsf_format_csv_host": (_i32, [_vp, _i32, _vp, _i32, _i64p, _i32, _vp, _i64, _i64p]),
+    "nsf_format_check": (_i32, [_f64p, _i64, _vp, _i32p]),
     "nsf_launch_count": (_i64, [_vp]),
     "nsf_set_profiling": (None, [_vp, _i32]),
     "nsf_stage_times_ms": (_i32, [_vp, _f32p, _i32]),

@@ -1376,6 +1376,67 @@ nsf_status nsf_extract_collect_host(nsf_ctx* ctx, const void* pcm_host, int32_t 
   });
 }
 
+// ---- audio_features.csv text ------------------------------------------------------------------------------
+nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_host, int32_t cols,
+                               const int64_t* row_off, int32_t n_files, char* text_host, int64_t text_capacity,
+                               int64_t* text_off) {
+  if (!ctx || !rows_host || !row_off || !text_host || !text_off || cols < 1 || n_files < 0) {
+    set_error("nsf_format_csv_host: NULL argument, cols < 1 or n_files < 0"); return NSF_ERR_BAD_ARG;
+  }
+  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_format_csv_host: bad dtype"); return NSF_ERR_BAD_ARG; }
+  for (int i = 0; i < n_files; ++i)
+    if (row_off[i + 1] < row_off[i]) { set_error("nsf_format_csv_host: offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+  const int64_t n_rows = row_off[n_files] - row_off[0];
+  if (text_capacity < nsf_csv_bytes_bound(n_rows, cols, n_files)) {
+    set_error("nsf_format_csv_host: text_capacity below nsf_csv_bytes_bound()"); return NSF_ERR_BAD_ARG;
+  }
+  text_off[0] = 0;
+  if (n_files == 0) return NSF_OK;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  const size_t row_bytes = static_cast<size_t>(cols) * (dtype == NSF_F64 ? 8 : 4);
+  const int64_t header = csv_header_bytes(cols);
+  std::vector<int64_t> cost(n_files + 1);   // file groups by value count
+  for (int i = 0; i <= n_files; ++i) cost[i] = (row_off[i] - row_off[0]) * cols;
+  const bool in_dma = dma_reachable(rows_host), out_dma = dma_reachable(text_host);
+  // device: in = [rows, row and header positions], out = [text, row lengths]
+  return run_groups(ctx, cost.data(), n_files, [&](int first, int last, Slot* sl) -> nsf_status {
+    const int64_t r0 = row_off[first] - row_off[0], nr = row_off[last] - row_off[first], nf = last - first;
+    if (nr + nf > INT32_MAX) { set_error("nsf_format_csv_host: more than 2^31 rows in one file"); return NSF_ERR_UNSUPPORTED; }
+    const size_t pos_bytes = static_cast<size_t>(nr + nf) * sizeof(int64_t), len_bytes = nr * sizeof(int64_t);
+    nsf_status st;
+    if ((st = sl->in[0].reserve(std::max<size_t>(nr * row_bytes, 1))) != NSF_OK) return st;
+    if ((st = sl->in[1].reserve(pos_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[1].reserve(std::max<size_t>(len_bytes, 1))) != NSF_OK) return st;
+    if ((st = sl->stage_in[1].reserve(pos_bytes)) != NSF_OK) return st;
+    if ((st = sl->stage_out[1].reserve(std::max<size_t>(len_bytes, 1))) != NSF_OK) return st;
+    if (nr > 0) {   // the group's row lengths, and with them its text size: the group's one wait
+      if ((st = upload(sl, 0, static_cast<const char*>(rows_host) + r0 * row_bytes, nr * row_bytes, in_dma)) != NSF_OK) return st;
+      const int m = launch_csv_lengths(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int64_t*>(sl->out[1].ptr));
+      if (m < 0) { set_error(cuda_msg("launch_csv_lengths", cudaGetLastError())); return NSF_ERR_CUDA; }
+      ctx->launches += m;
+      if ((st = download(sl, 1, sl->stage_out[1].ptr, len_bytes, len_bytes, 1, true)) != NSF_OK) return st;
+      NSF_CUDA(cudaStreamSynchronize(sl->stream));
+    }
+    // positions from the group's first byte: each file's header, then its rows
+    const int64_t* len = static_cast<const int64_t*>(sl->stage_out[1].ptr);
+    int64_t* pos = static_cast<int64_t*>(sl->stage_in[1].ptr);
+    int64_t at = 0;
+    for (int i = first; i < last; ++i) {
+      pos[nr + i - first] = at;
+      at += header;
+      for (int64_t r = row_off[i] - row_off[first]; r < row_off[i + 1] - row_off[first]; ++r) { pos[r] = at; at += len[r]; }
+      text_off[i + 1] = text_off[first] + at;
+    }
+    if ((st = upload(sl, 1, pos, pos_bytes, true)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(at)) != NSF_OK) return st;
+    const int m = launch_csv_write(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int32_t>(nf),
+                                   static_cast<const int64_t*>(sl->in[1].ptr), static_cast<char*>(sl->out[0].ptr));
+    if (m < 0) { set_error(cuda_msg("launch_csv_write", cudaGetLastError())); return NSF_ERR_CUDA; }
+    ctx->launches += m;
+    return download(sl, 0, text_host + text_off[first], at, at, 1, out_dma);
+  });
+}
+
 // ---- inference-side chunker ---------------------------------------------------------------------------
 int64_t nsf_chunk_count(int64_t n_rows, int32_t frame, int32_t overlap) {
   if (n_rows <= 0 || frame <= 0 || overlap < 0 || overlap >= frame) return 0;

@@ -146,6 +146,13 @@ constexpr int kWindowTileRows = 32;
 int launch_window_gather(cudaStream_t s, const WindowView& v, const float* audio, int a_cols, const float* facial,
                          int f_cols, float* out_a, float* out_f);
 
+// audio_features.csv text (nsf_csv.cu): row_len[r] = bytes of row r (k_csv_lengths, one block per row); then every
+// row at text + start[r] and the header of file f at text + start[n_rows + f] (k_csv_write).
+int64_t csv_header_bytes(int cols);
+int launch_csv_lengths(cudaStream_t s, int dtype, const void* rows, int64_t n_rows, int cols, int64_t* row_len);
+int launch_csv_write(cudaStream_t s, int dtype, const void* rows, int64_t n_rows, int cols, int32_t n_files,
+                     const int64_t* start, char* text);
+
 // One-time (per device) cudaFuncSetAttribute calls of each translation unit; nsf_ctx_create runs them so that no
 // launch path touches function attributes.
 bool init_kernel_attributes();        // nsf_kernels.cu

@@ -1,7 +1,8 @@
 """GPU-backed mirror of the reference's ``dataset/data_processing.py`` (dataset builders).
 
-Host side (unchanged semantics): folder scan, CSV cache of ``audio_features.csv``, the facial CSV
-minus ``Timecode`` / ``BlendshapeCount``, ``facial[:, :61] *= 100``.
+Host side (unchanged semantics): folder scan, reading the ``audio_features.csv`` cache, the facial CSV
+minus ``Timecode`` / ``BlendshapeCount``, ``facial[:, :61] *= 100``.  The cache's text is formatted on the device
+(``Engine.format_csv``), byte for byte what the reference's pandas writer produces.
 Device side: feature extraction (``extract_audio_features``) and the whole ``collect_features``
 augmentation - centre-trim, fast ``[::2]``, slow ``interpolate_slower`` (+ ``smooth_facial_data``),
 ``stack_with_blend`` - as one ``nsf_collect_host`` call in float64, bit-identical to the NumPy
@@ -138,10 +139,15 @@ def _read_feature_cache(path):
     return np.load(path) if path.endswith(".npy") else pd.read_csv(path).values
 
 
-def _write_feature_cache(cache_csv, rows, cache_format):
-    """The cache files of one take's feature rows (:115-120): the CSV from float64, the ``.npy`` from float32."""
+def _write_feature_cache(cache_csv, rows, cache_format, text=None):
+    """The cache files of one take's feature rows (:115-120): the CSV from float64, the ``.npy`` from float32.
+    The CSV is ``text``, the take's device-formatted bytes of ``Engine.format_csv`` (formatted here when None):
+    byte for byte what the reference's ``pd.DataFrame(rows).to_csv(path, index=False)`` writes."""
     if cache_format in ("csv", "both"):
-        pd.DataFrame(np.asarray(rows, dtype=np.float64)).to_csv(cache_csv, index=False)
+        if text is None:
+            text = _engine_any().format_csv(rows)[0]
+        with open(cache_csv, "wb") as fh:
+            fh.write(text)
         print(f"Audio features saved to {cache_csv}")
     if cache_format in ("npy", "both"):
         npy_path = _binary_cache_path(cache_csv)
@@ -155,7 +161,7 @@ def collect_features(audio_path, audio_features_csv_path, facial_csv_path, sr,
     """reference :108-177 -- same CSV cache side effects, same return shapes and dtypes.
 
     ``cache_format`` (extension, SURVEY section 8(f)-3; default from ``NSF_FEATURE_CACHE`` or "csv"):
-    "csv" = the reference's ``audio_features.csv`` (1.3 s and 9 MB per 30 s clip to write);
+    "csv" = the reference's ``audio_features.csv`` (9.5 MB per 30 s clip, formatted on the device);
     "npy" = a float32 ``audio_features.npy`` beside it (milliseconds, 1.8 MB); "both" writes both.
     An existing CSV cache is always honoured first, exactly like the reference."""
     cache_format = _cache_format(cache_format)
@@ -404,11 +410,11 @@ def _read_audio(eng, pool, paths, sr, then):
 
 
 def _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw):
-    """``(results, features)``: take -> augmented (audio, facial) rows, for the takes ``extract`` (PCM ``pcm`` at
-    ``off``) and those with ``loaded`` rows; take -> feature rows extracted.  float32 with augmentation fuses
-    extraction and augmentation in one ``nsf_extract_collect_host`` call; otherwise the extracted rows join the
-    loaded ones in the collect pass."""
-    results, features, rows = {}, {}, dict(loaded)
+    """``(results, feats, roff)``: take -> augmented (audio, facial) rows, for the takes ``extract`` (PCM ``pcm`` at
+    ``off``) and those with ``loaded`` rows; the feature rows extracted, packed in ``extract`` order at ``roff`` (None,
+    None without takes to extract).  float32 with augmentation fuses extraction and augmentation in one
+    ``nsf_extract_collect_host`` call; otherwise the extracted rows join the loaded ones in the collect pass."""
+    results, rows, feats, roff = {}, dict(loaded), None, None
     augment = kw["include_fast"] or kw["include_slow"]
     if extract:
         roff = eng.row_offsets(off)
@@ -429,11 +435,10 @@ def _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw):
                                      features_out=feats, **kw)
             for k, i in enumerate(extract):
                 results[i] = (out_a[o_off[k]:o_off[k + 1]], out_f[o_off[k]:o_off[k + 1]])
-                features[i] = feats[roff[k]:roff[k + 1]]
         else:
             feats = eng.extract_host(pcm, off, nv.PEAK_NORMALIZE)
             for k, i in enumerate(extract):
-                features[i] = rows[i] = feats[roff[k]:roff[k + 1]]
+                rows[i] = feats[roff[k]:roff[k + 1]]
     if rows:
         order = sorted(rows)
         rows_in = [np.ascontiguousarray(rows[i], dtype=dtype) for i in order]
@@ -446,7 +451,7 @@ def _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw):
         else:
             for r, i in zip(rows_in, order):
                 results[i] = tuple(np.array(x) for x in collect_arrays(r, facial[i], **kw))
-    return results, features
+    return results, feats, roff
 
 
 def _assemble(takes, mine, results, processed_folders):
@@ -515,10 +520,16 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
         loaded = {i: j.result() for i, j in loaded.items()}
         timing["facial_csv_wait"] = time.perf_counter() - t0
         t0 = time.perf_counter()
-        results, features = _device_pass(eng, pcm, off, list(extract), loaded, facial, dtype, kw)
+        extract = list(extract)
+        results, feats, roff = _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw)
         timing["device"] = time.perf_counter() - t0
         t0 = time.perf_counter()
-        list(pool.map(lambda i: _write_feature_cache(takes[i].cache_csv, features[i], cache_format), features))
+        if extract:
+            # every take's CSV in one device call; the pool only writes bytes
+            text, t_off = eng.format_csv(feats, roff) if cache_format in ("csv", "both") else (None, None)
+            list(pool.map(lambda k: _write_feature_cache(
+                takes[extract[k]].cache_csv, feats[roff[k]:roff[k + 1]], cache_format,
+                None if text is None else text[t_off[k]:t_off[k + 1]]), range(len(extract))))
         timing["write_cache"] = time.perf_counter() - t0
     finally:
         pool.shutdown(wait=True)

@@ -453,6 +453,33 @@ class Engine:
                                              int(blend_frames), nv.ptr(out_a), nv.ptr(out_f)))
         return out_a, out_f, o_off
 
+    def format_csv(self, rows, row_offsets=None):
+        """``audio_features.csv`` text of packed rows, formatted on the device (``nsf_format_csv_host``): file i is
+        ``rows[row_offsets[i]:row_offsets[i + 1]]`` (one file of every row if ``row_offsets`` is None), byte for byte
+        ``pd.DataFrame(rows_i.astype(np.float64)).to_csv(index=False)``.  ``rows``: 2-D, float32 or float64 (other
+        dtypes are cast to float64).  Returns ``(text uint8 array, text_offsets)``; file i is
+        ``text[text_offsets[i]:text_offsets[i + 1]]``."""
+        rows = np.asarray(rows)
+        if rows.dtype not in (np.float32, np.float64):
+            rows = rows.astype(np.float64)
+        if rows.ndim != 2:
+            raise ValueError("rows must be 2-D")
+        rows = np.ascontiguousarray(rows)
+        off, off_p = nv.i64_array([0, len(rows)] if row_offsets is None else row_offsets)
+        if len(off) < 1 or off[0] < 0 or off[-1] > len(rows):
+            raise ValueError("row_offsets must lie in [0, len(rows)]")
+        n_files, cols = len(off) - 1, rows.shape[1]
+        bound = int(nv.lib.nsf_csv_bytes_bound(int(off[-1] - off[0]), cols, n_files))
+        if bound < 0:
+            raise ValueError("rows need at least one column and row_offsets must be non-decreasing")
+        text = np.empty(bound, dtype=np.uint8)
+        text_off = np.empty(n_files + 1, dtype=np.int64)
+        with self._lock:
+            nv.check(nv.lib.nsf_format_csv_host(self.handle, nv.F64 if rows.dtype == np.float64 else nv.F32,
+                                                C.c_void_p(rows.ctypes.data + int(off[0]) * rows.strides[0]), cols,
+                                                off_p, n_files, nv.ptr(text), bound, text_off.ctypes.data_as(nv._i64p)))
+        return text[:int(text_off[-1])], text_off
+
     def rows_op(self, op, a, b=None, blend_frames=0):
         a = np.ascontiguousarray(a)
         if a.dtype not in (np.float32, np.float64):
