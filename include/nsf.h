@@ -408,6 +408,63 @@ NSF_API nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* 
  * compute path.  (data_processing.py:115-120) */
 NSF_API nsf_status nsf_format_check(const double* values, int64_t n, char* out, int32_t* lengths);
 
+/* ---- CSV text -> rows ------------------------------------------------------------------------------
+ * The reference's reads of the facial CSVs and of the audio_features.csv cache (dataset/data_processing.py:112-123):
+ * pd.read_csv(path).drop(columns=DROP).values, parsed on the device value for value.  A file is its header line
+ * (the first line, skipped here: names, duplicates and DROP are the caller's business) and data rows.  A row ends at
+ * '\n'; a '\r' directly before it is dropped; a line that is empty after that is skipped; the last line may lack its
+ * '\n'.  A field is empty (-> NaN), "inf" / "-inf", or [+-]? digits* ( . digits* )? ( [eE] [+-]? digits+ )? with
+ * at least one mantissa digit and at most 40 characters, valued by pandas' precise_xstrtod with the same IEEE double
+ * operations in the same order (not correctly rounded: up to 17 mantissa digits as number * 10 + d, then one
+ * multiplication or division by the double literal 1e<k>).  A column whose every field is an integer literal is
+ * int64 in pandas, so its -0 is +0.  float32 output is the double rounded to nearest (NumPy's astype).
+ * Anything else makes the file unaccepted and sets bits of its status word:
+ *   NSF_CSV_BAD_FIELD  a field outside the grammar (spaces, NaN spellings, non-ASCII or control bytes, a decimal
+ *                      exponent above 308, an overflow to inf) or longer than 40 characters;
+ *   NSF_CSV_BAD_SHAPE  a row with more or fewer fields than `cols`;
+ *   NSF_CSV_BAD_LINE   a quote character or a bare '\r' (pandas quotes / ends the line there);
+ *   NSF_CSV_BAD_INT    an integer literal of more than 15 digits, or a -0 literal in a column that also holds other
+ *                      fields (pandas' chunked reader types each chunk of rows on its own, so that zero's sign depends
+ *                      on where the chunk boundaries fall);
+ *   NSF_CSV_BAD_ROWS   row_offsets_host does not match the text.
+ * The rows of an unaccepted file are unspecified; read it with pandas instead. */
+#define NSF_CSV_BAD_FIELD 0x1u
+#define NSF_CSV_BAD_SHAPE 0x2u
+#define NSF_CSV_BAD_LINE 0x4u
+#define NSF_CSV_BAD_INT 0x8u
+#define NSF_CSV_BAD_ROWS 0x10u
+/* kinds of nsf_parse_check */
+#define NSF_CSV_KIND_NUMBER 0
+#define NSF_CSV_KIND_INTEGER 1 /* [+-]? digits: pandas' int64 when the whole column is such literals */
+#define NSF_CSV_KIND_EMPTY 2   /* NaN */
+#define NSF_CSV_KIND_INF 3
+#define NSF_CSV_KIND_BAD 4     /* unaccepted */
+/* Data rows per file: row_offsets_host[i] = data rows of the files before file i (n_files + 1 entries), file i being
+ * bytes [text_offsets_host[i], text_offsets_host[i+1]) of text_dev (header included; text_dev 16-byte aligned).
+ * The call's one host wait is the download of those n_files + 1 counts.  NSF_ERR_BAD_ARG for NULLs,
+ * n_files < 0, a negative first offset, decreasing offsets or an unaligned text_dev, before anything is launched;
+ * n_files == 0 launches nothing.  (data_processing.py:112-123) */
+NSF_API nsf_status nsf_csv_row_offsets(nsf_ctx* ctx, void* cuda_stream, const char* text_dev,
+                                       const int64_t* text_offsets_host, int32_t n_files, int64_t* row_offsets_host);
+/* The rows: file i's data rows go to out_dev rows [row_offsets_host[i], row_offsets_host[i+1]) (row_offsets_host as
+ * nsf_csv_row_offsets returned it, starting at 0), row r at out_dev + r * out_ld, of dtype NSF_F32 or NSF_F64; the
+ * file's column c goes to output column out_col_host[c] (cols entries, each in [-1, out_cols), -1 = dropped: not
+ * parsed, only checked for quotes and bare '\r', each output column used at most once).  file_status_dev[i]
+ * (uint32) == 0: file i's rows are final; else the NSF_CSV_BAD_* bits say why not.  Stream-ordered, no host wait:
+ * offsets, column map and row offsets travel through the descriptor ring.  NSF_ERR_BAD_ARG for NULLs, n_files < 0,
+ * cols < 1, bad offsets or alignment (as above), row offsets not starting at 0 or decreasing, a bad column map, a bad
+ * dtype or out_ld < out_cols; NSF_ERR_UNSUPPORTED above 2^31 rows; all before anything is launched.  n_files == 0
+ * launches nothing.  (data_processing.py:112-123) */
+NSF_API nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const char* text_dev,
+                                 const int64_t* text_offsets_host, int32_t n_files, int32_t cols,
+                                 const int32_t* out_col_host, int32_t out_cols, const int64_t* row_offsets_host,
+                                 void* out_dev, int64_t out_ld, uint32_t* file_status_dev);
+/* Verification aid, like nsf_format_check: the device's field routine run on the host.  Field i is
+ * text[field_offsets[i], field_offsets[i+1]) -> values[i], kinds[i] (NSF_CSV_KIND_*; values[i] is unspecified for
+ * NSF_CSV_KIND_BAD).  Not a compute path.  (data_processing.py:112-123) */
+NSF_API nsf_status nsf_parse_check(const char* text, const int64_t* field_offsets, int64_t n, double* values,
+                                   int32_t* kinds);
+
 /* ---- instrumentation -------------------------------------------------------------------------
  * Kernel launches issued by this context since creation (bench.py reports it as gpu_launches). */
 NSF_API int64_t nsf_launch_count(const nsf_ctx* ctx);

@@ -29,6 +29,8 @@ OPT_EDGE_ZERO_THRESHOLD = 0
 OPT_RESAMPLE_QUALITY = 1
 RESAMPLE_POLY, RESAMPLE_HQ = 0, 1
 POST_EDGEFIX, POST_CMVN, POST_DELTAS, POST_REDUCE = 0x1, 0x2, 0x4, 0x8
+CSV_BAD_FIELD, CSV_BAD_SHAPE, CSV_BAD_LINE, CSV_BAD_INT, CSV_BAD_ROWS = 0x1, 0x2, 0x4, 0x8, 0x10
+CSV_KIND_NUMBER, CSV_KIND_INTEGER, CSV_KIND_EMPTY, CSV_KIND_INF, CSV_KIND_BAD = range(5)
 ENC_U8, ENC_I16, ENC_I24, ENC_I32, ENC_F32, ENC_F64 = range(6)
 # nsf_pcm_source: one clip of the WAV conversion calls (raw data-chunk bytes -> mono float32)
 PCM_SOURCE = np.dtype([("byte_offset", "<i8"), ("frames", "<i8"), ("encoding", "<i4"), ("channels", "<i4"),
@@ -111,6 +113,9 @@ _SIGS = {
     "nsf_csv_bytes_bound": (_i64, [_i64, _i32, _i32]),
     "nsf_format_csv_host": (_i32, [_vp, _i32, _vp, _i32, _i64p, _i32, _vp, _i64, _i64p]),
     "nsf_format_check": (_i32, [_f64p, _i64, _vp, _i32p]),
+    "nsf_csv_row_offsets": (_i32, [_vp, _vp, _vp, _i64p, _i32, _i64p]),
+    "nsf_csv_parse": (_i32, [_vp, _vp, _i32, _vp, _i64p, _i32, _i32, _i32p, _i32, _i64p, _vp, _i64, _vp]),
+    "nsf_parse_check": (_i32, [_vp, _i64p, _i64, _f64p, _i32p]),
     "nsf_launch_count": (_i64, [_vp]),
     "nsf_set_profiling": (None, [_vp, _i32]),
     "nsf_stage_times_ms": (_i32, [_vp, _f32p, _i32]),

@@ -1437,6 +1437,136 @@ nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_hos
   });
 }
 
+// ---- CSV text -> rows ----------------------------------------------------------------------------------------
+namespace {
+// Checks shared by the two CSV calls; tile_off[i] = tiles of the files before file i.
+nsf_status csv_text_args(const char* fn, nsf_ctx* ctx, const char* text_dev, const int64_t* text_off, int32_t n_files,
+                         std::vector<int64_t>* tile_off) {
+  char buf[160];
+  if (!ctx || !text_off || n_files < 0) {
+    std::snprintf(buf, sizeof buf, "%s: NULL argument or n_files < 0", fn); set_error(buf); return NSF_ERR_BAD_ARG;
+  }
+  if (n_files == 0) return NSF_OK;
+  if (text_off[0] < 0) { std::snprintf(buf, sizeof buf, "%s: negative text offset", fn); set_error(buf); return NSF_ERR_BAD_ARG; }
+  tile_off->assign(n_files + 1, 0);
+  for (int i = 0; i < n_files; ++i) {
+    if (text_off[i + 1] < text_off[i]) {
+      std::snprintf(buf, sizeof buf, "%s: text offsets must be non-decreasing", fn); set_error(buf); return NSF_ERR_BAD_ARG;
+    }
+    (*tile_off)[i + 1] = (*tile_off)[i] + csv_tiles(text_off[i], text_off[i + 1]);
+  }
+  if (text_off[n_files] > text_off[0] && (!text_dev || reinterpret_cast<uintptr_t>(text_dev) % 16 != 0)) {
+    std::snprintf(buf, sizeof buf, "%s: text_dev is NULL or not 16-byte aligned", fn); set_error(buf); return NSF_ERR_BAD_ARG;
+  }
+  if ((*tile_off)[n_files] > INT32_MAX) {
+    std::snprintf(buf, sizeof buf, "%s: text too long for one call", fn); set_error(buf); return NSF_ERR_UNSUPPORTED;
+  }
+  return NSF_OK;
+}
+}  // namespace
+
+nsf_status nsf_csv_row_offsets(nsf_ctx* ctx, void* cuda_stream, const char* text_dev, const int64_t* text_off,
+                               int32_t n_files, int64_t* row_off) {
+  std::vector<int64_t> tile_off;
+  nsf_status st = csv_text_args("nsf_csv_row_offsets", ctx, text_dev, text_off, n_files, &tile_off);
+  if (st != NSF_OK) return st;
+  if (!row_off) { set_error("nsf_csv_row_offsets: row_offsets_host is NULL"); return NSF_ERR_BAD_ARG; }
+  row_off[0] = 0;
+  if (n_files == 0) return NSF_OK;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const size_t n1 = static_cast<size_t>(n_files) + 1, n_tiles = static_cast<size_t>(tile_off[n_files]);
+  // ring entry: host [text_off | tile_off | row_off (download)]; device [text_off | tile_off | row_off | tile_start |
+  // tile_rows]
+  const size_t desc = 2 * n1 * sizeof(int64_t), bytes = desc + n1 * sizeof(int64_t);
+  const size_t dev_bytes = bytes + (n_tiles + 1) * sizeof(int64_t) + std::max<size_t>(n_tiles, 1) * sizeof(int32_t);
+  DescEntry* de = nullptr;
+  if ((st = desc_acquire(ctx, bytes, &de)) != NSF_OK) return st;
+  if ((st = de->dev.reserve(dev_bytes)) != NSF_OK) return st;
+  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
+  std::memcpy(h, text_off, n1 * sizeof(int64_t));
+  std::memcpy(h + n1, tile_off.data(), n1 * sizeof(int64_t));
+  int64_t* d = static_cast<int64_t*>(de->dev.ptr);
+  NSF_CUDA(cudaMemcpyAsync(d, h, desc, cudaMemcpyHostToDevice, s));
+  CsvView v{};
+  v.text = text_dev; v.text_off = d; v.tile_off = d + n1; v.n_files = n_files; v.n_tiles = static_cast<int64_t>(n_tiles);
+  int64_t* d_rows = d + 2 * n1;
+  int64_t* d_tile_start = d + 3 * n1;
+  int32_t* d_tile_rows = reinterpret_cast<int32_t*>(d_tile_start + n_tiles + 1);
+  const int m = launch_csv_row_offsets(s, v, d_tile_rows, d_tile_start, d_rows);
+  if (m < 0) { set_error(cuda_msg("launch_csv_row_offsets", cudaGetLastError())); return NSF_ERR_CUDA; }
+  ctx->launches += m;
+  NSF_CUDA(cudaMemcpyAsync(h + 2 * n1, d_rows, n1 * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  if ((st = desc_commit(de, s)) != NSF_OK) return st;
+  NSF_CUDA(cudaStreamSynchronize(s));   // the call's one host wait
+  std::memcpy(row_off, h + 2 * n1, n1 * sizeof(int64_t));
+  return NSF_OK;
+}
+
+nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const char* text_dev, const int64_t* text_off,
+                         int32_t n_files, int32_t cols, const int32_t* out_col, int32_t out_cols, const int64_t* row_off,
+                         void* out_dev, int64_t out_ld, uint32_t* status_dev) {
+  std::vector<int64_t> tile_off;
+  nsf_status st = csv_text_args("nsf_csv_parse", ctx, text_dev, text_off, n_files, &tile_off);
+  if (st != NSF_OK) return st;
+  if (!out_col || !row_off || !status_dev || cols < 1 || out_cols < 0) {
+    set_error("nsf_csv_parse: NULL argument, cols < 1 or out_cols < 0"); return NSF_ERR_BAD_ARG;
+  }
+  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_csv_parse: bad dtype"); return NSF_ERR_BAD_ARG; }
+  if (out_ld < out_cols) { set_error("nsf_csv_parse: out_ld < out_cols"); return NSF_ERR_BAD_ARG; }
+  std::vector<char> used(out_cols, 0);
+  for (int c = 0; c < cols; ++c) {
+    const int oc = out_col[c];
+    if (oc < -1 || oc >= out_cols || (oc >= 0 && used[oc]++)) {
+      set_error("nsf_csv_parse: out_col entries must lie in [-1, out_cols) and name each output column at most once");
+      return NSF_ERR_BAD_ARG;
+    }
+  }
+  if (row_off[0] != 0) { set_error("nsf_csv_parse: row offsets must start at 0"); return NSF_ERR_BAD_ARG; }
+  for (int i = 0; i < n_files; ++i)
+    if (row_off[i + 1] < row_off[i]) { set_error("nsf_csv_parse: row offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+  const int64_t n_rows = row_off[n_files];
+  if (n_rows > 0 && !out_dev) { set_error("nsf_csv_parse: out_dev is NULL"); return NSF_ERR_BAD_ARG; }
+  if (n_rows > INT32_MAX) { set_error("nsf_csv_parse: more than 2^31 rows in one call"); return NSF_ERR_UNSUPPORTED; }
+  if (n_files == 0) return NSF_OK;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const size_t n1 = static_cast<size_t>(n_files) + 1, n_tiles = static_cast<size_t>(tile_off[n_files]);
+  // ring entry: [text_off | tile_off | row_off | out_col (int32)], then on the device only: tile_start, row_start,
+  // col_flags, tile_rows
+  const size_t desc = 3 * n1 * sizeof(int64_t) + align_up(static_cast<size_t>(cols) * sizeof(int32_t), 8);
+  const size_t flags_bytes = n1 * static_cast<size_t>(cols) * sizeof(uint32_t);
+  const size_t dev_bytes = desc + (n_tiles + 1 + static_cast<size_t>(n_rows)) * sizeof(int64_t) + flags_bytes +
+                           std::max<size_t>(n_tiles, 1) * sizeof(int32_t);
+  DescEntry* de = nullptr;
+  if ((st = desc_acquire(ctx, desc, &de)) != NSF_OK) return st;
+  if ((st = de->dev.reserve(dev_bytes)) != NSF_OK) return st;
+  char* h = static_cast<char*>(de->mem.ptr);
+  std::memcpy(h, text_off, n1 * sizeof(int64_t));
+  std::memcpy(h + n1 * 8, tile_off.data(), n1 * sizeof(int64_t));
+  std::memcpy(h + 2 * n1 * 8, row_off, n1 * sizeof(int64_t));
+  std::memcpy(h + 3 * n1 * 8, out_col, static_cast<size_t>(cols) * sizeof(int32_t));
+  char* d = static_cast<char*>(de->dev.ptr);
+  NSF_CUDA(cudaMemcpyAsync(d, h, desc, cudaMemcpyHostToDevice, s));
+  int64_t* d_tile_start = reinterpret_cast<int64_t*>(d + desc);
+  int64_t* d_row_start = d_tile_start + n_tiles + 1;
+  uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_row_start + n_rows);
+  int32_t* d_tile_rows = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(d_flags) + flags_bytes);
+  NSF_CUDA(cudaMemsetAsync(d_flags, 0, flags_bytes, s));
+  NSF_CUDA(cudaMemsetAsync(status_dev, 0, static_cast<size_t>(n_files) * sizeof(uint32_t), s));
+  CsvView v{};
+  v.text = text_dev;
+  v.text_off = reinterpret_cast<const int64_t*>(d);
+  v.tile_off = v.text_off + n1;
+  v.row_off = v.text_off + 2 * n1;
+  v.out_col = reinterpret_cast<const int32_t*>(d + 3 * n1 * 8);
+  v.n_files = n_files; v.cols = cols; v.n_tiles = static_cast<int64_t>(n_tiles); v.n_rows = n_rows;
+  const int m = launch_csv_parse(s, v, dtype, d_tile_rows, d_tile_start, d_row_start, d_flags, out_dev, out_ld, status_dev);
+  if (m < 0) { set_error(cuda_msg("launch_csv_parse", cudaGetLastError())); return NSF_ERR_CUDA; }
+  ctx->launches += m;
+  return desc_commit(de, s);
+}
+
 // ---- inference-side chunker ---------------------------------------------------------------------------
 int64_t nsf_chunk_count(int64_t n_rows, int32_t frame, int32_t overlap) {
   if (n_rows <= 0 || frame <= 0 || overlap < 0 || overlap >= frame) return 0;

@@ -153,6 +153,27 @@ int launch_csv_lengths(cudaStream_t s, int dtype, const void* rows, int64_t n_ro
 int launch_csv_write(cudaStream_t s, int dtype, const void* rows, int64_t n_rows, int cols, int32_t n_files,
                      const int64_t* start, char* text);
 
+// CSV text -> rows (nsf_csv_parse.cu).  File i is text[text_off[i], text_off[i+1]) (header line included); its
+// tiles [tile_off[i], tile_off[i+1]) are the kCsvTile-aligned blocks of the text clipped to the file (csv_tiles).
+// Data row r (rows of file i: [row_off[i], row_off[i+1]), row_off[0] = 0) goes to out + r * out_ld, column c of the
+// file to output column out_col[c] (-1: dropped).
+constexpr int64_t kCsvTile = 16384;
+struct CsvView {
+  const char* text;
+  const int64_t* text_off;   // [n_files + 1]
+  const int64_t* tile_off;   // [n_files + 1]
+  const int64_t* row_off;    // [n_files + 1], parse only
+  const int32_t* out_col;    // [cols], parse only
+  int32_t n_files, cols;
+  int64_t n_tiles, n_rows;
+};
+int64_t csv_tiles(int64_t begin, int64_t end);
+// tile_rows [n_tiles] int32, tile_start [n_tiles + 1]: workspace; row_off [n_files + 1] <- data rows before file i.
+int launch_csv_row_offsets(cudaStream_t s, const CsvView& v, int32_t* tile_rows, int64_t* tile_start, int64_t* row_off);
+// + row_start [n_rows], col_flags [n_files x cols] (zeroed by the caller), status [n_files] (zeroed by the caller).
+int launch_csv_parse(cudaStream_t s, const CsvView& v, int dtype, int32_t* tile_rows, int64_t* tile_start,
+                     int64_t* row_start, uint32_t* col_flags, void* out, int64_t out_ld, uint32_t* status);
+
 // One-time (per device) cudaFuncSetAttribute calls of each translation unit; nsf_ctx_create runs them so that no
 // launch path touches function attributes.
 bool init_kernel_attributes();        // nsf_kernels.cu

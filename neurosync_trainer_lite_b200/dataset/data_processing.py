@@ -2,7 +2,8 @@
 
 Host side (unchanged semantics): folder scan, reading the ``audio_features.csv`` cache, the facial CSV
 minus ``Timecode`` / ``BlendshapeCount``, ``facial[:, :61] *= 100``.  The cache's text is formatted on the device
-(``Engine.format_csv``), byte for byte what the reference's pandas writer produces.
+(``Engine.format_csv``), byte for byte what the reference's pandas writer produces, and the batched builder parses
+both kinds of CSV on the device (``Engine.parse_csv``), value for value what pandas reads.
 Device side: feature extraction (``extract_audio_features``) and the whole ``collect_features``
 augmentation - centre-trim, fast ``[::2]``, slow ``interpolate_slower`` (+ ``smooth_facial_data``),
 ``stack_with_blend`` - as one ``nsf_collect_host`` call in float64, bit-identical to the NumPy
@@ -301,23 +302,72 @@ def _read_into(path, offset, dst):
             got += n
 
 
+def _pandas_rows(path, drop, dtype):
+    """The reference's read of a CSV (:112-114, :123): ``pd.read_csv`` minus the columns ``drop``, cast to dtype."""
+    return np.ascontiguousarray(pd.read_csv(path).drop(columns=drop).values, dtype=dtype)
+
+
 def _facial_rows(path, dtype):
-    """The facial CSV minus Timecode / BlendshapeCount (:123).  float64: pandas' default parser, value for value
-    what the reference reads.  float32 (training format): Arrow's multi-threaded reader, 4x faster per file and
-    free of the GIL - its correctly rounded float64 values differ from pandas' fast parser by at most one ulp,
-    which the cast to float32 absorbs."""
-    if dtype == np.float32:
-        try:
-            import pyarrow.csv as pacsv
-            # single-threaded parse: the caller's thread pool already runs one file per core, and Arrow drops the GIL
-            table = pacsv.read_csv(path, read_options=pacsv.ReadOptions(use_threads=False)).drop_columns(COLUMNS_TO_DROP)
-            out = np.empty((table.num_rows, table.num_columns), dtype=np.float32)
-            for j, col in enumerate(table.columns):
-                out[:, j] = col.to_numpy()
-            return out
-        except Exception:      # noqa: BLE001 - anything Arrow cannot type as numbers goes the reference's way
-            pass
-    return np.ascontiguousarray(pd.read_csv(path).drop(columns=COLUMNS_TO_DROP).values, dtype=dtype)
+    """The facial CSV minus Timecode / BlendshapeCount (:123), read by pandas."""
+    return _pandas_rows(path, COLUMNS_TO_DROP, dtype)
+
+
+def _read_texts(pool, paths, tag):
+    """``(text, offsets, reads)``: the files ``paths`` back to back in the page-locked arena ``tag``, file k at
+    ``text[offsets[k]:offsets[k + 1]]``, once the pool jobs ``reads`` are done."""
+    off = _prefix([os.path.getsize(p) for p in paths])
+    text = _engine.scratch_pinned(tag, max(int(off[-1]), 1)).view(np.uint8, (int(off[-1]),))
+    return text, off, [pool.submit(_read_into, p, 0, text[off[k]:off[k + 1]]) for k, p in enumerate(paths)]
+
+
+_BOM = b"\xef\xbb\xbf"
+
+
+def _csv_header(head, drop):
+    """Column names of a CSV whose first bytes are ``head``, or None when the device route does not take the file:
+    the first line must be printable ASCII without quotes (a '\r' only before its '\n'), with unique, non-empty
+    names that include every name in ``drop``.  pandas handles the rest (BOMs, quoting, renamed duplicates, the
+    KeyError of a missing column)."""
+    if not head or head[:1] in (b"\r", b"\n") or head.startswith(_BOM):
+        return None
+    nl = head.find(b"\n")
+    line = head if nl < 0 else head[:nl]
+    if line.endswith(b"\r"):
+        line = line[:-1]
+    if any(c < 0x20 or c >= 0x7f or c == 0x22 for c in line):
+        return None
+    names = line.decode("ascii").split(",")
+    if "" in names or len(set(names)) != len(names) or any(d not in names for d in drop):
+        return None
+    return names
+
+
+def _parse_csvs(eng, pool, paths, text, off, drop, dtype):
+    """``[rows]`` of the files ``paths`` (read into ``text`` at ``off``), each ``_pandas_rows(path, drop, dtype)``:
+    files with the same header share one ``Engine.parse_csv`` call; a file the device does not accept (its header,
+    or a status bit) is read by pandas on ``pool``, so its result, or the exception it raises, is the reference's."""
+    groups, out = {}, [None] * len(paths)
+    for k in range(len(paths)):
+        head = bytes(text[off[k]:min(off[k + 1], off[k] + 65536)])      # a longer header line goes to pandas
+        names = _csv_header(head, drop) if b"\n" in head or len(head) == off[k + 1] - off[k] else None
+        if names is not None:
+            groups.setdefault(tuple(names), []).append(k)
+    for names, ks in groups.items():
+        kept = [n for n in names if n not in drop]
+        out_col = [-1 if n in drop else kept.index(n) for n in names]
+        if ks == list(range(len(paths))):
+            t, t_off = text, off
+        else:
+            t = np.concatenate([text[off[k]:off[k + 1]] for k in ks])
+            t_off = _prefix([off[k + 1] - off[k] for k in ks])
+        rows, r_off, status = eng.parse_csv(t, t_off, len(names), out_col, dtype)
+        for j, k in enumerate(ks):
+            if not status[j]:
+                out[k] = rows[r_off[j]:r_off[j + 1]]
+    fallback = {k: pool.submit(_pandas_rows, paths[k], drop, dtype) for k in range(len(paths)) if out[k] is None}
+    for k, job in fallback.items():
+        out[k] = job.result()
+    return out
 
 
 _Take = namedtuple("_Take", "folder video wav cache_csv facial_csv path")
@@ -353,21 +403,25 @@ def _partition(takes, rank, world):
 
 
 def _classify(takes, mine, cache_format, pool):
-    """``(loaded, extract)``: take -> pool job loading its feature cache, and take -> the audio file to extract
-    (``get_audio`` may run ffmpeg).  A take with neither is dropped, as ``process_folder`` returns (None, None)."""
-    loaded, extract = {}, {}
+    """``(loaded, cached_csv, extract)``: take -> pool job loading its ``.npy`` feature cache, take -> its CSV cache
+    (parsed with the facial CSVs), and take -> the audio file to extract (``get_audio`` may run ffmpeg).  A take with
+    none is dropped, as ``process_folder`` returns (None, None)."""
+    loaded, cached_csv, extract = {}, {}, {}
     for i in mine:
         t = takes[i]
         cache_path = _cached_features_path(t.cache_csv, cache_format)
         if cache_path:
             print(f"Loading audio features from {cache_path}")
-            loaded[i] = pool.submit(_read_feature_cache, cache_path)
+            if cache_path.endswith(".npy"):
+                loaded[i] = pool.submit(_read_feature_cache, cache_path)
+            else:
+                cached_csv[i] = cache_path
             continue
         audio_path = get_audio(t.video, t.wav, t.path) if (t.video or t.wav) else None
         if audio_path:
             print(f"Extracting audio features from {audio_path}")
             extract[i] = audio_path
-    return loaded, extract
+    return loaded, cached_csv, extract
 
 
 def _read_audio(eng, pool, paths, sr, then):
@@ -510,15 +564,22 @@ def load_data_batched(root_dir, sr, processed_folders, include_fast=True, includ
     pool = ThreadPoolExecutor(max_workers=threads)
     try:
         t0 = time.perf_counter()
-        loaded, extract = _classify(takes, mine, cache_format, pool)
-        keep = [i for i in mine if i in loaded or i in extract]
-        pcm, off, facial = _read_audio(eng, pool, list(extract.values()), sr, then=lambda: {
-            i: pool.submit(_facial_rows, takes[i].facial_csv, dtype) for i in keep})
+        loaded, cached_csv, extract = _classify(takes, mine, cache_format, pool)
+        keep = [i for i in mine if i in loaded or i in cached_csv or i in extract]
+        # the CSV texts are read into page-locked arenas behind the WAV payloads, then parsed on the device
+        facial_paths, cache_paths = [takes[i].facial_csv for i in keep], list(cached_csv.values())
+        pcm, off, (fac_text, cache_text) = _read_audio(eng, pool, list(extract.values()), sr, then=lambda: (
+            _read_texts(pool, facial_paths, "dataset_facial_csv"), _read_texts(pool, cache_paths, "dataset_cache_csv")))
         timing["read_audio"] = time.perf_counter() - t0
         t0 = time.perf_counter()
-        facial = {i: j.result() for i, j in facial.items()}
+        for j in fac_text[2] + cache_text[2]:
+            j.result()
         loaded = {i: j.result() for i, j in loaded.items()}
         timing["facial_csv_wait"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        facial = dict(zip(keep, _parse_csvs(eng, pool, facial_paths, *fac_text[:2], COLUMNS_TO_DROP, dtype)))
+        loaded.update(zip(cached_csv, _parse_csvs(eng, pool, cache_paths, *cache_text[:2], [], dtype)))
+        timing["parse_csv"] = time.perf_counter() - t0
         t0 = time.perf_counter()
         extract = list(extract)
         results, feats, roff = _device_pass(eng, pcm, off, extract, loaded, facial, dtype, kw)

@@ -480,6 +480,54 @@ class Engine:
                                                 off_p, n_files, nv.ptr(text), bound, text_off.ctypes.data_as(nv._i64p)))
         return text[:int(text_off[-1])], text_off
 
+    def parse_csv(self, text, text_offsets, cols, out_col, dtype=np.float64):
+        """CSV files parsed on the device (``nsf_csv_row_offsets`` + ``nsf_csv_parse``): file i is
+        ``text[text_offsets[i]:text_offsets[i + 1]]``, header line included, with ``cols`` columns; column c goes to
+        output column ``out_col[c]`` (-1 = dropped).  ``text``: host uint8 array, pageable or page-locked, uploaded
+        once.  Returns ``(rows [n, out_cols] of dtype, row_offsets, status)`` as host arrays: file i's rows are
+        ``rows[row_offsets[i]:row_offsets[i + 1]]``, value for value ``pd.read_csv(file).drop(columns=dropped).values``
+        cast to dtype, when ``status[i] == 0``; otherwise ``status[i]`` holds ``nv.CSV_BAD_*`` bits and the file's rows
+        are unspecified."""
+        import torch
+        text = np.ascontiguousarray(text).view(np.uint8).reshape(-1)
+        if not text.flags.writeable:          # torch.from_numpy wants a writable array
+            text = text.copy()
+        off, off_p = nv.i64_array(text_offsets)
+        if len(off) < 1 or off[0] < 0 or off[-1] > text.size:
+            raise ValueError("text_offsets must lie in [0, len(text)]")
+        oc = np.ascontiguousarray(out_col, dtype=np.int32)
+        if oc.size != int(cols):
+            raise ValueError("out_col needs one entry per column")
+        out_cols = int(oc.max(initial=-1)) + 1
+        dt = np.dtype(dtype)
+        if dt not in (np.float32, np.float64):
+            raise ValueError("dtype must be float32 or float64")
+        n_files = len(off) - 1
+        row_off = np.zeros(n_files + 1, dtype=np.int64)
+        dev = torch.device("cuda", self.device)
+        s = torch.cuda.current_stream(dev)
+        with self._lock:
+            d_text = torch.empty(max(text.size, 1), dtype=torch.uint8, device=dev)
+            if text.size:
+                d_text[:text.size].copy_(torch.from_numpy(text), non_blocking=True)
+            nv.check(nv.lib.nsf_csv_row_offsets(self.handle, C.c_void_p(s.cuda_stream), C.c_void_p(d_text.data_ptr()),
+                                                off_p, n_files, row_off.ctypes.data_as(nv._i64p)))
+            n = int(row_off[-1])
+            d_rows = torch.empty((max(n, 1), max(out_cols, 1)), dtype=getattr(torch, dt.name), device=dev)
+            d_status = torch.empty(max(n_files, 1), dtype=torch.int32, device=dev)
+            nv.check(nv.lib.nsf_csv_parse(self.handle, C.c_void_p(s.cuda_stream), nv.F64 if dt == np.float64 else nv.F32,
+                                          C.c_void_p(d_text.data_ptr()), off_p, n_files, int(cols),
+                                          oc.ctypes.data_as(nv._i32p), out_cols, row_off.ctypes.data_as(nv._i64p),
+                                          C.c_void_p(d_rows.data_ptr()), max(out_cols, 1),
+                                          C.c_void_p(d_status.data_ptr())))
+            rows = np.empty((n, out_cols), dtype=dt)
+            status = np.empty(n_files, dtype=np.uint32)
+            if rows.size:
+                torch.from_numpy(rows).copy_(d_rows[:n, :out_cols])
+            if n_files:
+                torch.from_numpy(status.view(np.int32)).copy_(d_status[:n_files])
+        return rows, row_off, status
+
     def rows_op(self, op, a, b=None, blend_frames=0):
         a = np.ascontiguousarray(a)
         if a.dtype not in (np.float32, np.float64):
