@@ -34,6 +34,34 @@ std::string cuda_msg(const char* what, cudaError_t e) {
     }                                                   \
   } while (0)
 
+// Runs a launcher (its kernel count, or < 0 when a launch failed) and counts its kernels in ctx->launches.
+#define NSF_LAUNCH(ctx, call)                           \
+  do {                                                  \
+    const int n__ = (call);                             \
+    if (n__ < 0) {                                      \
+      set_error(cuda_msg(#call, cudaGetLastError()));   \
+      return NSF_ERR_CUDA;                              \
+    }                                                   \
+    (ctx)->launches += n__;                             \
+  } while (0)
+
+nsf_status check_pcm_format(int32_t pcm_format) {
+  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
+  return NSF_OK;
+}
+
+nsf_status check_dtype(const char* fn, int32_t dtype) {
+  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error(std::string(fn) + ": bad dtype"); return NSF_ERR_BAD_ARG; }
+  return NSF_OK;
+}
+
+// off[0..n]: "<what> must be non-decreasing" unless every entry is >= the one before it.
+nsf_status check_nondecreasing(const std::string& what, const int64_t* off, int64_t n) {
+  for (int64_t i = 0; i < n; ++i)
+    if (off[i + 1] < off[i]) { set_error(what + " must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+  return NSF_OK;
+}
+
 inline size_t align_up(size_t v, size_t a = 256) { return (v + a - 1) / a * a; }
 
 // Bump allocator over a caller-provided (or context-owned) device buffer.
@@ -155,7 +183,7 @@ inline int64_t group_budget(int turn) {
 // Grid caps of the two front-end kernels inside the pipelined passes (nsf_kernels.cu, launch_absmax).
 constexpr int kPipelinedAbsmaxBlocks = 74, kPipelinedNormalizeBlocks = 148;
 
-struct Slot {  // one in-flight clip group of the host pipeline; slot 0 also serves the synchronous one-shot calls
+struct Slot {  // one in-flight clip group of the host pipeline
   cudaStream_t stream = nullptr;
   Arena in[2], out[3], work;   // device: the group's inputs, its results, kernel workspace
   // pinned twins of `in` / `out` for pageable caller buffers: an input is gathered into stage_in[i] before its
@@ -206,7 +234,6 @@ struct nsf_ctx {
   nsf::Slot slot[nsf::kSlots];
   int64_t launches = 0;
   bool profiling = false;
-  bool pipelined = false;     // set by the host passes around their nsf_extract_batch calls (front-end grid caps)
   cudaEvent_t stage_ev[nsf::kStages + 1] = {};
   bool stage_valid = false;
   std::vector<nsf::TapTable*> tap_tables;   // filter cache of the conversion calls, one per (rate pair, quality)
@@ -380,6 +407,24 @@ nsf_status desc_acquire(nsf_ctx* ctx, size_t bytes, DescEntry** out) {
   *out = &d;
   return NSF_OK;
 }
+// One descriptor block through the ring: fill(host) writes `bytes` into the next entry's pinned memory, and their upload
+// is queued on `s` to `dst`, or, when dst is NULL, to the entry's own device copy, reserved at dev_bytes >= bytes (a call
+// may keep device scratch behind its block).  The caller commits the entry once nothing on `s` reads it any more.
+template <typename Fill>
+nsf_status desc_upload(nsf_ctx* ctx, cudaStream_t s, size_t bytes, void* dst, size_t dev_bytes, DescEntry** out,
+                       Fill&& fill) {
+  DescEntry* de = nullptr;
+  nsf_status st = desc_acquire(ctx, bytes, &de);
+  if (st != NSF_OK) return st;
+  if (!dst) {
+    if ((st = de->dev.reserve(dev_bytes)) != NSF_OK) return st;
+    dst = de->dev.ptr;
+  }
+  fill(de->mem.ptr);
+  NSF_CUDA(cudaMemcpyAsync(dst, de->mem.ptr, bytes, cudaMemcpyHostToDevice, s));
+  *out = de;
+  return NSF_OK;
+}
 nsf_status desc_commit(DescEntry* d, cudaStream_t s) {
   NSF_CUDA(cudaEventRecord(d->copied, s));
   d->pending = true;
@@ -389,10 +434,20 @@ nsf_status desc_commit(DescEntry* d, cudaStream_t s) {
 // Host-side descriptor build + validation shared by the device and host entry points.
 nsf_status build_desc(const Plan& p, const int64_t* clip_offsets, int32_t n_clips, uint32_t flags,
                       const int64_t* out_row_offsets, HostDesc* d) {
+  if ((flags & NSF_NO_MFCC) && (flags & NSF_NO_AUTOCORR)) {
+    set_error("NSF_NO_MFCC | NSF_NO_AUTOCORR leaves nothing to compute"); return NSF_ERR_BAD_ARG;
+  }
+  // pad_signal=False exists for the autocorrelation branch only (librosa's STFT always centre-pads)
+  if ((flags & NSF_AC_NO_PAD) && !(flags & NSF_NO_MFCC)) {
+    set_error("NSF_AC_NO_PAD needs NSF_NO_MFCC: only the autocorrelation branch has a pad_signal switch");
+    return NSF_ERR_UNSUPPORTED;
+  }
   if (!clip_offsets || n_clips <= 0) {
     set_error("clip_offsets is NULL or n_clips <= 0");
     return NSF_ERR_BAD_ARG;
   }
+  const nsf_status st = check_nondecreasing("clip_offsets", clip_offsets, n_clips);
+  if (st != NSF_OK) return st;
   d->clip_off.resize(n_clips + 1);
   d->frame_off.resize(n_clips + 1);
   d->row_off.resize(n_clips + 1);
@@ -401,16 +456,14 @@ nsf_status build_desc(const Plan& p, const int64_t* clip_offsets, int32_t n_clip
   d->row_off[0] = out_row_offsets ? out_row_offsets[0] : 0;
   for (int i = 0; i < n_clips; ++i) {
     const int64_t len = clip_offsets[i + 1] - clip_offsets[i];
-    if (len < 0) { set_error("clip_offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
-    // NSF_AC_NO_PAD (pad_signal=False): frames are y[t H : t H + F], as many as fit
-    const bool no_pad = (flags & NSF_AC_NO_PAD) != 0;
-    const int64_t T = no_pad ? (len >= p.F ? nsf_guard_frames(len, p.F, p.H) : 0) : nsf_hop_frames(len, p.F, p.H);
+    int64_t R;
+    const int64_t T = clip_frames(len, p.F, p.H, flags, &R);
     // librosa.feature.delta(width=9) raises below 9 frames; the edge fix and reflect padding need
     // 2 frames and F/2 + 1 samples.  (The 9-frame *guard* of extract_features.py:16 counts
     // un-padded frames and belongs to the caller: see nsf_guard_frames.)
     const bool any_delta = (!(flags & NSF_NO_DELTAS) && !(flags & NSF_NO_MFCC)) ||
                            ((flags & NSF_AC_DELTAS) && !(flags & NSF_NO_AUTOCORR));
-    const int64_t need = any_delta ? kMinGuardFrames : (no_pad ? 1 : 2);
+    const int64_t need = any_delta ? kMinGuardFrames : ((flags & NSF_AC_NO_PAD) ? 1 : 2);
     if (T < need || len <= p.F / 2) {
       char buf[160];
       std::snprintf(buf, sizeof buf, "clip %d is too short: %lld hop-frames, required: %lld", i,
@@ -418,7 +471,6 @@ nsf_status build_desc(const Plan& p, const int64_t* clip_offsets, int32_t n_clip
       set_error(buf);
       return NSF_ERR_TOO_SHORT;
     }
-    const int64_t R = (flags & NSF_NO_REDUCE) ? T : (T + 1) / 2;
     d->clip_off[i] = clip_offsets[i] - origin;
     d->frame_off[i + 1] = d->frame_off[i] + T;
     if (out_row_offsets) {
@@ -502,17 +554,6 @@ nsf_status drain_slot(Slot* sl) {
   return NSF_OK;
 }
 
-// Slot 0, ready for a synchronous one-shot call: created, drained, owing no copy-out.
-nsf_status oneshot_slot(nsf_ctx* ctx, Slot** out) {
-  Slot* sl = &ctx->slot[0];
-  const nsf_status st = ensure_slot(sl);
-  if (st != NSF_OK) return st;
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  sl->n_pending = 0;
-  *out = sl;
-  return NSF_OK;
-}
-
 // Queues the copy of `bytes` of caller memory into the slot's device input i (reserved by the caller).  Pageable
 // memory is first gathered into the pinned stage_in[i] by the host, so that the copy itself stays asynchronous.
 nsf_status upload(Slot* sl, int i, const void* src, size_t bytes, bool dma) {
@@ -570,16 +611,152 @@ nsf_status run_groups(nsf_ctx* ctx, const int64_t* cost, int32_t n, Body&& body)
   return st;
 }
 
-// nsf_extract_batch of one group, from the slot's in[0] into its out[0], with the front-end grid caps of a pipelined
-// pass.
+// A synchronous host call as one group of run_groups: body(slot) reserves the slot's arenas and queues the uploads,
+// kernels and downloads.
+template <typename Body>
+nsf_status run_once(nsf_ctx* ctx, Body&& body) {
+  const int64_t cost[2] = {0, 0};
+  return run_groups(ctx, cost, 1, [&](int, int, Slot* sl) { return body(sl); });
+}
+
+// The body of nsf_extract_batch.  absmax_blocks / normalize_blocks cap the grids of the two front-end kernels (0: no
+// cap); the pipelined host passes cap them to stay off the copy engine's HBM share.
+nsf_status extract_enqueue(nsf_ctx* ctx, cudaStream_t s, const void* pcm_dev, int32_t pcm_format,
+                           const int64_t* clip_offsets_host, int32_t n_clips, uint32_t flags, float* out_dev,
+                           int64_t out_ld, const int64_t* out_row_offsets_host, float* y_norm_dev, void* workspace_dev,
+                           int64_t workspace_bytes, int absmax_blocks, int normalize_blocks) {
+  if (!ctx || !pcm_dev || !out_dev || !workspace_dev) { set_error("nsf_extract_batch: NULL argument"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_pcm_format(pcm_format);
+  if (st != NSF_OK) return st;
+  const Plan& p = ctx->plan->p;
+  const int cols = nsf_feature_cols(ctx->plan, flags);
+  if (out_ld < cols) { set_error("out_ld smaller than the feature width"); return NSF_ERR_BAD_ARG; }
+  if (workspace_bytes <= 0) { set_error("workspace_bytes must be positive; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
+  HostDesc& hd = ctx->hd_batch;
+  if ((st = build_desc(p, clip_offsets_host, n_clips, flags, out_row_offsets_host, &hd)) != NSF_OK) return st;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+
+  const bool normalize = (flags & NSF_PEAK_NORMALIZE) != 0;
+  const bool need_y = normalize || pcm_format == NSF_PCM_I16;
+  Sizes z;
+  z.total_samples = hd.total_samples; z.n_clips = n_clips;
+  z.frames_ub = hd.total_frames; z.rows_ub = hd.total_rows;
+  Layout L;
+  bool fits = false;
+  // 256-byte align the caller's pointer
+  char* wbase = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace_dev)));
+  const size_t wslack = static_cast<size_t>(wbase - static_cast<char*>(workspace_dev));
+  if (static_cast<size_t>(workspace_bytes) <= wslack) { set_error("workspace too small; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
+  const size_t wcap = static_cast<size_t>(workspace_bytes) - wslack;
+  plan_layout(p, z, flags, need_y && !y_norm_dev, wbase, wcap, &L, &fits);
+  if (!fits) { set_error("workspace too small; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
+
+  // descriptors: next entry of the pinned ring -> workspace, one stream-ordered upload, no host wait
+  const size_t n1 = static_cast<size_t>(n_clips) + 1;
+  const int64_t row_origin = hd.row_off[0];
+  DescEntry* de = nullptr;
+  st = desc_upload(ctx, s, 3 * n1 * sizeof(int64_t), L.clip_off, 0, &de, [&](void* mem) {
+    int64_t* h = static_cast<int64_t*>(mem);
+    for (size_t i = 0; i < n1; ++i) {
+      h[i] = hd.clip_off[i];
+      h[n1 + i] = hd.frame_off[i];
+      h[2 * n1 + i] = hd.row_off[i] - row_origin;
+    }
+  });
+  if (st != NSF_OK || (st = desc_commit(de, s)) != NSF_OK) return st;
+  NSF_CUDA(cudaMemsetAsync(wbase + L.zero_begin, 0, L.zero_bytes, s));
+
+  BatchView b;
+  b.clip_off = L.clip_off; b.frame_off = L.frame_off; b.row_off = L.row_off;
+  b.n_clips = n_clips; b.total_samples = hd.total_samples; b.total_frames = hd.total_frames;
+  b.total_rows = hd.total_rows;
+  float* out = out_dev + row_origin * out_ld;
+  const DeviceTables& t = ctx->tables;
+  StageTimer timer{ctx, s};
+
+  // stage 0: decode / peak normalise
+  timer.mark(0);
+  const float* y = static_cast<const float*>(pcm_dev);
+  if (need_y) {
+    float* ydst = y_norm_dev ? y_norm_dev : L.y;
+    if (normalize) NSF_LAUNCH(ctx, launch_absmax(s, pcm_dev, pcm_format, b, L.peak_bits, absmax_blocks));
+    NSF_LAUNCH(ctx, launch_normalize(s, pcm_dev, pcm_format, b, L.peak_bits, normalize, ydst, normalize_blocks));
+    y = ydst;
+  } else if (y_norm_dev) {
+    NSF_CUDA(cudaMemcpyAsync(y_norm_dev, pcm_dev, hd.total_samples * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  }
+
+  // the smoothing pass needs the un-smoothed rows in a scratch buffer
+  float* stage_out = (flags & NSF_SMOOTH) ? L.tmp_out : out;
+  const int64_t stage_ld = (flags & NSF_SMOOTH) ? cols : out_ld;
+  const bool reduce = !(flags & NSF_NO_REDUCE);
+  const bool deltas = !(flags & NSF_NO_DELTAS);
+  const bool do_mfcc = !(flags & NSF_NO_MFCC);
+  const int mfcc_cols = do_mfcc ? p.n_mfcc * (deltas ? 3 : 1) : 0;
+  DeviceTables t_ac = t;
+  if (flags & NSF_AC_NO_PAD) t_ac.pad = 0;    // autocorrelation only (build_desc)
+
+  // stages 1-3: STFT power -> mel -> dB (+ per-clip max)
+  bool fused_mel = false;
+  if (!do_mfcc) {
+    // autocorrelation block only
+  } else if (flags & NSF_DEBUG_SIMT_DFT) {
+    timer.mark(1);
+    NSF_LAUNCH(ctx, launch_fold32(s, t, b, y, L.a32));
+    timer.mark(2);
+    NSF_LAUNCH(ctx, launch_dft_simt(s, t, b, L.a32, L.power));
+  } else {
+    timer.mark(1);
+    NSF_LAUNCH(ctx, launch_stft_tc_fold(s, ctx->tc, t, b, y, L.tc_a));
+    timer.mark(2);
+    if (t.mel_col_ok && !(flags & NSF_DEBUG_UNFUSED_MEL)) {
+      // product path: STFT GEMM with the power -> mel -> dB epilogue fused (no power round trip)
+      NSF_LAUNCH(ctx, launch_stft_tc_mel(s, ctx->tc, t, b, L.tc_a, L.db, L.dbmax_key));
+      fused_mel = true;
+    } else {
+      NSF_LAUNCH(ctx, launch_stft_tc_gemm(s, ctx->tc, t, b, L.tc_a, L.power));
+    }
+  }
+  timer.mark(3);
+  if (do_mfcc && !fused_mel) NSF_LAUNCH(ctx, launch_mel_db(s, t, b, L.power, L.db, L.dbmax_key));
+  // stage 4: floor + DCT + CMVN statistics
+  timer.mark(4);
+  if (do_mfcc) {
+    NSF_LAUNCH(ctx, launch_dct_sum(s, t, b, L.db, L.dbmax_key, L.mfcc_raw, L.sum, L.sumsq));
+  }
+  // stage 5: CMVN + deltas + pair reduce -> columns [0, mfcc_cols)
+  timer.mark(5);
+  if (do_mfcc)
+    NSF_LAUNCH(ctx, launch_delta_reduce(s, b, L.mfcc_raw, p.n_mfcc, p.n_mfcc, L.sum, L.sumsq,
+                                        !(flags & NSF_NO_CMVN), deltas, reduce, stage_out, stage_ld, 0));
+  // stage 6: autocorrelation -> columns [mfcc_cols, ...)
+  timer.mark(6);
+  if (!(flags & NSF_NO_AUTOCORR)) {
+    if (flags & NSF_AC_DELTAS) {
+      BatchView bf = b;  // un-reduced: one row per hop-frame
+      bf.row_off = L.frame_off; bf.total_rows = hd.total_frames;
+      if (flags & NSF_DEBUG_FMA_AUTOCORR) NSF_LAUNCH(ctx, launch_autocorr(s, t_ac, bf, y, false, L.ac_raw, p.n_lags, 0));
+      else NSF_LAUNCH(ctx, launch_autocorr_mma(s, t_ac, bf, y, false, L.ac_raw, p.n_lags, 0));
+      NSF_LAUNCH(ctx, launch_delta_reduce(s, b, L.ac_raw, p.n_lags, p.n_lags, nullptr, nullptr, false, true,
+                                          reduce, stage_out, stage_ld, mfcc_cols));
+    } else {
+      if (flags & NSF_DEBUG_FMA_AUTOCORR) NSF_LAUNCH(ctx, launch_autocorr(s, t_ac, b, y, reduce, stage_out, stage_ld, mfcc_cols));
+      else NSF_LAUNCH(ctx, launch_autocorr_mma(s, t_ac, b, y, reduce, stage_out, stage_ld, mfcc_cols));
+    }
+  }
+  // stage 7: optional smoothing
+  timer.mark(7);
+  if (flags & NSF_SMOOTH) NSF_LAUNCH(ctx, launch_smooth(s, b, L.tmp_out, cols, cols, out, out_ld));
+  timer.finish();
+  return NSF_OK;
+}
+
+// extract_enqueue of one group of a pipelined host pass, from the slot's in[0] into its out[0].
 nsf_status extract_group(nsf_ctx* ctx, Slot* sl, int32_t pcm_format, const int64_t* clip_offsets, int32_t n,
                          uint32_t flags, int cols, float* y_norm_dev) {
-  ctx->pipelined = true;
-  const nsf_status st = nsf_extract_batch(ctx, sl->stream, sl->in[0].ptr, pcm_format, clip_offsets, n, flags,
-                                          static_cast<float*>(sl->out[0].ptr), cols, nullptr, y_norm_dev, sl->work.ptr,
-                                          static_cast<int64_t>(sl->work.bytes));
-  ctx->pipelined = false;
-  return st;
+  return extract_enqueue(ctx, sl->stream, sl->in[0].ptr, pcm_format, clip_offsets, n, flags,
+                         static_cast<float*>(sl->out[0].ptr), cols, nullptr, y_norm_dev, sl->work.ptr,
+                         static_cast<int64_t>(sl->work.bytes), kPipelinedAbsmaxBlocks, kPipelinedNormalizeBlocks);
 }
 
 // Enqueues k_collect_rows over n clips whose rows start at `audio` / `facial` and whose results start at `out_a` /
@@ -591,23 +768,20 @@ nsf_status collect_enqueue(nsf_ctx* ctx, cudaStream_t s, int32_t dtype, const vo
                            void* out_f) {
   const size_t n1 = static_cast<size_t>(n) + 1, bytes = 3 * n1 * sizeof(int64_t);
   DescEntry* de = nullptr;
-  nsf_status st = desc_acquire(ctx, bytes, &de);
+  const nsf_status st = desc_upload(ctx, s, bytes, nullptr, bytes, &de, [&](void* mem) {
+    int64_t* h = static_cast<int64_t*>(mem);
+    for (size_t i = 0; i < n1; ++i) {
+      h[i] = a_off[i] - a_off[0];
+      h[n1 + i] = f_off[i] - f_off[0];
+      h[2 * n1 + i] = o_off[i] - o_off[0];
+    }
+  });
   if (st != NSF_OK) return st;
-  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  for (size_t i = 0; i < n1; ++i) {
-    h[i] = a_off[i] - a_off[0];
-    h[n1 + i] = f_off[i] - f_off[0];
-    h[2 * n1 + i] = o_off[i] - o_off[0];
-  }
-  int64_t* d = static_cast<int64_t*>(de->dev.ptr);
-  NSF_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s));
+  const int64_t* d = static_cast<const int64_t*>(de->dev.ptr);
   CollectView v;
   v.a_off = d; v.f_off = d + n1; v.o_off = d + 2 * n1;
   v.n_clips = n; v.total_out_rows = o_off[n] - o_off[0]; v.flags = flags; v.blend_frames = blend_frames;
-  const int m = launch_collect(s, dtype, v, audio, a_cols, facial, f_cols, out_a, out_f);
-  if (m < 0) { set_error(cuda_msg("launch_collect", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += m;
+  NSF_LAUNCH(ctx, launch_collect(s, dtype, v, audio, a_cols, facial, f_cols, out_a, out_f));
   return desc_commit(de, s);     // recorded after the kernel: the entry (host and device) is reused only after it
 }
 
@@ -765,146 +939,8 @@ nsf_status nsf_extract_batch(nsf_ctx* ctx, void* cuda_stream, const void* pcm_de
                              const int64_t* clip_offsets_host, int32_t n_clips, uint32_t flags,
                              float* out_dev, int64_t out_ld, const int64_t* out_row_offsets_host,
                              float* y_norm_dev, void* workspace_dev, int64_t workspace_bytes) {
-  if (!ctx || !pcm_dev || !out_dev || !workspace_dev) { set_error("nsf_extract_batch: NULL argument"); return NSF_ERR_BAD_ARG; }
-  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
-  const Plan& p = ctx->plan->p;
-  const int cols = nsf_feature_cols(ctx->plan, flags);
-  if (out_ld < cols) { set_error("out_ld smaller than the feature width"); return NSF_ERR_BAD_ARG; }
-  if (workspace_bytes <= 0) { set_error("workspace_bytes must be positive; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
-  HostDesc& hd = ctx->hd_batch;
-  nsf_status st = build_desc(p, clip_offsets_host, n_clips, flags, out_row_offsets_host, &hd);
-  if (st != NSF_OK) return st;
-  NSF_CUDA(cudaSetDevice(ctx->device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-
-  const bool normalize = (flags & NSF_PEAK_NORMALIZE) != 0;
-  const bool need_y = normalize || pcm_format == NSF_PCM_I16;
-  Sizes z;
-  z.total_samples = hd.total_samples; z.n_clips = n_clips;
-  z.frames_ub = hd.total_frames; z.rows_ub = hd.total_rows;
-  Layout L;
-  bool fits = false;
-  // 256-byte align the caller's pointer
-  char* wbase = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace_dev)));
-  const size_t wslack = static_cast<size_t>(wbase - static_cast<char*>(workspace_dev));
-  if (static_cast<size_t>(workspace_bytes) <= wslack) { set_error("workspace too small; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
-  const size_t wcap = static_cast<size_t>(workspace_bytes) - wslack;
-  plan_layout(p, z, flags, need_y && !y_norm_dev, wbase, wcap, &L, &fits);
-  if (!fits) { set_error("workspace too small; size it with nsf_workspace_bytes()"); return NSF_ERR_WORKSPACE; }
-
-  // descriptors: next entry of the pinned ring -> device, one stream-ordered upload, no host wait
-  const size_t n1 = static_cast<size_t>(n_clips) + 1;
-  DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, 3 * n1 * sizeof(int64_t), &de)) != NSF_OK) return st;
-  int64_t* hstage = static_cast<int64_t*>(de->mem.ptr);
-  const int64_t row_origin = hd.row_off[0];
-  for (size_t i = 0; i < n1; ++i) {
-    hstage[i] = hd.clip_off[i];
-    hstage[n1 + i] = hd.frame_off[i];
-    hstage[2 * n1 + i] = hd.row_off[i] - row_origin;
-  }
-  NSF_CUDA(cudaMemcpyAsync(L.clip_off, hstage, 3 * n1 * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-  if ((st = desc_commit(de, s)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemsetAsync(wbase + L.zero_begin, 0, L.zero_bytes, s));
-
-  BatchView b;
-  b.clip_off = L.clip_off; b.frame_off = L.frame_off; b.row_off = L.row_off;
-  b.n_clips = n_clips; b.total_samples = hd.total_samples; b.total_frames = hd.total_frames;
-  b.total_rows = hd.total_rows;
-  float* out = out_dev + row_origin * out_ld;
-  const DeviceTables& t = ctx->tables;
-  StageTimer timer{ctx, s};
-  int launched = 0;
-#define NSF_LAUNCH(expr)                                                   \
-  do {                                                                     \
-    const int n__ = (expr);                                                \
-    if (n__ < 0) { set_error(cuda_msg(#expr, cudaGetLastError())); return NSF_ERR_CUDA; } \
-    launched += n__;                                                       \
-  } while (0)
-
-  // stage 0: decode / peak normalise
-  timer.mark(0);
-  const float* y = static_cast<const float*>(pcm_dev);
-  if (need_y) {
-    float* ydst = y_norm_dev ? y_norm_dev : L.y;
-    const bool capped = ctx->pipelined;           // inside a pipelined host pass: stay off the copy engine's HBM share
-    if (normalize) NSF_LAUNCH(launch_absmax(s, pcm_dev, pcm_format, b, L.peak_bits, capped ? kPipelinedAbsmaxBlocks : 0));
-    NSF_LAUNCH(launch_normalize(s, pcm_dev, pcm_format, b, L.peak_bits, normalize, ydst, capped ? kPipelinedNormalizeBlocks : 0));
-    y = ydst;
-  } else if (y_norm_dev) {
-    NSF_CUDA(cudaMemcpyAsync(y_norm_dev, pcm_dev, hd.total_samples * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  }
-
-  // the smoothing pass needs the un-smoothed rows in a scratch buffer
-  float* stage_out = (flags & NSF_SMOOTH) ? L.tmp_out : out;
-  const int64_t stage_ld = (flags & NSF_SMOOTH) ? cols : out_ld;
-  const bool reduce = !(flags & NSF_NO_REDUCE);
-  const bool deltas = !(flags & NSF_NO_DELTAS);
-  const bool do_mfcc = !(flags & NSF_NO_MFCC);
-  const int mfcc_cols = do_mfcc ? p.n_mfcc * (deltas ? 3 : 1) : 0;
-  if (!do_mfcc && (flags & NSF_NO_AUTOCORR)) { set_error("NSF_NO_MFCC | NSF_NO_AUTOCORR leaves nothing to compute"); return NSF_ERR_BAD_ARG; }
-  // pad_signal=False exists for the autocorrelation branch only (librosa's STFT always centre-pads)
-  DeviceTables t_ac = t;
-  if (flags & NSF_AC_NO_PAD) {
-    if (do_mfcc) { set_error("NSF_AC_NO_PAD needs NSF_NO_MFCC: only the autocorrelation branch has a pad_signal switch"); return NSF_ERR_UNSUPPORTED; }
-    t_ac.pad = 0;
-  }
-
-  // stages 1-3: STFT power -> mel -> dB (+ per-clip max)
-  bool fused_mel = false;
-  if (!do_mfcc) {
-    // autocorrelation block only
-  } else if (flags & NSF_DEBUG_SIMT_DFT) {
-    timer.mark(1);
-    NSF_LAUNCH(launch_fold32(s, t, b, y, L.a32));
-    timer.mark(2);
-    NSF_LAUNCH(launch_dft_simt(s, t, b, L.a32, L.power));
-  } else {
-    timer.mark(1);
-    NSF_LAUNCH(launch_stft_tc_fold(s, ctx->tc, t, b, y, L.tc_a));
-    timer.mark(2);
-    if (t.mel_col_ok && !(flags & NSF_DEBUG_UNFUSED_MEL)) {
-      // product path: STFT GEMM with the power -> mel -> dB epilogue fused (no power round trip)
-      NSF_LAUNCH(launch_stft_tc_mel(s, ctx->tc, t, b, L.tc_a, L.db, L.dbmax_key));
-      fused_mel = true;
-    } else {
-      NSF_LAUNCH(launch_stft_tc_gemm(s, ctx->tc, t, b, L.tc_a, L.power));
-    }
-  }
-  timer.mark(3);
-  if (do_mfcc && !fused_mel) NSF_LAUNCH(launch_mel_db(s, t, b, L.power, L.db, L.dbmax_key));
-  // stage 4: floor + DCT + CMVN statistics
-  timer.mark(4);
-  if (do_mfcc) {
-    NSF_LAUNCH(launch_dct_sum(s, t, b, L.db, L.dbmax_key, L.mfcc_raw, L.sum, L.sumsq));
-  }
-  // stage 5: CMVN + deltas + pair reduce -> columns [0, mfcc_cols)
-  timer.mark(5);
-  if (do_mfcc)
-    NSF_LAUNCH(launch_delta_reduce(s, b, L.mfcc_raw, p.n_mfcc, p.n_mfcc, L.sum, L.sumsq,
-                                   !(flags & NSF_NO_CMVN), deltas, reduce, stage_out, stage_ld, 0));
-  // stage 6: autocorrelation -> columns [mfcc_cols, ...)
-  timer.mark(6);
-  if (!(flags & NSF_NO_AUTOCORR)) {
-    if (flags & NSF_AC_DELTAS) {
-      BatchView bf = b;  // un-reduced: one row per hop-frame
-      bf.row_off = L.frame_off; bf.total_rows = hd.total_frames;
-      if (flags & NSF_DEBUG_FMA_AUTOCORR) NSF_LAUNCH(launch_autocorr(s, t_ac, bf, y, false, L.ac_raw, p.n_lags, 0));
-      else NSF_LAUNCH(launch_autocorr_mma(s, t_ac, bf, y, false, L.ac_raw, p.n_lags, 0));
-      NSF_LAUNCH(launch_delta_reduce(s, b, L.ac_raw, p.n_lags, p.n_lags, nullptr, nullptr, false, true,
-                                     reduce, stage_out, stage_ld, mfcc_cols));
-    } else {
-      if (flags & NSF_DEBUG_FMA_AUTOCORR) NSF_LAUNCH(launch_autocorr(s, t_ac, b, y, reduce, stage_out, stage_ld, mfcc_cols));
-      else NSF_LAUNCH(launch_autocorr_mma(s, t_ac, b, y, reduce, stage_out, stage_ld, mfcc_cols));
-    }
-  }
-  // stage 7: optional smoothing
-  timer.mark(7);
-  if (flags & NSF_SMOOTH) NSF_LAUNCH(launch_smooth(s, b, L.tmp_out, cols, cols, out, out_ld));
-  timer.finish();
-  ctx->launches += launched;
-#undef NSF_LAUNCH
-  return NSF_OK;
+  return extract_enqueue(ctx, static_cast<cudaStream_t>(cuda_stream), pcm_dev, pcm_format, clip_offsets_host, n_clips,
+                         flags, out_dev, out_ld, out_row_offsets_host, y_norm_dev, workspace_dev, workspace_bytes, 0, 0);
 }
 
 // ---- host-buffer pipeline ------------------------------------------------------------------------
@@ -914,14 +950,14 @@ nsf_status nsf_extract_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_form
   if (!ctx || !pcm_host || !out_host || !clip_offsets || n_clips <= 0) {
     set_error("nsf_extract_host: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_pcm_format(pcm_format);
+  if (st != NSF_OK) return st;
   const Plan& p = ctx->plan->p;
   const int cols = nsf_feature_cols(ctx->plan, flags);
   if (out_ld < cols) { set_error("out_ld smaller than the feature width"); return NSF_ERR_BAD_ARG; }
-  // validate everything up front so nothing is launched for a bad batch
+  // validate everything up front so nothing is queued for a bad batch
   HostDesc& all = ctx->hd_all;
-  nsf_status st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all);
-  if (st != NSF_OK) return st;
+  if ((st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all)) != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4, row_bytes = static_cast<size_t>(cols) * sizeof(float);
   // pageable caller buffers go through the slot's pinned staging arenas: the host copies group g + 1 in (and
@@ -953,46 +989,42 @@ nsf_status nsf_normalize_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_fo
   if (!ctx || !pcm_host || !clip_offsets || !y_host || n_clips <= 0) {
     set_error("nsf_normalize_host: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
-  for (int i = 0; i < n_clips; ++i)
-    if (clip_offsets[i + 1] < clip_offsets[i]) { set_error("clip_offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
-  NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = nullptr;
-  nsf_status st = oneshot_slot(ctx, &sl);
+  nsf_status st = check_pcm_format(pcm_format);
+  if (st == NSF_OK) st = check_nondecreasing("clip_offsets", clip_offsets, n_clips);
   if (st != NSF_OK) return st;
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
   const int64_t samples = clip_offsets[n_clips] - clip_offsets[0];
+  NSF_CUDA(cudaSetDevice(ctx->device));
   if (samples == 0) return NSF_OK;
   const size_t n1 = static_cast<size_t>(n_clips) + 1;
-  // work arena: [clip_off n1 x int64][peak n x u32]
-  const size_t off_b = align_up(n1 * sizeof(int64_t));
-  if ((st = sl->in[0].reserve(samples * esz)) != NSF_OK) return st;
-  if ((st = sl->out[0].reserve(samples * sizeof(float))) != NSF_OK) return st;
-  if ((st = sl->work.reserve(off_b + align_up(n_clips * sizeof(uint32_t)))) != NSF_OK) return st;
-  DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, n1 * sizeof(int64_t), &de)) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  for (size_t i = 0; i < n1; ++i) h[i] = clip_offsets[i] - clip_offsets[0];
-  int64_t* d_off = static_cast<int64_t*>(sl->work.ptr);
-  uint32_t* d_peak = reinterpret_cast<uint32_t*>(static_cast<char*>(sl->work.ptr) + off_b);
-  NSF_CUDA(cudaMemcpyAsync(d_off, h, n1 * sizeof(int64_t), cudaMemcpyHostToDevice, sl->stream));
-  if ((st = desc_commit(de, sl->stream)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemsetAsync(d_peak, 0, n_clips * sizeof(uint32_t), sl->stream));
-  const char* src = static_cast<const char*>(pcm_host) + clip_offsets[0] * esz;
-  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, src, samples * esz, cudaMemcpyHostToDevice, sl->stream));
-  BatchView b{};
-  b.clip_off = d_off; b.frame_off = d_off; b.row_off = d_off;
-  b.n_clips = n_clips; b.total_samples = samples;
-  int n = launch_absmax(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak);
-  if (n < 0) { set_error(cuda_msg("launch_absmax", cudaGetLastError())); return NSF_ERR_CUDA; }
-  int m = launch_normalize(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak, true, static_cast<float*>(sl->out[0].ptr));
-  if (m < 0) { set_error(cuda_msg("launch_normalize", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n + m;
-  NSF_CUDA(cudaMemcpyAsync(y_host, sl->out[0].ptr, samples * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-  if (peaks_host)  // float bits of a non-negative float: copy as-is
-    NSF_CUDA(cudaMemcpyAsync(peaks_host, d_peak, n_clips * sizeof(uint32_t), cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  return NSF_OK;
+  // in[0] = PCM, out[0] = y, out[1] = per-clip peaks, work = clip offsets
+  return run_once(ctx, [&](Slot* sl) -> nsf_status {
+    nsf_status st;
+    if ((st = sl->in[0].reserve(samples * esz)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(samples * sizeof(float))) != NSF_OK) return st;
+    if ((st = sl->out[1].reserve(n_clips * sizeof(uint32_t))) != NSF_OK) return st;
+    if ((st = sl->work.reserve(n1 * sizeof(int64_t))) != NSF_OK) return st;
+    int64_t* d_off = static_cast<int64_t*>(sl->work.ptr);
+    uint32_t* d_peak = static_cast<uint32_t*>(sl->out[1].ptr);
+    DescEntry* de = nullptr;
+    st = desc_upload(ctx, sl->stream, n1 * sizeof(int64_t), d_off, 0, &de, [&](void* mem) {
+      int64_t* h = static_cast<int64_t*>(mem);
+      for (size_t i = 0; i < n1; ++i) h[i] = clip_offsets[i] - clip_offsets[0];
+    });
+    if (st != NSF_OK || (st = desc_commit(de, sl->stream)) != NSF_OK) return st;
+    NSF_CUDA(cudaMemsetAsync(d_peak, 0, n_clips * sizeof(uint32_t), sl->stream));
+    if ((st = upload(sl, 0, static_cast<const char*>(pcm_host) + clip_offsets[0] * esz, samples * esz, true)) != NSF_OK)
+      return st;
+    BatchView b{};
+    b.clip_off = d_off; b.frame_off = d_off; b.row_off = d_off;
+    b.n_clips = n_clips; b.total_samples = samples;
+    NSF_LAUNCH(ctx, launch_absmax(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak));
+    NSF_LAUNCH(ctx, launch_normalize(sl->stream, sl->in[0].ptr, pcm_format, b, d_peak, true, static_cast<float*>(sl->out[0].ptr)));
+    const size_t y_bytes = samples * sizeof(float), p_bytes = n_clips * sizeof(uint32_t);
+    if ((st = download(sl, 0, y_host, y_bytes, y_bytes, 1, true)) != NSF_OK) return st;
+    // float bits of a non-negative float: copied as-is
+    return peaks_host ? download(sl, 1, peaks_host, p_bytes, p_bytes, 1, true) : NSF_OK;
+  });
 }
 
 // ---- sample-rate conversion + WAV conversion -----------------------------------------------------------
@@ -1135,21 +1167,15 @@ nsf_status convert_enqueue(nsf_ctx* ctx, cudaStream_t s, const void* payload_dev
   if (tiles[0] > INT32_MAX || tiles[1] > INT32_MAX) { set_error("nsf_convert: batch too large for one launch"); return NSF_ERR_UNSUPPORTED; }
   const size_t bytes = cl.size() * sizeof(ConvClip);
   DescEntry* de = nullptr;
-  nsf_status st = desc_acquire(ctx, bytes, &de);
+  const nsf_status st =
+      desc_upload(ctx, s, bytes, nullptr, bytes, &de, [&](void* mem) { std::memcpy(mem, cl.data(), bytes); });
   if (st != NSF_OK) return st;
-  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
-  std::memcpy(de->mem.ptr, cl.data(), bytes);
   const ConvClip* d = static_cast<const ConvClip*>(de->dev.ptr);
-  NSF_CUDA(cudaMemcpyAsync(de->dev.ptr, de->mem.ptr, bytes, cudaMemcpyHostToDevice, s));
-  int launched = 0;
   for (int kind = 0; kind < 2; ++kind) {
     const ConvClip* first = d + (kind == 0 ? 0 : n_kind[0]);
-    const int m = launch_convert(s, kind == 1, first, n_kind[kind], tiles[kind],
-                                 kind == 1 ? static_cast<size_t>(max_window) * sizeof(double) : 0, payload_dev, out_dev);
-    if (m < 0) { set_error(cuda_msg("launch_convert", cudaGetLastError())); return NSF_ERR_CUDA; }
-    launched += m;
+    NSF_LAUNCH(ctx, launch_convert(s, kind == 1, first, n_kind[kind], tiles[kind],
+                                   kind == 1 ? static_cast<size_t>(max_window) * sizeof(double) : 0, payload_dev, out_dev));
   }
-  ctx->launches += launched;
   return desc_commit(de, s);     // recorded after the kernels: the entry (host and device) is reused only after them
 }
 }  // namespace
@@ -1157,26 +1183,26 @@ nsf_status convert_enqueue(nsf_ctx* ctx, cudaStream_t s, const void* payload_dev
 nsf_status nsf_resample_host(nsf_ctx* ctx, const void* pcm_host, int32_t pcm_format, int64_t n_in, int32_t orig_sr,
                              int32_t target_sr, float* out_host, int64_t out_capacity) {
   if (!ctx || !pcm_host || !out_host || n_in <= 0) { set_error("nsf_resample_host: NULL argument or empty input"); return NSF_ERR_BAD_ARG; }
-  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
+  const nsf_status st = check_pcm_format(pcm_format);
+  if (st != NSF_OK) return st;
   if (orig_sr <= 0 || target_sr <= 0) { set_error("nsf_resample_host: rates must be positive"); return NSF_ERR_BAD_ARG; }
   const int64_t n_out = nsf_resample_len(n_in, orig_sr, target_sr);
   if (out_capacity < n_out) { set_error("nsf_resample_host: out_capacity < nsf_resample_len()"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = nullptr;
-  nsf_status st = oneshot_slot(ctx, &sl);
-  if (st != NSF_OK) return st;
   // one mono clip of the conversion kernel (float32 samples are its f32 encoding, int16 its i16 encoding)
   const nsf_pcm_source src{0, n_in, pcm_format == NSF_PCM_I16 ? NSF_ENC_I16 : NSF_ENC_F32, 1, orig_sr, 0};
-  const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
+  const size_t in_bytes = static_cast<size_t>(n_in) * (pcm_format == NSF_PCM_I16 ? 2 : 4);
+  const size_t out_bytes = static_cast<size_t>(n_out) * sizeof(float);
   const int64_t off[2] = {0, n_out};
-  if ((st = sl->in[0].reserve(static_cast<size_t>(n_in) * esz)) != NSF_OK) return st;
-  if ((st = sl->out[0].reserve(static_cast<size_t>(n_out) * sizeof(float))) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, pcm_host, static_cast<size_t>(n_in) * esz, cudaMemcpyHostToDevice, sl->stream));
-  if ((st = convert_enqueue(ctx, sl->stream, sl->in[0].ptr, &src, 1, target_sr, off, static_cast<float*>(sl->out[0].ptr),
-                            true)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(out_host, sl->out[0].ptr, static_cast<size_t>(n_out) * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  return NSF_OK;
+  return run_once(ctx, [&](Slot* sl) -> nsf_status {
+    nsf_status st;
+    if ((st = sl->in[0].reserve(in_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(out_bytes)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, pcm_host, in_bytes, true)) != NSF_OK) return st;
+    if ((st = convert_enqueue(ctx, sl->stream, sl->in[0].ptr, &src, 1, target_sr, off, static_cast<float*>(sl->out[0].ptr),
+                              true)) != NSF_OK) return st;
+    return download(sl, 0, out_host, out_bytes, out_bytes, 1, true);
+  });
 }
 
 nsf_status nsf_convert_offsets(const nsf_pcm_source* sources, int32_t n, int32_t target_sr, int64_t payload_bytes,
@@ -1244,15 +1270,21 @@ nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payl
 }
 
 // ---- collect ---------------------------------------------------------------------------------------
-static nsf_status collect_offsets(const int64_t* a_off, const int64_t* f_off, int32_t n, uint32_t flags,
-                                  int32_t blend_frames, const int64_t* o_off_in, std::vector<int64_t>* o_off) {
+// Checks shared by the collect calls (element type, column counts, offsets) and their output packing: o_off is the
+// prefix sum of nsf_collect_rows(), and must equal o_off_in when that is given.
+static nsf_status collect_offsets(int32_t dtype, int32_t a_cols, int32_t f_cols, const int64_t* a_off,
+                                  const int64_t* f_off, int32_t n, uint32_t flags, int32_t blend_frames,
+                                  const int64_t* o_off_in, std::vector<int64_t>* o_off) {
+  nsf_status st = check_dtype("nsf_collect", dtype);
+  if (st != NSF_OK) return st;
+  if (a_cols <= 0 || f_cols <= 0) { set_error("nsf_collect: column counts must be positive"); return NSF_ERR_BAD_ARG; }
   if (!a_off || !f_off || n <= 0) { set_error("nsf_collect: NULL offsets or n_clips <= 0"); return NSF_ERR_BAD_ARG; }
+  if ((st = check_nondecreasing("nsf_collect: offsets", a_off, n)) != NSF_OK ||
+      (st = check_nondecreasing("nsf_collect: offsets", f_off, n)) != NSF_OK) return st;
   o_off->resize(n + 1);
   (*o_off)[0] = 0;
   for (int i = 0; i < n; ++i) {
-    const int64_t na = a_off[i + 1] - a_off[i], nf = f_off[i + 1] - f_off[i];
-    if (na < 0 || nf < 0) { set_error("nsf_collect: offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
-    const int64_t r = nsf_collect_rows(na, nf, flags, blend_frames);
+    const int64_t r = nsf_collect_rows(a_off[i + 1] - a_off[i], f_off[i + 1] - f_off[i], flags, blend_frames);
     if (o_off_in && o_off_in[i + 1] - o_off_in[i] != r) {
       set_error("nsf_collect: out_offsets is not the prefix sum of nsf_collect_rows()");
       return NSF_ERR_BAD_ARG;
@@ -1270,12 +1302,9 @@ nsf_status nsf_collect_batch(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, con
   if (!ctx || !audio_dev || !facial_dev || !out_audio_dev || !out_facial_dev) {
     set_error("nsf_collect_batch: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if ((dtype != NSF_F32 && dtype != NSF_F64) || audio_cols <= 0 || facial_cols <= 0) {
-    set_error("nsf_collect_batch: bad dtype or column count"); return NSF_ERR_BAD_ARG;
-  }
   std::vector<int64_t> o_off;
-  nsf_status st = collect_offsets(audio_offsets_host, facial_offsets_host, n_clips, collect_flags,
-                                  blend_frames, out_offsets_host, &o_off);
+  nsf_status st = collect_offsets(dtype, audio_cols, facial_cols, audio_offsets_host, facial_offsets_host, n_clips,
+                                  collect_flags, blend_frames, out_offsets_host, &o_off);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
@@ -1295,33 +1324,29 @@ nsf_status nsf_collect_host(nsf_ctx* ctx, int32_t dtype, const void* audio_host,
   if (!ctx || !audio_host || !facial_host || !out_audio_host || !out_facial_host) {
     set_error("nsf_collect_host: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if ((dtype != NSF_F32 && dtype != NSF_F64) || audio_cols <= 0 || facial_cols <= 0) {
-    set_error("nsf_collect_host: bad dtype or column count"); return NSF_ERR_BAD_ARG;
-  }
   std::vector<int64_t> o_off;
-  nsf_status st = collect_offsets(a_off, f_off, n_clips, collect_flags, blend_frames, nullptr, &o_off);
+  nsf_status st = collect_offsets(dtype, audio_cols, facial_cols, a_off, f_off, n_clips, collect_flags, blend_frames,
+                                  nullptr, &o_off);
   if (st != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = nullptr;
-  if ((st = oneshot_slot(ctx, &sl)) != NSF_OK) return st;
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
   const size_t a_bytes = (a_off[n_clips] - a_off[0]) * audio_cols * esz, f_bytes = (f_off[n_clips] - f_off[0]) * facial_cols * esz;
   const size_t oa_bytes = o_off[n_clips] * audio_cols * esz, of_bytes = o_off[n_clips] * facial_cols * esz;
-  if ((st = sl->in[0].reserve(a_bytes)) != NSF_OK) return st;
-  if ((st = sl->in[1].reserve(f_bytes)) != NSF_OK) return st;
-  if ((st = sl->out[0].reserve(oa_bytes)) != NSF_OK) return st;
-  if ((st = sl->out[1].reserve(of_bytes)) != NSF_OK) return st;
-  const char* ah = static_cast<const char*>(audio_host) + a_off[0] * audio_cols * esz;
-  const char* fh = static_cast<const char*>(facial_host) + f_off[0] * facial_cols * esz;
-  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, ah, a_bytes, cudaMemcpyHostToDevice, sl->stream));
-  NSF_CUDA(cudaMemcpyAsync(sl->in[1].ptr, fh, f_bytes, cudaMemcpyHostToDevice, sl->stream));
-  if ((st = collect_enqueue(ctx, sl->stream, dtype, sl->in[0].ptr, audio_cols, a_off, sl->in[1].ptr, facial_cols, f_off,
-                            o_off.data(), n_clips, collect_flags, blend_frames, sl->out[0].ptr, sl->out[1].ptr)) != NSF_OK)
-    return st;
-  NSF_CUDA(cudaMemcpyAsync(out_audio_host, sl->out[0].ptr, oa_bytes, cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaMemcpyAsync(out_facial_host, sl->out[1].ptr, of_bytes, cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  return NSF_OK;
+  return run_once(ctx, [&](Slot* sl) -> nsf_status {
+    nsf_status st;
+    if ((st = sl->in[0].reserve(a_bytes)) != NSF_OK) return st;
+    if ((st = sl->in[1].reserve(f_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(oa_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[1].reserve(of_bytes)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, static_cast<const char*>(audio_host) + a_off[0] * audio_cols * esz, a_bytes, true)) != NSF_OK ||
+        (st = upload(sl, 1, static_cast<const char*>(facial_host) + f_off[0] * facial_cols * esz, f_bytes, true)) != NSF_OK)
+      return st;
+    if ((st = collect_enqueue(ctx, sl->stream, dtype, sl->in[0].ptr, audio_cols, a_off, sl->in[1].ptr, facial_cols, f_off,
+                              o_off.data(), n_clips, collect_flags, blend_frames, sl->out[0].ptr, sl->out[1].ptr)) != NSF_OK)
+      return st;
+    if ((st = download(sl, 0, out_audio_host, oa_bytes, oa_bytes, 1, true)) != NSF_OK) return st;
+    return download(sl, 1, out_facial_host, of_bytes, of_bytes, 1, true);
+  });
 }
 
 // ---- fused extract + collect (dataset builders) -------------------------------------------------------
@@ -1334,15 +1359,16 @@ nsf_status nsf_extract_collect_host(nsf_ctx* ctx, const void* pcm_host, int32_t 
       n_clips <= 0 || facial_cols <= 0) {
     set_error("nsf_extract_collect_host: NULL argument"); return NSF_ERR_BAD_ARG;
   }
-  if (pcm_format != NSF_PCM_F32 && pcm_format != NSF_PCM_I16) { set_error("unknown pcm_format"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_pcm_format(pcm_format);
+  if (st != NSF_OK) return st;
   const Plan& p = ctx->plan->p;
   const int cols = nsf_feature_cols(ctx->plan, flags);
   HostDesc& all = ctx->hd_all;
-  nsf_status st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all);
-  if (st != NSF_OK) return st;
+  if ((st = build_desc(p, clip_offsets, n_clips, flags, nullptr, &all)) != NSF_OK) return st;
   // output packing over the whole batch (validates the facial offsets)
   std::vector<int64_t> o_all;
-  if ((st = collect_offsets(all.row_off.data(), f_off, n_clips, collect_flags, blend_frames, nullptr, &o_all)) != NSF_OK) return st;
+  if ((st = collect_offsets(NSF_F32, cols, facial_cols, all.row_off.data(), f_off, n_clips, collect_flags, blend_frames,
+                            nullptr, &o_all)) != NSF_OK) return st;
   NSF_CUDA(cudaSetDevice(ctx->device));
   const size_t esz = pcm_format == NSF_PCM_I16 ? 2 : 4;
   const size_t row_bytes = static_cast<size_t>(cols) * sizeof(float), fac_row_bytes = static_cast<size_t>(facial_cols) * sizeof(float);
@@ -1383,9 +1409,9 @@ nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_hos
   if (!ctx || !rows_host || !row_off || !text_host || !text_off || cols < 1 || n_files < 0) {
     set_error("nsf_format_csv_host: NULL argument, cols < 1 or n_files < 0"); return NSF_ERR_BAD_ARG;
   }
-  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_format_csv_host: bad dtype"); return NSF_ERR_BAD_ARG; }
-  for (int i = 0; i < n_files; ++i)
-    if (row_off[i + 1] < row_off[i]) { set_error("nsf_format_csv_host: offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_dtype("nsf_format_csv_host", dtype);
+  if (st == NSF_OK) st = check_nondecreasing("nsf_format_csv_host: offsets", row_off, n_files);
+  if (st != NSF_OK) return st;
   const int64_t n_rows = row_off[n_files] - row_off[0];
   if (text_capacity < nsf_csv_bytes_bound(n_rows, cols, n_files)) {
     set_error("nsf_format_csv_host: text_capacity below nsf_csv_bytes_bound()"); return NSF_ERR_BAD_ARG;
@@ -1411,9 +1437,7 @@ nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_hos
     if ((st = sl->stage_out[1].reserve(std::max<size_t>(len_bytes, 1))) != NSF_OK) return st;
     if (nr > 0) {   // the group's row lengths, and with them its text size: the group's one wait
       if ((st = upload(sl, 0, static_cast<const char*>(rows_host) + r0 * row_bytes, nr * row_bytes, in_dma)) != NSF_OK) return st;
-      const int m = launch_csv_lengths(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int64_t*>(sl->out[1].ptr));
-      if (m < 0) { set_error(cuda_msg("launch_csv_lengths", cudaGetLastError())); return NSF_ERR_CUDA; }
-      ctx->launches += m;
+      NSF_LAUNCH(ctx, launch_csv_lengths(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int64_t*>(sl->out[1].ptr)));
       if ((st = download(sl, 1, sl->stage_out[1].ptr, len_bytes, len_bytes, 1, true)) != NSF_OK) return st;
       NSF_CUDA(cudaStreamSynchronize(sl->stream));
     }
@@ -1429,10 +1453,8 @@ nsf_status nsf_format_csv_host(nsf_ctx* ctx, int32_t dtype, const void* rows_hos
     }
     if ((st = upload(sl, 1, pos, pos_bytes, true)) != NSF_OK) return st;
     if ((st = sl->out[0].reserve(at)) != NSF_OK) return st;
-    const int m = launch_csv_write(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int32_t>(nf),
-                                   static_cast<const int64_t*>(sl->in[1].ptr), static_cast<char*>(sl->out[0].ptr));
-    if (m < 0) { set_error(cuda_msg("launch_csv_write", cudaGetLastError())); return NSF_ERR_CUDA; }
-    ctx->launches += m;
+    NSF_LAUNCH(ctx, launch_csv_write(sl->stream, dtype, sl->in[0].ptr, nr, cols, static_cast<int32_t>(nf),
+                                     static_cast<const int64_t*>(sl->in[1].ptr), static_cast<char*>(sl->out[0].ptr)));
     return download(sl, 0, text_host + text_off[first], at, at, 1, out_dma);
   });
 }
@@ -1448,13 +1470,10 @@ nsf_status csv_text_args(const char* fn, nsf_ctx* ctx, const char* text_dev, con
   }
   if (n_files == 0) return NSF_OK;
   if (text_off[0] < 0) { std::snprintf(buf, sizeof buf, "%s: negative text offset", fn); set_error(buf); return NSF_ERR_BAD_ARG; }
+  const nsf_status st = check_nondecreasing(std::string(fn) + ": text offsets", text_off, n_files);
+  if (st != NSF_OK) return st;
   tile_off->assign(n_files + 1, 0);
-  for (int i = 0; i < n_files; ++i) {
-    if (text_off[i + 1] < text_off[i]) {
-      std::snprintf(buf, sizeof buf, "%s: text offsets must be non-decreasing", fn); set_error(buf); return NSF_ERR_BAD_ARG;
-    }
-    (*tile_off)[i + 1] = (*tile_off)[i] + csv_tiles(text_off[i], text_off[i + 1]);
-  }
+  for (int i = 0; i < n_files; ++i) (*tile_off)[i + 1] = (*tile_off)[i] + csv_tiles(text_off[i], text_off[i + 1]);
   if (text_off[n_files] > text_off[0] && (!text_dev || reinterpret_cast<uintptr_t>(text_dev) % 16 != 0)) {
     std::snprintf(buf, sizeof buf, "%s: text_dev is NULL or not 16-byte aligned", fn); set_error(buf); return NSF_ERR_BAD_ARG;
   }
@@ -1476,30 +1495,27 @@ nsf_status nsf_csv_row_offsets(nsf_ctx* ctx, void* cuda_stream, const char* text
   NSF_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
   const size_t n1 = static_cast<size_t>(n_files) + 1, n_tiles = static_cast<size_t>(tile_off[n_files]);
-  // ring entry: host [text_off | tile_off | row_off (download)]; device [text_off | tile_off | row_off | tile_start |
-  // tile_rows]
-  const size_t desc = 2 * n1 * sizeof(int64_t), bytes = desc + n1 * sizeof(int64_t);
-  const size_t dev_bytes = bytes + (n_tiles + 1) * sizeof(int64_t) + std::max<size_t>(n_tiles, 1) * sizeof(int32_t);
+  // ring entry: host [text_off | tile_off], which the row counts overwrite on their way back (the download is queued
+  // behind the upload); device [text_off | tile_off | row_off | tile_start | tile_rows]
+  const size_t bytes = 2 * n1 * sizeof(int64_t);
+  const size_t dev_bytes = bytes + (n1 + n_tiles + 1) * sizeof(int64_t) + std::max<size_t>(n_tiles, 1) * sizeof(int32_t);
   DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, bytes, &de)) != NSF_OK) return st;
-  if ((st = de->dev.reserve(dev_bytes)) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  std::memcpy(h, text_off, n1 * sizeof(int64_t));
-  std::memcpy(h + n1, tile_off.data(), n1 * sizeof(int64_t));
+  st = desc_upload(ctx, s, bytes, nullptr, dev_bytes, &de, [&](void* mem) {
+    std::memcpy(mem, text_off, n1 * sizeof(int64_t));
+    std::memcpy(static_cast<int64_t*>(mem) + n1, tile_off.data(), n1 * sizeof(int64_t));
+  });
+  if (st != NSF_OK) return st;
   int64_t* d = static_cast<int64_t*>(de->dev.ptr);
-  NSF_CUDA(cudaMemcpyAsync(d, h, desc, cudaMemcpyHostToDevice, s));
   CsvView v{};
   v.text = text_dev; v.text_off = d; v.tile_off = d + n1; v.n_files = n_files; v.n_tiles = static_cast<int64_t>(n_tiles);
   int64_t* d_rows = d + 2 * n1;
   int64_t* d_tile_start = d + 3 * n1;
   int32_t* d_tile_rows = reinterpret_cast<int32_t*>(d_tile_start + n_tiles + 1);
-  const int m = launch_csv_row_offsets(s, v, d_tile_rows, d_tile_start, d_rows);
-  if (m < 0) { set_error(cuda_msg("launch_csv_row_offsets", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += m;
-  NSF_CUDA(cudaMemcpyAsync(h + 2 * n1, d_rows, n1 * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  NSF_LAUNCH(ctx, launch_csv_row_offsets(s, v, d_tile_rows, d_tile_start, d_rows));
+  NSF_CUDA(cudaMemcpyAsync(de->mem.ptr, d_rows, n1 * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   if ((st = desc_commit(de, s)) != NSF_OK) return st;
   NSF_CUDA(cudaStreamSynchronize(s));   // the call's one host wait
-  std::memcpy(row_off, h + 2 * n1, n1 * sizeof(int64_t));
+  std::memcpy(row_off, de->mem.ptr, n1 * sizeof(int64_t));
   return NSF_OK;
 }
 
@@ -1512,7 +1528,7 @@ nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const c
   if (!out_col || !row_off || !status_dev || cols < 1 || out_cols < 0) {
     set_error("nsf_csv_parse: NULL argument, cols < 1 or out_cols < 0"); return NSF_ERR_BAD_ARG;
   }
-  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_csv_parse: bad dtype"); return NSF_ERR_BAD_ARG; }
+  if ((st = check_dtype("nsf_csv_parse", dtype)) != NSF_OK) return st;
   if (out_ld < out_cols) { set_error("nsf_csv_parse: out_ld < out_cols"); return NSF_ERR_BAD_ARG; }
   std::vector<char> used(out_cols, 0);
   for (int c = 0; c < cols; ++c) {
@@ -1523,8 +1539,7 @@ nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const c
     }
   }
   if (row_off[0] != 0) { set_error("nsf_csv_parse: row offsets must start at 0"); return NSF_ERR_BAD_ARG; }
-  for (int i = 0; i < n_files; ++i)
-    if (row_off[i + 1] < row_off[i]) { set_error("nsf_csv_parse: row offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
+  if ((st = check_nondecreasing("nsf_csv_parse: row offsets", row_off, n_files)) != NSF_OK) return st;
   const int64_t n_rows = row_off[n_files];
   if (n_rows > 0 && !out_dev) { set_error("nsf_csv_parse: out_dev is NULL"); return NSF_ERR_BAD_ARG; }
   if (n_rows > INT32_MAX) { set_error("nsf_csv_parse: more than 2^31 rows in one call"); return NSF_ERR_UNSUPPORTED; }
@@ -1539,15 +1554,15 @@ nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const c
   const size_t dev_bytes = desc + (n_tiles + 1 + static_cast<size_t>(n_rows)) * sizeof(int64_t) + flags_bytes +
                            std::max<size_t>(n_tiles, 1) * sizeof(int32_t);
   DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, desc, &de)) != NSF_OK) return st;
-  if ((st = de->dev.reserve(dev_bytes)) != NSF_OK) return st;
-  char* h = static_cast<char*>(de->mem.ptr);
-  std::memcpy(h, text_off, n1 * sizeof(int64_t));
-  std::memcpy(h + n1 * 8, tile_off.data(), n1 * sizeof(int64_t));
-  std::memcpy(h + 2 * n1 * 8, row_off, n1 * sizeof(int64_t));
-  std::memcpy(h + 3 * n1 * 8, out_col, static_cast<size_t>(cols) * sizeof(int32_t));
+  st = desc_upload(ctx, s, desc, nullptr, dev_bytes, &de, [&](void* mem) {
+    char* h = static_cast<char*>(mem);
+    std::memcpy(h, text_off, n1 * sizeof(int64_t));
+    std::memcpy(h + n1 * 8, tile_off.data(), n1 * sizeof(int64_t));
+    std::memcpy(h + 2 * n1 * 8, row_off, n1 * sizeof(int64_t));
+    std::memcpy(h + 3 * n1 * 8, out_col, static_cast<size_t>(cols) * sizeof(int32_t));
+  });
+  if (st != NSF_OK) return st;
   char* d = static_cast<char*>(de->dev.ptr);
-  NSF_CUDA(cudaMemcpyAsync(d, h, desc, cudaMemcpyHostToDevice, s));
   int64_t* d_tile_start = reinterpret_cast<int64_t*>(d + desc);
   int64_t* d_row_start = d_tile_start + n_tiles + 1;
   uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_row_start + n_rows);
@@ -1561,9 +1576,7 @@ nsf_status nsf_csv_parse(nsf_ctx* ctx, void* cuda_stream, int32_t dtype, const c
   v.row_off = v.text_off + 2 * n1;
   v.out_col = reinterpret_cast<const int32_t*>(d + 3 * n1 * 8);
   v.n_files = n_files; v.cols = cols; v.n_tiles = static_cast<int64_t>(n_tiles); v.n_rows = n_rows;
-  const int m = launch_csv_parse(s, v, dtype, d_tile_rows, d_tile_start, d_row_start, d_flags, out_dev, out_ld, status_dev);
-  if (m < 0) { set_error(cuda_msg("launch_csv_parse", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += m;
+  NSF_LAUNCH(ctx, launch_csv_parse(s, v, dtype, d_tile_rows, d_tile_start, d_row_start, d_flags, out_dev, out_ld, status_dev));
   return desc_commit(de, s);
 }
 
@@ -1596,9 +1609,8 @@ nsf_status nsf_chunk_gather(nsf_ctx* ctx, void* cuda_stream, const float* rows_d
   const int64_t n_chunks = nsf_chunk_count(n_rows, frame, overlap);
   if (n_chunks <= 0) { set_error("nsf_chunk_gather: need n_rows > 0 and 0 <= overlap < frame"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  const int n = launch_chunk_gather(static_cast<cudaStream_t>(cuda_stream), rows_dev, n_rows, cols, ld, frame, overlap, n_chunks, chunks_dev);
-  if (n < 0) { set_error(cuda_msg("launch_chunk_gather", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n;
+  NSF_LAUNCH(ctx, launch_chunk_gather(static_cast<cudaStream_t>(cuda_stream), rows_dev, n_rows, cols, ld, frame, overlap,
+                                      n_chunks, chunks_dev));
   return NSF_OK;
 }
 
@@ -1613,10 +1625,8 @@ nsf_status nsf_chunk_blend(nsf_ctx* ctx, void* cuda_stream, const float* decoded
     return NSF_ERR_UNSUPPORTED;
   }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  const int n = launch_chunk_blend(static_cast<cudaStream_t>(cuda_stream), decoded_dev, n_rows, out_cols, frame, overlap, n_chunks,
-                                   scale_cols, divisor, out_dev);
-  if (n < 0) { set_error(cuda_msg("launch_chunk_blend", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n;
+  NSF_LAUNCH(ctx, launch_chunk_blend(static_cast<cudaStream_t>(cuda_stream), decoded_dev, n_rows, out_cols, frame, overlap,
+                                     n_chunks, scale_cols, divisor, out_dev));
   return NSF_OK;
 }
 
@@ -1626,11 +1636,12 @@ nsf_status nsf_window_offsets(const int64_t* a_off, const int64_t* f_off, int32_
   if (!a_off || !f_off || !w_off || n_clips < 1) { set_error("nsf_window_offsets: NULL argument or n_clips < 1"); return NSF_ERR_BAD_ARG; }
   if (window < 1) { set_error("nsf_window_offsets: window must be >= 1"); return NSF_ERR_BAD_ARG; }
   if (a_off[0] < 0 || f_off[0] < 0) { set_error("nsf_window_offsets: negative offset"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_nondecreasing("nsf_window_offsets: offsets", a_off, n_clips);
+  if (st != NSF_OK || (st = check_nondecreasing("nsf_window_offsets: offsets", f_off, n_clips)) != NSF_OK) return st;
   w_off[0] = 0;
   char buf[200];
   for (int i = 0; i < n_clips; ++i) {
     const int64_t na = a_off[i + 1] - a_off[i], nf = f_off[i + 1] - f_off[i];
-    if (na < 0 || nf < 0) { set_error("nsf_window_offsets: offsets must be non-decreasing"); return NSF_ERR_BAD_ARG; }
     const int64_t top = std::max(na, nf);
     if (top < window) {   // dataset.py:77-91 fails on such a clip (broadcast error in the tail branch)
       std::snprintf(buf, sizeof buf, "clip %d has %lld rows, fewer than the window of %d", i, static_cast<long long>(top), window);
@@ -1688,28 +1699,27 @@ nsf_status nsf_window_gather(nsf_ctx* ctx, void* cuda_stream, const float* audio
   // which is reused only after this call's kernel has run
   const size_t bytes = (3 * n1 + static_cast<size_t>(n)) * sizeof(int64_t);
   DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, bytes, &de)) != NSF_OK) return st;
-  if ((st = de->dev.reserve(bytes)) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  std::memcpy(h, a_off, n1 * sizeof(int64_t));
-  std::memcpy(h + n1, f_off, n1 * sizeof(int64_t));
-  std::memcpy(h + 2 * n1, w_off.data(), n1 * sizeof(int64_t));
-  std::memcpy(h + 3 * n1, indices, static_cast<size_t>(n) * sizeof(int64_t));
-  int64_t* d = static_cast<int64_t*>(de->dev.ptr);
-  NSF_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s));
+  st = desc_upload(ctx, s, bytes, nullptr, bytes, &de, [&](void* mem) {
+    int64_t* h = static_cast<int64_t*>(mem);
+    std::memcpy(h, a_off, n1 * sizeof(int64_t));
+    std::memcpy(h + n1, f_off, n1 * sizeof(int64_t));
+    std::memcpy(h + 2 * n1, w_off.data(), n1 * sizeof(int64_t));
+    std::memcpy(h + 3 * n1, indices, static_cast<size_t>(n) * sizeof(int64_t));
+  });
+  if (st != NSF_OK) return st;
+  const int64_t* d = static_cast<const int64_t*>(de->dev.ptr);
   WindowView v;
   v.a_off = d; v.f_off = d + n1; v.w_off = d + 2 * n1; v.index = d + 3 * n1;
   v.n_clips = n_clips; v.window = window; v.n = n;
-  const int m = launch_window_gather(s, v, audio_dev, audio_cols, facial_dev, facial_cols, out_audio_dev, out_facial_dev);
-  if (m < 0) { set_error(cuda_msg("launch_window_gather", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += m;
+  NSF_LAUNCH(ctx, launch_window_gather(s, v, audio_dev, audio_cols, facial_dev, facial_cols, out_audio_dev, out_facial_dev));
   return desc_commit(de, s);
 }
 
 nsf_status nsf_rows_host(nsf_ctx* ctx, int32_t op, int32_t dtype, const void* a_host, int64_t na,
                          const void* b_host, int64_t nb, int32_t cols, int32_t blend_frames, void* out_host) {
   if (!ctx || !a_host || !out_host || na <= 0 || cols <= 0) { set_error("nsf_rows_host: bad argument"); return NSF_ERR_BAD_ARG; }
-  if (dtype != NSF_F32 && dtype != NSF_F64) { set_error("nsf_rows_host: bad dtype"); return NSF_ERR_BAD_ARG; }
+  nsf_status st = check_dtype("nsf_rows_host", dtype);
+  if (st != NSF_OK) return st;
   int64_t out_rows = 0, k = 0;
   if (op == NSF_ROWS_INTERP_SLOWER) out_rows = 2 * na - 1;
   else if (op == NSF_ROWS_SMOOTH) out_rows = na;
@@ -1719,23 +1729,20 @@ nsf_status nsf_rows_host(nsf_ctx* ctx, int32_t op, int32_t dtype, const void* a_
     out_rows = na + nb - k;
   } else { set_error("nsf_rows_host: unknown op"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = nullptr;
-  nsf_status st = oneshot_slot(ctx, &sl);
-  if (st != NSF_OK) return st;
   const size_t esz = dtype == NSF_F64 ? 8 : 4;
   const bool two = op == NSF_ROWS_BLEND_STACK;
-  if ((st = sl->in[0].reserve(na * cols * esz)) != NSF_OK) return st;
-  if (two && (st = sl->in[1].reserve(nb * cols * esz)) != NSF_OK) return st;
-  if ((st = sl->out[0].reserve(out_rows * cols * esz)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(sl->in[0].ptr, a_host, na * cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  if (two) NSF_CUDA(cudaMemcpyAsync(sl->in[1].ptr, b_host, nb * cols * esz, cudaMemcpyHostToDevice, sl->stream));
-  const int n = launch_rows_op(sl->stream, op, dtype, sl->in[0].ptr, na, two ? sl->in[1].ptr : nullptr,
-                               nb, cols, k, sl->out[0].ptr, out_rows);
-  if (n < 0) { set_error(cuda_msg("launch_rows_op", cudaGetLastError())); return NSF_ERR_CUDA; }
-  ctx->launches += n;
-  NSF_CUDA(cudaMemcpyAsync(out_host, sl->out[0].ptr, out_rows * cols * esz, cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  return NSF_OK;
+  const size_t a_bytes = na * cols * esz, b_bytes = two ? nb * cols * esz : 0, out_bytes = out_rows * cols * esz;
+  return run_once(ctx, [&](Slot* sl) -> nsf_status {
+    nsf_status st;
+    if ((st = sl->in[0].reserve(a_bytes)) != NSF_OK) return st;
+    if (two && (st = sl->in[1].reserve(b_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(out_bytes)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, a_host, a_bytes, true)) != NSF_OK) return st;
+    if (two && (st = upload(sl, 1, b_host, b_bytes, true)) != NSF_OK) return st;
+    NSF_LAUNCH(ctx, launch_rows_op(sl->stream, op, dtype, sl->in[0].ptr, na, two ? sl->in[1].ptr : nullptr, nb, cols, k,
+                                   sl->out[0].ptr, out_rows));
+    return download(sl, 0, out_host, out_bytes, out_bytes, 1, true);
+  });
 }
 
 nsf_status nsf_post_host(nsf_ctx* ctx, const float* in_host, int64_t T, int32_t Cc, uint32_t pf, float* out_host) {
@@ -1743,51 +1750,40 @@ nsf_status nsf_post_host(nsf_ctx* ctx, const float* in_host, int64_t T, int32_t 
   if ((pf & NSF_POST_DELTAS) && T < 9) { set_error("nsf_post_host: delta needs at least 9 frames"); return NSF_ERR_TOO_SHORT; }
   if ((pf & NSF_POST_EDGEFIX) && T < 2) { set_error("nsf_post_host: edge fix needs 2 frames"); return NSF_ERR_BAD_ARG; }
   NSF_CUDA(cudaSetDevice(ctx->device));
-  Slot* sl = nullptr;
-  nsf_status st = oneshot_slot(ctx, &sl);
-  if (st != NSF_OK) return st;
   const bool reduce = (pf & NSF_POST_REDUCE) != 0, deltas = (pf & NSF_POST_DELTAS) != 0, cmvn = (pf & NSF_POST_CMVN) != 0;
   const int64_t rows = reduce ? (T + 1) / 2 : T;
   const int out_c = Cc * (deltas ? 3 : 1);
-  // device layout: [in T*C floats][out rows*out_c floats][desc 6 x int64][sum C][sumsq C]
-  const size_t in_b = align_up(T * Cc * sizeof(float)), out_b = align_up(rows * out_c * sizeof(float));
+  const size_t in_bytes = T * Cc * sizeof(float), out_bytes = rows * out_c * sizeof(float);
+  // in[0] = frames, out[0] = rows, work = [desc 6 x int64][sum C][sumsq C]
   const size_t desc_b = align_up(6 * sizeof(int64_t)), st_b = align_up(Cc * sizeof(double));
-  if ((st = sl->work.reserve(in_b + out_b + desc_b + 2 * st_b)) != NSF_OK) return st;
-  char* base = static_cast<char*>(sl->work.ptr);
-  float* d_in = reinterpret_cast<float*>(base);
-  float* d_out = reinterpret_cast<float*>(base + in_b);
-  int64_t* d_desc = reinterpret_cast<int64_t*>(base + in_b + out_b);
-  double* d_sum = reinterpret_cast<double*>(base + in_b + out_b + desc_b);
-  double* d_sq = reinterpret_cast<double*>(base + in_b + out_b + desc_b + st_b);
-  DescEntry* de = nullptr;
-  if ((st = desc_acquire(ctx, 6 * sizeof(int64_t), &de)) != NSF_OK) return st;
-  int64_t* h = static_cast<int64_t*>(de->mem.ptr);
-  h[0] = 0; h[1] = 0;           // clip_off (unused by the post kernels)
-  h[2] = 0; h[3] = T;           // frame_off
-  h[4] = 0; h[5] = rows;        // row_off
-  NSF_CUDA(cudaMemcpyAsync(d_desc, h, 6 * sizeof(int64_t), cudaMemcpyHostToDevice, sl->stream));
-  if ((st = desc_commit(de, sl->stream)) != NSF_OK) return st;
-  NSF_CUDA(cudaMemcpyAsync(d_in, in_host, T * Cc * sizeof(float), cudaMemcpyHostToDevice, sl->stream));
-  int launched = 0, n;
-  if (pf & NSF_POST_EDGEFIX) {
-    if ((n = launch_edge_fix(sl->stream, d_in, T, Cc, ctx->edge_zero_threshold)) < 0) { set_error(cuda_msg("launch_edge_fix", cudaGetLastError())); return NSF_ERR_CUDA; }
-    launched += n;
-  }
-  if (cmvn) {
-    if ((n = launch_col_stats(sl->stream, d_in, T, Cc, d_sum, d_sq)) < 0) { set_error(cuda_msg("launch_col_stats", cudaGetLastError())); return NSF_ERR_CUDA; }
-    launched += n;
-  }
-  BatchView b;
-  b.clip_off = d_desc; b.frame_off = d_desc + 2; b.row_off = d_desc + 4;
-  b.n_clips = 1; b.total_samples = 0; b.total_frames = T; b.total_rows = rows;
-  if ((n = launch_delta_reduce(sl->stream, b, d_in, Cc, Cc, d_sum, d_sq, cmvn, deltas, reduce, d_out, out_c, 0)) < 0) {
-    set_error(cuda_msg("launch_delta_reduce", cudaGetLastError())); return NSF_ERR_CUDA;
-  }
-  launched += n;
-  ctx->launches += launched;
-  NSF_CUDA(cudaMemcpyAsync(out_host, d_out, rows * out_c * sizeof(float), cudaMemcpyDeviceToHost, sl->stream));
-  NSF_CUDA(cudaStreamSynchronize(sl->stream));
-  return NSF_OK;
+  return run_once(ctx, [&](Slot* sl) -> nsf_status {
+    nsf_status st;
+    if ((st = sl->in[0].reserve(in_bytes)) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(out_bytes)) != NSF_OK) return st;
+    if ((st = sl->work.reserve(desc_b + 2 * st_b)) != NSF_OK) return st;
+    char* base = static_cast<char*>(sl->work.ptr);
+    float* d_in = static_cast<float*>(sl->in[0].ptr);
+    int64_t* d_desc = reinterpret_cast<int64_t*>(base);
+    double* d_sum = reinterpret_cast<double*>(base + desc_b);
+    double* d_sq = reinterpret_cast<double*>(base + desc_b + st_b);
+    DescEntry* de = nullptr;
+    st = desc_upload(ctx, sl->stream, 6 * sizeof(int64_t), d_desc, 0, &de, [&](void* mem) {
+      int64_t* h = static_cast<int64_t*>(mem);
+      h[0] = 0; h[1] = 0;           // clip_off (unused by the post kernels)
+      h[2] = 0; h[3] = T;           // frame_off
+      h[4] = 0; h[5] = rows;        // row_off
+    });
+    if (st != NSF_OK || (st = desc_commit(de, sl->stream)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, in_host, in_bytes, true)) != NSF_OK) return st;
+    if (pf & NSF_POST_EDGEFIX) NSF_LAUNCH(ctx, launch_edge_fix(sl->stream, d_in, T, Cc, ctx->edge_zero_threshold));
+    if (cmvn) NSF_LAUNCH(ctx, launch_col_stats(sl->stream, d_in, T, Cc, d_sum, d_sq));
+    BatchView b;
+    b.clip_off = d_desc; b.frame_off = d_desc + 2; b.row_off = d_desc + 4;
+    b.n_clips = 1; b.total_samples = 0; b.total_frames = T; b.total_rows = rows;
+    NSF_LAUNCH(ctx, launch_delta_reduce(sl->stream, b, d_in, Cc, Cc, d_sum, d_sq, cmvn, deltas, reduce,
+                                        static_cast<float*>(sl->out[0].ptr), out_c, 0));
+    return download(sl, 0, out_host, out_bytes, out_bytes, 1, true);
+  });
 }
 
 }  // extern "C"

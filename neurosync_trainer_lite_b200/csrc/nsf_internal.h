@@ -64,6 +64,14 @@ inline int64_t floordiv(int64_t a, int64_t b) {
   return (r != 0 && ((r < 0) != (b < 0))) ? q - 1 : q;
 }
 
+// Hop-frames of a clip of `len` samples under `flags`, and in *rows its feature rows.  Frames are centre-padded
+// unless NSF_AC_NO_PAD (pad_signal=False: y[t H : t H + F], as many as fit); rows are frame pairs unless NSF_NO_REDUCE.
+inline int64_t clip_frames(int64_t len, int32_t F, int32_t H, uint32_t flags, int64_t* rows) {
+  const int64_t T = (flags & NSF_AC_NO_PAD) ? (len >= F ? nsf_guard_frames(len, F, H) : 0) : nsf_hop_frames(len, F, H);
+  *rows = (flags & NSF_NO_REDUCE) ? T : (T + 1) / 2;
+  return T;
+}
+
 }  // namespace nsf
 
 struct nsf_plan {

@@ -372,15 +372,13 @@ int64_t nsf_feature_rows(int64_t n, int32_t F, int32_t H) {
 nsf_status nsf_row_offsets(int32_t F, int32_t H, const int64_t* clip_offsets, int32_t n_clips, uint32_t flags,
                            int64_t* row_offsets) {
   if (!clip_offsets || !row_offsets || n_clips < 0 || F <= 0 || H <= 0) return NSF_ERR_BAD_ARG;
-  const bool no_pad = (flags & NSF_AC_NO_PAD) != 0, no_reduce = (flags & NSF_NO_REDUCE) != 0;
   row_offsets[0] = 0;
   for (int32_t i = 0; i < n_clips; ++i) {
     const int64_t len = clip_offsets[i + 1] - clip_offsets[i];
     if (len < 0) return NSF_ERR_BAD_ARG;
-    int64_t T;
-    if (no_pad) T = len >= F ? std::max<int64_t>(0, nsf_guard_frames(len, F, H)) : 0;
-    else T = nsf_hop_frames(len, F, H);
-    row_offsets[i + 1] = row_offsets[i] + (no_reduce ? T : (T + 1) / 2);
+    int64_t rows;
+    nsf::clip_frames(len, F, H, flags, &rows);
+    row_offsets[i + 1] = row_offsets[i] + rows;
   }
   return NSF_OK;
 }
