@@ -356,6 +356,76 @@ NSF_API nsf_status nsf_convert_batch(nsf_ctx* ctx, void* cuda_stream, const void
 NSF_API nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes,
                                     const nsf_pcm_source* sources, int32_t n, int32_t target_sr, float* out_host);
 
+/* ---- FLAC decode -------------------------------------------------------------------------------------
+ * The decode half of librosa.load for FLAC files (utils/audio/load_audio.py:19, :25, :36; libsndfile reads FLAC
+ * natively).  The metadata blocks are container parsing and stay with the caller (load_audio.flac_layout); the
+ * frames are decoded on the device.  Stream i is described by sources[i]: its frame data is payload bytes
+ * [byte_offset, byte_offset + byte_length) and decodes to `frames` interleaved frames of `channels` samples of
+ * `bits` bits (STREAMINFO).  The output of stream i is the WAV data chunk holding those samples: u8 v + 128 for 8
+ * bits, little-endian i16 for 16, packed little-endian i24 for 24, at the prefix sum of frames * channels * (bits / 8).
+ * Decoded (RFC 9639): fixed and variable blocking, block sizes 1..65535, CONSTANT / VERBATIM / FIXED 0-4 / LPC 1-32
+ * subframes, wasted bits, both Rice methods with escaped partitions, the four channel assignments.  Every frame's
+ * header CRC-8 and frame CRC-16 are checked; the STREAMINFO MD5 is not.  Frames must follow each other from
+ * byte_offset, with consecutive frame numbers (fixed blocking) or first samples (variable blocking), tiling
+ * [0, frames) exactly; bytes after the last frame are ignored.  A frame whose channel count, bits per sample or
+ * explicit sample rate disagrees with the descriptor, or whose block is larger than max_block, is corrupt.
+ *   nsf_flac_decode_host  host payload -> host PCM bytes; synchronous, pipelined over stream groups like
+ *                         nsf_convert_host (pageable or page-locked buffers).  Descriptors are validated before
+ *                         anything is launched: the byte range inside payload_bytes and below 2^31 bytes,
+ *                         bits 8 / 16 / 24, channels 1..8, frames > 0, max_block 1..65535, sample_rate > 0
+ *                         (NSF_ERR_BAD_ARG).  A corrupt stream returns NSF_ERR_BAD_ARG, and nsf_last_error names the
+ *                         stream, the frame's byte offset in the payload and the reason.
+ *   nsf_flac_check        verification aid, like nsf_parse_check: the device's frame-header parser and frame decoder
+ *                         run on the host over the ONE frame that starts at source->byte_offset (and ends before
+ *                         byte_offset + byte_length).  Fills *frame (status NSF_FLAC_*: the call itself returns
+ *                         NSF_OK once its arguments are valid) and, when samples != NULL and the frame decodes, its
+ *                         samples channel by channel after the inter-channel decorrelation: samples[c * block + i],
+ *                         NSF_ERR_BAD_ARG when capacity < channels * block.  Not a compute path. */
+typedef struct nsf_flac_source {
+  int64_t byte_offset;  /* first byte of the first frame (after the metadata blocks)      */
+  int64_t byte_length;  /* bytes of frame data                                           */
+  int64_t frames;       /* STREAMINFO total samples per channel, > 0                      */
+  int32_t channels;     /* 1..8                                                           */
+  int32_t bits;         /* 8, 16 or 24                                                    */
+  int32_t sample_rate;  /* STREAMINFO                                                     */
+  int32_t max_block;    /* STREAMINFO maximum block size, 1..65535                         */
+} nsf_flac_source;
+/* status of one frame (nsf_flac_frame.status) */
+#define NSF_FLAC_OK 0
+#define NSF_FLAC_NO_SYNC 1       /* no frame sync code 0xFFF8 / 0xFFF9                                 */
+#define NSF_FLAC_TRUNCATED 2     /* the frame runs past the end of the stream                          */
+#define NSF_FLAC_BAD_NUMBER 3    /* malformed coded frame / sample number                              */
+#define NSF_FLAC_BAD_CRC8 4      /* header CRC-8 mismatch                                              */
+#define NSF_FLAC_RESERVED 5      /* a reserved or invalid code in the header or a subframe             */
+#define NSF_FLAC_CHANNELS 6      /* channel count disagrees with STREAMINFO                            */
+#define NSF_FLAC_BITS 7          /* bits per sample disagree with STREAMINFO                           */
+#define NSF_FLAC_RATE 8          /* sample rate disagrees with STREAMINFO                              */
+#define NSF_FLAC_BLOCK 9         /* block size above the STREAMINFO maximum                            */
+#define NSF_FLAC_WASTED 10       /* wasted bits leave no sample bits                                   */
+#define NSF_FLAC_LPC_SHIFT 11    /* negative LPC shift                                                 */
+#define NSF_FLAC_PARTITION 12    /* partition order does not divide the block, or a first partition
+                                    shorter than the predictor order                                 */
+#define NSF_FLAC_RANGE 13        /* a Rice-coded residual outside 32 bits                              */
+#define NSF_FLAC_BAD_CRC16 14    /* frame CRC-16 mismatch                                              */
+typedef struct nsf_flac_frame {
+  int64_t end;          /* first byte after the frame's CRC-16 (payload offset)                         */
+  int64_t number;       /* coded number: frame number (fixed blocking) or first sample (variable)      */
+  int32_t block;        /* block size                                                                   */
+  int32_t sample_rate;  /* from the header, the descriptor's when the header defers to STREAMINFO       */
+  int32_t bits;         /* likewise                                                                     */
+  int32_t assignment;   /* channel assignment code: 0-7 independent, 8 left/side, 9 side/right, 10 mid/side */
+  int32_t channels;
+  int32_t variable;     /* blocking strategy bit                                                        */
+  int32_t crc8_ok;      /* header CRC-8 matches                                                         */
+  int32_t crc16_ok;     /* frame CRC-16 matches (0 when the decode stopped before the CRC-16)           */
+  int32_t status;       /* NSF_FLAC_*                                                                   */
+  int32_t reserved;
+} nsf_flac_frame;
+NSF_API nsf_status nsf_flac_decode_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes,
+                                        const nsf_flac_source* sources, int32_t n, void* pcm_host);
+NSF_API nsf_status nsf_flac_check(const void* payload, const nsf_flac_source* source, nsf_flac_frame* frame,
+                                  int32_t* samples, int64_t capacity);
+
 /* ---- training windows ------------------------------------------------------------------------------
  * The consumer of the augmented rows at training time, AudioFacialDataset (dataset/dataset.py:58-98): every stride-1
  * window of `window` rows of each clip, plus one reflected tail window when the clip's length is not a multiple of

@@ -36,6 +36,17 @@ ENC_U8, ENC_I16, ENC_I24, ENC_I32, ENC_F32, ENC_F64 = range(6)
 PCM_SOURCE = np.dtype([("byte_offset", "<i8"), ("frames", "<i8"), ("encoding", "<i4"), ("channels", "<i4"),
                        ("sample_rate", "<i4"), ("reserved", "<i4")], align=True)
 assert PCM_SOURCE.itemsize == 32
+# nsf_flac_source: one FLAC stream of nsf_flac_decode_host (frame bytes -> WAV data-chunk bytes)
+FLAC_SOURCE = np.dtype([("byte_offset", "<i8"), ("byte_length", "<i8"), ("frames", "<i8"), ("channels", "<i4"),
+                        ("bits", "<i4"), ("sample_rate", "<i4"), ("max_block", "<i4")], align=True)
+assert FLAC_SOURCE.itemsize == 40
+# nsf_flac_frame: what nsf_flac_check reports for one frame
+FLAC_FRAME = np.dtype([("end", "<i8"), ("number", "<i8"), ("block", "<i4"), ("sample_rate", "<i4"), ("bits", "<i4"),
+                       ("assignment", "<i4"), ("channels", "<i4"), ("variable", "<i4"), ("crc8_ok", "<i4"),
+                       ("crc16_ok", "<i4"), ("status", "<i4"), ("reserved", "<i4")], align=True)
+assert FLAC_FRAME.itemsize == 56
+(FLAC_OK, FLAC_NO_SYNC, FLAC_TRUNCATED, FLAC_BAD_NUMBER, FLAC_BAD_CRC8, FLAC_RESERVED, FLAC_CHANNELS, FLAC_BITS,
+ FLAC_RATE, FLAC_BLOCK, FLAC_WASTED, FLAC_LPC_SHIFT, FLAC_PARTITION, FLAC_RANGE, FLAC_BAD_CRC16) = range(15)
 STAGE_NAMES = ("peak_normalize", "fold", "stft_gemm", "mel_db", "dct_stats", "cmvn_delta_reduce",
                "autocorr", "post")
 
@@ -108,6 +119,8 @@ _SIGS = {
     "nsf_convert_offsets": (_i32, [_vp, _i32, _i32, _i64, _i64p]),
     "nsf_convert_batch": (_i32, [_vp, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _i64p]),
     "nsf_convert_host": (_i32, [_vp, _vp, _i64, _vp, _i32, _i32, _vp]),
+    "nsf_flac_decode_host": (_i32, [_vp, _vp, _i64, _vp, _i32, _vp]),
+    "nsf_flac_check": (_i32, [_vp, _vp, _vp, _i32p, _i64]),
     "nsf_window_offsets": (_i32, [_i64p, _i64p, _i32, _i32, _i64p]),
     "nsf_window_gather": (_i32, [_vp, _vp, _vp, _i32, _i64p, _vp, _i32, _i64p, _i32, _i32, _i64p, _i64, _vp, _vp]),
     "nsf_csv_bytes_bound": (_i64, [_i64, _i32, _i32]),
@@ -171,6 +184,21 @@ def convert_offsets(sources, target_sr, payload_bytes):
     out = np.empty(len(src) + 1, dtype=np.int64)
     check(lib.nsf_convert_offsets(ptr(src), len(src), int(target_sr), int(payload_bytes), out.ctypes.data_as(_i64p)))
     return out
+
+
+def flac_check(data, source):
+    """The device's FLAC frame decoder run on the host over the one frame at ``source.byte_offset`` of ``data``
+    (``nsf_flac_check``, a verification aid): ``(FLAC_FRAME record, int32 samples [channels, block] or None)``."""
+    buf = np.frombuffer(bytes(data), dtype=np.uint8)
+    src = np.ascontiguousarray(np.asarray(source, dtype=FLAC_SOURCE).reshape(1))
+    frame = np.zeros(1, dtype=FLAC_FRAME)
+    ch = int(src["channels"][0])
+    samples = np.zeros(ch * 65536, dtype=np.int32)
+    check(lib.nsf_flac_check(ptr(buf), ptr(src), ptr(frame), samples.ctypes.data_as(_i32p), samples.size))
+    f = frame[0]
+    if int(f["status"]) != FLAC_OK:
+        return f, None
+    return f, samples[:ch * int(f["block"])].reshape(ch, -1).copy()
 
 
 def window_offsets(audio_offsets, facial_offsets, window):

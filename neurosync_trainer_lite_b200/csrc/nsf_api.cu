@@ -1269,6 +1269,185 @@ nsf_status nsf_convert_host(nsf_ctx* ctx, const void* payload_host, int64_t payl
   });
 }
 
+// ---- FLAC decode -------------------------------------------------------------------------------------
+namespace {
+// Validates every descriptor; out_off[i] = first output byte of stream i, cost[i] = int32 samples before stream i.
+nsf_status flac_offsets(const nsf_flac_source* src, int32_t n, int64_t payload_bytes, int64_t* out_off, int64_t* cost) {
+  if (!src || n <= 0) { set_error("nsf_flac_decode_host: NULL sources or n <= 0"); return NSF_ERR_BAD_ARG; }
+  if (payload_bytes < 0) { set_error("nsf_flac_decode_host: negative payload_bytes"); return NSF_ERR_BAD_ARG; }
+  out_off[0] = cost[0] = 0;
+  for (int i = 0; i < n; ++i) {
+    const nsf_flac_source& c = src[i];
+    char buf[200];
+    auto fail = [&](const char* what) {
+      std::snprintf(buf, sizeof buf, "nsf_flac_decode_host: source %d: %s", i, what);
+      set_error(buf);
+      return NSF_ERR_BAD_ARG;
+    };
+    if (c.bits != 8 && c.bits != 16 && c.bits != 24) return fail("bits must be 8, 16 or 24");
+    if (c.channels < 1 || c.channels > 8) return fail("channels must be in [1, 8]");
+    if (c.frames <= 0) return fail("frames must be positive");
+    if (c.max_block < 1 || c.max_block > 65535) return fail("max_block must be in [1, 65535]");
+    if (c.sample_rate <= 0) return fail("sample_rate must be positive");
+    if (c.byte_offset < 0 || c.byte_length < 0 || c.byte_offset > payload_bytes ||
+        c.byte_length > payload_bytes - c.byte_offset)
+      return fail("byte range outside the payload");
+    if (c.byte_length > INT32_MAX) return fail("byte_length must be below 2^31");
+    if (c.frames > (int64_t(1) << 36)) return fail("frames above 2^36");
+    out_off[i + 1] = out_off[i] + c.frames * c.channels * (c.bits / 8);
+    cost[i + 1] = cost[i] + c.frames * c.channels;
+  }
+  return NSF_OK;
+}
+
+// Walks stream s's frame chain over the group's candidates cand[c0, c1) (those of stream s, in byte order): the first
+// frame at the stream's first byte, each next one where the previous ended, numbers consecutive, samples tiling
+// [0, frames).  Appends the kept frames; on a broken chain sets the error (payload offsets) and returns false.
+bool flac_chain(const uint8_t* payload, int64_t b0, int s_index, const FlacStream& st, int64_t frames,
+                const FlacCand* cand, int64_t c0, int64_t c1, int64_t g_base, int64_t scratch_base,
+                std::vector<FlacKept>* kept) {
+  int64_t at = st.begin, sample = 0, index = 0, c = c0;
+  int variable = -1;
+  char buf[256];
+  auto fail = [&](const char* why) {
+    std::snprintf(buf, sizeof buf, "FLAC stream %d: frame at byte %lld: %s", s_index, static_cast<long long>(b0 + at), why);
+    set_error(buf);
+    return false;
+  };
+  while (sample < frames) {
+    if (at >= st.end) return fail("stream ends before its STREAMINFO total samples");
+    while (c < c1 && cand[c].start < at) ++c;
+    if (c == c1 || cand[c].start != at) {
+      const int why = flac_header_status(payload, at, st.end);
+      return fail(why == NSF_FLAC_OK ? "no frame header" : flac_status_text(why));
+    }
+    const FlacCand& f = cand[c];
+    if (f.status != NSF_FLAC_OK) return fail(flac_status_text(f.status));
+    const int var = f.assignment >> 4;
+    if (variable < 0) variable = var;
+    if (var != variable) return fail("blocking strategy changes within the stream");
+    if (f.number != (variable ? sample : index))
+      return fail(variable ? "first sample number out of sequence" : "frame number out of sequence");
+    if (f.block > frames - sample) return fail("frame runs past the STREAMINFO total samples");
+    kept->push_back(FlacKept{static_cast<int32_t>(c), 0, g_base + sample, sample, scratch_base + sample * st.channels});
+    sample += f.block;
+    ++index;
+    at = f.end;
+  }
+  return true;
+}
+}  // namespace
+
+nsf_status nsf_flac_decode_host(nsf_ctx* ctx, const void* payload_host, int64_t payload_bytes,
+                                const nsf_flac_source* sources, int32_t n, void* pcm_host) {
+  if (!ctx || !payload_host || !pcm_host) { set_error("nsf_flac_decode_host: NULL argument"); return NSF_ERR_BAD_ARG; }
+  std::vector<int64_t> out_off(n > 0 ? n + 1 : 1), cost(n > 0 ? n + 1 : 1);
+  nsf_status st = flac_offsets(sources, n, payload_bytes, out_off.data(), cost.data());
+  if (st != NSF_OK) return st;
+  NSF_CUDA(cudaSetDevice(ctx->device));
+  const uint8_t* payload = static_cast<const uint8_t*>(payload_host);
+  const bool in_dma = dma_reachable(payload_host), out_dma = dma_reachable(pcm_host);
+  std::vector<FlacStream> gs;
+  std::vector<FlacKept> kept;
+  // stream groups by decoded samples
+  return run_groups(ctx, cost.data(), n, [&](int first, int last, Slot* sl) -> nsf_status {
+    int64_t b0 = INT64_MAX, b1 = 0, scan = 0, cap = 0, out_frames = 0;
+    int max_ch = 1;
+    for (int i = first; i < last; ++i) {
+      b0 = std::min(b0, sources[i].byte_offset);
+      b1 = std::max(b1, sources[i].byte_offset + sources[i].byte_length);
+    }
+    gs.clear();
+    for (int i = first; i < last; ++i) {
+      const nsf_flac_source& c = sources[i];
+      gs.push_back(FlacStream{c.byte_offset - b0, c.byte_offset + c.byte_length - b0, scan, out_off[i] - out_off[first],
+                              c.channels, c.bits, c.sample_rate, c.max_block});
+      scan += c.byte_length;
+      cap += 2 * ((c.frames + c.max_block - 1) / c.max_block) + 16;   // room for a few false syncs per stream
+      out_frames += c.frames;
+      max_ch = std::max(max_ch, c.channels);
+    }
+    const int ng = last - first;
+    const int64_t in_bytes = b1 - b0, out_bytes = out_off[last] - out_off[first], samples = cost[last] - cost[first];
+    if (scan == 0) return NSF_OK;   // unreachable: frames > 0 needs bytes, and the chain reports their absence
+    nsf_status st;
+    if ((st = sl->in[0].reserve(std::max<int64_t>(in_bytes, 1))) != NSF_OK) return st;
+    if ((st = sl->out[0].reserve(out_bytes)) != NSF_OK) return st;
+    if ((st = upload(sl, 0, payload + b0, in_bytes, in_dma)) != NSF_OK) return st;
+    const size_t streams_bytes = ng * sizeof(FlacStream);
+    DescEntry* de_streams = nullptr;
+    st = desc_upload(ctx, sl->stream, streams_bytes, nullptr, streams_bytes, &de_streams,
+                     [&](void* mem) { std::memcpy(mem, gs.data(), streams_bytes); });
+    if (st != NSF_OK) return st;
+    const FlacStream* d_streams = static_cast<const FlacStream*>(de_streams->dev.ptr);
+    const uint8_t* d_payload = static_cast<const uint8_t*>(sl->in[0].ptr);
+    const int64_t n_blk = (scan + kFlacScanTile - 1) / kFlacScanTile;
+    // work: [scratch | tile counts | tile offsets | total | positions | candidates]; the table comes back to the
+    // pinned stage_out[1] as [total | candidates].  One wait, unless the candidates overflow `cap` (false syncs
+    // beyond the allowance): then the scan runs again with room for all of them.
+    FlacCand* d_cand = nullptr;
+    int64_t* d_total = nullptr;
+    int32_t* d_scratch = nullptr;
+    const FlacCand* cand = nullptr;
+    int64_t total = 0;
+    for (;;) {
+      Carver sizer(reinterpret_cast<void*>(0x1000), ~size_t(0) >> 1);
+      auto carve = [&](Carver& c) {
+        d_scratch = c.take<int32_t>(samples);
+        int32_t* d_count = c.take<int32_t>(n_blk);
+        int64_t* d_off = c.take<int64_t>(n_blk);
+        d_total = c.take<int64_t>(1);
+        int64_t* d_pos = c.take<int64_t>(cap);
+        d_cand = c.take<FlacCand>(cap);
+        return std::make_pair(d_count, std::make_pair(d_off, d_pos));
+      };
+      carve(sizer);
+      if ((st = sl->work.reserve(sizer.used)) != NSF_OK) return st;
+      Carver cv(sl->work.ptr, sl->work.bytes);
+      const auto ptrs = carve(cv);
+      const size_t table_bytes = sizeof(int64_t) + cap * sizeof(FlacCand);
+      if ((st = sl->stage_out[1].reserve(table_bytes)) != NSF_OK) return st;
+      NSF_LAUNCH(ctx, launch_flac_scan_parse(sl->stream, d_streams, ng, scan, d_payload, ptrs.first, ptrs.second.first,
+                                             d_total, ptrs.second.second, d_cand, cap));
+      char* table = static_cast<char*>(sl->stage_out[1].ptr);
+      NSF_CUDA(cudaMemcpyAsync(table, d_total, sizeof(int64_t), cudaMemcpyDeviceToHost, sl->stream));
+      NSF_CUDA(cudaMemcpyAsync(table + sizeof(int64_t), d_cand, cap * sizeof(FlacCand), cudaMemcpyDeviceToHost,
+                               sl->stream));
+      NSF_CUDA(cudaStreamSynchronize(sl->stream));
+      std::memcpy(&total, table, sizeof total);
+      cand = reinterpret_cast<const FlacCand*>(table + sizeof(int64_t));
+      if (total <= cap) break;
+      cap = total;
+    }
+    // each stream's chain; candidates are in scan order, so stream by stream
+    kept.clear();
+    int64_t c0 = 0, g_base = 0, scratch_base = 0;
+    for (int s = 0; s < ng; ++s) {
+      int64_t c1 = c0;
+      while (c1 < total && cand[c1].stream == s) ++c1;
+      const size_t k0 = kept.size();
+      if (!flac_chain(payload + b0, b0, first + s, gs[s], sources[first + s].frames, cand, c0, c1, g_base, scratch_base,
+                      &kept))
+        return NSF_ERR_BAD_ARG;
+      for (size_t k = k0; k < kept.size(); ++k) kept[k].stream = s;
+      g_base += sources[first + s].frames;
+      scratch_base += sources[first + s].frames * sources[first + s].channels;
+      c0 = c1;
+    }
+    if (kept.size() > static_cast<size_t>(INT32_MAX)) { set_error("nsf_flac_decode_host: too many frames"); return NSF_ERR_UNSUPPORTED; }
+    const size_t kept_bytes = kept.size() * sizeof(FlacKept);
+    DescEntry* de_kept = nullptr;
+    st = desc_upload(ctx, sl->stream, kept_bytes, nullptr, kept_bytes, &de_kept,
+                     [&](void* mem) { std::memcpy(mem, kept.data(), kept_bytes); });
+    if (st != NSF_OK) return st;
+    NSF_LAUNCH(ctx, launch_flac_decode(sl->stream, d_streams, d_cand, static_cast<const FlacKept*>(de_kept->dev.ptr),
+                                       static_cast<int>(kept.size()), max_ch, out_frames, d_payload, d_scratch,
+                                       static_cast<uint8_t*>(sl->out[0].ptr)));
+    if ((st = desc_commit(de_streams, sl->stream)) != NSF_OK || (st = desc_commit(de_kept, sl->stream)) != NSF_OK) return st;
+    return download(sl, 0, static_cast<uint8_t*>(pcm_host) + out_off[first], out_bytes, out_bytes, 1, out_dma);
+  });
+}
+
 // ---- collect ---------------------------------------------------------------------------------------
 // Checks shared by the collect calls (element type, column counts, offsets) and their output packing: o_off is the
 // prefix sum of nsf_collect_rows(), and must equal o_off_in when that is given.

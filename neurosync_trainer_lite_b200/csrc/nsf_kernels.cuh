@@ -174,6 +174,42 @@ int launch_csv_row_offsets(cudaStream_t s, const CsvView& v, int32_t* tile_rows,
 int launch_csv_parse(cudaStream_t s, const CsvView& v, int dtype, int32_t* tile_rows, int64_t* tile_start,
                      int64_t* row_start, uint32_t* col_flags, void* out, int64_t out_ld, uint32_t* status);
 
+// FLAC frames (nsf_flac.cu).  Byte positions are relative to the group's payload; a stream's scan positions are
+// [scan0, scan0 + end - begin) of the group's scan space (the streams' frame bytes one after the other, so that
+// streams sharing payload bytes are each scanned).
+struct FlacStream {
+  int64_t begin, end;   // frame bytes of the stream
+  int64_t scan0;        // first scan position
+  int64_t out0;         // first output byte
+  int32_t channels, bits, sample_rate, max_block;
+};
+struct FlacCand {       // a sync candidate: header fields and the result of decoding the frame that starts there
+  int64_t start, end;   // frame bytes [start, end)
+  int64_t number;       // coded number
+  int32_t stream, block, status, assignment;   // status NSF_FLAC_*; assignment | variable << 4
+  uint32_t sub_bit[8];  // first bit of each subframe, from `start`
+};
+struct FlacKept {       // a frame on a stream's frame chain
+  int32_t cand, stream;
+  int64_t g0;           // first output frame of the frame in the group (sorted)
+  int64_t first;        // first sample of the frame in its stream
+  int64_t scratch0;     // its samples in the int32 scratch: channel c at scratch0 + c * block
+};
+constexpr int kFlacScanTile = 4096;   // scan positions per block of the sync scan
+// k_flac_count + k_flac_scan + k_flac_write + k_flac_parse: candidates in scan order; cand_total <- their count,
+// of which the first min(count, cap) are parsed into cand.  blk_count / blk_off: one entry per scan tile.
+int launch_flac_scan_parse(cudaStream_t s, const FlacStream* streams, int n_streams, int64_t scan_total,
+                           const uint8_t* payload, int32_t* blk_count, int64_t* blk_off, int64_t* cand_total,
+                           int64_t* cand_pos, FlacCand* cand, int64_t cap);
+// k_flac_decode (one thread per kept frame and channel) + k_flac_interleave (one thread per output frame)
+int launch_flac_decode(cudaStream_t s, const FlacStream* streams, const FlacCand* cand, const FlacKept* kept,
+                       int n_kept, int max_channels, int64_t out_frames, const uint8_t* payload, int32_t* scratch,
+                       uint8_t* out);
+// The header at payload[pos] of a stream ending at `end`: NSF_FLAC_OK or why no frame starts there (no sync,
+// truncated, bad number, CRC-8).  Host-side diagnosis of a broken frame chain.
+int flac_header_status(const uint8_t* payload, int64_t pos, int64_t end);
+const char* flac_status_text(int status);
+
 // One-time (per device) cudaFuncSetAttribute calls of each translation unit; nsf_ctx_create runs them so that no
 // launch path touches function attributes.
 bool init_kernel_attributes();        // nsf_kernels.cu

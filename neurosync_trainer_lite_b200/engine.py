@@ -279,6 +279,26 @@ class Engine:
                                               C.c_void_p(out.data_ptr()), off.ctypes.data_as(nv._i64p)))
         return out[:int(off[-1])], off
 
+    # ---- FLAC decode: frame bytes -> WAV data-chunk bytes ---------------------------------------------------
+    def flac_decode_host(self, payload, sources):
+        """Decode FLAC streams on the device (``nsf_flac_decode_host``).
+
+        ``payload``: 1-D uint8 host array (or bytes); ``sources``: ``nv.FLAC_SOURCE`` array, one record per stream
+        (its frame bytes and STREAMINFO).  Returns ``(uint8 PCM, byte offsets)``: stream i is
+        ``pcm[offsets[i]:offsets[i + 1]]``, the WAV data chunk of its samples (u8, i16 or packed i24, interleaved).
+        A corrupt stream raises ``NsfError`` (status ``ERR_BAD_ARG``) naming the stream, frame offset and reason."""
+        payload = np.frombuffer(payload, dtype=np.uint8) if isinstance(payload, (bytes, bytearray)) else \
+            np.ascontiguousarray(payload).view(np.uint8).reshape(-1)
+        src = np.ascontiguousarray(np.asarray(sources, dtype=nv.FLAC_SOURCE).reshape(-1))
+        sizes = src["frames"] * src["channels"] * (src["bits"] // 8)
+        off = np.zeros(len(src) + 1, dtype=np.int64)
+        np.cumsum(sizes, out=off[1:])
+        out = np.empty(int(off[-1]), dtype=np.uint8)
+        with self._lock:
+            nv.check(nv.lib.nsf_flac_decode_host(self.handle, nv.ptr(payload), payload.nbytes, nv.ptr(src), len(src),
+                                                 nv.ptr(out)))
+        return out, off
+
     # ---- training windows of a packed dataset (dataset/dataset.py:58-98) ------------------------------
     @staticmethod
     def window_offsets(audio_offsets, facial_offsets, window):

@@ -1,11 +1,17 @@
 """Audio loaders with the reference's names and return conventions (``utils/audio/load_audio.py``).
 
 Division of labour
-* **decode** (RIFF/WAV container -> PCM) stays on the host: it is container parsing, not arithmetic
-  (SURVEY.md section 8(f)-2 lists on-device decode/resample as a later row).  The reference decodes
-  through ``librosa.load`` -> soundfile; here a small RIFF reader does the same conversions
-  (int16 / 32768, int24 / 2**23, int32 / 2**31, uint8 (v - 128) / 128, float32 as is, channels
-  averaged) because neither librosa nor soundfile is installable in this image.
+* **decode** (container -> PCM).  The reference decodes through ``librosa.load`` -> soundfile (libsndfile); neither
+  is installable in this image, so ``decode`` dispatches on the stream's first bytes:
+  - RIFF/WAVE: a small RIFF reader on the host (container parsing, not arithmetic; SURVEY.md section 8(f)-2) does
+    soundfile's conversions (int16 / 32768, int24 / 2**23, int32 / 2**31, uint8 (v - 128) / 128, float32 as is,
+    channels averaged);
+  - FLAC (``fLaC``): ``flac_layout`` reads the metadata blocks on the host and the frames (Rice codes and linear
+    prediction over every sample) are decoded on the GPU through ``nsf_flac_decode_host``, which writes the WAV data
+    chunk of the decoded samples; the same host tail as for WAV turns it into the array, so a FLAC file gives exactly
+    what the WAV holding its samples gives.  Bits per sample 8, 16 and 24; each frame's CRC-8 and CRC-16 are
+    checked, the STREAMINFO MD5 is not;
+  - anything else (MP3, Ogg, ...) raises ``ValueError``.
 * **peak normalisation** ``y / max|y|`` (reference ``load_audio.py:12-14``) runs on the GPU through
   ``nsf_normalize_host`` - or, on the feature path, fused into ``nsf_extract_host`` via
   ``NSF_PEAK_NORMALIZE`` so the PCM crosses PCIe once, as int16 when the file is int16.
@@ -34,6 +40,8 @@ WAV_ENCODINGS = {(1, 8): nv.ENC_U8, (1, 16): nv.ENC_I16, (1, 24): nv.ENC_I24, (1
                  (3, 32): nv.ENC_F32, (3, 64): nv.ENC_F64}
 
 WavLayout = namedtuple("WavLayout", "tag channels rate bits data_offset data_bytes")
+FlacLayout = namedtuple("FlacLayout", "channels rate bits frames max_block data_offset data_bytes")
+FLAC_BITS = (8, 16, 24)
 
 
 def wav_layout(fh):
@@ -71,11 +79,16 @@ def decode_wav(data):
     """RIFF/WAVE bytes -> (pcm, native_sr).  pcm is int16 (mono PCM16 files, kept as is so it can
     be uploaded at 2 bytes/sample) or float32 in [-1, 1) (everything else, soundfile scaling)."""
     code, channels, sr, bits, off, n = wav_layout(io.BytesIO(data))
-    payload = data[off:off + n]
+    return _samples(code, channels, bits, data[off:off + n]), sr
+
+
+def _samples(code, channels, bits, payload):
+    """The samples of a WAV data chunk as ``decode_wav`` returns them: int16 for mono PCM16, else float32 in
+    [-1, 1) with soundfile's scaling, channels averaged."""
     if code == 1 and bits == 16:
         pcm = np.frombuffer(payload, dtype="<i2", count=len(payload) // 2)
         if channels == 1:
-            return pcm.copy(), sr
+            return pcm.copy()
         x = pcm.astype(np.float32) / np.float32(32768)
     elif code == 1 and bits == 8:
         x = (np.frombuffer(payload, dtype=np.uint8).astype(np.float32) - 128) / np.float32(128)
@@ -93,7 +106,79 @@ def decode_wav(data):
         x = np.frombuffer(payload, dtype="<f8", count=len(payload) // 8).astype(np.float32)
     if channels > 1:
         x = x[: len(x) // channels * channels].reshape(-1, channels).mean(axis=1, dtype=np.float32)
-    return np.ascontiguousarray(x, dtype=np.float32), sr
+    return np.ascontiguousarray(x, dtype=np.float32)
+
+
+def flac_layout(fh):
+    """``FlacLayout`` of the seekable binary FLAC stream ``fh``, read from its metadata blocks: STREAMINFO's
+    channels, rate, bits per sample, total samples per channel and maximum block size, and the byte range of the
+    frames (everything after the last metadata block).  Blocks after STREAMINFO (padding, seek table, tags,
+    pictures, ...) are skipped.  ``ValueError`` for every stream ``decode_flac`` does not decode: no ``fLaC``
+    marker (an ID3v2 tag or an Ogg page in front included), a missing, misplaced or repeated STREAMINFO, an
+    invalid block type, a truncated block, no frame data, 12-, 20- or 32-bit samples, an unknown length (total
+    samples 0)."""
+    size = fh.seek(0, io.SEEK_END)
+    fh.seek(0)
+    magic = fh.read(4)
+    if magic != b"fLaC":
+        if magic[:3] == b"ID3":
+            raise ValueError("FLAC stream behind an ID3v2 tag is not supported")
+        if magic == b"OggS":
+            raise ValueError("Ogg-encapsulated FLAC is not supported")
+        raise ValueError("not a FLAC stream (no fLaC marker)")
+    pos, info, last = 4, None, False
+    while not last:
+        head = fh.read(4)
+        if len(head) < 4:
+            raise ValueError(f"truncated FLAC metadata block header at byte {pos}")
+        last, kind, n = head[0] >> 7, head[0] & 0x7F, int.from_bytes(head[1:4], "big")
+        if kind == 127:
+            raise ValueError(f"invalid FLAC metadata block type 127 at byte {pos}")
+        if pos + 4 + n > size:
+            raise ValueError(f"truncated FLAC metadata block at byte {pos}")
+        if (kind == 0) != (info is None):
+            raise ValueError("STREAMINFO is not the first FLAC metadata block" if info is None
+                             else "more than one STREAMINFO block")
+        if kind == 0:
+            if n != 34:
+                raise ValueError(f"STREAMINFO block of {n} bytes (34 expected)")
+            info = int.from_bytes(fh.read(34)[:18], "big")
+        else:
+            fh.seek(n, io.SEEK_CUR)
+        pos += 4 + n
+    max_block = (info >> 112) & 0xFFFF
+    rate = (info >> 44) & 0xFFFFF
+    channels = ((info >> 41) & 7) + 1
+    bits = ((info >> 36) & 31) + 1
+    frames = info & ((1 << 36) - 1)
+    if bits not in FLAC_BITS:
+        raise ValueError(f"unsupported FLAC bits per sample {bits} (8, 16 and 24 are decoded)")
+    if frames == 0:
+        raise ValueError("FLAC STREAMINFO total samples is 0 (unknown length)")
+    if rate == 0:
+        raise ValueError("FLAC STREAMINFO sample rate is 0")
+    if max_block == 0:
+        raise ValueError("FLAC STREAMINFO maximum block size is 0")
+    if pos >= size:
+        raise ValueError("truncated FLAC stream: no frame data")
+    return FlacLayout(channels, rate, bits, frames, max_block, pos, size - pos)
+
+
+def decode_flac(data):
+    """FLAC bytes -> (pcm, native_sr): what ``decode_wav`` returns for the WAV holding the same samples.  The frames
+    are decoded on the GPU into the WAV data chunk (u8 v + 128, i16, packed i24); ``ValueError`` for a stream
+    ``flac_layout`` rejects and for a corrupt frame (naming its byte offset and the reason)."""
+    lay = flac_layout(io.BytesIO(data))
+    src = np.array([(lay.data_offset, lay.data_bytes, lay.frames, lay.channels, lay.bits, lay.rate, lay.max_block)],
+                   dtype=nv.FLAC_SOURCE)
+    f, h = _engine.frame_params(REFERENCE_RATE)
+    try:
+        pcm, _ = _engine.get_engine(REFERENCE_RATE, f, h).flac_decode_host(np.frombuffer(data, dtype=np.uint8), src)
+    except nv.NsfError as e:
+        if e.status != nv.ERR_BAD_ARG:
+            raise
+        raise ValueError(nv.last_error() or str(e)) from None
+    return _samples(1, lay.channels, lay.bits, pcm), lay.rate
 
 
 def _resample(y, orig_sr, target_sr):
@@ -113,7 +198,8 @@ def _read(source):
 
 def decode(source, sr):
     """``librosa.load(source, sr=sr)`` without the normalisation: (pcm int16|float32, sr)."""
-    pcm, native = decode_wav(_read(source))
+    data = _read(source)
+    pcm, native = decode_flac(data) if data[:4] == b"fLaC" else decode_wav(data)
     if sr is not None and native != sr:
         pcm = _resample(pcm, native, sr)
         native = sr
