@@ -38,7 +38,6 @@ namespace nsf {
 
 namespace {
 
-constexpr int kSmCount = 148;
 constexpr int kFrontMargin = 16;   // halfs of zeros before X(0)  (B reads back to X(-7))
 constexpr int kBackMargin = 160;   // halfs of zeros after the last K-block (the A prefetch of one block beyond reads up to +151)
 constexpr int kVals = 6;           // lags per thread that can be <= 191
@@ -955,7 +954,8 @@ int launch_autocorr_mma(cudaStream_t s, const DeviceTables& t, const BatchView& 
     if (pgrid > kSmCount) pgrid = kSmCount;
     if (pgrid < 1) pgrid = 1;
     k_autocorr_pipe<23, 92, kPipeWarps, 1><<<static_cast<int>(pgrid), kPipeWarps * 32, pipe_smem, s>>>(t, b, y, reduce, out, out_ld, col0);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    NSF_CHECK_LAUNCH();
+    return 1;
   }
   const int per_sm = smem <= 113 * 1024 ? 2 : 1;
   int64_t grid = (b.total_rows + warps - 1) / warps;
@@ -965,7 +965,8 @@ int launch_autocorr_mma(cudaStream_t s, const DeviceTables& t, const BatchView& 
   auto go = [&](auto k_five, auto k_six) {
     if (use_six) k_six<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
     else k_five<<<static_cast<int>(grid), threads, smem, s>>>(t, b, y, reduce, out, out_ld, col0);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    NSF_CHECK_LAUNCH();
+    return 1;
   };
 #define NSF_AC_GO(IT, EX) go(k_autocorr_sym<IT, EX, true>, k_autocorr_sym<IT, EX, false>)
   if (iters == 23) return NSF_AC_GO(23, true);    // 88.2 kHz: F = 1470

@@ -4,10 +4,8 @@
 #include <cstdint>
 
 #include "nsf.h"
+#include "nsf_device_utils.cuh"
 #include "nsf_kernels.cuh"
-
-#define NSF_CHECK_LAUNCH() \
-  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
 
 namespace nsf {
 namespace {
@@ -83,21 +81,12 @@ __device__ __forceinline__ float decode_frame(const uint8_t* clip, int64_t n, in
   return s / static_cast<float>(channels);
 }
 
-__device__ __forceinline__ int find_clip(const ConvClip* c, int n, int64_t tile) {
-  int lo = 0, hi = n - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (c[mid].tile0 <= tile) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
 }  // namespace
 
 // Same-rate clips: decode + downmix only.  kConvDecodeTile frames per block.
 __global__ void __launch_bounds__(256) k_convert_decode(const ConvClip* __restrict__ clips, int n_clips,
                                                         const uint8_t* __restrict__ payload, float* __restrict__ out) {
-  const ConvClip c = clips[find_clip(clips, n_clips, blockIdx.x)];
+  const ConvClip c = clips[last_le(n_clips, blockIdx.x, [&](int i) { return clips[i].tile0; })];
   const int64_t f0 = (blockIdx.x - c.tile0) * kConvDecodeTile;
   const int64_t f1 = min(f0 + kConvDecodeTile, c.frames);
   const uint8_t* src = payload + c.byte_off;
@@ -117,7 +106,7 @@ __global__ void __launch_bounds__(256) k_convert_resample(const ConvClip* __rest
                                                           const uint8_t* __restrict__ payload,
                                                           float* __restrict__ out) {
   extern __shared__ double s_x[];
-  const ConvClip c = clips[find_clip(clips, n_clips, blockIdx.x)];
+  const ConvClip c = clips[last_le(n_clips, blockIdx.x, [&](int i) { return clips[i].tile0; })];
   const int64_t span = static_cast<int64_t>(c.slots) * c.reps;
   const int64_t j0 = (blockIdx.x - c.tile0) * span;
   const int64_t lo = ((j0 + c.n_pre_remove) * c.down - c.n_pre_pad) / c.up - (c.kmax - 1);

@@ -14,11 +14,9 @@
 #include <cstring>
 
 #include "nsf.h"
+#include "nsf_device_utils.cuh"
 #include "nsf_internal.h"
 #include "nsf_kernels.cuh"
-
-#define NSF_CHECK_LAUNCH() \
-  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
 
 namespace nsf {
 namespace {
@@ -224,34 +222,15 @@ __host__ __device__ __forceinline__ int64_t header_pos(int64_t c) {
 __device__ __forceinline__ double csv_value(const float* p) { return static_cast<double>(__ldg(p)); }
 __device__ __forceinline__ double csv_value(const double* p) { return __ldg(p); }
 
-// Block reduction / exclusive scan helpers over kCsvThreads threads.
-__device__ __forceinline__ int warp_inclusive_scan(int v, int lane) {
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int t = __shfl_up_sync(0xffffffffu, v, o);
-    if (lane >= o) v += t;
-  }
-  return v;
-}
-
 // One block per row: row_len[r] = bytes of row r, separators and newline included.
 template <typename T>
 __global__ void __launch_bounds__(kCsvThreads) k_csv_lengths(const T* __restrict__ rows, int cols,
                                                              int64_t* __restrict__ row_len) {
-  __shared__ int64_t s_warp[kCsvThreads / 32];
   const T* row = rows + static_cast<int64_t>(blockIdx.x) * cols;
   int64_t sum = 0;
   for (int c = threadIdx.x; c < cols; c += kCsvThreads) sum += field_bytes(make_field(csv_value(row + c)), cols);
-#pragma unroll
-  for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-  if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = sum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int64_t t = 0;
-#pragma unroll
-    for (int w = 0; w < kCsvThreads / 32; ++w) t += s_warp[w];
-    row_len[blockIdx.x] = t;
-  }
+  sum = block_sum<kCsvThreads>(sum);
+  if (threadIdx.x == 0) row_len[blockIdx.x] = sum;
 }
 
 // Blocks [0, n_rows): row b at text + start[b].  Blocks [n_rows, n_rows + n_files): the header of file b - n_rows
@@ -262,7 +241,6 @@ template <typename T>
 __global__ void __launch_bounds__(kCsvThreads) k_csv_write(const T* __restrict__ rows, int64_t n_rows, int cols,
                                                            const int64_t* __restrict__ start, char* __restrict__ text) {
   __shared__ __align__(16) char s_buf[kCsvThreads * kCsvFieldMax + 16];
-  __shared__ int s_warp[kCsvThreads / 32];
   const int64_t b = blockIdx.x;
   int64_t pos = start[b];
   if (b >= n_rows) {
@@ -276,7 +254,6 @@ __global__ void __launch_bounds__(kCsvThreads) k_csv_write(const T* __restrict__
     return;
   }
   const T* row = rows + b * cols;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int c0 = 0; c0 < cols; c0 += kCsvThreads) {
     const int c = c0 + static_cast<int>(threadIdx.x);
     Field f{};
@@ -285,19 +262,12 @@ __global__ void __launch_bounds__(kCsvThreads) k_csv_write(const T* __restrict__
       f = make_field(csv_value(row + c));
       len = field_bytes(f, cols);
     }
-    const int incl = warp_inclusive_scan(len, lane);
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    int before = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < kCsvThreads / 32; ++w) {
-      const int t = s_warp[w];
-      before += w < warp ? t : 0;
-      total += t;
-    }
+    // the scan's first barrier also orders this tile's s_buf writes after the previous tile's stores
+    int total;
+    const int before = block_exclusive_scan<kCsvThreads>(len, &total);
     const int head = static_cast<int>(pos & 15);
     if (c < cols) {
-      char* p = s_buf + head + before + incl - len;
+      char* p = s_buf + head + before;
       if (f.kind == kNan && cols == 1) { p[0] = '"'; p[1] = '"'; }
       else put_field(f, p);
       p[len - 1] = c == cols - 1 ? '\n' : ',';
@@ -314,7 +284,6 @@ __global__ void __launch_bounds__(kCsvThreads) k_csv_write(const T* __restrict__
       }
     }
     pos += total;
-    __syncthreads();   // s_buf and s_warp are the next tile's
   }
 }
 

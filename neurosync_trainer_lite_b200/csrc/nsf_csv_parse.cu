@@ -8,7 +8,7 @@
 // by the double literal 1e<k> (two divisions below 1e-308).  The first 15 digits accumulate in a uint64_t, where
 // every intermediate is exact, as it is in the double chain; digits 16 and 17 continue in doubles.  nvcc would
 // contract number * 10 + d into a DFMA (--fmad=true), which rounds once instead of twice: the device code spells
-// every operation with __dmul_rn / __dadd_rn / __ddiv_rn.
+// every operation with mul_rn / add_rn / div_rn (nsf_device_utils.cuh).
 //
 // Kernels of one parse call (the row-offsets call runs the first two):
 //   k_csv_count   one block per text tile (16 KB, never across a file boundary): data rows starting in the tile
@@ -24,11 +24,9 @@
 #include <cstring>
 
 #include "nsf.h"
+#include "nsf_device_utils.cuh"
 #include "nsf_internal.h"
 #include "nsf_kernels.cuh"
-
-#define NSF_CHECK_LAUNCH() \
-  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
 
 namespace nsf {
 namespace {
@@ -53,27 +51,6 @@ __host__ __device__ __forceinline__ double e10(int k) {
   return __ldg(d_e10 + k);
 #else
   return h_e10[k];
-#endif
-}
-__host__ __device__ __forceinline__ double mul_rn(double a, double b) {
-#ifdef __CUDA_ARCH__
-  return __dmul_rn(a, b);
-#else
-  return a * b;
-#endif
-}
-__host__ __device__ __forceinline__ double add_rn(double a, double b) {
-#ifdef __CUDA_ARCH__
-  return __dadd_rn(a, b);
-#else
-  return a + b;
-#endif
-}
-__host__ __device__ __forceinline__ double div_rn(double a, double b) {
-#ifdef __CUDA_ARCH__
-  return __ddiv_rn(a, b);
-#else
-  return a / b;
 #endif
 }
 __host__ __device__ __forceinline__ double from_bits(uint64_t b) {
@@ -187,18 +164,9 @@ __device__ __forceinline__ uint32_t byte_of(const uint4& w, int k) {
 
 struct Tile { int64_t fb, fe, lo, hi; int file; };   // file bytes, tile bytes [lo, hi)
 
-__device__ __forceinline__ int upper_file(const int64_t* off, int n, int64_t x) {   // last i < n with off[i] <= x
-  int a = 0, b = n - 1;
-  while (a < b) {
-    const int m = (a + b + 1) >> 1;
-    if (__ldg(off + m) <= x) a = m; else b = m - 1;
-  }
-  return a;
-}
-
 __device__ __forceinline__ Tile tile_of(const CsvView& v, int64_t t) {
   Tile r;
-  r.file = upper_file(v.tile_off, v.n_files, t);
+  r.file = find_segment(v.tile_off, v.n_files, t);
   r.fb = __ldg(v.text_off + r.file);
   r.fe = __ldg(v.text_off + r.file + 1);
   const int64_t a = (r.fb / kCsvTile + (t - __ldg(v.tile_off + r.file))) * kCsvTile;
@@ -233,43 +201,10 @@ __device__ __forceinline__ uint64_t row_starts(const char* text, const Tile& t, 
 }
 
 __global__ void __launch_bounds__(kTileThreads) k_csv_count(CsvView v, int32_t* __restrict__ tile_rows) {
-  __shared__ int s_warp[kTileThreads / 32];
   const Tile t = tile_of(v, blockIdx.x);
   const int64_t base = t.lo / kCsvTile * kCsvTile + 64 * threadIdx.x;
-  int c = __popcll(row_starts(v.text, t, base));
-#pragma unroll
-  for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int s = 0;
-#pragma unroll
-    for (int w = 0; w < kTileThreads / 32; ++w) s += s_warp[w];
-    tile_rows[blockIdx.x] = s;
-  }
-}
-
-template <int kThreads>
-__device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t* s_warp, int64_t* total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int64_t incl = x;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int64_t y = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += y;
-  }
-  if (lane == 31) s_warp[warp] = incl;
-  __syncthreads();
-  int64_t before = 0, all = 0;
-#pragma unroll
-  for (int w = 0; w < kThreads / 32; ++w) {
-    const int64_t s = s_warp[w];
-    before += w < warp ? s : 0;
-    all += s;
-  }
-  __syncthreads();   // s_warp is free for the next scan
-  *total = all;
-  return before + incl - x;
+  const int c = block_sum<kTileThreads>(__popcll(row_starts(v.text, t, base)));
+  if (threadIdx.x == 0) tile_rows[blockIdx.x] = c;
 }
 
 // One block: tile_start[t] = data rows before tile t (n_tiles + 1 entries); row_off[i] = rows before file i.  With
@@ -277,14 +212,7 @@ __device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t* s_wa
 __global__ void __launch_bounds__(kScanThreads) k_csv_scan(CsvView v, const int32_t* __restrict__ tile_rows,
                                                            int64_t* __restrict__ tile_start, int64_t* __restrict__ row_off,
                                                            const int64_t* __restrict__ given, uint32_t* __restrict__ status) {
-  __shared__ int64_t s_warp[kScanThreads / 32];
-  const int64_t n = v.n_tiles, per = (n + kScanThreads - 1) / kScanThreads;
-  const int64_t a = min(n, per * threadIdx.x), b = min(n, a + per);
-  int64_t sum = 0;
-  for (int64_t t = a; t < b; ++t) sum += tile_rows[t];
-  int64_t total;
-  int64_t run = block_exclusive_scan<kScanThreads>(sum, s_warp, &total);
-  for (int64_t t = a; t < b; ++t) { tile_start[t] = run; run += tile_rows[t]; }
+  const int64_t n = v.n_tiles, total = scan_counts<kScanThreads>(tile_rows, n, tile_start);
   if (threadIdx.x == 0) tile_start[n] = total;
   __syncthreads();
   for (int i = threadIdx.x; i <= v.n_files; i += kScanThreads) {
@@ -300,12 +228,11 @@ __global__ void __launch_bounds__(kScanThreads) k_csv_scan(CsvView v, const int3
 // row_start[r] = byte position of data row r, for r < n_rows.
 __global__ void __launch_bounds__(kTileThreads) k_csv_starts(CsvView v, const int64_t* __restrict__ tile_start,
                                                              int64_t n_rows, int64_t* __restrict__ row_start) {
-  __shared__ int64_t s_warp[kTileThreads / 32];
   const Tile t = tile_of(v, blockIdx.x);
   const int64_t base = t.lo / kCsvTile * kCsvTile + 64 * threadIdx.x;
   uint64_t m = row_starts(v.text, t, base);
   int64_t total;
-  int64_t r = tile_start[blockIdx.x] + block_exclusive_scan<kTileThreads>(__popcll(m), s_warp, &total);
+  int64_t r = tile_start[blockIdx.x] + block_exclusive_scan<kTileThreads>(int64_t(__popcll(m)), &total);
   for (; m; m &= m - 1, ++r)
     if (r < n_rows) row_start[r] = base + __ffsll(static_cast<long long>(m)) - 1;
 }
@@ -329,7 +256,7 @@ __global__ void __launch_bounds__(32 * kFieldWarps) k_csv_fields(CsvView v, cons
   int16_t* term = s_term[wb];
   for (int64_t r = static_cast<int64_t>(blockIdx.x) * kFieldWarps + wb; r < v.n_rows;
        r += static_cast<int64_t>(gridDim.x) * kFieldWarps) {
-    const int f = upper_file(v.row_off, v.n_files, r);
+    const int f = find_segment(v.row_off, v.n_files, r);
     const int64_t fb = __ldg(v.text_off + f), fe = __ldg(v.text_off + f + 1);
     int64_t cur = row_start[r];
     uint32_t bad = 0;
@@ -358,12 +285,7 @@ __global__ void __launch_bounds__(32 * kFieldWarps) k_csv_fields(CsvView v, cons
       uint32_t tm = comma & (mine >= 16 ? 0xffffu : mine <= 0 ? 0u : (1u << mine) - 1);
       if (mine >= 0 && mine < 16) tm |= 1u << mine;
       const int cnt = __popc(tm);
-      int incl = cnt;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += y;
-      }
+      const int incl = warp_inclusive_scan(cnt);
       const int total = __shfl_sync(0xffffffffu, incl, 31);
       for (int k = incl - cnt; tm; tm &= tm - 1, ++k) term[k] = static_cast<int16_t>(16 * lane + __ffs(tm) - 1);
       __syncwarp();
@@ -464,10 +386,7 @@ int launch_csv_parse(cudaStream_t s, const CsvView& v, int dtype, int32_t* tile_
   if (v.n_rows == 0 || v.n_tiles == 0) return m;   // (rows without text: the scan has marked every file)
   k_csv_starts<<<static_cast<unsigned>(v.n_tiles), kTileThreads, 0, s>>>(v, tile_start, v.n_rows, row_start);
   NSF_CHECK_LAUNCH();
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int64_t blocks = std::min<int64_t>((v.n_rows + kFieldWarps - 1) / kFieldWarps, int64_t(sms) * 8);
+  const int64_t blocks = std::min<int64_t>((v.n_rows + kFieldWarps - 1) / kFieldWarps, int64_t(kSmCount) * 8);
   if (dtype == NSF_F64) {
     k_csv_fields<double><<<static_cast<unsigned>(blocks), 32 * kFieldWarps, 0, s>>>(
         v, row_start, static_cast<double*>(out), out_ld, col_flags, status);

@@ -18,11 +18,9 @@
 #include <cstring>
 
 #include "nsf.h"
+#include "nsf_device_utils.cuh"
 #include "nsf_internal.h"
 #include "nsf_kernels.cuh"
-
-#define NSF_CHECK_LAUNCH() \
-  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
 
 #define HD __host__ __device__ __forceinline__
 
@@ -332,19 +330,10 @@ HD int decode_frame(const uint8_t* d, int64_t pos, const FlacStream& st, const u
   return fc->status = (crc == stored ? NSF_FLAC_OK : NSF_FLAC_BAD_CRC16);
 }
 
-// Stream owning scan position p (streams sorted by scan0).
-__device__ __forceinline__ int find_stream(const FlacStream* s, int n, int64_t p) {
-  int lo = 0, hi = n - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (s[mid].scan0 <= p) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
-// Is scan position p a candidate: a sync code whose header parses and passes its CRC-8?
+// Is scan position p a candidate: a sync code whose header parses and passes its CRC-8?  The stream owning p is the
+// last one whose scan0 <= p (streams sorted by scan0).
 __device__ __forceinline__ bool is_candidate(const FlacStream* streams, int n, const uint8_t* d, int64_t p) {
-  const FlacStream& st = streams[find_stream(streams, n, p)];
+  const FlacStream& st = streams[last_le(n, p, [&](int i) { return streams[i].scan0; })];
   const int64_t pos = st.begin + (p - st.scan0);
   if (d[pos] != 0xFF) return false;
   Header h;
@@ -364,24 +353,11 @@ __global__ void __launch_bounds__(256) k_flac_count(const FlacStream* __restrict
   if (threadIdx.x == 0) blk_count[blockIdx.x] = count;
 }
 
-// Exclusive scan of the tile counts by one block of 1024 threads: each thread owns a contiguous run of tiles.
+// Exclusive scan of the tile counts by one block of 1024 threads.
 __global__ void __launch_bounds__(1024) k_flac_scan(const int32_t* __restrict__ blk_count, int64_t n_blk,
                                                     int64_t* __restrict__ blk_off, int64_t* __restrict__ cand_total) {
-  __shared__ int64_t s[1024];
-  const int64_t per = (n_blk + 1023) / 1024, b0 = threadIdx.x * per, b1 = min(b0 + per, n_blk);
-  int64_t sum = 0;
-  for (int64_t b = b0; b < b1; ++b) sum += blk_count[b];
-  s[threadIdx.x] = sum;
-  __syncthreads();
-  for (int off = 1; off < 1024; off <<= 1) {
-    const int64_t v = threadIdx.x >= off ? s[threadIdx.x - off] : 0;
-    __syncthreads();
-    s[threadIdx.x] += v;
-    __syncthreads();
-  }
-  int64_t run = s[threadIdx.x] - sum;
-  for (int64_t b = b0; b < b1; ++b) { blk_off[b] = run; run += blk_count[b]; }
-  if (threadIdx.x == 1023) *cand_total = s[1023];
+  const int64_t total = scan_counts<1024>(blk_count, n_blk, blk_off);
+  if (threadIdx.x == 0) *cand_total = total;
 }
 
 // The candidates of a tile at blk_off[tile] + their rank in byte order (position rows of 256, warps in order).
@@ -420,7 +396,7 @@ __global__ void __launch_bounds__(kParseThreads) k_flac_parse(const FlacStream* 
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= min(*cand_total, cap)) return;
   const int64_t p = cand_pos[i];
-  const int s = find_stream(streams, n, p);
+  const int s = last_le(n, p, [&](int j) { return streams[j].scan0; });
   FlacCand fc;
   fc.stream = s;
   decode_frame(d, streams[s].begin + (p - streams[s].scan0), streams[s], crc_tab, &fc, nullptr);
@@ -456,12 +432,7 @@ __global__ void __launch_bounds__(256) k_flac_interleave(const FlacStream* __res
                                                          const int32_t* __restrict__ scratch, uint8_t* __restrict__ out) {
   const int64_t g = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (g >= n_out) return;
-  int lo = 0, hi = n_kept - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (kept[mid].g0 <= g) lo = mid; else hi = mid - 1;
-  }
-  const FlacKept kf = kept[lo];
+  const FlacKept kf = kept[last_le(n_kept, g, [&](int i) { return kept[i].g0; })];
   const FlacStream& st = streams[kf.stream];
   const int block = cand[kf.cand].block, assignment = cand[kf.cand].assignment & 15;
   const int64_t i = g - kf.g0;

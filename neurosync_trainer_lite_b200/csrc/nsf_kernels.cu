@@ -23,8 +23,6 @@ namespace nsf {
 
 namespace {
 
-constexpr int kSmCount = 148;
-
 template <typename T> __device__ __forceinline__ float decode_pcm(T v);
 template <> __device__ __forceinline__ float decode_pcm<float>(float v) { return v; }
 template <> __device__ __forceinline__ float decode_pcm<int16_t>(int16_t v) {
@@ -1071,16 +1069,6 @@ __global__ void __launch_bounds__(256) k_smooth(BatchView b, const float* __rest
 // collect_features augmentation.  One warp per output row, every warp walking short runs of consecutive rows;
 // the row's provenance (which version, blend weights) is resolved once, then the lanes stream the 256 + 61 columns.
 // ------------------------------------------------------------------------------------------------
-template <typename T> struct Arith;
-template <> struct Arith<double> {
-  static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
-  static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
-};
-template <> struct Arith<float> {
-  static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
-  static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
-};
-
 // np.linspace(start, stop, n)[i] exactly as numpy evaluates it (arange * step + start, endpoint set)
 __device__ __forceinline__ double linspace_at(double start, double stop, int64_t n, int64_t i) {
   if (n == 1) return start;
@@ -1094,16 +1082,15 @@ __device__ __forceinline__ double linspace_at(double start, double stop, int64_t
 template <typename T>
 __device__ __forceinline__ T version_value(const T* __restrict__ src, int64_t ld, int ver, int64_t j,
                                            int c, bool smooth_slow) {
-  using A = Arith<T>;
   auto at = [&](int64_t row) { return src[row * ld + c]; };
   auto slow = [&](int64_t k) -> T {
     if ((k & 1) == 0) return at(k >> 1);
-    return A::mul(A::add(at(k >> 1), at((k >> 1) + 1)), static_cast<T>(0.5));
+    return mul_rn(add_rn(at(k >> 1), at((k >> 1) + 1)), static_cast<T>(0.5));
   };
   if (ver == 0) return at(j);
   if (ver == 1) return at(2 * j);
   if (!smooth_slow || j == 0) return slow(j);
-  return A::mul(A::add(slow(j - 1), slow(j)), static_cast<T>(0.5));  // smooth_facial_data
+  return mul_rn(add_rn(slow(j - 1), slow(j)), static_cast<T>(0.5));  // smooth_facial_data
 }
 
 // float4 form of version_value for the float32 audio block (256 columns): four columns per lane and load,
@@ -1114,7 +1101,7 @@ __device__ __forceinline__ float4 add4(float4 a, float4 b) {
 __device__ __forceinline__ float4 mul4(float4 a, float s) {
   return make_float4(__fmul_rn(a.x, s), __fmul_rn(a.y, s), __fmul_rn(a.z, s), __fmul_rn(a.w, s));
 }
-__device__ __forceinline__ float4 mul4s(float s, float4 a) {      // scalar first, like A::mul(w, val)
+__device__ __forceinline__ float4 mul4s(float s, float4 a) {      // scalar first, like mul_rn(w, val)
   return make_float4(__fmul_rn(s, a.x), __fmul_rn(s, a.y), __fmul_rn(s, a.z), __fmul_rn(s, a.w));
 }
 __device__ __forceinline__ float4 version_value4(const float* __restrict__ src, int64_t ld, int ver, int64_t j,
@@ -1133,13 +1120,12 @@ __device__ __forceinline__ float4 version_value4(const float* __restrict__ src, 
 // The stack geometry of a clip (trim offsets, version lengths, blend zones) is derived once per clip and kept in
 // registers - round 1's block-per-row kernel recomputed it, behind a chain of dependent loads, with all 128 threads
 // of a block for every single row - and the lanes stream the 256 + 61 columns of the row with fully coalesced
-// 128-byte requests.  Arith<T>, linspace_at and version_value keep the float64 variant bit-exact.
+// 128-byte requests.  add_rn / mul_rn, linspace_at and version_value keep the float64 variant bit-exact.
 constexpr int kCollectRun = 4;      // consecutive rows per warp and tile
 template <typename T>
 __global__ void __launch_bounds__(256, 5) k_collect_rows(CollectView v, const T* __restrict__ audio, int a_cols,
                                                       const T* __restrict__ facial, int f_cols,
                                                       T* __restrict__ out_audio, T* __restrict__ out_facial) {
-  using A = Arith<T>;
   const int lane = threadIdx.x & 31, wr = threadIdx.x >> 5, wpb = blockDim.x >> 5;
   // Row order: the grid sweeps the output in TILES of wpb x kCollectRun consecutive rows (block b takes tiles b,
   // b + gridDim.x, ...; a warp takes kCollectRun consecutive rows of the tile), so at any time all resident warps
@@ -1247,7 +1233,7 @@ __global__ void __launch_bounds__(256, 5) k_collect_rows(CollectView v, const T*
         T val = version_value<T>(src, ld, term_ver, term_row, c, smooth_slow);
         for (int bi = n_blend - 1; bi >= 0; --bi) {
           const T nv_val = version_value<T>(src, ld, ver[blend_level[bi]], blend_q[bi], c, smooth_slow);
-          val = A::add(A::mul(w1[bi], val), A::mul(w2[bi], nv_val));
+          val = add_rn(mul_rn(w1[bi], val), mul_rn(w2[bi], nv_val));
         }
         dst[c] = val;
       }
@@ -1279,7 +1265,6 @@ template <typename T>
 __global__ void __launch_bounds__(256) k_rows_op(int op, const T* __restrict__ a, int64_t na,
                                                  const T* __restrict__ b, int64_t nb, int cols,
                                                  int64_t k, T* __restrict__ out, int64_t out_rows) {
-  using A = Arith<T>;
   const int64_t total = out_rows * cols;
   for (int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; e < total;
        e += static_cast<int64_t>(gridDim.x) * blockDim.x) {
@@ -1287,17 +1272,17 @@ __global__ void __launch_bounds__(256) k_rows_op(int op, const T* __restrict__ a
     const int c = static_cast<int>(e - r * cols);
     T v;
     if (op == NSF_ROWS_INTERP_SLOWER) {
-      v = (r & 1) ? A::mul(A::add(a[(r >> 1) * cols + c], a[((r >> 1) + 1) * cols + c]), static_cast<T>(0.5))
+      v = (r & 1) ? mul_rn(add_rn(a[(r >> 1) * cols + c], a[((r >> 1) + 1) * cols + c]), static_cast<T>(0.5))
                   : a[(r >> 1) * cols + c];
     } else if (op == NSF_ROWS_SMOOTH) {
-      v = r == 0 ? a[c] : A::mul(A::add(a[(r - 1) * cols + c], a[r * cols + c]), static_cast<T>(0.5));
+      v = r == 0 ? a[c] : mul_rn(add_rn(a[(r - 1) * cols + c], a[r * cols + c]), static_cast<T>(0.5));
     } else {  // NSF_ROWS_BLEND_STACK
       if (r < na - k) v = a[r * cols + c];
       else if (r < na) {
         const int64_t q = r - (na - k);
         const T w1 = static_cast<T>(linspace_at(1.0, 0.0, k, q));
         const T w2 = static_cast<T>(linspace_at(0.0, 1.0, k, q));
-        v = A::add(A::mul(w1, a[r * cols + c]), A::mul(w2, b[q * cols + c]));
+        v = add_rn(mul_rn(w1, a[r * cols + c]), mul_rn(w2, b[q * cols + c]));
       } else v = b[(r - na + k) * cols + c];
     }
     out[e] = v;
@@ -1307,26 +1292,15 @@ __global__ void __launch_bounds__(256) k_rows_op(int op, const T* __restrict__ a
 // one block per channel: float64 moments sum x and sum x^2
 __global__ void __launch_bounds__(256) k_col_stats(const float* __restrict__ in, int64_t T, int C,
                                                    double* __restrict__ sum, double* __restrict__ sumsq) {
-  __shared__ double s_red[8];
   const int c = blockIdx.x;
-  auto block_sum = [&](double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
-    __syncthreads();
-    double r = 0.0;
-    for (int w = 0; w < 8; ++w) r += s_red[w];
-    __syncthreads();
-    return r;
-  };
   double acc = 0.0, acc2 = 0.0;
   for (int64_t t = threadIdx.x; t < T; t += blockDim.x) {
     const double v = static_cast<double>(in[t * C + c]);
     acc += v;
     acc2 = fma(v, v, acc2);
   }
-  const double tot = block_sum(acc);
-  const double sq = block_sum(acc2);
+  const double tot = block_sum<256>(acc);
+  const double sq = block_sum<256>(acc2);
   if (threadIdx.x == 0) { sum[c] = tot; sumsq[c] = sq; }
 }
 
@@ -1469,7 +1443,7 @@ __device__ __forceinline__ void win_copy(const float* __restrict__ rows, int col
 }
 
 // Block b copies rows [r0, r0 + kWindowTileRows) of output window b / tiles.  Thread 0 resolves the window to its clip
-// (binary search over the window offsets) and to the two streams' sources once; the copy itself is pure data movement.
+// (find_segment over the window offsets) and to the two streams' sources once; the copy itself is pure data movement.
 // V = 4: audio rows as float4 (cols % 4 == 0 and 16-byte aligned bases); facial rows are always scalar (61 columns,
 // 244-byte rows), read by consecutive threads.
 template <int V>
@@ -1482,11 +1456,7 @@ __global__ void __launch_bounds__(kWinThreads) k_window_gather(WindowView v, int
   const int n_rows = min(kWindowTileRows, v.window - r0);
   if (threadIdx.x == 0) {
     const int64_t idx = v.index[k];
-    int lo = 0, hi = v.n_clips;                 // last clip c with w_off[c] <= idx (every clip has >= 1 window)
-    while (hi - lo > 1) {
-      const int mid = (lo + hi) >> 1;
-      if (__ldg(v.w_off + mid) <= idx) lo = mid; else hi = mid;
-    }
+    const int lo = find_segment(v.w_off, v.n_clips, idx);   // every clip has >= 1 window
     const int64_t j = idx - __ldg(v.w_off + lo);
     const int64_t a0 = __ldg(v.a_off + lo), f0 = __ldg(v.f_off + lo);
     const int64_t na = __ldg(v.a_off + lo + 1) - a0, nf = __ldg(v.f_off + lo + 1) - f0;
@@ -1519,9 +1489,6 @@ int grid_for(int64_t items, int per_block, int max_blocks) {
 // ------------------------------------------------------------------------------------------------
 // launchers (return number of kernels launched, or -1 on launch error)
 // ------------------------------------------------------------------------------------------------
-#define NSF_CHECK_LAUNCH() \
-  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
-
 // 16-byte vector loads / stores need 16-byte aligned array bases (library arenas always are; caller-owned device
 // pointers of the stream-ordered entry points may not be: those take the scalar instantiation)
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }

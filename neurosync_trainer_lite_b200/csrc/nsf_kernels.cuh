@@ -5,7 +5,14 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+// Launchers return the number of kernels they launched, or -1 when a launch failed.
+#define NSF_CHECK_LAUNCH() \
+  do { if (cudaGetLastError() != cudaSuccess) return -1; } while (0)
+
 namespace nsf {
+
+// SMs of the one target, the B200 (sm_100a): grids sized in waves of resident blocks are multiples of it.
+constexpr int kSmCount = 148;
 
 // Segment descriptors of one batch of clips, all in device memory.
 struct BatchView {

@@ -1370,11 +1370,12 @@ int launch_stft_tc_fold(cudaStream_t s, const StftTcTables& tc, const DeviceTabl
   int per_sm = static_cast<int>((224 * 1024) / (smem + 1024));
   per_sm = per_sm < 1 ? 1 : (per_sm > 6 ? 6 : per_sm);
   int64_t grid = (b.total_frames + kFoldWarps - 1) / kFoldWarps;
-  if (grid > 148 * per_sm) grid = 148 * per_sm;
+  if (grid > kSmCount * per_sm) grid = kSmCount * per_sm;
   if (grid < 1) grid = 1;
   auto go = [&](auto kernel) {
     kernel<<<static_cast<int>(grid), kFoldWarps * 32, smem, s>>>(t, b, y, v.planes, v.rows, v.row_exp, buf_floats, wp_pairs);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    NSF_CHECK_LAUNCH();
+    return 1;
   };
   if (reg_path) {
     if (iters <= 2) return go(k_tc_fold_r<2>);       // F <= 508   (16 kHz: 266, 22.05 kHz: 367 odd -> kp 192: 3)
@@ -1384,7 +1385,8 @@ int launch_stft_tc_fold(cudaStream_t s, const StftTcTables& tc, const DeviceTabl
     return go(k_tc_fold_r<8>);
   }
   k_tc_fold<<<static_cast<int>(grid), kFoldWarps * 32, smem, s>>>(t, b, y, v.planes, v.rows, v.row_exp, buf_floats);
-  return cudaGetLastError() == cudaSuccess ? 1 : -1;
+  NSF_CHECK_LAUNCH();
+  return 1;
 }
 
 int launch_stft_tc_mel(cudaStream_t s, const StftTcTables& tc, const DeviceTables& t, const BatchView& b,
@@ -1398,18 +1400,20 @@ int launch_stft_tc_mel(cudaStream_t s, const StftTcTables& tc, const DeviceTable
   const int kblocks = (tc.kp + BK - 1) / BK;
   if (kblocks >= 4) {
     int64_t pairs = v.rows / (2 * BM);
-    if (pairs > 74) pairs = 74;
+    if (pairs > kSmCount / 2) pairs = kSmCount / 2;
     if (pairs < 1) pairs = 1;
     k_tc_stft_mel_pair<<<static_cast<unsigned>(2 * pairs), kFusedThreads, kPairSmem, s>>>(
         map_a, tc.map_b_half, t, b, v.rows, tc.kp, tc.np_ld, v.row_exp, db, dbmax_key);
-    return cudaGetLastError() == cudaSuccess ? 1 : -1;
+    NSF_CHECK_LAUNCH();
+    return 1;
   }
   int64_t grid = v.rows / BM;
-  if (grid > 148) grid = 148;
+  if (grid > kSmCount) grid = kSmCount;
   if (grid < 1) grid = 1;
   k_tc_stft_mel<<<static_cast<unsigned>(grid), kFusedThreads, kFusedSmem, s>>>(map_a, tc.map_b, t, b, v.rows, tc.kp,
                                                                              tc.np_ld, v.row_exp, db, dbmax_key);
-  return cudaGetLastError() == cudaSuccess ? 1 : -1;
+  NSF_CHECK_LAUNCH();
+  return 1;
 }
 
 int launch_stft_tc_gemm(cudaStream_t s, const StftTcTables& tc, const DeviceTables& t, const BatchView& b,
@@ -1425,7 +1429,8 @@ int launch_stft_tc_gemm(cudaStream_t s, const StftTcTables& tc, const DeviceTabl
   k_tc_gemm<<<static_cast<unsigned>(grid), kThreads, kSmemBytes, s>>>(
       map_a, tc.map_b, b.total_frames, v.rows, n_tiles, tc.chains, tc.kp, tc.np_ld, tc.np[0], tc.np[1],
       tc.col_off[1], t.bins_ld, v.row_exp, power);
-  return cudaGetLastError() == cudaSuccess ? 1 : -1;
+  NSF_CHECK_LAUNCH();
+  return 1;
 }
 
 // Opt-in shared-memory limits, once per device (nsf_ctx_create, after cudaSetDevice).
