@@ -146,5 +146,19 @@ __device__ __forceinline__ float key_float(uint32_t k) {
   return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
+// max_key[clip] = max(max_key[clip], key) for every lane of a converged warp; clip < 0: the lane has no value.  A warp
+// whose lanes share one clip (the usual case: clips are far longer than 32 frames) reduces first and makes one atomic.
+__device__ __forceinline__ void warp_clip_max(uint32_t* __restrict__ max_key, int clip, uint32_t key) {
+  const int first_clip = __shfl_sync(0xffffffffu, clip, 0);
+  if (__all_sync(0xffffffffu, clip == first_clip || clip < 0)) {
+    uint32_t k = clip >= 0 ? key : 0u;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) k = max(k, __shfl_xor_sync(0xffffffffu, k, o));
+    if ((threadIdx.x & 31) == 0 && first_clip >= 0) atomicMax(max_key + first_clip, k);
+  } else if (clip >= 0) {
+    atomicMax(max_key + clip, key);
+  }
+}
+
 }  // namespace nsf
 #endif  // NSF_DEVICE_UTILS_CUH_

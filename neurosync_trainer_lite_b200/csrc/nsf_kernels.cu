@@ -324,22 +324,8 @@ __global__ void __launch_bounds__(kMelWarps * 32) k_mel_db(DeviceTables t, Batch
     // coalesced dB rows out
     for (int f = warp; f < nf; f += kMelWarps)
       for (int m = lane; m < t.n_mels; m += 32) db[(g0 + f) * t.n_mels + m] = s_out[f * out_pitch + m];
-    if (warp == 0) {
-      // one global atomic per run of frames that share a clip (normally one per tile)
-      const int64_t g = g0 + lane;
-      const int clip = lane < nf ? find_segment(b.frame_off, b.n_clips, g) : -1;
-      const uint32_t key = lane < nf ? s_max[lane] : 0u;
-      const int first_clip = __shfl_sync(0xffffffffu, clip, 0);
-      const bool uniform = __all_sync(0xffffffffu, clip == first_clip || clip < 0);
-      if (uniform) {
-        uint32_t k = key;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) k = max(k, __shfl_xor_sync(0xffffffffu, k, o));
-        if (lane == 0) atomicMax(dbmax_key + first_clip, k);
-      } else if (clip >= 0) {
-        atomicMax(dbmax_key + clip, key);
-      }
-    }
+    if (warp == 0)   // one global atomic per tile, unless the tile spans clips
+      warp_clip_max(dbmax_key, lane < nf ? find_segment(b.frame_off, b.n_clips, g0 + lane) : -1, s_max[lane]);
   }
 }
 

@@ -14,8 +14,12 @@
 // would be 1e-2..1e-1 off on the CMVN'd features (SURVEY.md section 7.3).
 //
 // Kernels
-//   k_tc_fold : signal -> folded, scaled, split fp16 operands   (HBM bound, elementwise)
-//   k_tc_gemm : warp-specialised TMA -> tcgen05.mma -> TMEM -> |.|^2 epilogue
+//   k_tc_fold_r, k_tc_fold : signal -> folded, scaled, split fp16 operands (HBM bound, elementwise);
+//                            k_tc_fold_r keeps a frame in registers (kp <= 512), k_tc_fold serves longer frames
+//   k_tc_stft_mel_pair,      persistent warp-specialised TMA -> tcgen05.mma -> TMEM -> |.|^2 -> mel -> dB, one body
+//   k_tc_stft_mel            on CTA pairs (cta_group::2) and on single CTAs (short K)
+//   k_tc_gemm              : TMA -> tcgen05.mma -> TMEM -> |.|^2 written to HBM (NSF_DEBUG_UNFUSED_MEL, and plans
+//                            whose mel filters overlap more than pairwise)
 #include <cuda_fp16.h>
 
 #include <cmath>
@@ -43,8 +47,23 @@ constexpr int kFusedThreads = 320;                  // fused kernels: warps 2-5 
 constexpr size_t kSmemBytes = 1024 + static_cast<size_t>(kStages) * kStageBytes + 256;
 
 // ---- PTX wrappers --------------------------------------------------------------------------
+// CTA pairs (cta_group::2): two CTAs of one cluster (same TPC) execute ONE tcgen05.mma of M = 256: each
+// supplies its own 128 rows of A and HALF of the N rows of B from its own shared memory, and receives its
+// 128 accumulator rows in its own TMEM.  Only the leader (cluster rank 0) issues MMAs; both issue TMA loads
+// whose completion bytes land on the LEADER's mbarrier (peer bit of the shared::cluster address cleared).
+// The wrappers that depend on the CTA group take it as kCtas = 1 (one CTA) or 2 (a pair).
+constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
+}
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync_all() {
+  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
@@ -53,8 +72,13 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
                : "memory");
 }
+// kCtas = 2: arrives on the leader's (even CTA's) barrier at this offset
+template <int kCtas>
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+  if constexpr (kCtas == 1)
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+  else
+    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBitMask) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
@@ -76,12 +100,21 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
+// kCtas = 2: the bytes complete on the leader's barrier at this offset
+template <int kCtas>
 __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar,
                                             int32_t x, int32_t y) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(x), "r"(y)
-      : "memory");
+  if constexpr (kCtas == 1)
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(x), "r"(y)
+        : "memory");
+  else
+    asm volatile(
+        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & kPeerBitMask),
+          "r"(x), "r"(y)
+        : "memory");
 }
 __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
@@ -92,80 +125,58 @@ __device__ __forceinline__ void tcgen05_fence_before() {
 __device__ __forceinline__ void tcgen05_fence_after() {
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 }
+template <int kCtas>
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
-               "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  if constexpr (kCtas == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
+                 "r"(cols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
+                 "r"(cols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  }
 }
+template <int kCtas>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+  if constexpr (kCtas == 1)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+  else
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem]^T, 16-bit inputs, fp32 accumulation
+template <int kCtas>
 __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
+  if constexpr (kCtas == 1)
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+  else
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
 }
-// mbarrier arrives once every previously issued tcgen05.mma of this thread has completed
+// mbarrier arrives once every previously issued tcgen05.mma of this thread has completed; kCtas = 2: on the
+// barrier at this offset in BOTH CTAs
+template <int kCtas>
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// ---- CTA-pair (cta_group::2) variants -----------------------------------------------------------
-// Two CTAs of one cluster (same TPC) execute ONE tcgen05.mma of M = 256: each supplies its own 128 rows
-// of A and HALF of the N rows of B from its own shared memory, and receives its 128 accumulator rows in
-// its own TMEM.  Only the leader (cluster rank 0) issues MMAs; both issue TMA loads whose completion
-// bytes land on the LEADER's mbarrier (peer bit of the shared::cluster address cleared).
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* map, uint64_t* leader_bar,
-                                                 int32_t x, int32_t y) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(leader_bar) & kPeerBitMask),
-        "r"(x), "r"(y)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_leader(uint64_t* bar) {      // arrive on the even CTA's barrier
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBitMask) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
-               "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_f16_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                              uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrives on the barrier at this offset in BOTH CTAs once the pair's previous MMAs have completed
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(static_cast<uint16_t>(3))
-      : "memory");
+  if constexpr (kCtas == 1)
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
+                 : "memory");
+  else
+    asm volatile(
+        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+        ::"r"(smem_u32(bar)), "h"(static_cast<uint16_t>(3))
+        : "memory");
 }
 __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, float (&v)[32]) {
   uint32_t r[32];
@@ -629,7 +640,7 @@ k_tc_gemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
     mbar_init(tmem_full_bar, 1);
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
+  if (warp == 1) tmem_alloc<1>(tmem_slot, kTmemCols);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -647,11 +658,11 @@ k_tc_gemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
         mbar_expect_tx(full_bar + stage, kStageBytes);
         const int kx = kb * BK;
         const int64_t a_row = static_cast<int64_t>(cp * 2) * plane_rows + g0;
-        tma_load_2d(st + 0 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row));
-        tma_load_2d(st + 1 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row + plane_rows));
+        tma_load_2d<1>(st + 0 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row));
+        tma_load_2d<1>(st + 1 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row + plane_rows));
         const int b_row = (cp * 2) * np_ld + n0;
-        tma_load_2d(st + 2 * kTileBytes, &map_b, full_bar + stage, kx, b_row);
-        tma_load_2d(st + 3 * kTileBytes, &map_b, full_bar + stage, kx, b_row + np_ld);
+        tma_load_2d<1>(st + 2 * kTileBytes, &map_b, full_bar + stage, kx, b_row);
+        tma_load_2d<1>(st + 3 * kTileBytes, &map_b, full_bar + stage, kx, b_row + np_ld);
       }
     }
   } else if (warp == 1) {
@@ -672,13 +683,13 @@ k_tc_gemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
           const uint64_t a_lo = make_smem_desc(st + 1 * kTileBytes + koff);
           const uint64_t b_hi = make_smem_desc(st + 2 * kTileBytes + koff);
           const uint64_t b_lo = make_smem_desc(st + 3 * kTileBytes + koff);
-          umma_f16(d_tmem, a_hi, b_hi, idesc, (kb | k) != 0 ? 1u : 0u);
-          umma_f16(d_tmem, a_hi, b_lo, idesc, 1u);
-          umma_f16(d_tmem, a_lo, b_hi, idesc, 1u);
+          umma_f16<1>(d_tmem, a_hi, b_hi, idesc, (kb | k) != 0 ? 1u : 0u);
+          umma_f16<1>(d_tmem, a_hi, b_lo, idesc, 1u);
+          umma_f16<1>(d_tmem, a_lo, b_hi, idesc, 1u);
         }
-        umma_commit(empty_bar + stage);          // smem slot reusable once these MMAs retire
+        umma_commit<1>(empty_bar + stage);          // smem slot reusable once these MMAs retire
       }
-      umma_commit(tmem_full_bar);                // accumulators complete
+      umma_commit<1>(tmem_full_bar);                // accumulators complete
     }
   } else {
     const int quarter = warp & 3;                // TMEM lane quarter this warp may access
@@ -715,7 +726,7 @@ k_tc_gemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    tmem_dealloc(tmem_base, kTmemCols);
+    tmem_dealloc<1>(tmem_base, kTmemCols);
   }
 }
 
@@ -807,10 +818,8 @@ __device__ __forceinline__ void pair_sync(int quarter) {
   asm volatile("bar.sync %0, 64;" ::"r"(quarter + 1) : "memory");
 }
 
-// The epilogue of the fused kernels for one thread: `upper` selects the column half, the thread owns frame
-// row `row` of the tile (TMEM lane).  Called by warps 2..9; see k_tc_stft_mel for the surrounding protocol.
 // ------------------------------------------------------------------------------------------------
-// k_tc_stft_mel: PERSISTENT fused kernel, one CTA per SM looping over tiles of 128 hop-frames.
+// k_tc_stft_mel / k_tc_stft_mel_pair: PERSISTENT fused kernel, looping over tiles of 128 hop-frames per CTA.
 // For every tile it runs the (chain, 128-bin) sub-tiles back to back; TMEM holds two 256-column
 // accumulator buffers (Re | Im), so the tensor pipe works on sub-tile s+1 while the epilogue warps
 // drain sub-tile s.  The epilogue never writes the power spectrum: it squares, undoes the scaling and
@@ -819,8 +828,22 @@ __device__ __forceinline__ void pair_sync(int quarter) {
 // last sub-tile writes 10 log10(max(1e-10, mel)) plus the per-clip dB maximum.
 //   warp 0 : TMA producer      warp 1 : TMEM alloc + tcgen05.mma issuer      warps 2-9 : epilogue
 //   (two warps per TMEM lane quarter, 64 of the 128 accumulator columns each)
+// One body, kCtas CTAs per MMA:
+//   k_tc_stft_mel       kCtas = 1, two pipeline stages.  Used for short K (fewer than four K blocks), where the
+//                       pair's longer hand-off is exposed.
+//   k_tc_stft_mel_pair  kCtas = 2 (product path).  With one CTA the kernel is bound by operand delivery
+//                       L2 -> shared memory (every CTA streams the whole DFT matrix for each 128 frames; it sustains
+//                       ~80 % of the L2 throughput cap with the tensor pipe 40 % active).  A cluster of two CTAs works
+//                       on 256 frames with tcgen05.mma.cta_group::2 (M = 256): each CTA still loads its own 128 frame
+//                       rows of A but only HALF of every DFT-matrix tile (64 of the 128 bin rows), the tensor cores
+//                       read the other half from the peer's shared memory.  Operand bytes per CTA and stage drop from
+//                       64 KB to 48 KB, which also makes room for a third pipeline stage.
+// Hand-off of a pair: full[s]       leader's barrier; the leader's producer posts the bytes of BOTH CTAs, both
+//                                   CTAs' TMA loads complete on it (peer bit cleared)
+//                     empty[s]      per CTA; tcgen05.commit multicast from the leader's MMA thread
+//                     tmem_full[b]  per CTA; tcgen05.commit multicast
+//                     tmem_empty[b] leader's barrier, 16 arrivals: the eight epilogue warps of both CTAs
 // ------------------------------------------------------------------------------------------------
-constexpr int kFStages = 2;
 constexpr int kMelPitch = 129;                       // floats per frame row of the mel tile
 // Finished dB rows of the mel tile -> global memory, one warp per 16 consecutive frame rows (`src` = the first of them in
 // the tile, `g0` its frame index).  Four rows (sixteen loads) are in flight per warp: as one load -> store pair per
@@ -851,53 +874,69 @@ __device__ __forceinline__ void store_db_rows(const float* __restrict__ src, flo
 // BM frame rows + one scratch row (sink for rows beyond the batch), rounded so the mbarriers that follow
 // stay 8-byte aligned
 constexpr size_t kMelTileBytes = (static_cast<size_t>(BM + 1) * kMelPitch * sizeof(float) + 15) / 16 * 16;
-constexpr size_t kFusedSmem = 1024 + static_cast<size_t>(kFStages) * kStageBytes +
-                              kMelTileBytes + 256;
+// Pipeline stages and operand bytes per stage of the fused kernels: A_hi, A_lo (BM frame rows each), B_hi, B_lo
+// (BN / ctas bin rows each)
+__host__ __device__ constexpr int fused_stages(int ctas) { return ctas == 1 ? 2 : 3; }
+__host__ __device__ constexpr int fused_stage_bytes(int ctas) { return 2 * kTileBytes + 2 * (BN / ctas) * BK * 2; }
+constexpr size_t fused_smem_bytes(int ctas) {
+  return 1024 + static_cast<size_t>(fused_stages(ctas)) * fused_stage_bytes(ctas) + kMelTileBytes + 256;
+}
+constexpr size_t kFusedSmem = fused_smem_bytes(1);
+constexpr size_t kPairSmem = fused_smem_bytes(2);
 
-__global__ void __launch_bounds__(kFusedThreads, 1)
-k_tc_stft_mel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-              DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
-              const int32_t* __restrict__ row_exp, float* __restrict__ db, uint32_t* __restrict__ dbmax_key) {
+template <int kCtas>
+__device__ __forceinline__ void stft_mel_body(const CUtensorMap& map_a, const CUtensorMap& map_b, const DeviceTables& t,
+                                              const BatchView& b, int64_t plane_rows, int kp, int np_ld,
+                                              const int32_t* __restrict__ row_exp, float* __restrict__ db,
+                                              uint32_t* __restrict__ dbmax_key) {
+  constexpr int kFStages = fused_stages(kCtas), kFStageBytes = fused_stage_bytes(kCtas);
+  constexpr int kBRows = BN / kCtas;                 // bin rows of a B tile this CTA loads
+  constexpr int kTileB = kBRows * BK * 2;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment (128-byte swizzle) by OFFSETTING the shared array, not by rounding a generic pointer:
   // the compiler then keeps the shared address space and emits LDS / STS for the mel tile
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* tiles = smem;
-  float* mel_acc = reinterpret_cast<float*>(smem + kFStages * kStageBytes);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kFStages * kStageBytes + kMelTileBytes);
+  float* mel_acc = reinterpret_cast<float*>(smem + kFStages * kFStageBytes);
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kFStages * kFStageBytes + kMelTileBytes);
   uint64_t* empty_bar = full_bar + kFStages;
   uint64_t* tmem_full = empty_bar + kFStages;     // [2]
   uint64_t* tmem_empty = tmem_full + 2;           // [2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t rank = kCtas == 1 ? 0u : cluster_ctarank();
   const int kblocks = (kp + BK - 1) / BK;
   const int ntile[2] = {(t.np[0] + BN - 1) / BN, t.chains > 1 ? (t.np[1] + BN - 1) / BN : 0};
   const int n_sub = ntile[0] + ntile[1];
-  const int64_t n_tiles = (b.total_frames + BM - 1) / BM;
+  // A unit is the kCtas * BM frames of one cluster, rank r owns frames [r BM, (r + 1) BM) of it.  Each role's loop
+  // derives its first unit from blockIdx.x in its own header: hoisted above the role branches, the 64-bit start lands
+  // in vector registers and the MMA issuer's loop loses its uniform (UR / BRA.U) control flow.
+  const int64_t n_units = (b.total_frames + kCtas * BM - 1) / (kCtas * BM);
 
   if (threadIdx.x == 0) {
     prefetch_tensormap(&map_a);
     prefetch_tensormap(&map_b);
     for (int i = 0; i < kFStages; ++i) { mbar_init(full_bar + i, 1); mbar_init(empty_bar + i, 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(tmem_full + i, 1); mbar_init(tmem_empty + i, 8); }
+    for (int i = 0; i < 2; ++i) { mbar_init(tmem_full + i, 1); mbar_init(tmem_empty + i, 8 * kCtas); }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc(tmem_slot, 512);
+  if (warp == 1) tmem_alloc<kCtas>(tmem_slot, 512);
   for (int i = threadIdx.x; i < BM * kMelPitch; i += blockDim.x) mel_acc[i] = 0.0f;
   tcgen05_fence_before();
   __syncthreads();
+  if constexpr (kCtas == 2) cluster_sync_all();     // the peer's barriers are initialised before any remote arrive
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {
       uint32_t it = 0;
-      for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int64_t g0 = tile * BM;
+      for (int64_t unit = blockIdx.x / kCtas; unit < n_units; unit += gridDim.x / kCtas) {
+        const int64_t g0 = unit * kCtas * BM + static_cast<int64_t>(rank) * BM;      // this CTA's 128 frames
         for (int sub = 0; sub < n_sub; ++sub) {
           const int chain = sub < ntile[0] ? 0 : 1;
-          const int n0 = (chain == 0 ? sub : sub - ntile[0]) * BN;
+          const int n0 = (chain == 0 ? sub : sub - ntile[0]) * BN + static_cast<int>(rank) * kBRows;
           for (int part = 0; part < 2; ++part) {
             const int cp = chain * 2 + part;
             const int64_t a_row = static_cast<int64_t>(cp * 2) * plane_rows + g0;
@@ -905,261 +944,52 @@ k_tc_stft_mel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
             for (int kb = 0; kb < kblocks; ++kb, ++it) {
               const int stage = it % kFStages;
               mbar_wait(empty_bar + stage, ((it / kFStages) & 1) ^ 1);
-              uint8_t* st = tiles + stage * kStageBytes;
-              mbar_expect_tx(full_bar + stage, kStageBytes);
+              uint8_t* st = tiles + stage * kFStageBytes;
+              if (rank == 0) mbar_expect_tx(full_bar + stage, kCtas * kFStageBytes);  // the bytes of all kCtas CTAs
               const int kx = kb * BK;
-              tma_load_2d(st + 0 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row));
-              tma_load_2d(st + 1 * kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row + plane_rows));
-              tma_load_2d(st + 2 * kTileBytes, &map_b, full_bar + stage, kx, b_row);
-              tma_load_2d(st + 3 * kTileBytes, &map_b, full_bar + stage, kx, b_row + np_ld);
+              tma_load_2d<kCtas>(st, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row));
+              tma_load_2d<kCtas>(st + kTileBytes, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row + plane_rows));
+              tma_load_2d<kCtas>(st + 2 * kTileBytes, &map_b, full_bar + stage, kx, b_row);
+              tma_load_2d<kCtas>(st + 2 * kTileBytes + kTileB, &map_b, full_bar + stage, kx, b_row + np_ld);
             }
           }
         }
       }
     }
   } else if (warp == 1) {
-    // all 32 lanes walk the schedule (and wait on the barriers) together; one elected lane issues.
-    // Descriptors of a stage are formed once; a K step of 16 fp16 = 32 bytes is +2 in the address field.
-    constexpr uint32_t idesc = make_idesc(BM, BN);
-    uint32_t it = 0, acc_it = 0;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int sub = 0; sub < n_sub; ++sub, ++acc_it) {
-        const uint32_t buf = acc_it & 1u;
-        mbar_wait(tmem_empty + buf, ((acc_it >> 1) & 1u) ^ 1u);     // epilogue has drained this buffer
-        tcgen05_fence_after();
-        for (int part = 0; part < 2; ++part) {
-          const uint32_t d_tmem = tmem_base + buf * 256u + static_cast<uint32_t>(part * BN);
-          for (int kb = 0; kb < kblocks; ++kb, ++it) {
-            const int stage = it % kFStages;
-            mbar_wait(full_bar + stage, (it / kFStages) & 1);
-            tcgen05_fence_after();
-            if (elect_one()) {
-              const uint32_t st = smem_u32(tiles + stage * kStageBytes);
-              const uint64_t a_hi = make_smem_desc(st + 0 * kTileBytes), a_lo = make_smem_desc(st + 1 * kTileBytes);
-              const uint64_t b_hi = make_smem_desc(st + 2 * kTileBytes), b_lo = make_smem_desc(st + 3 * kTileBytes);
-              const int ksteps = min(BK / UK, (kp - kb * BK + UK - 1) / UK);
-#pragma unroll
-              for (int k = 0; k < BK / UK; ++k) {
-                if (k < ksteps) {
-                  const uint64_t ko = static_cast<uint64_t>(k * ((UK * 2) >> 4));
-                  umma_f16(d_tmem, a_hi + ko, b_hi + ko, idesc, (kb | k) != 0 ? 1u : 0u);
-                  umma_f16(d_tmem, a_hi + ko, b_lo + ko, idesc, 1u);
-                  umma_f16(d_tmem, a_lo + ko, b_hi + ko, idesc, 1u);
-                }
-              }
-              umma_commit(empty_bar + stage);
-              if (part == 1 && kb == kblocks - 1) umma_commit(tmem_full + buf);
-            }
-            __syncwarp();
-          }
-        }
-      }
-    }
-  } else {
-    const int quarter = warp & 3;                 // TMEM lane quarter this warp may access
-    const bool upper = warp >= 6;                 // warps 2-5: columns 0-63 of a sub-tile, warps 6-9: 64-127
-    const int row = quarter * 32 + lane;          // frame row of the tile owned by this thread (and its partner)
-    float* my_acc = mel_acc + row * kMelPitch;
-    float* scratch_row = mel_acc + BM * kMelPitch;   // sink for rows beyond the batch (never read)
-    const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
-    uint32_t acc_it = 0;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const int64_t tile0 = tile * BM;
-      const int64_t g = tile0 + row;
-      const bool row_ok = g < b.total_frames;
-      const int32_t row_info = row_ok ? __ldg(row_exp + g) : 0;
-      const float sc2 = row_ok ? ldexpf(1.0f, -2 * (row_info_exp(row_info) + kTcBScaleExp)) : 0.0f;
-      float* acc_row = row_ok ? my_acc : scratch_row;
-      for (int sub = 0; sub < n_sub; ++sub, ++acc_it) {
-        const int chain = sub < ntile[0] ? 0 : 1;
-        const int n0 = (chain == 0 ? sub : sub - ntile[0]) * BN;
-        const float4* tab = t.mel_col[chain] + n0;
-        const uint32_t buf = acc_it & 1u;
-        mbar_wait(tmem_full + buf, (acc_it >> 1) & 1u);
-        tcgen05_fence_after();
-        MelDeferred def;
-        const int live_chunks = (min(BN, t.np[chain] - n0) + 15) / 16, lower_chunks = (live_chunks + 1) / 2;
-        if (upper) mel_accumulate_half<true>(lane_addr + buf * 256u, tab, acc_row, sc2, def, lower_chunks, live_chunks);
-        else mel_accumulate_half<false>(lane_addr + buf * 256u, tab, acc_row, sc2, def, 0, lower_chunks);
-        // all TMEM reads of this warp are complete (tcgen05.wait::ld inside the routine)
-        tcgen05_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(tmem_empty + buf);
-        pair_sync(quarter);                        // the lower half has flushed everything
-        if (upper) apply_deferred(acc_row, def);
-      }
-      pair_sync(quarter);                          // deferred sums are in: the rows of this quarter are complete
-      // tile finished: dB (each warp its 64 mels), per-clip maximum, coalesced store, reset of the rows
-      const int m_lo = upper ? t.n_mels / 2 : 0, m_hi = upper ? t.n_mels : t.n_mels / 2;
-      float vmax = -INFINITY;
-      int m = m_lo;
-      for (; m + 8 <= m_hi; m += 8) {               // eight independent load -> log -> store chains in flight
-        float v8[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) v8[i] = my_acc[m + i];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          v8[i] = 10.0f * log10f(fmaxf(1e-10f, v8[i]));
-          vmax = fmaxf(vmax, v8[i]);
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) my_acc[m + i] = v8[i];
-      }
-      for (; m < m_hi; ++m) {
-        const float v = 10.0f * log10f(fmaxf(1e-10f, my_acc[m]));
-        my_acc[m] = v;
-        vmax = fmaxf(vmax, v);
-      }
-      pair_sync(quarter);
-      const int64_t gw = tile0 + quarter * 32;          // first frame of this quarter's 32 rows
-      store_db_rows(mel_acc + (quarter * 32 + (upper ? 16 : 0)) * kMelPitch, db, gw + (upper ? 16 : 0), b.total_frames,
-                    t.n_mels, lane);
-      pair_sync(quarter);
-      for (int m = upper ? kMelPitch / 2 : 0; m < (upper ? kMelPitch : kMelPitch / 2); ++m) my_acc[m] = 0.0f;
-      {
-        const int clip = row_ok ? row_info_clip(row_info) : -1;      // written by the fold kernel
-        const uint32_t key = row_ok ? float_key(vmax) : 0u;
-        const int first_clip = __shfl_sync(0xffffffffu, clip, 0);
-        const bool uniform = __all_sync(0xffffffffu, clip == first_clip || clip < 0);
-        if (uniform) {
-          uint32_t k = key;
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) k = max(k, __shfl_xor_sync(0xffffffffu, k, o));
-          if (lane == 0 && first_clip >= 0) atomicMax(dbmax_key + first_clip, k);
-        } else if (clip >= 0) {
-          atomicMax(dbmax_key + clip, key);
-        }
-      }
-    }
-    tcgen05_fence_before();
-  }
-  __syncthreads();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// k_tc_stft_mel_pair: the fused kernel on CTA PAIRS (product path).  k_tc_stft_mel is bound by operand
-// delivery L2 -> shared memory (every CTA streams the whole DFT matrix for each 128 frames; the kernel
-// sustains ~80 % of the L2 throughput cap with the tensor pipe 40 % active).  Here a cluster of two CTAs
-// works on 256 frames with tcgen05.mma.cta_group::2 (M = 256): each CTA still loads its own 128 frame rows
-// of A but only HALF of every DFT-matrix tile (64 of the 128 bin rows), the tensor cores read the other
-// half from the peer's shared memory.  Operand bytes per CTA and stage drop from 64 KB to 48 KB, which
-// also makes room for a third pipeline stage.
-//   hand-off: full[s]       leader's barrier; the leader's producer posts the bytes of BOTH CTAs, both
-//                           CTAs' TMA loads complete on it (peer bit cleared)
-//             empty[s]      per CTA; tcgen05.commit multicast from the leader's MMA thread
-//             tmem_full[b]  per CTA; tcgen05.commit multicast
-//             tmem_empty[b] leader's barrier, 16 arrivals: the eight epilogue warps of both CTAs
-// Epilogue, mel accumulation and outputs are those of k_tc_stft_mel (each CTA owns its 128 rows).
-// ------------------------------------------------------------------------------------------------
-constexpr int kPStages = 3;
-constexpr int kPTileA = BM * BK * 2;                 // 16 KiB: 128 frame rows
-constexpr int kPTileB = (BN / 2) * BK * 2;           // 8 KiB: 64 of the 128 bin rows
-constexpr int kPStageBytes = 2 * kPTileA + 2 * kPTileB;
-constexpr size_t kPairSmem = 1024 + static_cast<size_t>(kPStages) * kPStageBytes +
-                             kMelTileBytes + 256;
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1)
-k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-                   DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
-                   const int32_t* __restrict__ row_exp, float* __restrict__ db, uint32_t* __restrict__ dbmax_key) {
-  extern __shared__ uint8_t smem_raw[];
-  // 1024-byte alignment (128-byte swizzle) by OFFSETTING the shared array, not by rounding a generic pointer:
-  // the compiler then keeps the shared address space and emits LDS / STS for the mel tile
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* tiles = smem;
-  float* mel_acc = reinterpret_cast<float*>(smem + kPStages * kPStageBytes);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kPStages * kPStageBytes + kMelTileBytes);
-  uint64_t* empty_bar = full_bar + kPStages;
-  uint64_t* tmem_full = empty_bar + kPStages;     // [2]
-  uint64_t* tmem_empty = tmem_full + 2;           // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int kblocks = (kp + BK - 1) / BK;
-  const int ntile[2] = {(t.np[0] + BN - 1) / BN, t.chains > 1 ? (t.np[1] + BN - 1) / BN : 0};
-  const int n_sub = ntile[0] + ntile[1];
-  const int64_t n_ptiles = (b.total_frames + 2 * BM - 1) / (2 * BM);
-  const int64_t pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-
-  if (threadIdx.x == 0) {
-    prefetch_tensormap(&map_a);
-    prefetch_tensormap(&map_b);
-    for (int i = 0; i < kPStages; ++i) { mbar_init(full_bar + i, 1); mbar_init(empty_bar + i, 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(tmem_full + i, 1); mbar_init(tmem_empty + i, 16); }
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc_pair(tmem_slot, 512);
-  for (int i = threadIdx.x; i < BM * kMelPitch; i += blockDim.x) mel_acc[i] = 0.0f;
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();                               // the peer's barriers are initialised before any remote arrive
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t it = 0;
-      for (int64_t pt = pair; pt < n_ptiles; pt += n_pairs) {
-        const int64_t g0 = pt * 2 * BM + static_cast<int64_t>(rank) * BM;      // this CTA's 128 frames
-        for (int sub = 0; sub < n_sub; ++sub) {
-          const int chain = sub < ntile[0] ? 0 : 1;
-          const int n0 = (chain == 0 ? sub : sub - ntile[0]) * BN + static_cast<int>(rank) * (BN / 2);
-          for (int part = 0; part < 2; ++part) {
-            const int cp = chain * 2 + part;
-            const int64_t a_row = static_cast<int64_t>(cp * 2) * plane_rows + g0;
-            const int b_row = (cp * 2) * np_ld + n0;
-            for (int kb = 0; kb < kblocks; ++kb, ++it) {
-              const int stage = it % kPStages;
-              mbar_wait(empty_bar + stage, ((it / kPStages) & 1) ^ 1);
-              uint8_t* st = tiles + stage * kPStageBytes;
-              if (leader) mbar_expect_tx(full_bar + stage, 2 * kPStageBytes);  // both CTAs' bytes
-              const int kx = kb * BK;
-              tma_load_2d_pair(st, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row));
-              tma_load_2d_pair(st + kPTileA, &map_a, full_bar + stage, kx, static_cast<int32_t>(a_row + plane_rows));
-              tma_load_2d_pair(st + 2 * kPTileA, &map_b, full_bar + stage, kx, b_row);
-              tma_load_2d_pair(st + 2 * kPTileA + kPTileB, &map_b, full_bar + stage, kx, b_row + np_ld);
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (leader) {                                    // warp-uniform: the whole warp walks the schedule
-      constexpr uint32_t idesc = make_idesc(2 * BM, BN);
+    // The leader issues the MMAs of its cluster.  All 32 lanes walk the schedule (and wait on the barriers) together;
+    // one elected lane issues.  Descriptors of a stage are formed once; a K step of 16 fp16 = 32 bytes is +2 in the
+    // address field.
+    if (rank == 0) {
+      constexpr uint32_t idesc = make_idesc(kCtas * BM, BN);
       uint32_t it = 0, acc_it = 0;
-      for (int64_t pt = pair; pt < n_ptiles; pt += n_pairs) {
+      for (int64_t unit = blockIdx.x / kCtas; unit < n_units; unit += gridDim.x / kCtas) {
         for (int sub = 0; sub < n_sub; ++sub, ++acc_it) {
           const uint32_t buf = acc_it & 1u;
-          mbar_wait(tmem_empty + buf, ((acc_it >> 1) & 1u) ^ 1u);     // both epilogues have drained this buffer
+          mbar_wait(tmem_empty + buf, ((acc_it >> 1) & 1u) ^ 1u);     // the epilogues have drained this buffer
           tcgen05_fence_after();
           for (int part = 0; part < 2; ++part) {
             const uint32_t d_tmem = tmem_base + buf * 256u + static_cast<uint32_t>(part * BN);
             for (int kb = 0; kb < kblocks; ++kb, ++it) {
-              const int stage = it % kPStages;
-              mbar_wait(full_bar + stage, (it / kPStages) & 1);
+              const int stage = it % kFStages;
+              mbar_wait(full_bar + stage, (it / kFStages) & 1);
               tcgen05_fence_after();
               if (elect_one()) {
-                const uint32_t st = smem_u32(tiles + stage * kPStageBytes);
-                const uint64_t a_hi = make_smem_desc(st), a_lo = make_smem_desc(st + kPTileA);
-                const uint64_t b_hi = make_smem_desc(st + 2 * kPTileA), b_lo = make_smem_desc(st + 2 * kPTileA + kPTileB);
+                const uint32_t st = smem_u32(tiles + stage * kFStageBytes);
+                const uint64_t a_hi = make_smem_desc(st), a_lo = make_smem_desc(st + kTileBytes);
+                const uint64_t b_hi = make_smem_desc(st + 2 * kTileBytes), b_lo = make_smem_desc(st + 2 * kTileBytes + kTileB);
                 const int ksteps = min(BK / UK, (kp - kb * BK + UK - 1) / UK);
 #pragma unroll
                 for (int k = 0; k < BK / UK; ++k) {
                   if (k < ksteps) {
                     const uint64_t ko = static_cast<uint64_t>(k * ((UK * 2) >> 4));
-                    umma_f16_pair(d_tmem, a_hi + ko, b_hi + ko, idesc, (kb | k) != 0 ? 1u : 0u);
-                    umma_f16_pair(d_tmem, a_hi + ko, b_lo + ko, idesc, 1u);
-                    umma_f16_pair(d_tmem, a_lo + ko, b_hi + ko, idesc, 1u);
+                    umma_f16<kCtas>(d_tmem, a_hi + ko, b_hi + ko, idesc, (kb | k) != 0 ? 1u : 0u);
+                    umma_f16<kCtas>(d_tmem, a_hi + ko, b_lo + ko, idesc, 1u);
+                    umma_f16<kCtas>(d_tmem, a_lo + ko, b_hi + ko, idesc, 1u);
                   }
                 }
-                umma_commit_pair(empty_bar + stage);
-                if (part == 1 && kb == kblocks - 1) umma_commit_pair(tmem_full + buf);
+                umma_commit<kCtas>(empty_bar + stage);
+                if (part == 1 && kb == kblocks - 1) umma_commit<kCtas>(tmem_full + buf);
               }
               __syncwarp();
             }
@@ -1175,8 +1005,8 @@ k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_const
     float* scratch_row = mel_acc + BM * kMelPitch;   // sink for rows beyond the batch (never read)
     const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
     uint32_t acc_it = 0;
-    for (int64_t pt = pair; pt < n_ptiles; pt += n_pairs) {
-      const int64_t tile0 = pt * 2 * BM + static_cast<int64_t>(rank) * BM;
+    for (int64_t unit = blockIdx.x / kCtas; unit < n_units; unit += gridDim.x / kCtas) {
+      const int64_t tile0 = unit * kCtas * BM + static_cast<int64_t>(rank) * BM;
       const int64_t g = tile0 + row;
       const bool row_ok = g < b.total_frames;
       const int32_t row_info = row_ok ? __ldg(row_exp + g) : 0;
@@ -1196,7 +1026,7 @@ k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_const
         // all TMEM reads of this warp are complete (tcgen05.wait::ld inside the routine)
         tcgen05_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive_leader(tmem_empty + buf);
+        if (lane == 0) mbar_arrive<kCtas>(tmem_empty + buf);
         pair_sync(quarter);                        // the lower half has flushed everything
         if (upper) apply_deferred(acc_row, def);
       }
@@ -1228,29 +1058,31 @@ k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_const
                     t.n_mels, lane);
       pair_sync(quarter);
       for (int m = upper ? kMelPitch / 2 : 0; m < (upper ? kMelPitch : kMelPitch / 2); ++m) my_acc[m] = 0.0f;
-      {
-        const int clip = row_ok ? row_info_clip(row_info) : -1;      // written by the fold kernel
-        const uint32_t key = row_ok ? float_key(vmax) : 0u;
-        const int first_clip = __shfl_sync(0xffffffffu, clip, 0);
-        const bool uniform = __all_sync(0xffffffffu, clip == first_clip || clip < 0);
-        if (uniform) {
-          uint32_t k = key;
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) k = max(k, __shfl_xor_sync(0xffffffffu, k, o));
-          if (lane == 0 && first_clip >= 0) atomicMax(dbmax_key + first_clip, k);
-        } else if (clip >= 0) {
-          atomicMax(dbmax_key + clip, key);
-        }
-      }
+      // the clip index was written by the fold kernel
+      warp_clip_max(dbmax_key, row_ok ? row_info_clip(row_info) : -1, float_key(vmax));
     }
     tcgen05_fence_before();
   }
   __syncthreads();
-  cluster_sync_all();                               // neither CTA leaves while the pair's MMAs may still read it
+  if constexpr (kCtas == 2) cluster_sync_all();     // neither CTA leaves while the pair's MMAs may still read it
   if (warp == 1) {
     tcgen05_fence_after();
-    tmem_dealloc_pair(tmem_base, 512);
+    tmem_dealloc<kCtas>(tmem_base, 512);
   }
+}
+
+__global__ void __launch_bounds__(kFusedThreads, 1)
+k_tc_stft_mel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
+              DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
+              const int32_t* __restrict__ row_exp, float* __restrict__ db, uint32_t* __restrict__ dbmax_key) {
+  stft_mel_body<1>(map_a, map_b, t, b, plane_rows, kp, np_ld, row_exp, db, dbmax_key);
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1)
+k_tc_stft_mel_pair(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
+                   DeviceTables t, BatchView b, int64_t plane_rows, int kp, int np_ld,
+                   const int32_t* __restrict__ row_exp, float* __restrict__ db, uint32_t* __restrict__ dbmax_key) {
+  stft_mel_body<2>(map_a, map_b, t, b, plane_rows, kp, np_ld, row_exp, db, dbmax_key);
 }
 
 // ---- host side ----------------------------------------------------------------------------------
